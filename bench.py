@@ -2,6 +2,7 @@
 """bench.py -- output Mpx/s of MewZoom.upscale on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2|cfg3|cfg4a|cfg4b|cfg4c|cfg5] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (FiLM table, stem, 2L fused 3x3 convolutions, head) over one batch of
 synthetic frames.  Default workload = BASELINE.json configs[1]: MewZoom-2X-Ctrl (48 ch / 20 layers), batch 16 of
@@ -212,6 +213,33 @@ def run_reference(args):
     emit(line)
 
 
+DUMP_MAX_ELEMENTS = 4 << 20   # float32 values + float64 indices of a sampled output: 48 MB, under 64 MB
+
+
+def dump_output(out_dir: str, name: str, y) -> None:
+    """--dump-outputs: write `y`, what the timed path returned in its last step, as out_dir/<name>.npy in float32 (an
+    8-bit image as its values 0..255).  An output of more than DUMP_MAX_ELEMENTS elements is sampled: the flattened
+    output is cut into DUMP_MAX_ELEMENTS equal blocks and one element of each is taken at an offset drawn from a fixed
+    seed, its flat indices in out_dir/<name>_index.npy (float64, exact).  The same arguments give the same inputs,
+    indices and files, so two builds compare element for element."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    path = os.path.join(out_dir, name + ".npy")
+    y = y.detach()
+    if y.numel() <= DUMP_MAX_ELEMENTS:
+        np.save(path, y.float().cpu().numpy())
+        print(f"bench: wrote {path}, the whole output {tuple(y.shape)}", file=sys.stderr)
+        return
+    edges = torch.arange(DUMP_MAX_ELEMENTS + 1, dtype=torch.int64) * y.numel() // DUMP_MAX_ELEMENTS
+    u = torch.rand(DUMP_MAX_ELEMENTS, dtype=torch.float64, generator=torch.Generator().manual_seed(0))
+    idx = edges[:-1] + (u * (edges[1:] - edges[:-1])).long()
+    np.save(path, y.reshape(-1)[idx.to(y.device)].float().cpu().numpy())
+    np.save(os.path.join(out_dir, name + "_index.npy"), idx.double().numpy())
+    print(f"bench: wrote {path}, {DUMP_MAX_ELEMENTS} sampled elements of the output {tuple(y.shape)}", file=sys.stderr)
+
+
 _REAL_STDOUT = None
 
 
@@ -257,7 +285,14 @@ def main():
     ap.add_argument("--unet-ops", action="store_true", help="add the U-Net operator microbenchmarks to the line (default with cfg2 at N = 1)")
     ap.add_argument("--no-also", action="store_true",
                     help="skip the secondary records (4X-Ctrl frame, 3X-Ctrl frame, halo-tiled 8K frame)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the output of the workload's last step (rank 0) to DIR/upscale.npy "
+                         "(float32; a fixed sample of a larger output, its indices in DIR/upscale_index.npy)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3  # timing rule: at least three warm-up steps
     if args.impl == "reference":
@@ -304,11 +339,12 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    def measure(workload: str, steps: int, warmup: int, want_e2e: bool, sample_clocks: bool, operands=None):
+    def measure(workload: str, steps: int, warmup: int, want_e2e: bool, sample_clocks: bool, operands=None, dump=False):
         """W untimed + exactly K timed steps (CUDA events on the launching stream, barrier + synchronize on both
-        sides, max over ranks) of one workload; optionally the end-to-end leg with host buffers."""
+        sides, max over ranks) of one workload; optionally the end-to-end leg with host buffers.  `dump`: write the
+        last timed step's output to --dump-outputs."""
         if workload == "cfg5":
-            return measure_tiled(steps, warmup, want_e2e, sample_clocks)
+            return measure_tiled(steps, warmup, want_e2e, sample_clocks, dump)
         model_name, B, H, W, desc = WORKLOADS[workload]
         cfg = MODEL_CONFIGS[model_name]
         r = cfg["upscale_ratio"]
@@ -337,12 +373,16 @@ def main():
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         sampler.mark_begin()
         ev0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             model.upscale(x, c)
+        y = model.upscale(x, c)                             # the last step's output, for --dump-outputs
         ev1.record()
         barrier()
         ms_total = ev0.elapsed_time(ev1)
         clocks = sampler.stop() if (rank == 0 and sample_clocks) else None
+        if dump and rank == 0:
+            dump_output(args.dump_outputs, "upscale", y)
+        del y
         conv_ms = C.c_float()
         _native.check(eng.lib.mz_model_conv_stack_ms(eng.handle, C.byref(conv_ms)))
         _native.check(eng.lib.mz_model_enable_timing(eng.handle, 0))
@@ -410,7 +450,7 @@ def main():
         torch.cuda.empty_cache()
         return res
 
-    def measure_tiled(steps: int, warmup: int, want_e2e: bool, sample_clocks: bool):
+    def measure_tiled(steps: int, warmup: int, want_e2e: bool, sample_clocks: bool, dump=False):
         """cfg5 (BASELINE configs[4]), strong scaling: ONE 1080p -> 8K MewZoom-4X-Ctrl frame, `world` halo-padded tiles
         (sharding.best_grid / plan_tiles, columns sized for the kernel's 128-pixel tiles), one per rank.  Every rank
         runs the whole network on its tile and its head kernel stores the tile's core straight into the frame that
@@ -483,6 +523,8 @@ def main():
         executed = sum((t_.hy1 - t_.hy0) * (t_.hx1 - t_.hx0) for t_ in plan) / (H * W)
         err = None
         if rank == 0:                                       # every rank's stores landed before the barrier returned
+            if dump:
+                dump_output(args.dump_outputs, "upscale", frame)
             full = model.upscale(x, c)
             err = float((full.float() - frame.float()).abs().max())
             del full
@@ -694,15 +736,15 @@ def main():
             "bicubic_standalone": timed(lambda: ops.bicubic(x, r), npx * (12 + 12 * r * r)),
         }
 
-    main_res = measure(args.workload, args.steps, args.warmup, not args.no_e2e, True)
+    main_res = measure(args.workload, args.steps, args.warmup, not args.no_e2e, True, dump=bool(args.dump_outputs))
     # The north_star's efficiency target is stated on MewZoom-4X-Ctrl and its hard multi-GPU case is the spatial split:
     # the default line carries those as first-class records (own clocks; 4X-Ctrl with its own e2e) under "also".
     also = {}
     if args.workload == "cfg2" and not args.no_also:
-        k = max(3, args.steps)
+        k = args.steps
         also["cfg4a"] = measure("cfg4a", k, args.warmup, not args.no_e2e, True)
         also["cfg3"] = measure("cfg3", k, args.warmup, False, True)
-        also["cfg5"] = measure("cfg5", max(3, min(args.steps, 5)), args.warmup, False, True)
+        also["cfg5"] = measure("cfg5", k, args.warmup, False, True)
         # the same headline workload with the other 16-bit operand type (same tcgen05 rate and bytes; see operands_for)
         other = "float16" if main_res["operands"] == "bfloat16" else "bfloat16"
         also["cfg2_fp16" if other == "float16" else "cfg2_bf16"] = measure("cfg2", k, args.warmup, False, True, operands=other)

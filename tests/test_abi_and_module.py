@@ -196,11 +196,8 @@ def test_bench_arms_describe_one_workload():
     """VERDICT r1: the driver compares the `config` objects of `bench.py` and `bench.py --impl reference`; both come
     from one function, for every workload."""
     import argparse
-    import importlib.util
 
-    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
-    bench = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(bench)
+    bench = _bench_module()
     args = argparse.Namespace(io="float32", residual_stream="auto", operands="float16", tune="")
     for w in bench.WORKLOADS:
         a, b = bench.config_of(w, 1, args), bench.config_of(w, 1, args)
@@ -212,3 +209,59 @@ def test_bench_arms_describe_one_workload():
     assert bench.config_of("cfg2", 1, auto)["mma_operands"] == "bfloat16"
     assert all(bench.config_of(w, 1, auto)["mma_operands"] == "float16" for w in ("cfg3", "cfg4a", "cfg4b", "cfg5"))
     assert bench.config_of("cfg2", 1, auto, "float16")["mma_operands"] == "float16"
+
+
+def test_current_library_is_found_without_writing(monkeypatch):
+    """bench.py may run from a read-only tree: a current library is returned without a lock file or a directory."""
+    import builtins
+
+    from ultrazoom_b200 import build as b
+
+    b.build_locked()
+    real_open = builtins.open
+
+    def read_only_open(path, mode="r", *a, **kw):
+        if set(mode) & set("wax+"):
+            raise PermissionError(f"read-only tree: {path}")
+        return real_open(path, mode, *a, **kw)
+
+    def no_makedirs(path, *a, **kw):
+        raise PermissionError(f"read-only tree: {path}")
+
+    monkeypatch.setattr(builtins, "open", read_only_open)
+    monkeypatch.setattr(b.os, "makedirs", no_makedirs)
+    assert b.build_locked() == b.LIB
+
+
+def _bench_module():
+    import importlib.util
+
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    return bench
+
+
+def test_bench_dump_outputs(tmp_path):
+    """--dump-outputs: a small output is written whole, a large one as a fixed sample with its flat indices; float32,
+    within 64 MB, the same files for the same output."""
+    import numpy as np
+
+    bench = _bench_module()
+    small = torch.rand(1, 3, 8, 10)
+    bench.dump_output(str(tmp_path / "a"), "upscale", small)
+    got = np.load(tmp_path / "a" / "upscale.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, small.numpy())
+    assert not (tmp_path / "a" / "upscale_index.npy").exists()
+
+    big = (torch.arange(2 * 3 * 1030 * 1024) % 251).to(torch.uint8).reshape(2, 3, 1030, 1024)
+    for d in ("b", "c"):
+        bench.dump_output(str(tmp_path / d), "upscale", big)
+    vals, idx = np.load(tmp_path / "b" / "upscale.npy"), np.load(tmp_path / "b" / "upscale_index.npy")
+    assert vals.dtype == np.float32 and idx.dtype == np.float64 and vals.shape == idx.shape == (bench.DUMP_MAX_ELEMENTS,)
+    block = -(-big.numel() // bench.DUMP_MAX_ELEMENTS)                 # the sample spans the whole output
+    assert np.all(np.diff(idx) > 0) and 0 <= idx[0] < block and big.numel() - block <= idx[-1] < big.numel()
+    assert np.array_equal(vals, big.reshape(-1)[torch.from_numpy(idx).long()].float().numpy())
+    assert sum(os.path.getsize(p) for p in (tmp_path / "b").iterdir()) <= 64 << 20
+    for name in ("upscale.npy", "upscale_index.npy"):
+        assert (tmp_path / "b" / name).read_bytes() == (tmp_path / "c" / name).read_bytes()

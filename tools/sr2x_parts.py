@@ -1,5 +1,5 @@
 import os, sys, torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from ultrazoom_b200 import unet as N, ops
 dev = torch.device("cuda", 0)
 def timed(fn, iters=10):

@@ -18,6 +18,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 OBJDIR = os.path.join(HERE, "build")
 LIB = os.path.join(LIBDIR, "libmewzoom_b200.so")
+STAMP = os.path.join(LIBDIR, "libmewzoom_b200.sha256")
 # (source, extra defines, object name).  conv_tc.cu is compiled once per epilogue mode 0..2 (its template instantiations
 # dominate the build time) and once (part 4) for its host side; see the MZ_TC_PART comment in the file.
 SOURCES = [(f"{n}.cu", [], f"{n}.o") for n in ("host_util", "small_kernels", "api", "model", "probe", "block_fused", "unet_ops", "unet_tc")] + [
@@ -49,13 +50,20 @@ def _digest() -> str:
     return h.hexdigest()
 
 
+def is_current() -> bool:
+    """The library exists and was built from the present sources and flags."""
+    if not (os.path.exists(LIB) and os.path.exists(STAMP)):
+        return False
+    with open(STAMP) as f:
+        return f.read().strip() == _digest()
+
+
 def build(force: bool = False, verbose: bool = False) -> str:
+    if not force and is_current():
+        return LIB
     os.makedirs(LIBDIR, exist_ok=True)
     os.makedirs(OBJDIR, exist_ok=True)
-    stamp = os.path.join(LIBDIR, "libmewzoom_b200.sha256")
     digest = _digest()
-    if not force and os.path.exists(LIB) and os.path.exists(stamp) and open(stamp).read().strip() == digest:
-        return LIB
     nvcc = _nvcc()
 
     def compile_one(unit) -> str:
@@ -76,15 +84,19 @@ def build(force: bool = False, verbose: bool = False) -> str:
     r = subprocess.run([nvcc, "-shared", "-o", LIB, *objs, "-cudart", "static"], capture_output=True, text=True)
     if r.returncode != 0:
         raise RuntimeError(f"link failed:\n{r.stdout}\n{r.stderr}")
-    with open(stamp, "w") as f:
+    with open(STAMP, "w") as f:
         f.write(digest)
     return LIB
 
 
 def build_locked(force: bool = False, verbose: bool = False) -> str:
-    """build() under an inter-process file lock (one process per GPU: every rank calls this at import)."""
+    """build() under an inter-process file lock (one process per GPU: every rank calls this at import).
+
+    A current library is returned without taking the lock, so that a built tree is only read: it may be read-only."""
     import fcntl
 
+    if not force and is_current():
+        return LIB
     os.makedirs(LIBDIR, exist_ok=True)
     with open(os.path.join(LIBDIR, ".build.lock"), "w") as lock:
         fcntl.flock(lock, fcntl.LOCK_EX)
