@@ -54,6 +54,13 @@ typedef enum mz_status {
                                   /* test_compare.py:89).  Needs MZ_FLAG_CLAMP01.  4x less image traffic on PCIe / HBM.  */
 #define MZ_FLAG_U8_TRUNC 16u      /* with MZ_FLAG_IO_U8: y8 = floor(255 clamp(y)) (ToPILImage, README.md:81)             */
 #define MZ_FLAG_SKIP_FROM_BUFFER 4u /* head reads a precomputed bicubic image (mz_bicubic_f32 output in y) instead of recomputing it in its epilogue */
+/* Interleaved (channels-last) images, for callers that hold pixels as numpy / PIL / OpenCV arrays or rgb24 video frames:
+ * the stem reads and the head writes them directly, so neither side needs a transpose.  The two flags are independent, fp32
+ * or 8-bit (MZ_FLAG_IO_U8) alike, and apply to mz_upscale, mz_upscale_window, mz_upscale_stage, mz_upscale_host and
+ * mz_upscale_host_async.  Images stay 3HW (3 rH rW) elements apart, so byte counts and per-image chunking are unchanged.
+ * Neither combines with MZ_FLAG_SKIP_FROM_BUFFER (MZ_ERR_INVALID); an interleaved image must be below 2^31 elements. */
+#define MZ_FLAG_X_NHWC 32u        /* x is (B,H,W,3): colour c of LR pixel (y, x) at ((b H + y) W + x) 3 + c             */
+#define MZ_FLAG_Y_NHWC 64u        /* y is (B,rH,rW,3); windowed output: see mz_upscale_window                          */
 
 /* Constructor kwargs of the 0.2.x-style MewZoom (README.md:254-258, model.py:52-69). */
 typedef struct mz_config {
@@ -126,10 +133,10 @@ int mz_model_saturated(mz_model* m, int32_t reset, int32_t* saturated);
 int mz_workspace_bytes(const mz_model* m, int32_t B, int32_t H, int32_t W, size_t* bytes);
 
 /* ---- the hot path: replaces MewZoom.forward / MewZoom.upscale (model.py:149-179) ----
- * x_dev : (B,3,H,W) fp32 NCHW in [0,1]   (uint8 with MZ_FLAG_IO_U8)
+ * x_dev : (B,3,H,W) fp32 NCHW in [0,1]   (uint8 with MZ_FLAG_IO_U8; (B,H,W,3) with MZ_FLAG_X_NHWC)
  * c_dev : NULL for non-control models, else (B, control_features) fp32 (c_rows == B)
  *         or (1, control_features) (c_rows == 1, broadcast) -- validate.py:73-94
- * y_dev : (B,3,rH,rW) fp32 NCHW          (uint8 with MZ_FLAG_IO_U8)
+ * y_dev : (B,3,rH,rW) fp32 NCHW          (uint8 with MZ_FLAG_IO_U8; (B,rH,rW,3) with MZ_FLAG_Y_NHWC)
  * flags : MZ_FLAG_CLAMP01 => upscale(), 0 => forward()
  */
 int mz_upscale(mz_model* m, const void* x_dev, const float* c_dev, int32_t c_rows, void* y_dev,
@@ -141,7 +148,12 @@ int mz_upscale(mz_model* m, const void* x_dev, const float* c_dev, int32_t c_row
  * straight into an assembled frame: y_dev is where HR pixel (win_y0 * r, win_x0 * r) of plane 0 of image 0 lands,
  * HR rows are y_row_pitch elements apart and the three colour planes (and then the images) y_plane_pitch elements.
  * y_dev may be another GPU's memory with peer access enabled (mz_enable_peer_access): the head kernel's stores then ARE
- * the transfer over NVLink -- no tile output buffer, no copy, no collective.  The bicubic skip is always recomputed. */
+ * the transfer over NVLink -- no tile output buffer, no copy, no collective.  The bicubic skip is always recomputed.
+ * With MZ_FLAG_Y_NHWC (interleaved output): y_dev is where colour 0 of HR pixel (win_y0 * r, win_x0 * r) of image 0
+ * lands, y_row_pitch is the number of elements between HR rows (at least 3 * r * (win_x1 - win_x0)) and y_plane_pitch the
+ * number between images.
+ * y_dev and both pitches must be aligned to the head's vector stores: fp32 8 / 16 / 4 bytes at r = 2 / 4 / 3, 8-bit
+ * 2 / 4 / 1 bytes -- in either layout. */
 int mz_upscale_window(mz_model* m, const void* x_dev, const float* c_dev, int32_t c_rows, void* y_dev,
                       int64_t y_row_pitch, int64_t y_plane_pitch, int32_t B, int32_t H, int32_t W, int32_t win_y0,
                       int32_t win_y1, int32_t win_x0, int32_t win_x1, void* workspace_dev, size_t workspace_bytes,

@@ -107,7 +107,8 @@ __host__ __device__ inline SmemPlan plan_smem(const TcParams& p) {
 // instead of 3R: the 128 x 16 activation tile -- 4 KB of shared-memory operand fetch per UMMA, what bounds the small-N
 // shapes -- is fetched once per input row instead of once per (output row, tap).  Every UMMA accumulates; the epilogue
 // zeroes each accumulator column group right after reading it.
-template <int MODE, int KT, int ROWS, int VAR>
+// LAY (head only): bit 0 interleaved input image, bit 1 interleaved output image (EpiParams::x_nhwc / y_nhwc).
+template <int MODE, int KT, int ROWS, int VAR, int LAY = 0>
 __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_constant__ TcParams p) {
   constexpr bool PAIR = VAR == 1, FUSE = VAR == 2;
   extern __shared__ uint8_t smem_raw[];
@@ -935,10 +936,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
             if (ok) {
               const bool interior = xw >= 2 && xw + 33 < p.epi.W;  // (warp-uniform) no clamped column in this warp
               const bool second = y + 1 < p.epi.H;
-              if (p.epi.x8 != nullptr)
-                epi_head2_pair<uint8_t>(p.epi, p.epi.x8, b, y, x, v0, v1, interior, second);
-              else
-                epi_head2_pair<float>(p.epi, p.epi.x, b, y, x, v0, v1, interior, second);
+              epi_head2<(LAY & 1) != 0, (LAY & 2) != 0>(p.epi, b, y, x, v0, v1, interior, second);
             }
           }
         }
@@ -980,12 +978,13 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
           }
           if (ok) {
             const bool interior = xw >= 2 && xw + 33 < p.epi.W;  // (warp-uniform) no clamped column in this warp
+            constexpr bool XN = (LAY & 1) != 0, YN = (LAY & 2) != 0;
             if (p.epi.r == 4)
-              epi_head_r<4>(p.epi, b, y, x, acc, interior);
+              epi_head_r<4, XN, YN>(p.epi, b, y, x, acc, interior);
             else if (p.epi.r == 2)
-              epi_head_r<2>(p.epi, b, y, x, acc, interior);
+              epi_head_r<2, XN, YN>(p.epi, b, y, x, acc, interior);
             else
-              epi_head_r<3>(p.epi, b, y, x, acc, interior);
+              epi_head_r<3, XN, YN>(p.epi, b, y, x, acc, interior);
           }
         } else if (MODE == 1) {
           if (k > 0 && !all_rows) load_residual(k, k + 1);
@@ -1157,18 +1156,22 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
 // ---- kernel lookup -------------------------------------------------------------------------------------------------
 // One lookup function per epilogue mode, so that the build can compile the instantiations of each mode in its own
 // translation unit: build.py compiles this file four times, with -DMZ_TC_PART=<mode> for the kernels of modes 0..2 and
-// -DMZ_TC_PART=4 for the host side.  Without the define (a plain `nvcc -c conv_tc.cu`) everything lands in one object.
+// -DMZ_TC_PART=4 for the host side, and the heads for interleaved images (LAY 1..3) with -DMZ_TC_PART=5..7.  Without
+// the define (a plain `nvcc -c conv_tc.cu`) everything lands in one object.
 //   var 0: one CTA per patch, 1: CTA pair (cta_group::2), 2: fused rows.  Returns nullptr for a shape that has no kernel.
 const void* tc_kernel_mode0(int ks, int rows, int var);
 const void* tc_kernel_mode1(int ks, int rows, int var);
 const void* tc_kernel_mode2(int ks, int rows, int var);
+const void* tc_kernel_mode2_lay1(int ks, int rows, int var);
+const void* tc_kernel_mode2_lay2(int ks, int rows, int var);
+const void* tc_kernel_mode2_lay3(int ks, int rows, int var);
 
-template <int M, int K>
+template <int M, int K, int LAY = 0>
 static const void* tc_kernel_rows(int rows, int var) {
   if (var == 0) {
-    if (rows == 1) return reinterpret_cast<const void*>(conv_tc_kernel<M, K, 1, 0>);
-    if (rows == 2) return reinterpret_cast<const void*>(conv_tc_kernel<M, K, 2, 0>);
-    if (rows == 4) return reinterpret_cast<const void*>(conv_tc_kernel<M, K, 4, 0>);
+    if (rows == 1) return reinterpret_cast<const void*>(conv_tc_kernel<M, K, 1, 0, LAY>);
+    if (rows == 2) return reinterpret_cast<const void*>(conv_tc_kernel<M, K, 2, 0, LAY>);
+    if (rows == 4) return reinterpret_cast<const void*>(conv_tc_kernel<M, K, 4, 0, LAY>);
   }
   if constexpr (M != 2 && K != 3) {  // pairs: the shapes the 64/96/128-channel encoders use (the head has no pair form)
     if (var == 1 && rows == 1) return reinterpret_cast<const void*>(conv_tc_kernel<M, K, 1, 1>);
@@ -1177,17 +1180,17 @@ static const void* tc_kernel_rows(int rows, int var) {
   if constexpr (M != 2) {
     if (var == 2 && rows == 2) return reinterpret_cast<const void*>(conv_tc_kernel<M, K, 2, 2>);
   }
-  if (var == 2 && rows == 4) return reinterpret_cast<const void*>(conv_tc_kernel<M, K, 4, 2>);  // (head: four-row patches only)
+  if (var == 2 && rows == 4) return reinterpret_cast<const void*>(conv_tc_kernel<M, K, 4, 2, LAY>);  // (head: four-row patches only)
   return nullptr;
 }
 
-template <int M>
+template <int M, int LAY = 0>
 static const void* tc_kernel_lookup(int ks, int rows, int var) {
   switch (ks) {
-    case 1: return tc_kernel_rows<M, 1>(rows, var);
-    case 2: return tc_kernel_rows<M, 2>(rows, var);
-    case 3: return tc_kernel_rows<M, 3>(rows, var);
-    case 4: return tc_kernel_rows<M, 4>(rows, var);
+    case 1: return tc_kernel_rows<M, 1, LAY>(rows, var);
+    case 2: return tc_kernel_rows<M, 2, LAY>(rows, var);
+    case 3: return tc_kernel_rows<M, 3, LAY>(rows, var);
+    case 4: return tc_kernel_rows<M, 4, LAY>(rows, var);
     default: return nullptr;
   }
 }
@@ -1200,6 +1203,15 @@ const void* tc_kernel_mode1(int ks, int rows, int var) { return tc_kernel_lookup
 #endif
 #if !defined(MZ_TC_PART) || MZ_TC_PART == 2
 const void* tc_kernel_mode2(int ks, int rows, int var) { return tc_kernel_lookup<2>(ks, rows, var); }
+#endif
+#if !defined(MZ_TC_PART) || MZ_TC_PART == 5
+const void* tc_kernel_mode2_lay1(int ks, int rows, int var) { return tc_kernel_lookup<2, 1>(ks, rows, var); }
+#endif
+#if !defined(MZ_TC_PART) || MZ_TC_PART == 6
+const void* tc_kernel_mode2_lay2(int ks, int rows, int var) { return tc_kernel_lookup<2, 2>(ks, rows, var); }
+#endif
+#if !defined(MZ_TC_PART) || MZ_TC_PART == 7
+const void* tc_kernel_mode2_lay3(int ks, int rows, int var) { return tc_kernel_lookup<2, 3>(ks, rows, var); }
 #endif
 
 #if !defined(MZ_TC_PART) || MZ_TC_PART == 4  // ---- host side ----------------------------------------------------------
@@ -1269,7 +1281,19 @@ struct ConvLaunchImpl {
   int grid, k;
   uint32_t smem;
   int mode, n_pad;
+  int ks, var, lay;  // what `fn` was looked up for (the head's image layouts are patched per call)
 };
+
+// the head kernel for image layouts `lay` (bit 0 interleaved input, bit 1 interleaved output)
+static const void* tc_kernel_head(int lay, int ks, int rows, int var) {
+  switch (lay) {
+    case 0: return tc_kernel_mode2(ks, rows, var);
+    case 1: return tc_kernel_mode2_lay1(ks, rows, var);
+    case 2: return tc_kernel_mode2_lay2(ks, rows, var);
+    default: return tc_kernel_mode2_lay3(ks, rows, var);
+  }
+}
+static int head_layout(const EpiParams& e) { return (e.x_nhwc ? 1 : 0) | (e.y_nhwc ? 2 : 0); }
 static_assert(sizeof(ConvLaunchImpl) <= sizeof(ConvLaunch::storage), "ConvLaunch::storage too small");
 
 static int run_prepared(ConvLaunchImpl& L, cudaStream_t s) {
@@ -1328,8 +1352,17 @@ int run_conv_tc(ConvLaunch& launch, cudaStream_t s) {
   return run_prepared(*reinterpret_cast<ConvLaunchImpl*>(launch.storage), s);
 }
 
-void patch_conv_epi(ConvLaunch& launch, const EpiParams& e) {
-  EpiParams& d = reinterpret_cast<ConvLaunchImpl*>(launch.storage)->p.epi;
+int patch_conv_epi(ConvLaunch& launch, const EpiParams& e) {
+  ConvLaunchImpl& L = *reinterpret_cast<ConvLaunchImpl*>(launch.storage);
+  const int lay = head_layout(e);
+  if (lay != L.lay) {  // same geometry, the instantiation for the other layouts
+    const void* fn = tc_kernel_head(lay, L.ks, L.p.rows, L.var);
+    MZ_REQUIRE(fn != nullptr, "conv: no head kernel for image layouts %d", lay);
+    MZ_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem));
+    L.fn = fn;
+    L.lay = lay;
+  }
+  EpiParams& d = L.p.epi;
   d.x = e.x;
   d.y = e.y;
   d.x8 = e.x8;
@@ -1343,6 +1376,9 @@ void patch_conv_epi(ConvLaunch& launch, const EpiParams& e) {
   d.wx1 = e.wx1;
   d.y_row = e.y_row;
   d.y_plane = e.y_plane;
+  d.x_nhwc = e.x_nhwc;
+  d.y_nhwc = e.y_nhwc;
+  return MZ_OK;
 }
 
 int launch_conv_tc(const ConvArgs& a, const ConvTcTune& tune, int device, cudaStream_t s) {
@@ -1628,7 +1664,7 @@ int prepare_conv_tc(const ConvArgs& a, const ConvTcTune& tune, int device, ConvL
   const int var = p.fuse_g ? 2 : (p.pair ? 1 : 0);
   const void* fn = e.mode == 0   ? tc_kernel_mode0(ks, p.rows, var)
                    : e.mode == 1 ? tc_kernel_mode1(ks, p.rows, var)
-                                 : tc_kernel_mode2(ks, p.rows, var);
+                                 : tc_kernel_head(head_layout(e), ks, p.rows, var);
   if (!fn) {
     set_error("conv: no %s kernel for mode %d, %d k-steps, %d rows", var == 2 ? "fused-row" : (var == 1 ? "CTA-pair" : "tcgen05"),
               e.mode, ks, p.rows);
@@ -1642,6 +1678,9 @@ int prepare_conv_tc(const ConvArgs& a, const ConvTcTune& tune, int device, ConvL
   L.smem = smem;
   L.mode = e.mode;
   L.n_pad = e.n_pad;
+  L.ks = ks;
+  L.var = var;
+  L.lay = e.mode == 2 ? head_layout(e) : 0;
   out->valid = true;
   return MZ_OK;
 }

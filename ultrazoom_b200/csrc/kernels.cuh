@@ -62,6 +62,10 @@ struct EpiParams {
   // colour planes y_plane elements apart -- a tile's core written straight into an assembled (possibly remote) frame.
   int wy0, wy1, wx0, wx1;
   long long y_row, y_plane;
+  // Interleaved images (MZ_FLAG_X_NHWC / MZ_FLAG_Y_NHWC): x is (B,H,W,3), y is (B,rH,rW,3) -- colour c of a pixel at
+  // pixel * 3 + c, images 3HW (3 rH rW) elements apart as in the planar layout.  For a windowed y_nhwc output y / y8
+  // points at colour 0 of HR pixel (wy0 r, wx0 r), y_row is the element pitch of HR rows and y_plane that of images.
+  int x_nhwc, y_nhwc;
   // fp16 range guard: a kernel that is about to round a value beyond +-65504 into a 16-bit fp16 operand (where
   // cvt.rn.satfinite would clip it silently) writes 1 here.  Points at a host-mapped word owned by the mz_model
   // (mz_model_saturated); nullptr = not tracked (per-kernel entry points).
@@ -72,13 +76,23 @@ struct EpiParams {
 // largest finite fp16: a pre-rounding magnitude above it saturates the operand
 #define MZ_F16_MAX 65504.0f
 
-// address of HR pixel (oy, ox) of colour plane (b, c) in the output of mode 2, or -1 outside the window
-__host__ __device__ inline long long head_out_index(const EpiParams& p, int b, int c, int y, int x, int i, int j) {
+// address of colour c of HR pixel (y r + i, x r + j) of image b in the output of mode 2, or -1 outside the window;
+// YN: interleaved output (EpiParams::y_nhwc)
+template <bool YN>
+__host__ __device__ inline long long head_out_index_l(const EpiParams& p, int b, int c, int y, int x, int i, int j) {
   const long long WR = static_cast<long long>(p.W) * p.r, HR = static_cast<long long>(p.H) * p.r;
   if (p.wy1 > 0 && (y < p.wy0 || y >= p.wy1 || x < p.wx0 || x >= p.wx1)) return -1;
+  if (YN) {
+    const long long row = p.y_row ? p.y_row : 3 * WR, img = p.y_plane ? p.y_plane : 3 * HR * WR;
+    return static_cast<long long>(b) * img + (static_cast<long long>(y - p.wy0) * p.r + i) * row +
+           (static_cast<long long>(x - p.wx0) * p.r + j) * 3 + c;
+  }
   const long long row = p.y_row ? p.y_row : WR, plane = p.y_plane ? p.y_plane : HR * WR;
   return (static_cast<long long>(b) * 3 + c) * plane + (static_cast<long long>(y - p.wy0) * p.r + i) * row +
          static_cast<long long>(x - p.wx0) * p.r + j;
+}
+__host__ __device__ inline long long head_out_index(const EpiParams& p, int b, int c, int y, int x, int i, int j) {
+  return p.y_nhwc ? head_out_index_l<true>(p, b, c, y, x, i, j) : head_out_index_l<false>(p, b, c, y, x, i, j);
 }
 
 // One 3x3 convolution launch (both kernels).
@@ -125,8 +139,9 @@ struct alignas(64) ConvLaunch {
 };
 int prepare_conv_tc(const ConvArgs& a, const ConvTcTune& tune, int device, ConvLaunch* out);
 int run_conv_tc(ConvLaunch& launch, cudaStream_t s);
-// head (mode 2) only: replace the image pointers, output window and image-epilogue flags of a prepared launch
-void patch_conv_epi(ConvLaunch& launch, const EpiParams& e);
+// head (mode 2) only: replace the image pointers, output window, image layouts and image-epilogue flags of a prepared
+// launch (a new layout swaps the kernel instantiation)
+int patch_conv_epi(ConvLaunch& launch, const EpiParams& e);
 // ---- one encoder block as one kernel (block_fused.cu): zf += conv2(SiLU(FiLM(conv1(zb_in)))), zb_out = round16(zf) ----
 struct FusedBlockArgs {
   const uint16_t* zb_in;  // (B,H,W,48) 16-bit: read with a halo, so the output goes to a second buffer
@@ -168,9 +183,10 @@ int launch_seg_gemm_tc(const SgArgs& a, cudaStream_t s);
 
 int launch_bicubic(const float* x, float* y, int planes, int H, int W, int r, cudaStream_t s);
 // fp32 stream zf + 16-bit shadow zb (pitch zb_pitch).
-// x8 != nullptr: the image is 8-bit (B,3,H,W) and read as x8 / 255.
+// x8 != nullptr: the image is 8-bit (B,3,H,W) and read as x8 / 255.  x_nhwc: the image is interleaved (B,H,W,3).
 int launch_stem(const float* x, const uint8_t* x8, const float* w, const float* bias, float* zf, uint16_t* zb, int bf16,
-                int B, int H, int W, int Cp, int zb_pitch, cudaStream_t s, unsigned int* sat = nullptr);
+                int B, int H, int W, int Cp, int zb_pitch, cudaStream_t s, unsigned int* sat = nullptr,
+                bool x_nhwc = false);
 // film: [L][hCp / ns][B][2][ns] -- one [B][2][ns] table (scale row, shift row) per conv1 launch; ns == hCp normally
 int launch_film(const float* c, int c_rows, const float* w, const float* b, float* film, int L, int B, int F,
                 int hC, int hCp, int ns, cudaStream_t s);
@@ -272,9 +288,10 @@ __device__ __forceinline__ uint8_t to_u8(float v, int trunc) {
   return static_cast<uint8_t>(static_cast<int>(fmaf(v, 255.f, trunc ? 0.f : 0.5f)));
 }
 
-// Bicubic value of HR pixel (oy, ox) of one plane (H x W, fp32 | u8): 16 clamped taps, rows first.
+// Bicubic value of HR pixel (oy, ox) of one colour (H x W, fp32 | u8, pixels `ps` elements apart: 1 planar, 3
+// interleaved): 16 clamped taps, rows first.
 template <typename T>
-__device__ __forceinline__ float bicubic_at(const T* __restrict__ plane, int H, int W, const BicubicTable& bt,
+__device__ __forceinline__ float bicubic_at(const T* __restrict__ plane, int H, int W, int ps, const BicubicTable& bt,
                                             int oy, int ox) {
   const int r = bt.r;
   const int py = oy % r, px = ox % r;
@@ -283,12 +300,12 @@ __device__ __forceinline__ float bicubic_at(const T* __restrict__ plane, int H, 
 #pragma unroll
   for (int k = 0; k < 4; ++k) {
     const int yy = min(max(by + k, 0), H - 1);
-    const T* row = plane + static_cast<size_t>(yy) * W;
+    const T* row = plane + static_cast<size_t>(yy) * W * ps;
     float h = 0.f;
 #pragma unroll
     for (int m = 0; m < 4; ++m) {
       const int xx = min(max(bx + m, 0), W - 1);
-      h = fmaf(lr_px(row + xx), bt.w[px][m], h);
+      h = fmaf(lr_px(row + static_cast<size_t>(xx) * ps), bt.w[px][m], h);
     }
     acc = fmaf(h, bt.w[py][k], acc);
   }
@@ -312,8 +329,11 @@ __device__ __forceinline__ void epi_head(const EpiParams& p, int b, int y, int x
       if (p.skip_mode == 1) {
         v += p.y[di];
       } else if (p.skip_mode == 2) {
-        const size_t pl = (static_cast<size_t>(b) * 3 + c) * p.H * p.W;
-        v += p.x8 != nullptr ? bicubic_at(p.x8 + pl, p.H, p.W, p.bt, oy, ox) : bicubic_at(p.x + pl, p.H, p.W, p.bt, oy, ox);
+        const size_t HW = static_cast<size_t>(p.H) * p.W;
+        const size_t pl = p.x_nhwc ? static_cast<size_t>(b) * 3 * HW + c : (static_cast<size_t>(b) * 3 + c) * HW;
+        const int ps = p.x_nhwc ? 3 : 1;
+        v += p.x8 != nullptr ? bicubic_at(p.x8 + pl, p.H, p.W, ps, p.bt, oy, ox)
+                             : bicubic_at(p.x + pl, p.H, p.W, ps, p.bt, oy, ox);
       }
       if (p.clamp01) v = fminf(fmaxf(v, 0.f), 1.f);
       if (p.y8 != nullptr)
@@ -323,6 +343,50 @@ __device__ __forceinline__ void epi_head(const EpiParams& p, int b, int y, int x
     }
   }
 }
+// One interleaved HR row segment of an LR pixel: v = R pixels x 3 colours, stored at element d of y / y8 as three
+// vectors (fp32: float2 at R = 2, float4 at R = 4; 8-bit: u16 / u32) or, at R = 3, element by element.
+template <int R>
+__device__ __forceinline__ void store_hr_row_nhwc(const EpiParams& p, size_t d, float (&v)[3 * R]) {
+  if (p.y8 != nullptr) {
+    uint8_t q[3 * R];
+#pragma unroll
+    for (int e = 0; e < 3 * R; ++e) q[e] = to_u8(v[e], p.u8_trunc);
+    uint8_t* rowp = p.y8 + d;
+    if constexpr (R == 4) {
+#pragma unroll
+      for (int k = 0; k < 3; ++k)
+        reinterpret_cast<uint32_t*>(rowp)[k] = static_cast<uint32_t>(q[4 * k]) | (static_cast<uint32_t>(q[4 * k + 1]) << 8) |
+                                               (static_cast<uint32_t>(q[4 * k + 2]) << 16) |
+                                               (static_cast<uint32_t>(q[4 * k + 3]) << 24);
+    } else if constexpr (R == 2) {
+#pragma unroll
+      for (int k = 0; k < 3; ++k)
+        reinterpret_cast<uint16_t*>(rowp)[k] =
+            static_cast<uint16_t>(static_cast<uint32_t>(q[2 * k]) | (static_cast<uint32_t>(q[2 * k + 1]) << 8));
+    } else {
+#pragma unroll
+      for (int e = 0; e < 3 * R; ++e) rowp[e] = q[e];
+    }
+    return;
+  }
+  if (p.clamp01) {
+#pragma unroll
+    for (int e = 0; e < 3 * R; ++e) v[e] = fminf(fmaxf(v[e], 0.f), 1.f);
+  }
+  float* rowp = p.y + d;
+  if constexpr (R == 4) {
+#pragma unroll
+    for (int k = 0; k < 3; ++k)
+      reinterpret_cast<float4*>(rowp)[k] = make_float4(v[4 * k], v[4 * k + 1], v[4 * k + 2], v[4 * k + 3]);
+  } else if constexpr (R == 2) {
+#pragma unroll
+    for (int k = 0; k < 3; ++k) reinterpret_cast<float2*>(rowp)[k] = make_float2(v[2 * k], v[2 * k + 1]);
+  } else {
+#pragma unroll
+    for (int e = 0; e < 3 * R; ++e) rowp[e] = v[e];
+  }
+}
+
 // Same as epi_head with the ratio known at compile time: the 5x5 LR neighbourhood of the pixel is loaded once per
 // colour, interpolated horizontally for the R phases (5 rows x R values) and then vertically (R x R values) --
 // 25 loads + 20R + 4R^2 FMAs per colour instead of 16 loads + 20 FMAs per HR pixel -- and every HR row segment of
@@ -333,15 +397,19 @@ __device__ __forceinline__ void epi_head(const EpiParams& p, int b, int y, int x
 // the first FMA; skip-from-buffer reads all its row segments before the first store (a store to y orders every
 // later load from y behind it).  Columns are only clamped in the first and last warp of an image row: the others
 // (interior) read each neighbourhood row through one pointer with immediate offsets.
-template <int R, typename T>
+// XN / YN: interleaved input / output (EpiParams::x_nhwc / y_nhwc) -- compile-time, so that the planar instantiation is
+// the code it was.  Interleaved, the taps of one colour are 3 elements apart (same FMA order per colour: bit-identical
+// results) and each HR row of the pixel leaves as 3R contiguous values.
+template <int R, typename T, bool XN, bool YN>
 __device__ __forceinline__ void epi_head_rt(const EpiParams& p, const T* __restrict__ lr, int b, int y, int x,
                                             const float (&acc)[48], bool interior) {
   const int H = p.H, W = p.W;
-  const long long first = head_out_index(p, b, 0, y, x, 0, 0);
+  const long long first = head_out_index_l<YN>(p, b, 0, y, x, 0, 0);
   if (first < 0) return;  // outside the output window
-  const size_t row_pitch = p.y_row ? static_cast<size_t>(p.y_row) : static_cast<size_t>(W) * R;
+  const size_t row_pitch = p.y_row ? static_cast<size_t>(p.y_row) : static_cast<size_t>(W) * R * (YN ? 3 : 1);
   const size_t plane_pitch = p.y_plane ? static_cast<size_t>(p.y_plane) : static_cast<size_t>(H) * R * W * R;
   constexpr int NC = (R == 2) ? 3 : 1;  // colours whose taps are in flight together
+  constexpr int PS = XN ? 3 : 1;        // elements between horizontally adjacent LR pixels of one colour
   float out[3][R][R];
 #pragma unroll
   for (int c = 0; c < 3; ++c)
@@ -353,23 +421,24 @@ __device__ __forceinline__ void epi_head_rt(const EpiParams& p, const T* __restr
   if (p.skip_mode == 2) {
     const size_t HW = static_cast<size_t>(H) * W;
     const T* img = lr + static_cast<size_t>(b) * 3 * HW;
-    int xo[5], ro[5];  // (a colour plane is below 2^31 pixels: prepare_conv_tc checks)
+    int xo[5], ro[5];  // (a colour plane is below 2^31 pixels: prepare_conv_tc checks; an interleaved image is below
+                       // 2^31 elements: upscale_impl checks)
 #pragma unroll
-    for (int m = 0; m < 5; ++m) xo[m] = min(max(x - 2 + m, 0), W - 1);
+    for (int m = 0; m < 5; ++m) xo[m] = min(max(x - 2 + m, 0), W - 1) * PS;
 #pragma unroll
-    for (int k = 0; k < 5; ++k) ro[k] = min(max(y - 2 + k, 0), H - 1) * W;
+    for (int k = 0; k < 5; ++k) ro[k] = min(max(y - 2 + k, 0), H - 1) * W * PS;
 #pragma unroll
     for (int c0 = 0; c0 < 3; c0 += NC) {
       float nb[NC][5][5];
 #pragma unroll
       for (int cc = 0; cc < NC; ++cc) {
-        const T* pl = img + (c0 + cc) * HW;
+        const T* pl = img + (XN ? (c0 + cc) : (c0 + cc) * HW);
         if (interior) {  // warp-uniform: no column of the warp's neighbourhoods is clamped -> one pointer per row
 #pragma unroll
           for (int k = 0; k < 5; ++k) {
-            const T* rp = pl + (ro[k] + (x - 2));
+            const T* rp = pl + (ro[k] + (x - 2) * PS);
 #pragma unroll
-            for (int m = 0; m < 5; ++m) nb[cc][k][m] = lr_px(rp + m);
+            for (int m = 0; m < 5; ++m) nb[cc][k][m] = lr_px(rp + m * PS);
           }
         } else {
 #pragma unroll
@@ -406,6 +475,18 @@ __device__ __forceinline__ void epi_head_rt(const EpiParams& p, const T* __restr
     }
   }
 
+  if constexpr (YN) {  // (no skip-from-buffer: the API refuses it with interleaved images)
+#pragma unroll
+    for (int i = 0; i < R; ++i) {
+      float v[3 * R];
+#pragma unroll
+      for (int j = 0; j < R; ++j)
+#pragma unroll
+        for (int c = 0; c < 3; ++c) v[3 * j + c] = out[c][i][j];
+      store_hr_row_nhwc<R>(p, static_cast<size_t>(first) + static_cast<size_t>(i) * row_pitch, v);
+    }
+    return;
+  }
   if (p.y8 != nullptr) {  // 8-bit output: R bytes per HR row segment (a warp writes 32 * R contiguous bytes)
 #pragma unroll
     for (int c = 0; c < 3; ++c)
@@ -474,28 +555,31 @@ __device__ __forceinline__ void epi_head_rt(const EpiParams& p, const T* __restr
     }
 }
 // interior: warp-uniform promise that x - 2 >= 0 and x + 2 < W for every lane of the calling warp
-template <int R>
+// (the layouts are template parameters of the calling kernel: one runtime branch over four layouts in the same kernel
+// raises the planar head's registers and makes it spill)
+template <int R, bool XN, bool YN>
 __device__ __forceinline__ void epi_head_r(const EpiParams& p, int b, int y, int x, const float (&acc)[48], bool interior) {
   if (p.x8 != nullptr)
-    epi_head_rt<R, uint8_t>(p, p.x8, b, y, x, acc, interior);
+    epi_head_rt<R, uint8_t, XN, YN>(p, p.x8, b, y, x, acc, interior);
   else
-    epi_head_rt<R, float>(p, p.x, b, y, x, acc, interior);
+    epi_head_rt<R, float, XN, YN>(p, p.x, b, y, x, acc, interior);
 }
 // r = 2, TWO vertically adjacent LR pixels (y, x) and (y + 1, x) per thread: their 5x5 neighbourhoods share four of
 // five rows, so the pair costs 6 x 5 loads and 6 x 2 horizontal interpolations per colour instead of 2 x (5 x 5) and
 // 2 x (5 x 2), and -- what matters for the latency-bound epilogue warps -- ONE exposed load latency instead of two.
 // Same FMA order per output as epi_head_rt<2>: the results are bit-identical.  v0 / v1: the twelve head channels of the
-// two pixels as they come out of TMEM; second: row y + 1 exists (y + 1 < H).
-template <typename T>
+// two pixels as they come out of TMEM; second: row y + 1 exists (y + 1 < H).  XN / YN as in epi_head_rt.
+template <typename T, bool XN, bool YN>
 __device__ __forceinline__ void epi_head2_pair(const EpiParams& p, const T* __restrict__ lr, int b, int y, int x,
                                                const uint32_t (&v0)[16], const uint32_t (&v1)[16], bool interior,
                                                bool second) {
   const int H = p.H, W = p.W;
   long long first[2];
-  first[0] = head_out_index(p, b, 0, y, x, 0, 0);
-  first[1] = second ? head_out_index(p, b, 0, y + 1, x, 0, 0) : -1;
+  first[0] = head_out_index_l<YN>(p, b, 0, y, x, 0, 0);
+  first[1] = second ? head_out_index_l<YN>(p, b, 0, y + 1, x, 0, 0) : -1;
   if (first[0] < 0 && first[1] < 0) return;  // both outside the output window
-  const size_t row_pitch = p.y_row ? static_cast<size_t>(p.y_row) : static_cast<size_t>(W) * 2;
+  const size_t row_pitch = p.y_row ? static_cast<size_t>(p.y_row) : static_cast<size_t>(W) * 2 * (YN ? 3 : 1);
+  constexpr int PS = XN ? 3 : 1;  // elements between horizontally adjacent LR pixels of one colour
   const size_t plane_pitch = p.y_plane ? static_cast<size_t>(p.y_plane) : static_cast<size_t>(H) * 2 * W * 2;
   float out[2][3][2][2];
 #pragma unroll
@@ -512,19 +596,19 @@ __device__ __forceinline__ void epi_head2_pair(const EpiParams& p, const T* __re
     const T* img = lr + static_cast<size_t>(b) * 3 * HW;
     int xo[5], ro[6];
 #pragma unroll
-    for (int m = 0; m < 5; ++m) xo[m] = min(max(x - 2 + m, 0), W - 1);
+    for (int m = 0; m < 5; ++m) xo[m] = min(max(x - 2 + m, 0), W - 1) * PS;
 #pragma unroll
-    for (int k = 0; k < 6; ++k) ro[k] = min(max(y - 2 + k, 0), H - 1) * W;
+    for (int k = 0; k < 6; ++k) ro[k] = min(max(y - 2 + k, 0), H - 1) * W * PS;
     float nb[3][6][5];
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
-      const T* pl = img + c * HW;
+      const T* pl = img + (XN ? c : c * HW);
       if (interior) {
 #pragma unroll
         for (int k = 0; k < 6; ++k) {
-          const T* rp = pl + (ro[k] + (x - 2));
+          const T* rp = pl + (ro[k] + (x - 2) * PS);
 #pragma unroll
-          for (int m = 0; m < 5; ++m) nb[c][k][m] = lr_px(rp + m);
+          for (int m = 0; m < 5; ++m) nb[c][k][m] = lr_px(rp + m * PS);
         }
       } else {
 #pragma unroll
@@ -557,6 +641,22 @@ __device__ __forceinline__ void epi_head2_pair(const EpiParams& p, const T* __re
             out[rr][c][i][j] += a;
           }
     }
+  }
+  if constexpr (YN) {  // (no skip-from-buffer: the API refuses it with interleaved images)
+#pragma unroll
+    for (int rr = 0; rr < 2; ++rr) {
+      if (first[rr] < 0) continue;
+#pragma unroll
+      for (int i = 0; i < 2; ++i) {
+        float v[6];
+#pragma unroll
+        for (int j = 0; j < 2; ++j)
+#pragma unroll
+          for (int c = 0; c < 3; ++c) v[3 * j + c] = out[rr][c][i][j];
+        store_hr_row_nhwc<2>(p, static_cast<size_t>(first[rr]) + static_cast<size_t>(i) * row_pitch, v);
+      }
+    }
+    return;
   }
   if (p.skip_mode == 1 && p.y8 == nullptr) {  // y already holds the bicubic image: every segment is read before the first store
     float2 sk[2][3][2];
@@ -598,6 +698,14 @@ __device__ __forceinline__ void epi_head2_pair(const EpiParams& p, const T* __re
         }
       }
   }
+}
+template <bool XN, bool YN>
+__device__ __forceinline__ void epi_head2(const EpiParams& p, int b, int y, int x, const uint32_t (&v0)[16],
+                                          const uint32_t (&v1)[16], bool interior, bool second) {
+  if (p.x8 != nullptr)
+    epi_head2_pair<uint8_t, XN, YN>(p, p.x8, b, y, x, v0, v1, interior, second);
+  else
+    epi_head2_pair<float, XN, YN>(p, p.x, b, y, x, v0, v1, interior, second);
 }
 #endif  // __CUDACC__
 

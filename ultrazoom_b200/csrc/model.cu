@@ -161,12 +161,16 @@ static int run_conv(mz_model* m, int slot, const ConvArgs& a, const ConvTcTune& 
     key.a.epi.u8_trunc = key.a.epi.skip_mode = key.a.epi.clamp01 = 0;
     key.a.epi.wy0 = key.a.epi.wy1 = key.a.epi.wx0 = key.a.epi.wx1 = 0;
     key.a.epi.y_row = key.a.epi.y_plane = 0;
+    key.a.epi.x_nhwc = key.a.epi.y_nhwc = 0;
   }
   // kWays prepared launches per convolution: the host lanes, the engine workspace and captured graphs alternate operands
   for (int way = 0; way < kWays; ++way) {
     const int i = kWays * slot + way;
     if (m->prepared[i].valid && memcmp(&key, &m->keys[i], sizeof(key)) == 0) {
-      if (a.epi.mode == 2) patch_conv_epi(m->prepared[i], a.epi);
+      if (a.epi.mode == 2) {
+        const int rc = patch_conv_epi(m->prepared[i], a.epi);
+        if (rc != MZ_OK) return rc;
+      }
       return run_conv_tc(m->prepared[i], s);
     }
   }
@@ -572,6 +576,11 @@ static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, in
   const bool io8 = (flags & MZ_FLAG_IO_U8) != 0;
   MZ_REQUIRE(!io8 || ((flags & MZ_FLAG_CLAMP01) && !(flags & MZ_FLAG_SKIP_FROM_BUFFER)),
              "upscale: 8-bit image I/O needs MZ_FLAG_CLAMP01 and recomputes the skip (no MZ_FLAG_SKIP_FROM_BUFFER)");
+  const bool x_nhwc = (flags & MZ_FLAG_X_NHWC) != 0, y_nhwc = (flags & MZ_FLAG_Y_NHWC) != 0;
+  MZ_REQUIRE(!((x_nhwc || y_nhwc) && (flags & MZ_FLAG_SKIP_FROM_BUFFER)),
+             "upscale: interleaved images (MZ_FLAG_X_NHWC / MZ_FLAG_Y_NHWC) recompute the skip (no MZ_FLAG_SKIP_FROM_BUFFER)");
+  MZ_REQUIRE(!(x_nhwc || y_nhwc) || static_cast<long long>(H) * W * 3 < (1LL << 31),
+             "upscale: an interleaved %d x %d image exceeds 2^31 elements", H, W);
   const float* x_dev = io8 ? nullptr : static_cast<const float*>(x_dev_v);
   float* y_dev = io8 ? nullptr : static_cast<float*>(y_dev_v);
   const uint8_t* x8 = io8 ? static_cast<const uint8_t*>(x_dev_v) : nullptr;
@@ -614,7 +623,7 @@ static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, in
   rc = MZ_OK;
   if (front)
     rc = launch_stem(x_dev, x8, m->stem_w, m->stem_b, zf, zb, m->bf16, B, H, W, m->Cpm, m->Czm, s,
-                     m->sat_dev);
+                     m->sat_dev, x_nhwc);
   if (rc != MZ_OK) return rc;
 
   const int slot = m->timing_calls % kTimingSlots;
@@ -737,6 +746,8 @@ static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, in
   a.epi.r = m->r;
   a.epi.skip_mode = skip_mode;
   a.epi.clamp01 = (flags & MZ_FLAG_CLAMP01) ? 1 : 0;
+  a.epi.x_nhwc = x_nhwc ? 1 : 0;
+  a.epi.y_nhwc = y_nhwc ? 1 : 0;
   if (win) {
     a.epi.wy0 = win->y0;
     a.epi.wy1 = win->y1;
@@ -764,12 +775,13 @@ int mz_upscale_window(mz_model* m, const void* x_dev, const float* c_dev, int32_
   MZ_REQUIRE(0 <= win_y0 && win_y0 < win_y1 && win_y1 <= H && 0 <= win_x0 && win_x0 < win_x1 && win_x1 <= W,
              "upscale_window: window [%d, %d) x [%d, %d) is not inside the %d x %d input", win_y0, win_y1, win_x0, win_x1,
              H, W);
-  const int64_t r = m->r;
-  MZ_REQUIRE(y_row_pitch >= (win_x1 - win_x0) * r && y_plane_pitch >= y_row_pitch * (win_y1 - win_y0) * r,
+  const int64_t r = m->r, ch = (flags & MZ_FLAG_Y_NHWC) ? 3 : 1;  // (elements per HR pixel in a row)
+  MZ_REQUIRE(y_row_pitch >= (win_x1 - win_x0) * r * ch && y_plane_pitch >= y_row_pitch * (win_y1 - win_y0) * r,
              "upscale_window: pitches (%lld, %lld) are smaller than the window", static_cast<long long>(y_row_pitch),
              static_cast<long long>(y_plane_pitch));
   MZ_REQUIRE(!(flags & MZ_FLAG_SKIP_FROM_BUFFER), "upscale_window: the bicubic skip is recomputed (no MZ_FLAG_SKIP_FROM_BUFFER)");
-  const int es = (flags & MZ_FLAG_IO_U8) ? 1 : 4, vec = m->r == 3 ? es : es * m->r;  // bytes of one vector store
+  // bytes of one vector store: the same in both layouts (an interleaved HR row segment of a pixel is three of them)
+  const int es = (flags & MZ_FLAG_IO_U8) ? 1 : 4, vec = m->r == 3 ? es : es * m->r;
   MZ_REQUIRE(reinterpret_cast<uintptr_t>(y_dev) % vec == 0 && (y_row_pitch * es) % vec == 0 && (y_plane_pitch * es) % vec == 0,
              "upscale_window: y and its pitches must be aligned to %d bytes", vec);
   const OutWindow w{win_y0, win_y1, win_x0, win_x1, y_row_pitch, y_plane_pitch};

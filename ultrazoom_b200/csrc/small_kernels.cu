@@ -159,6 +159,8 @@ int launch_bicubic(const float* x, float* y, int planes, int H, int W, int r, cu
 // store 256 (the first version's 8 channels per thread wrote every other 16 bytes of a 1 KB span per instruction:
 // 1.67 x the L2 sectors, ncu l1tex 75 % busy at 62 % of the DRAM peak).  The block first stages the three colour
 // planes of its pixel range in shared memory with coalesced loads, so the store loop never waits for a global load.
+// x_nhwc: x is interleaved (B,H,W,3); images are 3HW elements apart in both layouts, so the block's pixel range is one
+// contiguous run of 3n elements even across images, read with coalesced loads into the same planar staging.
 // ----------------------------------------------------------------------------------------------
 __device__ __forceinline__ void st_global_v2(void* p, uint32_t a, uint32_t b) {
   asm volatile("st.global.v2.b32 [%0], {%1, %2};" ::"l"(p), "r"(a), "r"(b) : "memory");
@@ -168,7 +170,7 @@ __global__ void __launch_bounds__(256) stem_kernel(const float* __restrict__ x, 
                                                    const float* __restrict__ w,
                                                    const float* __restrict__ bias, float* __restrict__ zf,
                                                    uint16_t* __restrict__ zb, int bf16, int B, int H, int W, int Cp,
-                                                   int Cz, int ppb, unsigned int* sat) {
+                                                   int Cz, int ppb, unsigned int* sat, int x_nhwc) {
   extern __shared__ float xs[];  // [3][ppb]: the block's pixels, colour planes apart
   // blockDim = (channel groups of 4, pixels per pass): a thread keeps ITS four channels' weights and bias in registers
   const int g = threadIdx.x;
@@ -185,7 +187,14 @@ __global__ void __launch_bounds__(256) stem_kernel(const float* __restrict__ x, 
   const size_t npix = static_cast<size_t>(B) * plane;
   const size_t p0 = static_cast<size_t>(blockIdx.x) * ppb;
   const int n = static_cast<int>((p0 + ppb < npix ? p0 + ppb : npix) - p0);
-  {
+  if (x_nhwc) {
+    const int tid = threadIdx.y * blockDim.x + threadIdx.x, nt = blockDim.x * blockDim.y;
+    const size_t e0 = p0 * 3;
+    for (int e = tid; e < 3 * n; e += nt) {
+      const int j = e / 3, c = e - 3 * j;
+      xs[c * ppb + j] = x8 != nullptr ? __fdiv_rn(static_cast<float>(__ldg(x8 + e0 + e)), 255.f) : __ldg(x + e0 + e);
+    }
+  } else {
     const size_t b0 = p0 / plane, rem0 = p0 - b0 * plane;  // (one division per block; the range may cross images)
     const int tid = threadIdx.y * blockDim.x + threadIdx.x, nt = blockDim.x * blockDim.y;
     for (int j = tid; j < n; j += nt) {
@@ -222,7 +231,7 @@ __global__ void __launch_bounds__(256) stem_kernel(const float* __restrict__ x, 
 }
 
 int launch_stem(const float* x, const uint8_t* x8, const float* w, const float* bias, float* zf, uint16_t* zb, int bf16,
-                int B, int H, int W, int Cp, int zb_pitch, cudaStream_t s, unsigned int* sat) {
+                int B, int H, int W, int Cp, int zb_pitch, cudaStream_t s, unsigned int* sat, bool x_nhwc) {
   MZ_REQUIRE(Cp > 0 && Cp % 8 == 0, "stem: padded channel count must be a multiple of 8, %d given", Cp);
   MZ_REQUIRE(B > 0 && H > 0 && W > 0, "stem: empty input");
   MZ_REQUIRE(zf != nullptr, "stem: null fp32 stream");
@@ -241,7 +250,7 @@ int launch_stem(const float* x, const uint8_t* x8, const float* w, const float* 
   MZ_REQUIRE(blocks < (1LL << 31), "stem: too many pixels");
   const size_t smem = static_cast<size_t>(3) * ppb * sizeof(float);
   stem_kernel<<<static_cast<unsigned>(blocks), dim3(groups, py), smem, s>>>(x, x8, w, bias, zf, zb, bf16, B, H, W, Cp, Cz,
-                                                                         static_cast<int>(ppb), sat);
+                                                                         static_cast<int>(ppb), sat, x_nhwc ? 1 : 0);
   MZ_CUDA(cudaGetLastError());
   return MZ_OK;
 }

@@ -25,6 +25,38 @@ except Exception:  # pragma: no cover - hub not installed
 from . import _native
 
 
+def _is_nhwc(t: Tensor) -> bool:
+    """``t`` holds interleaved pixels: (B,3,H,W) in ``channels_last`` strides -- what a numpy / PIL / video frame becomes
+    through ``torch.from_numpy(frames).permute(0, 3, 1, 2)`` -- and not also plainly contiguous."""
+    return t.is_contiguous(memory_format=torch.channels_last) and not t.is_contiguous()
+
+
+def _input_image(x: Tensor, io8: bool):
+    """``(x, flag)``: the image as the kernels read it -- uint8 as it is, anything else as float32 -- kept interleaved
+    when it is (``MZ_FLAG_X_NHWC``, no transpose), otherwise made contiguous NCHW."""
+    nhwc = _is_nhwc(x)
+    x = x.detach() if io8 else x.detach().to(torch.float32)
+    x = x.contiguous(memory_format=torch.channels_last if nhwc else torch.contiguous_format)
+    return x, (_native.FLAG_X_NHWC if nhwc else 0)
+
+
+def _output_flag(memory_format) -> int:
+    assert memory_format in (torch.contiguous_format, torch.channels_last), (
+        "memory_format must be torch.contiguous_format or torch.channels_last")
+    return _native.FLAG_Y_NHWC if memory_format == torch.channels_last else 0
+
+
+def _frame_layout(frame: Tensor):
+    """``(flag, row pitch, image-or-plane pitch)`` of an assembled output frame (B,3,H',W'): interleaved (channels-last
+    strides: ``stride(1) == 1``, ``stride(3) == 3``; rows and images at any pitch) or planar (``stride(3) == 1``, evenly
+    spaced planes)."""
+    if frame.stride(1) == 1 and frame.stride(3) == 3:
+        return _native.FLAG_Y_NHWC, frame.stride(2), frame.stride(0)
+    assert frame.stride(3) == 1, "frame must be planar (stride(3) == 1) or interleaved (stride(1) == 1, stride(3) == 3)"
+    assert frame.stride(0) == 3 * frame.stride(1), "frame planes must be evenly spaced"
+    return 0, frame.stride(2), frame.stride(1)
+
+
 class FanOutProjection(nn.Module):
     """Parameter holder for the 1x1 stem (reference model.py:212-242)."""
 
@@ -367,7 +399,8 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         assert c.shape[0] in (1, x.shape[0]), "Batch size of c must match x."
         return c
 
-    def _run(self, x: Tensor, c: Optional[Tensor], flags: int, ws: Optional[Tensor] = None) -> Tensor:
+    def _run(self, x: Tensor, c: Optional[Tensor], flags: int, ws: Optional[Tensor] = None,
+             memory_format=torch.contiguous_format) -> Tensor:
         c = self._check_inputs(x, c)
         if not x.is_cuda:
             raise RuntimeError("ultrazoom_b200.MewZoom runs on sm_100a CUDA kernels only; move the input to a "
@@ -377,7 +410,8 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         if io8:
             assert flags & _native.FLAG_CLAMP01, "uint8 images are supported by upscale(), not forward()"
             flags |= _native.FLAG_IO_U8 | (_native.FLAG_U8_TRUNC if self.u8_truncate else 0)
-        x = x.detach().contiguous() if io8 else x.detach().to(torch.float32).contiguous()
+        x, xflag = _input_image(x, io8)
+        flags |= xflag | _output_flag(memory_format)
         if c is not None:
             c = c.detach().to(device=dev, dtype=torch.float32).contiguous()
         B, _, H, W = x.shape
@@ -395,7 +429,8 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
                         "(model.saturated(reset=True) clears the flag).")
                 self._auto_dtype = "bfloat16"
                 continue
-            y = torch.empty((B, 3, H * r, W * r), dtype=torch.uint8 if io8 else torch.float32, device=dev)
+            y = torch.empty((B, 3, H * r, W * r), dtype=torch.uint8 if io8 else torch.float32, device=dev,
+                            memory_format=memory_format)
             stream = torch.cuda.current_stream(dev)
             eng.begin(stream)
             w = ws if ws is not None else eng.workspace(B, H, W, stream)
@@ -414,19 +449,25 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
             return y
 
     # ---- reference model.py:149-179 ----
-    def forward(self, x: Tensor, c: Optional[Tensor] = None) -> Tensor:
-        """bicubic(x) + residual network, un-clamped (reference model.py:149-164)."""
-        return self._run(x, c, 0)
+    def forward(self, x: Tensor, c: Optional[Tensor] = None, *, memory_format=torch.contiguous_format) -> Tensor:
+        """bicubic(x) + residual network, un-clamped (reference model.py:149-164).  See ``upscale`` for the layouts."""
+        return self._run(x, c, 0, memory_format=memory_format)
 
     @torch.inference_mode()
-    def upscale(self, x: Tensor, c: Optional[Tensor] = None) -> Tensor:
+    def upscale(self, x: Tensor, c: Optional[Tensor] = None, *, memory_format=torch.contiguous_format) -> Tensor:
         """``clamp(forward(x, c), 0, 1)`` (reference model.py:166-179); the clamp is fused in the head kernel.
 
         A ``torch.uint8`` image (what ``decode_image`` returns, reference test_compare.py:53) is read as ``x / 255``
         (``ToDtype(float32, scale=True)``, test_compare.py:55-57) and the result comes back as uint8,
         ``floor(255 * y + 0.5)`` as ``save_image`` writes it (test_compare.py:89) -- or ``floor(255 * y)`` as
-        ``ToPILImage`` does (README.md:81) when ``model.u8_truncate`` is set: a quarter of the image traffic."""
-        return self._run(x, c, _native.FLAG_CLAMP01)
+        ``ToPILImage`` does (README.md:81) when ``model.u8_truncate`` is set: a quarter of the image traffic.
+
+        Interleaved images need no transpose on either side: an ``x`` in ``channels_last`` strides (and not also plainly
+        contiguous), e.g. ``torch.from_numpy(hwc_frames).permute(0, 3, 1, 2)``, is read as it is, and
+        ``memory_format=torch.channels_last`` returns ``y`` in channels-last strides, so ``y.permute(0, 2, 3, 1)`` is a
+        contiguous (B,rH,rW,3) array.  The default output is contiguous NCHW whatever the input's layout.  The results
+        are bit-identical in every layout."""
+        return self._run(x, c, _native.FLAG_CLAMP01, memory_format=memory_format)
 
     @torch.inference_mode()
     def test_compare(self, x: Tensor, c: Optional[Tensor] = None):
@@ -442,7 +483,8 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         """Halo-tiled inference without a tile output: ``upscale`` the LR tile ``x`` and write only its core -- the LR
         pixels ``window = (y0, y1, x0, x1)`` of the tile -- straight into ``frame`` (B,3,rH',rW'), whose HR pixel
         ``at = (fy, fx)`` receives the core's first pixel (mz_upscale_window).  ``frame`` may live on another GPU
-        (``sharding.share_frame``): the head kernel's stores are then the transfer over NVLink."""
+        (``sharding.share_frame``): the head kernel's stores are then the transfer over NVLink.  ``frame`` is planar or
+        interleaved (channels-last strides, any row and image pitch, e.g. a view into a wider HWC buffer)."""
         c = self._check_inputs(x, c)
         if not x.is_cuda:
             raise RuntimeError("ultrazoom_b200.MewZoom runs on sm_100a CUDA kernels only (no CPU fallback).")
@@ -452,7 +494,7 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         flags = _native.FLAG_CLAMP01 | self._flags_extra
         if io8:
             flags |= _native.FLAG_IO_U8 | (_native.FLAG_U8_TRUNC if self.u8_truncate else 0)
-        x = x.detach().contiguous() if io8 else x.detach().to(torch.float32).contiguous()
+        x, xflag = _input_image(x, io8)
         if c is not None:
             c = c.detach().to(device=dev, dtype=torch.float32).contiguous()
         B, _, H, W = x.shape
@@ -460,8 +502,9 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         y0, y1, x0, x1 = window
         fy, fx = at
         assert frame.is_cuda and frame.dim() == 4 and frame.shape[0] == B and frame.shape[1] == 3, "frame must be (B,3,H',W')"
-        assert frame.dtype == (torch.uint8 if io8 else torch.float32) and frame.stride(3) == 1
-        assert frame.stride(0) == 3 * frame.stride(1), "frame planes must be evenly spaced"
+        assert frame.dtype == (torch.uint8 if io8 else torch.float32)
+        yflag, row_pitch, img_pitch = _frame_layout(frame)
+        flags |= xflag | yflag
         assert 0 <= fy and fy + (y1 - y0) * r <= frame.shape[2] and 0 <= fx and fx + (x1 - x0) * r <= frame.shape[3], (
             "the window does not fit into the frame at that position")
         if frame.device != dev:
@@ -473,7 +516,7 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         dst = frame[0, 0, fy, fx].data_ptr() if frame.numel() else 0
         _native.check(eng.lib.mz_upscale_window(
             eng.handle, x.data_ptr(), c.data_ptr() if c is not None else None, c.shape[0] if c is not None else 0,
-            dst, frame.stride(2), frame.stride(1), B, H, W, y0, y1, x0, x1, ws_ptr,
+            dst, row_pitch, img_pitch, B, H, W, y0, y1, x0, x1, ws_ptr,
             ws.numel() - (ws_ptr - ws.data_ptr()), flags, stream.cuda_stream))
         eng.end(stream)
 
@@ -493,15 +536,16 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         flags = _native.FLAG_CLAMP01 | self._flags_extra
         if io8:
             flags |= _native.FLAG_IO_U8 | (_native.FLAG_U8_TRUNC if self.u8_truncate else 0)
-        x = x.contiguous()
+        x, xflag = _input_image(x, io8)
         if c is not None:
             c = c.detach().to(device=dev, dtype=torch.float32).contiguous()
         B, _, H, W = x.shape
         r = self.upscale_ratio
         y0, y1, x0, x1 = window
         fy, fx = at
-        assert frame.is_cuda and frame.dim() == 4 and frame.shape[0] == B and frame.shape[1] == 3 and frame.stride(3) == 1
-        assert frame.stride(0) == 3 * frame.stride(1), "frame planes must be evenly spaced"
+        assert frame.is_cuda and frame.dim() == 4 and frame.shape[0] == B and frame.shape[1] == 3
+        yflag, row_pitch, img_pitch = _frame_layout(frame)
+        flags |= xflag | yflag
         if frame.device != dev:
             _native.check(eng.lib.mz_enable_peer_access(dev.index or 0, frame.device.index or 0))
         stream = torch.cuda.current_stream(dev)
@@ -509,7 +553,7 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         dst = frame[0, 0, fy, fx].data_ptr()
         _native.check(eng.lib.mz_upscale_stage(
             eng.handle, x.data_ptr(), c.data_ptr() if c is not None else None, c.shape[0] if c is not None else 0,
-            dst, frame.stride(2), frame.stride(1), B, H, W, y0, y1, x0, x1, ws_ptr, ws.numel() - (ws_ptr - ws.data_ptr()),
+            dst, row_pitch, img_pitch, B, H, W, y0, y1, x0, x1, ws_ptr, ws.numel() - (ws_ptr - ws.data_ptr()),
             flags, stream.cuda_stream, layer_begin, layer_end))
 
     def stage_workspace(self, shape, device: torch.device) -> Tensor:
@@ -537,38 +581,48 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         z16 = ws[base + off: base + off + npix * pitch * 2].view(dt16).view(B, H, W, pitch)
         return zf, z16
 
-    def capture(self, x: Tensor, c: Optional[Tensor] = None, clamp: bool = True) -> "GraphedUpscale":
+    def capture(self, x: Tensor, c: Optional[Tensor] = None, clamp: bool = True, *,
+                memory_format=torch.contiguous_format) -> "GraphedUpscale":
         """Record one ``upscale`` (``clamp=False``: ``forward``) call at the shape of ``x`` into a CUDA graph.
 
         A frame of a few hundred pixels a side is launch-bound (2L + 3 kernels, most of them cluster launches of
         15-20 us of host time each); replaying the recorded graph removes the host from that loop.  The dependent-launch
-        edges between the kernels are kept by the capture.  See ``GraphedUpscale``."""
-        return GraphedUpscale(self, x, c, _native.FLAG_CLAMP01 if clamp else 0)
+        edges between the kernels are kept by the capture.  The graph reads its input in the layout of ``x`` and writes
+        its output in ``memory_format`` (see ``upscale``).  See ``GraphedUpscale``."""
+        return GraphedUpscale(self, x, c, _native.FLAG_CLAMP01 if clamp else 0, memory_format)
 
     @torch.inference_mode()
     def upscale_host(self, x: Tensor, c: Optional[Tensor] = None, out: Optional[Tensor] = None,
-                     device: int = 0, lane: Optional[int] = None) -> Tensor:
+                     device: int = 0, lane: Optional[int] = None, *, memory_format=torch.contiguous_format) -> Tensor:
         """End-to-end call with HOST tensors: H2D copy, kernels, D2H copy (mz_upscale_host).
 
         ``lane=None``: synchronous; a batch is cut into chunks whose copies overlap the kernels of their neighbours.
         ``lane=0|1``: frame-stream form (mz_upscale_host_async) -- the call only enqueues and returns ``out`` at once;
         ``out`` is valid after ``host_wait(lane)``.  Alternating lanes double-buffers a stream of frames.  ``x``, ``c``
-        and ``out`` should be pinned and must not be touched until the wait."""
+        and ``out`` should be pinned and must not be touched until the wait.
+
+        Layouts as in ``upscale``: a channels-last ``x`` is copied as it is (no transpose on the CPU), and the result is
+        interleaved with ``memory_format=torch.channels_last``.  A caller's ``out`` sets the output layout itself: it
+        must be contiguous NCHW or contiguous channels-last."""
         c = self._check_inputs(x, c)
         assert not x.is_cuda, "upscale_host takes host tensors"
         assert lane in (None, 0, 1), "lane must be None, 0 or 1"
         eng = self._engine(torch.device("cuda", device))
         io8 = x.dtype == torch.uint8
-        x = x.contiguous() if io8 else x.to(torch.float32).contiguous()
+        x, xflag = _input_image(x, io8)
         if c is not None:
             c = c.to(device="cpu", dtype=torch.float32).contiguous()
         B, _, H, W = x.shape
         r = self.upscale_ratio
         odt = torch.uint8 if io8 else torch.float32
         if out is None:
-            out = torch.empty((B, 3, H * r, W * r), dtype=odt)
-        assert out.is_contiguous() and tuple(out.shape) == (B, 3, H * r, W * r) and out.dtype == odt
-        flags = _native.FLAG_CLAMP01 | self._flags_extra
+            out = torch.empty((B, 3, H * r, W * r), dtype=odt, memory_format=memory_format)
+            yflag = _output_flag(memory_format)
+        else:
+            yflag = _native.FLAG_Y_NHWC if _is_nhwc(out) else 0
+            assert out.is_contiguous() or yflag, "out must be contiguous NCHW or contiguous channels-last"
+        assert tuple(out.shape) == (B, 3, H * r, W * r) and out.dtype == odt
+        flags = _native.FLAG_CLAMP01 | self._flags_extra | xflag | yflag
         if io8:
             flags |= _native.FLAG_IO_U8 | (_native.FLAG_U8_TRUNC if self.u8_truncate else 0)
         cp, cr = (c.data_ptr(), c.shape[0]) if c is not None else (None, 0)
@@ -599,12 +653,14 @@ class GraphedUpscale:
     ``g.x`` / ``g.c`` yourself).  The graph reads the engine's packed weights in place: parameters changed after the
     capture are picked up by the next ordinary call (which re-packs them), not by a replay on its own."""
 
-    def __init__(self, model: MewZoom, x: Tensor, c: Optional[Tensor], flags: int):
+    def __init__(self, model: MewZoom, x: Tensor, c: Optional[Tensor], flags: int,
+                 memory_format=torch.contiguous_format):
         c = model._check_inputs(x, c)
         if not x.is_cuda:
             raise RuntimeError("MewZoom.capture needs a CUDA input (there is no CPU fallback).")
         self.model = model
-        self.x = (x.detach() if x.dtype == torch.uint8 else x.detach().to(torch.float32)).contiguous().clone()
+        # (the input buffer keeps the layout of x: the graph reads it as _run reads x; a replay copies either layout in)
+        self.x = _input_image(x, x.dtype == torch.uint8)[0].clone()
         self.c = None if c is None else c.detach().to(device=x.device, dtype=torch.float32).contiguous().clone()
         # The graph bakes in raw pointers: it owns everything they point at -- its input / output tensors, a PRIVATE
         # workspace (the engine's cached one is dropped and re-allocated when a later call needs a larger one) and the
@@ -618,11 +674,11 @@ class GraphedUpscale:
             side = torch.cuda.Stream(device=x.device)
             side.wait_stream(torch.cuda.current_stream(x.device))
             with torch.cuda.stream(side):        # warm-up: packs the weights, prepares the launches
-                model._run(self.x, self.c, flags, ws=self.ws)
+                model._run(self.x, self.c, flags, ws=self.ws, memory_format=memory_format)
             torch.cuda.current_stream(x.device).wait_stream(side)
             self.graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(self.graph):
-                self.y = model._run(self.x, self.c, flags, ws=self.ws)
+                self.y = model._run(self.x, self.c, flags, ws=self.ws, memory_format=memory_format)
 
     def replay(self) -> Tensor:
         self.graph.replay()
