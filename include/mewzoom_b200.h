@@ -126,7 +126,11 @@ int mz_model_set_weight_dev(mz_model* m, int32_t kind, int32_t layer, const floa
  * of the residual stream, or a device-packed weight -- also sets a host-mapped flag.  *saturated = 1 if any kernel
  * that has COMPLETED so far did (the call does not synchronise; synchronise the stream first for a definite answer
  * about a particular mz_upscale).  reset != 0 clears the flag.  A saturated result is wrong: re-run the frame on a
- * model created with MZ_DTYPE_BF16 (same range as fp32).  mz_model_set_weight rejects out-of-range weights at once. */
+ * model created with MZ_DTYPE_BF16 (same range as fp32).  mz_model_set_weight rejects out-of-range weights at once.
+ * No entry point of this ABI checks the flag itself (mz_upscale_host included): callers read it.  The Python mirror
+ * (MewZoom) checks it at every entry point: upscale_host, host_wait and capture raise in the call, the others on the
+ * next call; operand_dtype="auto" re-runs forward / upscale / upscale_into / upscale_host with bf16 operands.  The U-Net
+ * operators (mz_adaptive_mix, mz_pixel_crush, ...) and the per-kernel entry points do not track the range. */
 int mz_model_saturated(mz_model* m, int32_t reset, int32_t* saturated);
 
 /* Bytes of device scratch mz_upscale needs for a (B,3,H,W) input. */

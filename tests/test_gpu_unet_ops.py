@@ -11,6 +11,7 @@ import torch
 
 from oracle import unet_oracle as U
 from tests.helpers import GOLDEN
+from tests.test_gpu_fp16_range import same16
 
 pytestmark = pytest.mark.gpu
 
@@ -126,8 +127,9 @@ def test_mix_and_crush_against_the_oracle_at_other_shapes(dev, C, shape):
 @pytest.mark.parametrize("math", ["tf32", "fp32"])
 @pytest.mark.parametrize("dt", [torch.float16, torch.bfloat16])
 def test_sixteen_bit_shadow_is_the_rounded_output(dev, math, dt):
-    """Both operators can also write the 16-bit copy the tcgen05 convolutions read: exactly round16(out); many tiles per
-    CTA (more tiles than SMs) and a deterministic result."""
+    """Both operators (and the pixel shuffle) can also write the 16-bit copy the tcgen05 convolutions read: exactly
+    round16(out), i.e. ``out.to(dt)`` -- beyond the fp16 range too, where that is +-inf (the shadow replaces the cast, it
+    does not clip); NaN compared by NaN-ness.  Many tiles per CTA (more tiles than SMs) and a deterministic result."""
     from ultrazoom_b200 import unet as N
 
     g = torch.Generator().manual_seed(11)
@@ -144,6 +146,17 @@ def test_sixteen_bit_shadow_is_the_rounded_output(dev, math, dt):
     assert tuple(out.shape) == (2, 75, 150, 96) and torch.equal(sh, out.to(dt))
     want = U.pixel_crush(N.to_nchw(x).cpu(), wc, 2)
     _close(out, want, TF32_TOL * want.abs().max().item() if math == "tf32" else 2e-5)
+    # beyond the fp16 range: outputs up to ~1e5, a few inputs at the edge, inf and NaN
+    xw, zw = x * 3e4, z * 3e4
+    xw[0, 7, 11, :8] = torch.tensor([float("inf"), -float("inf"), float("nan"), 1e5, -65519.99, 65520.0, 3e38, 2.0**-25])
+    out, sh = N.adaptive_residual_mix(xw, zw, w, torch.tensor(0.3), math, shadow=dt)
+    assert float(out.abs().nan_to_num(0, 0, 0).max()) > 65520
+    same16(sh, out.to(dt))
+    out, sh = N.pixel_crush(xw, wc, 2, math, shadow=dt)
+    assert float(out.abs().nan_to_num(0, 0, 0).max()) > 65520
+    same16(sh, out.to(dt))
+    out = N.pixel_shuffle_nhwc(xw, 2, shadow=dt)
+    same16(out._mz16[0], out.to(dt))
 
 
 @pytest.mark.parametrize("C,hidden_ratio,shape", [(96, 2, (1, 24, 150)), (192, 2, (1, 10, 140)), (384, 2, (1, 6, 40)), (64, 4, (2, 9, 70))])

@@ -429,9 +429,19 @@ __device__ __forceinline__ uint32_t pack_f16x2(float lo, float hi) {  // saturat
   asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
   return r;
 }
+__device__ __forceinline__ uint32_t pack_f16x2_rn(float lo, float hi) {  // plain rounding: +-inf beyond the range, as torch
+  uint32_t r;
+  asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+  return r;
+}
 // MMA-operand element type of the activations / weights: 0 = fp16 (default), 1 = bf16.
 __device__ __forceinline__ uint32_t pack_op2(int bf16, float lo, float hi) {
   return bf16 ? pack_bf16x2(lo, hi) : pack_f16x2(lo, hi);
+}
+// A 16-bit shadow of an fp32 tensor that is not range-tracked: exactly what `x.to(dtype)` gives, so that it can stand in
+// for that cast (out-of-range values become inf, not a silently clipped +-65504).
+__device__ __forceinline__ uint32_t pack_shadow2(int bf16, float lo, float hi) {
+  return bf16 ? pack_bf16x2(lo, hi) : pack_f16x2_rn(lo, hi);
 }
 // two packed 16-bit operands -> floats (x = low half)
 __device__ __forceinline__ float2 unpack_op2(int bf16, uint32_t u) {

@@ -840,7 +840,11 @@ static int host_enqueue(mz_model* m, int li, const void* x_host, const float* c_
   if ((rc = ensure(reinterpret_cast<void**>(&L.hx), &L.hx_bytes, xb)) != MZ_OK) return rc;
   if ((rc = ensure(reinterpret_cast<void**>(&L.hy), &L.hy_bytes, yb)) != MZ_OK) return rc;
   if (cb && (rc = ensure(reinterpret_cast<void**>(&L.hc), &L.hc_bytes, cb)) != MZ_OK) return rc;
-  if ((rc = ensure(&L.ws, &L.ws_bytes, wsb)) != MZ_OK) return rc;
+  // (cudaMalloc only promises 256-byte alignment, and where a small block lands depends on what the process allocated
+  // before; the workspace must start on a 1024-byte boundary)
+  if ((rc = ensure(&L.ws, &L.ws_bytes, wsb + 1024)) != MZ_OK) return rc;
+  uint8_t* ws = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(L.ws) + 1023) & ~static_cast<uintptr_t>(1023));
+  const size_t ws_bytes = L.ws_bytes - static_cast<size_t>(ws - static_cast<uint8_t*>(L.ws));
   MZ_CUDA(cudaMemcpyAsync(L.hx, x_host, xb, cudaMemcpyHostToDevice, L.stream));
   if (cb) MZ_CUDA(cudaMemcpyAsync(L.hc, c_host, cb, cudaMemcpyHostToDevice, L.stream));
   // The two lanes take turns on the SMs: this lane's kernels start when the other lane's have finished, so that one
@@ -848,7 +852,7 @@ static int host_enqueue(mz_model* m, int li, const void* x_host, const float* c_
   // proceed on the copy engines -- instead of the kernels of two steps interleaving and both finishing late.
   mz_model::HostLane& O = m->lane[li ^ 1];
   if (O.has_work) MZ_CUDA(cudaStreamWaitEvent(L.stream, O.kernels_done, 0));
-  rc = mz_upscale(m, L.hx, cb ? L.hc : nullptr, c_rows, L.hy, B, H, W, L.ws, L.ws_bytes, flags, L.stream);
+  rc = mz_upscale(m, L.hx, cb ? L.hc : nullptr, c_rows, L.hy, B, H, W, ws, ws_bytes, flags, L.stream);
   if (rc != MZ_OK) return rc;
   MZ_CUDA(cudaEventRecord(L.kernels_done, L.stream));
   L.has_work = true;

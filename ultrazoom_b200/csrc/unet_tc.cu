@@ -312,10 +312,10 @@ __global__ void __launch_bounds__(sg::kMaxThreads, 1) seg_gemm_tc_kernel(const _
           sts128(slot + swz[kk], __float_as_uint(o[kk].x), __float_as_uint(o[kk].y), __float_as_uint(o[kk].z), __float_as_uint(o[kk].w));
         if (p.has16) {
           if (p.mix) __syncwarp();  // the shadow goes where z was: every lane has read its z row
-          sts128(slot + sg::kSlotX + swz16_0, pack_op2(p.bf16, o[0].x, o[0].y), pack_op2(p.bf16, o[0].z, o[0].w),
-                 pack_op2(p.bf16, o[1].x, o[1].y), pack_op2(p.bf16, o[1].z, o[1].w));
-          sts128(slot + sg::kSlotX + swz16_1, pack_op2(p.bf16, o[2].x, o[2].y), pack_op2(p.bf16, o[2].z, o[2].w),
-                 pack_op2(p.bf16, o[3].x, o[3].y), pack_op2(p.bf16, o[3].z, o[3].w));
+          sts128(slot + sg::kSlotX + swz16_0, pack_shadow2(p.bf16, o[0].x, o[0].y), pack_shadow2(p.bf16, o[0].z, o[0].w),
+                 pack_shadow2(p.bf16, o[1].x, o[1].y), pack_shadow2(p.bf16, o[1].z, o[1].w));
+          sts128(slot + sg::kSlotX + swz16_1, pack_shadow2(p.bf16, o[2].x, o[2].y), pack_shadow2(p.bf16, o[2].z, o[2].w),
+                 pack_shadow2(p.bf16, o[3].x, o[3].y), pack_shadow2(p.bf16, o[3].z, o[3].w));
         }
         fence_proxy_async_smem();
         __syncwarp();

@@ -232,9 +232,12 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         """``operand_dtype``: element type of the tensor-core operands ("float16" default, "bfloat16", or "auto").
         Both run at the same tcgen05 rate with fp32 accumulation; fp16's 10-bit mantissa keeps max|err| vs the fp32
         reference ~8x smaller (DESIGN.md, "Numerics"), but its range ends at 65504: every kernel that rounds a larger
-        magnitude into an fp16 operand raises a flag (``saturated()``); with "float16" the next call then raises
-        instead of returning clipped images, with "auto" every call is checked (one stream synchronisation) and a
-        saturated one is re-run -- like all later ones -- with bfloat16 operands.
+        magnitude into an fp16 operand raises a flag (``saturated()``).  With "float16" a call that synchronises anyway
+        (``upscale_host``, ``host_wait``, ``capture``) raises itself; every other call returns at once and the NEXT call
+        on the model (any entry point, a graph's ``__call__`` included) raises -- a clipped result is never passed
+        over in silence.  With "auto", ``forward``, ``upscale``, ``upscale_into`` and ``upscale_host`` are checked
+        (one stream synchronisation) and a saturated one is re-run -- like all later calls -- with bfloat16 operands;
+        stages, lanes and graphs cannot be re-run and raise as with "float16" (the model then runs with bfloat16).
         ``residual_stream``: "auto" | "float32" -- the residual stream lives in HBM as fp32 + a 16-bit shadow (the next
         block's tensor-core operand)."""
         super().__init__()
@@ -265,6 +268,8 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         self.u8_truncate = False
         self._auto_dtype = "float16"      # operand_dtype="auto": what the next call runs with
         self._param_cache = None
+        self._host_keep: dict = {}          # (device, lane) -> (engine, x, c, out) of the frame in flight on that lane
+        self._host_clipped: set = set()     # (device, lane) whose frame was in flight when the range flag was found up
 
     # ---- reference model.py:94-115 ----
     @property
@@ -378,6 +383,37 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         eng = self._engines.get((dev.type, dev.index, "float16"))
         return eng.saturated(reset) if eng is not None else False
 
+    def _range_guard(self, eng: _Engine, rerun: bool = False) -> bool:
+        """The fp16 range policy of every entry point: True when no COMPLETED kernel of ``eng`` has clipped a value.
+
+        Otherwise a result was clipped.  With "float16" this raises (the flag stays up until ``saturated(reset=True)``).
+        With "auto" the model switches to bfloat16 operands for good and clears the flag; then a caller that can still
+        repeat its own call (``rerun``: the flag is its own -- it synchronised the device before its launch -- and
+        nothing clipped has reached the caller yet) gets False and repeats it, anyone else gets the error: a clipped
+        result that was already handed out is never passed over silently.  The flag is one word per engine, so a frame
+        still in flight on one of the engine's host lanes when it is found up is reported as clipped by its
+        ``host_wait`` too."""
+        if eng.operand_dtype != "float16" or not eng.saturated():
+            return True
+        if self.operand_dtype == "auto":
+            eng.saturated(reset=True)
+            self._auto_dtype = "bfloat16"
+            if rerun:
+                return False
+        self._host_clipped.update(k for k, v in self._host_keep.items() if v[0] is eng)
+        raise self._clipped_error()
+
+    def _clipped_error(self) -> RuntimeError:
+        if self.operand_dtype == "auto":
+            return RuntimeError(
+                "a call on this model rounded a value beyond the fp16 range (65504) into a tensor-core operand: its "
+                "result was clipped.  The model now runs with bfloat16 operands ('auto'); repeat the call (a captured "
+                "graph must be captured again).")
+        return RuntimeError(
+            "a call on this model rounded a value beyond the fp16 range (65504) into a tensor-core operand: its result "
+            "was clipped.  Use operand_dtype='bfloat16' or 'auto' for this checkpoint (model.saturated(reset=True) "
+            "clears the flag).")
+
     def set_conv_tune(self, which: int = -1, device: Optional[torch.device] = None, **kw) -> None:
         """Override the tcgen05 kernel's tunables (see mz_conv_tune); for benches and tests."""
         dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
@@ -420,15 +456,10 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         auto = self.operand_dtype == "auto" and not capturing
         while True:
             eng = self._engine(dev)
-            f16 = eng.operand_dtype == "float16"
-            if f16 and not capturing and eng.saturated(reset=auto):
-                if not auto:
-                    raise RuntimeError(
-                        "an earlier call on this model rounded a value beyond the fp16 range (65504) into a tensor-core "
-                        "operand: its result was clipped.  Use operand_dtype='bfloat16' or 'auto' for this checkpoint "
-                        "(model.saturated(reset=True) clears the flag).")
-                self._auto_dtype = "bfloat16"
-                continue
+            if auto and eng.operand_dtype == "float16":
+                torch.cuda.synchronize(dev)    # (the flag of an earlier asynchronous call is not this call's to absorb)
+            if not capturing:
+                self._range_guard(eng)
             y = torch.empty((B, 3, H * r, W * r), dtype=torch.uint8 if io8 else torch.float32, device=dev,
                             memory_format=memory_format)
             stream = torch.cuda.current_stream(dev)
@@ -441,10 +472,9 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
                 c.shape[0] if c is not None else 0, y.data_ptr(), B, H, W, ws_ptr, ws_bytes,
                 flags | self._flags_extra, stream.cuda_stream))
             eng.end(stream)
-            if auto and f16:
+            if auto and eng.operand_dtype == "float16":
                 stream.synchronize()       # "auto": a saturated fp16 call is repeated with bfloat16 operands
-                if eng.saturated(reset=True):
-                    self._auto_dtype = "bfloat16"
+                if not self._range_guard(eng, rerun=True):
                     continue
             return y
 
@@ -490,6 +520,11 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
             raise RuntimeError("ultrazoom_b200.MewZoom runs on sm_100a CUDA kernels only (no CPU fallback).")
         dev = x.device
         eng = self._engine(dev)
+        auto = self.operand_dtype == "auto" and eng.operand_dtype == "float16"
+        if auto:
+            torch.cuda.synchronize(dev)        # (as in upscale: only this call's flag may be absorbed by its re-run)
+        self._range_guard(eng)
+        x_in, c_in = x, c
         io8 = x.dtype == torch.uint8
         flags = _native.FLAG_CLAMP01 | self._flags_extra
         if io8:
@@ -519,6 +554,10 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
             dst, row_pitch, img_pitch, B, H, W, y0, y1, x0, x1, ws_ptr,
             ws.numel() - (ws_ptr - ws.data_ptr()), flags, stream.cuda_stream))
         eng.end(stream)
+        if auto:
+            stream.synchronize()          # as in upscale: a saturated window is written again with bfloat16 operands
+            if not self._range_guard(eng, rerun=True):
+                self.upscale_into(x_in, c_in, frame, window, at)
 
     @torch.inference_mode()
     def upscale_stage(self, x: Tensor, c: Optional[Tensor], frame: Tensor, window: tuple, at: tuple, layer_begin: int,
@@ -532,6 +571,7 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         assert x.is_cuda and x.dtype in (torch.float32, torch.uint8), "upscale_stage takes a CUDA image (float32 or uint8)"
         dev = x.device
         eng = self._engine(dev)
+        self._range_guard(eng)            # (stages run asynchronously: a saturated stage is reported by the next call)
         io8 = x.dtype == torch.uint8
         flags = _native.FLAG_CLAMP01 | self._flags_extra
         if io8:
@@ -599,7 +639,8 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         ``lane=None``: synchronous; a batch is cut into chunks whose copies overlap the kernels of their neighbours.
         ``lane=0|1``: frame-stream form (mz_upscale_host_async) -- the call only enqueues and returns ``out`` at once;
         ``out`` is valid after ``host_wait(lane)``.  Alternating lanes double-buffers a stream of frames.  ``x``, ``c``
-        and ``out`` should be pinned and must not be touched until the wait.
+        and ``out`` should be pinned and must not be touched until the wait.  A frame clipped to the fp16 range raises
+        in the synchronous call itself ("auto": it is repeated with bfloat16 operands), on a lane at ``host_wait``.
 
         Layouts as in ``upscale``: a channels-last ``x`` is copied as it is (no transpose on the CPU), and the result is
         interleaved with ``memory_format=torch.channels_last``.  A caller's ``out`` sets the output layout itself: it
@@ -608,6 +649,9 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         assert not x.is_cuda, "upscale_host takes host tensors"
         assert lane in (None, 0, 1), "lane must be None, 0 or 1"
         eng = self._engine(torch.device("cuda", device))
+        if lane is None and self.operand_dtype == "auto" and eng.operand_dtype == "float16":
+            torch.cuda.synchronize(torch.device("cuda", device))   # (as in upscale; lanes included)
+        self._range_guard(eng)
         io8 = x.dtype == torch.uint8
         x, xflag = _input_image(x, io8)
         if c is not None:
@@ -628,20 +672,30 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         cp, cr = (c.data_ptr(), c.shape[0]) if c is not None else (None, 0)
         if lane is None:
             _native.check(eng.lib.mz_upscale_host(eng.handle, x.data_ptr(), cp, cr, out.data_ptr(), B, H, W, flags))
+            if not self._range_guard(eng, rerun=True):     # (the call has synchronised: "auto" repeats it with bf16)
+                return self.upscale_host(x, c, out, device)
         else:
-            self._host_keep = getattr(self, "_host_keep", {})
-            self._host_keep[(device, lane)] = (x, c, out)      # keep the (possibly converted) inputs alive until the wait
+            # keep the (possibly converted) inputs alive until the wait, and the engine whose lane runs the frame
+            self._host_keep[(device, lane)] = (eng, x, c, out)
             _native.check(eng.lib.mz_upscale_host_async(eng.handle, lane, x.data_ptr(), cp, cr, out.data_ptr(), B, H, W,
                                                         flags))
         return out
 
     def host_wait(self, lane: int = -1, device: int = 0) -> None:
-        """Block until the frames enqueued with ``upscale_host(..., lane=...)`` on that lane (-1: both) are done."""
-        eng = self._engine(torch.device("cuda", device))
-        _native.check(eng.lib.mz_upscale_host_wait(eng.handle, lane))
-        keep = getattr(self, "_host_keep", {})
-        for k in [k for k in keep if k[0] == device and (lane < 0 or k[1] == lane)]:
-            del keep[k]
+        """Block until the frames enqueued with ``upscale_host(..., lane=...)`` on that lane (-1: both) are done; raises
+        when one of them was clipped to the fp16 range (see ``_range_guard``).  It waits on the engine that ran each
+        frame, which is not the current one when "auto" has switched to bfloat16 since the frame was enqueued."""
+        lanes = (0, 1) if lane < 0 else (lane,)
+        done = [self._host_keep.pop((device, ln)) for ln in lanes if (device, ln) in self._host_keep]
+        engines = list({id(d[0]): d[0] for d in done}.values()) or [self._engine(torch.device("cuda", device))]
+        for eng in engines:
+            _native.check(eng.lib.mz_upscale_host_wait(eng.handle, lane))
+        clipped = any((device, ln) in self._host_clipped for ln in lanes)
+        self._host_clipped.difference_update((device, ln) for ln in lanes)
+        for eng in engines:
+            self._range_guard(eng)
+        if clipped:
+            raise self._clipped_error()
 
 
 class GraphedUpscale:
@@ -664,27 +718,35 @@ class GraphedUpscale:
         self.c = None if c is None else c.detach().to(device=x.device, dtype=torch.float32).contiguous().clone()
         # The graph bakes in raw pointers: it owns everything they point at -- its input / output tensors, a PRIVATE
         # workspace (the engine's cached one is dropped and re-allocated when a later call needs a larger one) and the
-        # engine itself (packed weights, FiLM parameters).
-        self.engine = model._engine(x.device)
+        # engine itself (packed weights, FiLM parameters): the one the warm-up left current, which "auto" may have
+        # switched to bfloat16.
+        eng = model._engine(x.device)
         need = C.c_size_t()
         B, _, H, W = self.x.shape
-        _native.check(self.engine.lib.mz_workspace_bytes(self.engine.handle, B, H, W, C.byref(need)))
+        _native.check(eng.lib.mz_workspace_bytes(eng.handle, B, H, W, C.byref(need)))
         self.ws = torch.empty(need.value + 1024, dtype=torch.uint8, device=x.device)
         with torch.inference_mode():
             side = torch.cuda.Stream(device=x.device)
             side.wait_stream(torch.cuda.current_stream(x.device))
             with torch.cuda.stream(side):        # warm-up: packs the weights, prepares the launches
                 model._run(self.x, self.c, flags, ws=self.ws, memory_format=memory_format)
+            side.synchronize()
+            self.engine = model._engine(x.device)
+            model._range_guard(self.engine)      # a checkpoint that saturates is not recorded
             torch.cuda.current_stream(x.device).wait_stream(side)
             self.graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(self.graph):
                 self.y = model._run(self.x, self.c, flags, ws=self.ws, memory_format=memory_format)
 
     def replay(self) -> Tensor:
+        """Replay as it is: the 3-5 us path, so it does not consult the fp16 range flag.  A clipped replay is reported
+        by the next ``__call__`` or call on the model, or read with ``model.saturated()``."""
         self.graph.replay()
         return self.y
 
     def __call__(self, x: Tensor, c: Optional[Tensor] = None) -> Tensor:
+        """Copy ``x`` / ``c`` in and replay; raises first when an earlier replay was clipped to the fp16 range."""
+        self.model._range_guard(self.engine)
         assert tuple(x.shape) == tuple(self.x.shape) and (x.dtype == torch.uint8) == (self.x.dtype == torch.uint8), (
             f"Graph was captured for input {tuple(self.x.shape)} {self.x.dtype}, got {tuple(x.shape)} {x.dtype}.")
         self.x.copy_(x, non_blocking=True)
