@@ -61,6 +61,13 @@ typedef enum mz_status {
  * Neither combines with MZ_FLAG_SKIP_FROM_BUFFER (MZ_ERR_INVALID); an interleaved image must be below 2^31 elements. */
 #define MZ_FLAG_X_NHWC 32u        /* x is (B,H,W,3): colour c of LR pixel (y, x) at ((b H + y) W + x) 3 + c             */
 #define MZ_FLAG_Y_NHWC 64u        /* y is (B,rH,rW,3); windowed output: see mz_upscale_window                          */
+/* 16-bit images, for 16-bit PNG / TIFF stills and 10/12-bit video decoded to rgb48le: x and y are uint16 in either
+ * layout, 6 bytes per pixel instead of fp32's 12, without 8-bit's loss of precision.  x = x16 / 65535 (the IEEE quotient:
+ * ToDtype(float32, scale=True)), y16 = floor(65535 clamp(y) + 0.5) -- the result equals the fp32 call on x16 / 65535,
+ * quantised so.  Needs MZ_FLAG_CLAMP01; MZ_FLAG_IO_U8, MZ_FLAG_U8_TRUNC and MZ_FLAG_SKIP_FROM_BUFFER are refused
+ * (MZ_ERR_INVALID).  Applies to mz_upscale, mz_upscale_window, mz_upscale_stage, mz_upscale_host and
+ * mz_upscale_host_async. */
+#define MZ_FLAG_IO_U16 128u
 
 /* Constructor kwargs of the 0.2.x-style MewZoom (README.md:254-258, model.py:52-69). */
 typedef struct mz_config {
@@ -137,10 +144,10 @@ int mz_model_saturated(mz_model* m, int32_t reset, int32_t* saturated);
 int mz_workspace_bytes(const mz_model* m, int32_t B, int32_t H, int32_t W, size_t* bytes);
 
 /* ---- the hot path: replaces MewZoom.forward / MewZoom.upscale (model.py:149-179) ----
- * x_dev : (B,3,H,W) fp32 NCHW in [0,1]   (uint8 with MZ_FLAG_IO_U8; (B,H,W,3) with MZ_FLAG_X_NHWC)
+ * x_dev : (B,3,H,W) fp32 NCHW in [0,1]   (uint8 / uint16 with MZ_FLAG_IO_U8 / _U16; (B,H,W,3) with MZ_FLAG_X_NHWC)
  * c_dev : NULL for non-control models, else (B, control_features) fp32 (c_rows == B)
  *         or (1, control_features) (c_rows == 1, broadcast) -- validate.py:73-94
- * y_dev : (B,3,rH,rW) fp32 NCHW          (uint8 with MZ_FLAG_IO_U8; (B,rH,rW,3) with MZ_FLAG_Y_NHWC)
+ * y_dev : (B,3,rH,rW) fp32 NCHW          (uint8 / uint16 with MZ_FLAG_IO_U8 / _U16; (B,rH,rW,3) with MZ_FLAG_Y_NHWC)
  * flags : MZ_FLAG_CLAMP01 => upscale(), 0 => forward()
  */
 int mz_upscale(mz_model* m, const void* x_dev, const float* c_dev, int32_t c_rows, void* y_dev,
@@ -157,7 +164,7 @@ int mz_upscale(mz_model* m, const void* x_dev, const float* c_dev, int32_t c_row
  * lands, y_row_pitch is the number of elements between HR rows (at least 3 * r * (win_x1 - win_x0)) and y_plane_pitch the
  * number between images.
  * y_dev and both pitches must be aligned to the head's vector stores: fp32 8 / 16 / 4 bytes at r = 2 / 4 / 3, 8-bit
- * 2 / 4 / 1 bytes -- in either layout. */
+ * 2 / 4 / 1 bytes, 16-bit 4 / 8 / 2 bytes -- in either layout. */
 int mz_upscale_window(mz_model* m, const void* x_dev, const float* c_dev, int32_t c_rows, void* y_dev,
                       int64_t y_row_pitch, int64_t y_plane_pitch, int32_t B, int32_t H, int32_t W, int32_t win_y0,
                       int32_t win_y1, int32_t win_x0, int32_t win_x1, void* workspace_dev, size_t workspace_bytes,

@@ -1,17 +1,18 @@
-"""Planar against interleaved (channels-last) images: device step time, head kernel time and frame-stream wall time.
+"""Image element types and layouts: device step time, head kernel time and frame-stream wall time.
 
     python tools/time_layouts.py --out DIR [--rounds 5] [--iters 10]
 
 Writes JSON lines to DIR/time_layouts.jsonl (and prints them):
   * "gpu": card name and power limit (nvidia-smi, read-only query), so the numbers below carry what they were measured on;
+  * "bytes": image bytes per HR pixel of each element type (computed, not measured): 12 fp32, 6 uint16, 3 uint8;
   * "step": device time per upscale call (CUDA events around `iters` calls after a warm-up) at cfg2 (MewZoom-2X-Ctrl,
     batch 16, 960x540 -> 1920x1080) and cfg4a (MewZoom-4X-Ctrl, 960x540 -> 3840x2160), for the four input / output layout
-    combinations, fp32 and uint8.  The variants alternate round by round; min, median and max over the rounds are given.
-    The images and the workspace (0.1 - 2 GB) exceed the 126 MB L2;
-  * "head": the head kernel's mean time per call in each layout, from a separate torch.profiler run (with the stem's);
-  * "stream": wall time per frame of 960x540 uint8 frames through upscale_host at 4X, interleaved pinned frames in and
-    out, against the planar route a caller with interleaved frames had before: CPU transpose HWC -> CHW, planar call,
-    CPU transpose of the HR frame CHW -> HWC.
+    combinations, fp32, uint8 and uint16.  The variants alternate round by round; min, median and max over the rounds are
+    given.  The images and the workspace (0.1 - 2 GB) exceed the 126 MB L2;
+  * "head": the head kernel's mean time per call in each variant, from a separate torch.profiler run (with the stem's);
+  * "stream": wall time per frame of 960x540 frames through upscale_host at 4X: interleaved pinned frames in and out as
+    uint8, uint16 and fp32, and the planar route a caller with interleaved uint8 frames had before interleaved images:
+    CPU transpose HWC -> CHW, planar call, CPU transpose of the HR frame CHW -> HWC.
 """
 import argparse
 import json
@@ -37,11 +38,23 @@ def gpu_info():
     return {"kind": "gpu", "nvidia_smi": q.stdout.strip().splitlines()[:1], "torch_name": torch.cuda.get_device_name(0)}
 
 
+def _channels_last(t):
+    """(uint16 tensors are re-laid out through an int16 view: torch's CUDA support of uint16 is partial)"""
+    if t.dtype == torch.uint16:
+        return t.view(torch.int16).contiguous(memory_format=CL).view(torch.uint16)
+    return t.contiguous(memory_format=CL)
+
+
+def _bits(t):
+    return t.view(torch.int16) if t.dtype == torch.uint16 else t
+
+
 def variants(x):
     x8 = (x * 255).to(torch.uint8)
+    x16 = (x.cpu() * 65535).round().to(torch.uint16).to(x.device)
     out = {}
-    for dt, xx in (("fp32", x), ("u8", x8)):
-        for xin_name, xin in (("nchw", xx), ("nhwc", xx.contiguous(memory_format=CL))):
+    for dt, xx in (("fp32", x), ("u8", x8), ("u16", x16)):
+        for xin_name, xin in (("nchw", xx), ("nhwc", _channels_last(xx))):
             for fmt_name, fmt in (("nchw", NCHW), ("nhwc", CL)):
                 out[f"{dt} {xin_name}->{fmt_name}"] = (xin, fmt)
     return out
@@ -65,7 +78,7 @@ def time_steps(cfg_name, dev, rounds, iters, emit):
         y = m.upscale(xin, c, memory_format=fmt)
         base = k.split()[0] + " nchw->nchw"
         if base in ref:
-            assert torch.equal(y, ref[base]), k
+            assert torch.equal(_bits(y), _bits(ref[base])), k
         else:
             ref[base] = y
     del ref
@@ -112,32 +125,40 @@ def time_stream(dev, frames, emit):
     r = m.upscale_ratio
     H, W = 540, 960
     g = torch.Generator().manual_seed(2)
-    hwc = [(torch.rand(1, H, W, 3, generator=g) * 255).to(torch.uint8).pin_memory() for _ in range(2)]
+    base = [torch.rand(1, H, W, 3, generator=g) for _ in range(2)]
+    hwc = {"uint8": [(b * 255).to(torch.uint8).pin_memory() for b in base],
+           "uint16": [(b * 65535).round().to(torch.uint16).pin_memory() for b in base],
+           "float32": [b.pin_memory() for b in base]}
     c = torch.rand(1, 3, generator=g)
-    out_hwc = torch.empty(1, H * r, W * r, 3, dtype=torch.uint8).pin_memory()
+    out_hwc = {k: torch.empty(1, H * r, W * r, 3, dtype=v[0].dtype).pin_memory() for k, v in hwc.items()}
     out_planar = torch.empty(1, 3, H * r, W * r, dtype=torch.uint8).pin_memory()
     x_planar = torch.empty(1, 3, H, W, dtype=torch.uint8).pin_memory()
 
-    def interleaved(i):
-        m.upscale_host(hwc[i % 2].permute(0, 3, 1, 2), c, out=out_hwc.permute(0, 3, 1, 2))
-        return out_hwc
+    def interleaved(dt):
+        def route(i):
+            m.upscale_host(hwc[dt][i % 2].permute(0, 3, 1, 2), c, out=out_hwc[dt].permute(0, 3, 1, 2))
+            return out_hwc[dt]
+        return route
 
     def planar_route(i):
-        x_planar.copy_(hwc[i % 2].permute(0, 3, 1, 2))                # CPU transpose HWC -> CHW
+        x_planar.copy_(hwc["uint8"][i % 2].permute(0, 3, 1, 2))       # CPU transpose HWC -> CHW
         m.upscale_host(x_planar, c, out=out_planar)
         return out_planar.permute(0, 2, 3, 1).contiguous()            # CPU transpose CHW -> HWC of the HR frame
 
-    assert torch.equal(interleaved(0), planar_route(0))
+    assert torch.equal(interleaved("uint8")(0), planar_route(0))
+    routes = [("uint8 interleaved", "uint8", interleaved("uint8")), ("uint8 planar+transposes", "uint8", planar_route),
+              ("uint16 interleaved", "uint16", interleaved("uint16")), ("float32 interleaved", "float32", interleaved("float32"))]
     res = {}
-    for _ in range(3):                                                # alternate the two routes
-        for name, fn in (("interleaved", interleaved), ("planar+transposes", planar_route)):
+    for _ in range(3):                                                # alternate the routes
+        for name, _, fn in routes:
             fn(0)
             t0 = time.perf_counter()
             for i in range(frames):
                 fn(i)
             res.setdefault(name, []).append((time.perf_counter() - t0) / frames * 1e3)
-    for name, t in res.items():
-        emit({"kind": "stream", "route": name, "frame": "1x960x540 uint8 -> 4X", "ms_per_frame_min": min(t),
+    for name, dt, _ in routes:
+        t = res[name]
+        emit({"kind": "stream", "route": name, "frame": f"1x960x540 {dt} -> 4X", "ms_per_frame_min": min(t),
               "ms_per_frame_median": statistics.median(t), "frames": frames, "cpu_threads": torch.get_num_threads()})
 
 
@@ -160,6 +181,9 @@ def main():
             f.flush()
 
         emit(gpu_info())
+        emit({"kind": "bytes", "per_hr_pixel": {dt: 3 * torch.empty((), dtype=d).element_size()
+                                                for dt, d in (("fp32", torch.float32), ("u16", torch.uint16),
+                                                              ("u8", torch.uint8))}})
         for cfg_name in CONFIGS:
             m, x, c, vs = time_steps(cfg_name, dev, args.rounds, args.iters, emit)
             time_head(cfg_name, m, c, vs, emit)

@@ -28,6 +28,7 @@ FLAG_IO_U8 = 8
 FLAG_U8_TRUNC = 16
 FLAG_X_NHWC = 32
 FLAG_Y_NHWC = 64
+FLAG_IO_U16 = 128
 
 DTYPE_F16, DTYPE_BF16 = 0, 1
 MATH_TF32, MATH_FP32 = 0, 1

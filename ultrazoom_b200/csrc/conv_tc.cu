@@ -107,7 +107,8 @@ __host__ __device__ inline SmemPlan plan_smem(const TcParams& p) {
 // instead of 3R: the 128 x 16 activation tile -- 4 KB of shared-memory operand fetch per UMMA, what bounds the small-N
 // shapes -- is fetched once per input row instead of once per (output row, tap).  Every UMMA accumulates; the epilogue
 // zeroes each accumulator column group right after reading it.
-// LAY (head only): bit 0 interleaved input image, bit 1 interleaved output image (EpiParams::x_nhwc / y_nhwc).
+// LAY (head only): bit 0 interleaved input image, bit 1 interleaved output image (EpiParams::x_nhwc / y_nhwc), bit 2
+// 16-bit images (EpiParams::x16 / y16).
 template <int MODE, int KT, int ROWS, int VAR, int LAY = 0>
 __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_constant__ TcParams p) {
   constexpr bool PAIR = VAR == 1, FUSE = VAR == 2;
@@ -936,7 +937,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
             if (ok) {
               const bool interior = xw >= 2 && xw + 33 < p.epi.W;  // (warp-uniform) no clamped column in this warp
               const bool second = y + 1 < p.epi.H;
-              epi_head2<(LAY & 1) != 0, (LAY & 2) != 0>(p.epi, b, y, x, v0, v1, interior, second);
+              epi_head2<(LAY & 1) != 0, (LAY & 2) != 0, (LAY & 4) != 0>(p.epi, b, y, x, v0, v1, interior, second);
             }
           }
         }
@@ -978,13 +979,13 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
           }
           if (ok) {
             const bool interior = xw >= 2 && xw + 33 < p.epi.W;  // (warp-uniform) no clamped column in this warp
-            constexpr bool XN = (LAY & 1) != 0, YN = (LAY & 2) != 0;
+            constexpr bool XN = (LAY & 1) != 0, YN = (LAY & 2) != 0, I16 = (LAY & 4) != 0;
             if (p.epi.r == 4)
-              epi_head_r<4, XN, YN>(p.epi, b, y, x, acc, interior);
+              epi_head_r<4, XN, YN, I16>(p.epi, b, y, x, acc, interior);
             else if (p.epi.r == 2)
-              epi_head_r<2, XN, YN>(p.epi, b, y, x, acc, interior);
+              epi_head_r<2, XN, YN, I16>(p.epi, b, y, x, acc, interior);
             else
-              epi_head_r<3, XN, YN>(p.epi, b, y, x, acc, interior);
+              epi_head_r<3, XN, YN, I16>(p.epi, b, y, x, acc, interior);
           }
         } else if (MODE == 1) {
           if (k > 0 && !all_rows) load_residual(k, k + 1);
@@ -1156,8 +1157,9 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
 // ---- kernel lookup -------------------------------------------------------------------------------------------------
 // One lookup function per epilogue mode, so that the build can compile the instantiations of each mode in its own
 // translation unit: build.py compiles this file four times, with -DMZ_TC_PART=<mode> for the kernels of modes 0..2 and
-// -DMZ_TC_PART=4 for the host side, and the heads for interleaved images (LAY 1..3) with -DMZ_TC_PART=5..7.  Without
-// the define (a plain `nvcc -c conv_tc.cu`) everything lands in one object.
+// -DMZ_TC_PART=4 for the host side, the heads for interleaved images (LAY 1..3) with -DMZ_TC_PART=5..7 and those for
+// 16-bit images (LAY 4..7) with -DMZ_TC_PART=8..11.  Without the define (a plain `nvcc -c conv_tc.cu`) everything lands
+// in one object.
 //   var 0: one CTA per patch, 1: CTA pair (cta_group::2), 2: fused rows.  Returns nullptr for a shape that has no kernel.
 const void* tc_kernel_mode0(int ks, int rows, int var);
 const void* tc_kernel_mode1(int ks, int rows, int var);
@@ -1165,6 +1167,10 @@ const void* tc_kernel_mode2(int ks, int rows, int var);
 const void* tc_kernel_mode2_lay1(int ks, int rows, int var);
 const void* tc_kernel_mode2_lay2(int ks, int rows, int var);
 const void* tc_kernel_mode2_lay3(int ks, int rows, int var);
+const void* tc_kernel_mode2_lay4(int ks, int rows, int var);
+const void* tc_kernel_mode2_lay5(int ks, int rows, int var);
+const void* tc_kernel_mode2_lay6(int ks, int rows, int var);
+const void* tc_kernel_mode2_lay7(int ks, int rows, int var);
 
 template <int M, int K, int LAY = 0>
 static const void* tc_kernel_rows(int rows, int var) {
@@ -1212,6 +1218,18 @@ const void* tc_kernel_mode2_lay2(int ks, int rows, int var) { return tc_kernel_l
 #endif
 #if !defined(MZ_TC_PART) || MZ_TC_PART == 7
 const void* tc_kernel_mode2_lay3(int ks, int rows, int var) { return tc_kernel_lookup<2, 3>(ks, rows, var); }
+#endif
+#if !defined(MZ_TC_PART) || MZ_TC_PART == 8
+const void* tc_kernel_mode2_lay4(int ks, int rows, int var) { return tc_kernel_lookup<2, 4>(ks, rows, var); }
+#endif
+#if !defined(MZ_TC_PART) || MZ_TC_PART == 9
+const void* tc_kernel_mode2_lay5(int ks, int rows, int var) { return tc_kernel_lookup<2, 5>(ks, rows, var); }
+#endif
+#if !defined(MZ_TC_PART) || MZ_TC_PART == 10
+const void* tc_kernel_mode2_lay6(int ks, int rows, int var) { return tc_kernel_lookup<2, 6>(ks, rows, var); }
+#endif
+#if !defined(MZ_TC_PART) || MZ_TC_PART == 11
+const void* tc_kernel_mode2_lay7(int ks, int rows, int var) { return tc_kernel_lookup<2, 7>(ks, rows, var); }
 #endif
 
 #if !defined(MZ_TC_PART) || MZ_TC_PART == 4  // ---- host side ----------------------------------------------------------
@@ -1284,16 +1302,22 @@ struct ConvLaunchImpl {
   int ks, var, lay;  // what `fn` was looked up for (the head's image layouts are patched per call)
 };
 
-// the head kernel for image layouts `lay` (bit 0 interleaved input, bit 1 interleaved output)
+// the head kernel for image layouts `lay` (bit 0 interleaved input, bit 1 interleaved output, bit 2 16-bit images)
 static const void* tc_kernel_head(int lay, int ks, int rows, int var) {
   switch (lay) {
     case 0: return tc_kernel_mode2(ks, rows, var);
     case 1: return tc_kernel_mode2_lay1(ks, rows, var);
     case 2: return tc_kernel_mode2_lay2(ks, rows, var);
-    default: return tc_kernel_mode2_lay3(ks, rows, var);
+    case 3: return tc_kernel_mode2_lay3(ks, rows, var);
+    case 4: return tc_kernel_mode2_lay4(ks, rows, var);
+    case 5: return tc_kernel_mode2_lay5(ks, rows, var);
+    case 6: return tc_kernel_mode2_lay6(ks, rows, var);
+    default: return tc_kernel_mode2_lay7(ks, rows, var);
   }
 }
-static int head_layout(const EpiParams& e) { return (e.x_nhwc ? 1 : 0) | (e.y_nhwc ? 2 : 0); }
+static int head_layout(const EpiParams& e) {
+  return (e.x_nhwc ? 1 : 0) | (e.y_nhwc ? 2 : 0) | (e.y16 != nullptr ? 4 : 0);
+}
 static_assert(sizeof(ConvLaunchImpl) <= sizeof(ConvLaunch::storage), "ConvLaunch::storage too small");
 
 static int run_prepared(ConvLaunchImpl& L, cudaStream_t s) {
@@ -1367,6 +1391,8 @@ int patch_conv_epi(ConvLaunch& launch, const EpiParams& e) {
   d.y = e.y;
   d.x8 = e.x8;
   d.y8 = e.y8;
+  d.x16 = e.x16;
+  d.y16 = e.y16;
   d.u8_trunc = e.u8_trunc;
   d.skip_mode = e.skip_mode;
   d.clamp01 = e.clamp01;

@@ -5,6 +5,7 @@
 
 #include <string.h>
 
+#include <type_traits>
 #include <vector>
 
 #include "common.cuh"
@@ -66,6 +67,11 @@ struct EpiParams {
   // pixel * 3 + c, images 3HW (3 rH rW) elements apart as in the planar layout.  For a windowed y_nhwc output y / y8
   // points at colour 0 of HR pixel (wy0 r, wx0 r), y_row is the element pitch of HR rows and y_plane that of images.
   int x_nhwc, y_nhwc;
+  // 16-bit image I/O (MZ_FLAG_IO_U16), either layout: when set they replace x / y.  x16 is read as the IEEE quotient
+  // x16 / 65535 (ToDtype(float32, scale=True)); y16 = floor(65535 * clamp(v, 0, 1) + 0.5).  A head kernel of its own
+  // (conv_tc_kernel's LAY bit 2) reads and writes them.
+  const uint16_t* x16;
+  uint16_t* y16;
   // fp16 range guard: a kernel that is about to round a value beyond +-65504 into a 16-bit fp16 operand (where
   // cvt.rn.satfinite would clip it silently) writes 1 here.  Points at a host-mapped word owned by the mz_model
   // (mz_model_saturated); nullptr = not tracked (per-kernel entry points).
@@ -183,10 +189,11 @@ int launch_seg_gemm_tc(const SgArgs& a, cudaStream_t s);
 
 int launch_bicubic(const float* x, float* y, int planes, int H, int W, int r, cudaStream_t s);
 // fp32 stream zf + 16-bit shadow zb (pitch zb_pitch).
-// x8 != nullptr: the image is 8-bit (B,3,H,W) and read as x8 / 255.  x_nhwc: the image is interleaved (B,H,W,3).
+// x8 != nullptr: the image is 8-bit (B,3,H,W) and read as x8 / 255; x16 != nullptr: 16-bit, read as x16 / 65535.
+// x_nhwc: the image is interleaved (B,H,W,3).
 int launch_stem(const float* x, const uint8_t* x8, const float* w, const float* bias, float* zf, uint16_t* zb, int bf16,
                 int B, int H, int W, int Cp, int zb_pitch, cudaStream_t s, unsigned int* sat = nullptr,
-                bool x_nhwc = false);
+                bool x_nhwc = false, const uint16_t* x16 = nullptr);
 // film: [L][hCp / ns][B][2][ns] -- one [B][2][ns] table (scale row, shift row) per conv1 launch; ns == hCp normally
 int launch_film(const float* c, int c_rows, const float* w, const float* b, float* film, int L, int B, int F,
                 int hC, int hCp, int ns, cudaStream_t s);
@@ -282,13 +289,30 @@ __device__ __forceinline__ void epi_store16(const EpiParams& p, int b, int y, in
 // LR pixel as float: fp32 planes as they are, 8-bit planes scaled by 1/255 (ToDtype(float32, scale=True))
 __device__ __forceinline__ float lr_px(const float* p) { return __ldg(p); }
 __device__ __forceinline__ float lr_px(const uint8_t* p) { return static_cast<float>(__ldg(p)) * (1.0f / 255.0f); }
+// 16-bit planes: exactly the IEEE quotient x16 / 65535 -- what the stem computes with __fdiv_rn, so that a 16-bit call
+// equals the fp32 call on x16.float() / 65535 bit for bit.  A reciprocal multiply and one FMA correction (the residual
+// x - 65535 q is exact); checked against the quotient for all 65536 codes on the CPU (tests/test_gpu_u16_io.py).  The
+// product alone is 1 ulp off for 512 codes.
+__device__ __forceinline__ float lr_px(const uint16_t* p) {
+  constexpr float kRcp = 1.0f / 65535.0f;
+  const float x = static_cast<float>(__ldg(p)), q = __fmul_rn(x, kRcp);
+  return fmaf(fmaf(-q, 65535.f, x), kRcp, q);
+}
 // [0,1] -> 8 bits: floor(255 v + 0.5) (save_image) or floor(255 v) (ToPILImage); v is clamped here in any case
 __device__ __forceinline__ uint8_t to_u8(float v, int trunc) {
   v = fminf(fmaxf(v, 0.f), 1.f);
   return static_cast<uint8_t>(static_cast<int>(fmaf(v, 255.f, trunc ? 0.f : 0.5f)));
 }
+// [0,1] -> 16 bits: floor(65535 v + 0.5), one fmaf then truncation as to_u8; v is clamped here
+__device__ __forceinline__ uint16_t to_u16(float v) {
+  v = fminf(fmaxf(v, 0.f), 1.f);
+  return static_cast<uint16_t>(static_cast<int>(fmaf(v, 65535.f, 0.5f)));
+}
+__device__ __forceinline__ uint32_t pack_u16x2(uint16_t lo, uint16_t hi) {
+  return static_cast<uint32_t>(lo) | (static_cast<uint32_t>(hi) << 16);
+}
 
-// Bicubic value of HR pixel (oy, ox) of one colour (H x W, fp32 | u8, pixels `ps` elements apart: 1 planar, 3
+// Bicubic value of HR pixel (oy, ox) of one colour (H x W, fp32 | u8 | u16, pixels `ps` elements apart: 1 planar, 3
 // interleaved): 16 clamped taps, rows first.
 template <typename T>
 __device__ __forceinline__ float bicubic_at(const T* __restrict__ plane, int H, int W, int ps, const BicubicTable& bt,
@@ -332,21 +356,43 @@ __device__ __forceinline__ void epi_head(const EpiParams& p, int b, int y, int x
         const size_t HW = static_cast<size_t>(p.H) * p.W;
         const size_t pl = p.x_nhwc ? static_cast<size_t>(b) * 3 * HW + c : (static_cast<size_t>(b) * 3 + c) * HW;
         const int ps = p.x_nhwc ? 3 : 1;
-        v += p.x8 != nullptr ? bicubic_at(p.x8 + pl, p.H, p.W, ps, p.bt, oy, ox)
-                             : bicubic_at(p.x + pl, p.H, p.W, ps, p.bt, oy, ox);
+        v += p.x16 != nullptr ? bicubic_at(p.x16 + pl, p.H, p.W, ps, p.bt, oy, ox)
+             : p.x8 != nullptr ? bicubic_at(p.x8 + pl, p.H, p.W, ps, p.bt, oy, ox)
+                               : bicubic_at(p.x + pl, p.H, p.W, ps, p.bt, oy, ox);
       }
       if (p.clamp01) v = fminf(fmaxf(v, 0.f), 1.f);
-      if (p.y8 != nullptr)
+      if (p.y16 != nullptr)
+        p.y16[di] = to_u16(v);
+      else if (p.y8 != nullptr)
         p.y8[di] = to_u8(v, p.u8_trunc);
       else
         p.y[di] = v;
     }
   }
 }
-// One interleaved HR row segment of an LR pixel: v = R pixels x 3 colours, stored at element d of y / y8 as three
-// vectors (fp32: float2 at R = 2, float4 at R = 4; 8-bit: u16 / u32) or, at R = 3, element by element.
-template <int R>
+// One interleaved HR row segment of an LR pixel: v = R pixels x 3 colours, stored at element d of y / y8 / y16 as three
+// vectors (fp32: float2 at R = 2, float4 at R = 4; 8-bit: u16 / u32; 16-bit: u32 / 8 bytes) or, at R = 3, element by
+// element.  O16: the output is 16-bit (y16).
+template <int R, bool O16 = false>
 __device__ __forceinline__ void store_hr_row_nhwc(const EpiParams& p, size_t d, float (&v)[3 * R]) {
+  if constexpr (O16) {
+    uint16_t q[3 * R];
+#pragma unroll
+    for (int e = 0; e < 3 * R; ++e) q[e] = to_u16(v[e]);
+    uint16_t* rowp = p.y16 + d;
+    if constexpr (R == 4) {
+#pragma unroll
+      for (int k = 0; k < 3; ++k)
+        reinterpret_cast<uint2*>(rowp)[k] = make_uint2(pack_u16x2(q[4 * k], q[4 * k + 1]), pack_u16x2(q[4 * k + 2], q[4 * k + 3]));
+    } else if constexpr (R == 2) {
+#pragma unroll
+      for (int k = 0; k < 3; ++k) reinterpret_cast<uint32_t*>(rowp)[k] = pack_u16x2(q[2 * k], q[2 * k + 1]);
+    } else {
+#pragma unroll
+      for (int e = 0; e < 3 * R; ++e) rowp[e] = q[e];
+    }
+    return;
+  }
   if (p.y8 != nullptr) {
     uint8_t q[3 * R];
 #pragma unroll
@@ -400,9 +446,11 @@ __device__ __forceinline__ void store_hr_row_nhwc(const EpiParams& p, size_t d, 
 // XN / YN: interleaved input / output (EpiParams::x_nhwc / y_nhwc) -- compile-time, so that the planar instantiation is
 // the code it was.  Interleaved, the taps of one colour are 3 elements apart (same FMA order per colour: bit-identical
 // results) and each HR row of the pixel leaves as 3R contiguous values.
+// T = uint16_t: 16-bit images on both sides (MZ_FLAG_IO_U16, y16) -- the 16-bit heads are instantiations of their own.
 template <int R, typename T, bool XN, bool YN>
 __device__ __forceinline__ void epi_head_rt(const EpiParams& p, const T* __restrict__ lr, int b, int y, int x,
                                             const float (&acc)[48], bool interior) {
+  constexpr bool O16 = std::is_same_v<T, uint16_t>;
   const int H = p.H, W = p.W;
   const long long first = head_out_index_l<YN>(p, b, 0, y, x, 0, 0);
   if (first < 0) return;  // outside the output window
@@ -483,8 +531,28 @@ __device__ __forceinline__ void epi_head_rt(const EpiParams& p, const T* __restr
       for (int j = 0; j < R; ++j)
 #pragma unroll
         for (int c = 0; c < 3; ++c) v[3 * j + c] = out[c][i][j];
-      store_hr_row_nhwc<R>(p, static_cast<size_t>(first) + static_cast<size_t>(i) * row_pitch, v);
+      store_hr_row_nhwc<R, O16>(p, static_cast<size_t>(first) + static_cast<size_t>(i) * row_pitch, v);
     }
+    return;
+  }
+  if constexpr (O16) {  // 16-bit output: 2R bytes per HR row segment -- one u32 at R = 2, one 8-byte store at R = 4
+#pragma unroll
+    for (int c = 0; c < 3; ++c)
+#pragma unroll
+      for (int i = 0; i < R; ++i) {
+        uint16_t* rowp = p.y16 + static_cast<size_t>(first) + c * plane_pitch + static_cast<size_t>(i) * row_pitch;
+        uint16_t q[R];
+#pragma unroll
+        for (int j = 0; j < R; ++j) q[j] = to_u16(out[c][i][j]);
+        if constexpr (R == 4) {
+          *reinterpret_cast<uint2*>(rowp) = make_uint2(pack_u16x2(q[0], q[1]), pack_u16x2(q[2], q[3]));
+        } else if constexpr (R == 2) {
+          *reinterpret_cast<uint32_t*>(rowp) = pack_u16x2(q[0], q[1]);
+        } else {
+#pragma unroll
+          for (int j = 0; j < R; ++j) rowp[j] = q[j];
+        }
+      }
     return;
   }
   if (p.y8 != nullptr) {  // 8-bit output: R bytes per HR row segment (a warp writes 32 * R contiguous bytes)
@@ -555,11 +623,13 @@ __device__ __forceinline__ void epi_head_rt(const EpiParams& p, const T* __restr
     }
 }
 // interior: warp-uniform promise that x - 2 >= 0 and x + 2 < W for every lane of the calling warp
-// (the layouts are template parameters of the calling kernel: one runtime branch over four layouts in the same kernel
-// raises the planar head's registers and makes it spill)
-template <int R, bool XN, bool YN>
+// (the layouts and the 16-bit image type, I16, are template parameters of the calling kernel: one runtime branch over
+// four layouts in the same kernel raises the planar head's registers and makes it spill)
+template <int R, bool XN, bool YN, bool I16>
 __device__ __forceinline__ void epi_head_r(const EpiParams& p, int b, int y, int x, const float (&acc)[48], bool interior) {
-  if (p.x8 != nullptr)
+  if constexpr (I16)
+    epi_head_rt<R, uint16_t, XN, YN>(p, p.x16, b, y, x, acc, interior);
+  else if (p.x8 != nullptr)
     epi_head_rt<R, uint8_t, XN, YN>(p, p.x8, b, y, x, acc, interior);
   else
     epi_head_rt<R, float, XN, YN>(p, p.x, b, y, x, acc, interior);
@@ -573,6 +643,7 @@ template <typename T, bool XN, bool YN>
 __device__ __forceinline__ void epi_head2_pair(const EpiParams& p, const T* __restrict__ lr, int b, int y, int x,
                                                const uint32_t (&v0)[16], const uint32_t (&v1)[16], bool interior,
                                                bool second) {
+  constexpr bool O16 = std::is_same_v<T, uint16_t>;  // 16-bit images on both sides, as in epi_head_rt
   const int H = p.H, W = p.W;
   long long first[2];
   first[0] = head_out_index_l<YN>(p, b, 0, y, x, 0, 0);
@@ -653,12 +724,12 @@ __device__ __forceinline__ void epi_head2_pair(const EpiParams& p, const T* __re
         for (int j = 0; j < 2; ++j)
 #pragma unroll
           for (int c = 0; c < 3; ++c) v[3 * j + c] = out[rr][c][i][j];
-        store_hr_row_nhwc<2>(p, static_cast<size_t>(first[rr]) + static_cast<size_t>(i) * row_pitch, v);
+        store_hr_row_nhwc<2, O16>(p, static_cast<size_t>(first[rr]) + static_cast<size_t>(i) * row_pitch, v);
       }
     }
     return;
   }
-  if (p.skip_mode == 1 && p.y8 == nullptr) {  // y already holds the bicubic image: every segment is read before the first store
+  if (!O16 && p.skip_mode == 1 && p.y8 == nullptr) {  // y already holds the bicubic image: every segment is read before the first store
     float2 sk[2][3][2];
 #pragma unroll
     for (int rr = 0; rr < 2; ++rr)
@@ -687,7 +758,9 @@ __device__ __forceinline__ void epi_head2_pair(const EpiParams& p, const T* __re
 #pragma unroll
       for (int i = 0; i < 2; ++i) {
         const size_t d = static_cast<size_t>(first[rr]) + c * plane_pitch + static_cast<size_t>(i) * row_pitch;
-        if (p.y8 != nullptr) {
+        if constexpr (O16) {
+          *reinterpret_cast<uint32_t*>(p.y16 + d) = pack_u16x2(to_u16(out[rr][c][i][0]), to_u16(out[rr][c][i][1]));
+        } else if (p.y8 != nullptr) {
           const uint32_t w = static_cast<uint32_t>(to_u8(out[rr][c][i][0], p.u8_trunc)) |
                              (static_cast<uint32_t>(to_u8(out[rr][c][i][1], p.u8_trunc)) << 8);
           *reinterpret_cast<uint16_t*>(p.y8 + d) = static_cast<uint16_t>(w);
@@ -699,10 +772,12 @@ __device__ __forceinline__ void epi_head2_pair(const EpiParams& p, const T* __re
       }
   }
 }
-template <bool XN, bool YN>
+template <bool XN, bool YN, bool I16>
 __device__ __forceinline__ void epi_head2(const EpiParams& p, int b, int y, int x, const uint32_t (&v0)[16],
                                           const uint32_t (&v1)[16], bool interior, bool second) {
-  if (p.x8 != nullptr)
+  if constexpr (I16)
+    epi_head2_pair<uint16_t, XN, YN>(p, p.x16, b, y, x, v0, v1, interior, second);
+  else if (p.x8 != nullptr)
     epi_head2_pair<uint8_t, XN, YN>(p, p.x8, b, y, x, v0, v1, interior, second);
   else
     epi_head2_pair<float, XN, YN>(p, p.x, b, y, x, v0, v1, interior, second);

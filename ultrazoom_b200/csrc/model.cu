@@ -158,6 +158,8 @@ static int run_conv(mz_model* m, int slot, const ConvArgs& a, const ConvTcTune& 
     key.a.epi.y = nullptr;
     key.a.epi.x8 = nullptr;
     key.a.epi.y8 = nullptr;
+    key.a.epi.x16 = nullptr;
+    key.a.epi.y16 = nullptr;
     key.a.epi.u8_trunc = key.a.epi.skip_mode = key.a.epi.clamp01 = 0;
     key.a.epi.wy0 = key.a.epi.wy1 = key.a.epi.wx0 = key.a.epi.wx1 = 0;
     key.a.epi.y_row = key.a.epi.y_plane = 0;
@@ -563,6 +565,21 @@ struct OutWindow {
   long long row_pitch, plane_pitch;
 };
 
+// the image element type flags: 8 or 16 bits need MZ_FLAG_CLAMP01, recompute the skip and exclude each other
+static int check_image_flags(uint32_t flags) {
+  MZ_REQUIRE(!(flags & MZ_FLAG_IO_U8) || ((flags & MZ_FLAG_CLAMP01) && !(flags & MZ_FLAG_SKIP_FROM_BUFFER)),
+             "upscale: 8-bit image I/O needs MZ_FLAG_CLAMP01 and recomputes the skip (no MZ_FLAG_SKIP_FROM_BUFFER)");
+  MZ_REQUIRE(!(flags & MZ_FLAG_IO_U16) ||
+                 ((flags & MZ_FLAG_CLAMP01) && !(flags & (MZ_FLAG_SKIP_FROM_BUFFER | MZ_FLAG_IO_U8 | MZ_FLAG_U8_TRUNC))),
+             "upscale: 16-bit image I/O needs MZ_FLAG_CLAMP01, recomputes the skip (no MZ_FLAG_SKIP_FROM_BUFFER) and "
+             "excludes MZ_FLAG_IO_U8 and MZ_FLAG_U8_TRUNC");
+  return MZ_OK;
+}
+// bytes per image element: fp32, 8 or 16 bits
+static size_t image_elem_bytes(uint32_t flags) {
+  return (flags & MZ_FLAG_IO_U8) ? 1 : ((flags & MZ_FLAG_IO_U16) ? 2 : sizeof(float));
+}
+
 // layer_begin / layer_end: the encoder blocks [layer_begin, layer_end) of this call (mz_upscale_stage).  The FiLM table and
 // the stem run when layer_begin == 0, the head when layer_end == L; in between the state lives in the workspace.
 static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, int32_t c_rows, void* y_dev_v, int32_t B,
@@ -573,18 +590,20 @@ static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, in
   MZ_REQUIRE(0 <= layer_begin && layer_begin <= layer_end && layer_end <= m->L, "upscale: bad layer range [%d, %d) of %d",
              layer_begin, layer_end, m->L);
   const bool front = layer_begin == 0, back = layer_end == m->L;
-  const bool io8 = (flags & MZ_FLAG_IO_U8) != 0;
-  MZ_REQUIRE(!io8 || ((flags & MZ_FLAG_CLAMP01) && !(flags & MZ_FLAG_SKIP_FROM_BUFFER)),
-             "upscale: 8-bit image I/O needs MZ_FLAG_CLAMP01 and recomputes the skip (no MZ_FLAG_SKIP_FROM_BUFFER)");
+  const int frc = check_image_flags(flags);
+  if (frc != MZ_OK) return frc;
+  const bool io8 = (flags & MZ_FLAG_IO_U8) != 0, io16 = (flags & MZ_FLAG_IO_U16) != 0;
   const bool x_nhwc = (flags & MZ_FLAG_X_NHWC) != 0, y_nhwc = (flags & MZ_FLAG_Y_NHWC) != 0;
   MZ_REQUIRE(!((x_nhwc || y_nhwc) && (flags & MZ_FLAG_SKIP_FROM_BUFFER)),
              "upscale: interleaved images (MZ_FLAG_X_NHWC / MZ_FLAG_Y_NHWC) recompute the skip (no MZ_FLAG_SKIP_FROM_BUFFER)");
   MZ_REQUIRE(!(x_nhwc || y_nhwc) || static_cast<long long>(H) * W * 3 < (1LL << 31),
              "upscale: an interleaved %d x %d image exceeds 2^31 elements", H, W);
-  const float* x_dev = io8 ? nullptr : static_cast<const float*>(x_dev_v);
-  float* y_dev = io8 ? nullptr : static_cast<float*>(y_dev_v);
+  const float* x_dev = io8 || io16 ? nullptr : static_cast<const float*>(x_dev_v);
+  float* y_dev = io8 || io16 ? nullptr : static_cast<float*>(y_dev_v);
   const uint8_t* x8 = io8 ? static_cast<const uint8_t*>(x_dev_v) : nullptr;
   uint8_t* y8 = io8 ? static_cast<uint8_t*>(y_dev_v) : nullptr;
+  const uint16_t* x16 = io16 ? static_cast<const uint16_t*>(x_dev_v) : nullptr;
+  uint16_t* y16 = io16 ? static_cast<uint16_t*>(y_dev_v) : nullptr;
   MZ_REQUIRE(B > 0 && H > 0 && W > 0, "upscale: empty input (B %d, H %d, W %d)", B, H, W);
   if (m->F > 0) {
     MZ_REQUIRE(c_dev != nullptr, "Control vector c is required for control models.");
@@ -623,7 +642,7 @@ static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, in
   rc = MZ_OK;
   if (front)
     rc = launch_stem(x_dev, x8, m->stem_w, m->stem_b, zf, zb, m->bf16, B, H, W, m->Cpm, m->Czm, s,
-                     m->sat_dev, x_nhwc);
+                     m->sat_dev, x_nhwc, x16);
   if (rc != MZ_OK) return rc;
 
   const int slot = m->timing_calls % kTimingSlots;
@@ -742,6 +761,8 @@ static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, in
   a.epi.y = y_dev;
   a.epi.x8 = x8;
   a.epi.y8 = y8;
+  a.epi.x16 = x16;
+  a.epi.y16 = y16;
   a.epi.u8_trunc = (flags & MZ_FLAG_U8_TRUNC) ? 1 : 0;
   a.epi.r = m->r;
   a.epi.skip_mode = skip_mode;
@@ -781,7 +802,7 @@ int mz_upscale_window(mz_model* m, const void* x_dev, const float* c_dev, int32_
              static_cast<long long>(y_plane_pitch));
   MZ_REQUIRE(!(flags & MZ_FLAG_SKIP_FROM_BUFFER), "upscale_window: the bicubic skip is recomputed (no MZ_FLAG_SKIP_FROM_BUFFER)");
   // bytes of one vector store: the same in both layouts (an interleaved HR row segment of a pixel is three of them)
-  const int es = (flags & MZ_FLAG_IO_U8) ? 1 : 4, vec = m->r == 3 ? es : es * m->r;
+  const int es = (flags & MZ_FLAG_IO_U8) ? 1 : ((flags & MZ_FLAG_IO_U16) ? 2 : 4), vec = m->r == 3 ? es : es * m->r;
   MZ_REQUIRE(reinterpret_cast<uintptr_t>(y_dev) % vec == 0 && (y_row_pitch * es) % vec == 0 && (y_plane_pitch * es) % vec == 0,
              "upscale_window: y and its pitches must be aligned to %d bytes", vec);
   const OutWindow w{win_y0, win_y1, win_x0, win_x1, y_row_pitch, y_plane_pitch};
@@ -821,7 +842,7 @@ int mz_workspace_layout(const mz_model* m, int32_t B, int32_t H, int32_t W, size
 static int host_enqueue(mz_model* m, int li, const void* x_host, const float* c_host, int32_t c_rows, void* y_host,
                         int32_t B, int32_t H, int32_t W, uint32_t flags) {
   mz_model::HostLane& L = m->lane[li];
-  const size_t xb = ((flags & MZ_FLAG_IO_U8) ? 1 : sizeof(float)) * 3 * B * H * W;
+  const size_t xb = image_elem_bytes(flags) * 3 * B * H * W;
   const size_t yb = xb * m->r * m->r;
   const size_t cb = c_host ? sizeof(float) * c_rows * (m->F > 0 ? m->F : 1) : 0;
   size_t wsb = 0;
@@ -865,6 +886,8 @@ int mz_upscale_host_async(mz_model* m, int32_t lane, const void* x_host, const f
   MZ_REQUIRE(m && x_host && y_host, "upscale_host_async: null pointer");
   MZ_REQUIRE(lane == 0 || lane == 1, "upscale_host_async: lane must be 0 or 1, %d given", lane);
   MZ_REQUIRE(B > 0 && H > 0 && W > 0, "upscale_host_async: empty input (B %d, H %d, W %d)", B, H, W);
+  const int frc = check_image_flags(flags);  // (before the copies are enqueued)
+  if (frc != MZ_OK) return frc;
   DeviceGuard g(m->cfg.device);
   return host_enqueue(m, lane, x_host, c_host, c_rows, y_host, B, H, W, flags);
 }
@@ -880,11 +903,13 @@ int mz_upscale_host_wait(mz_model* m, int32_t lane) {
 
 int mz_upscale_host(mz_model* m, const void* x_host_v, const float* c_host, int32_t c_rows, void* y_host_v, int32_t B,
                     int32_t H, int32_t W, uint32_t flags) {
-  const size_t esz = (flags & MZ_FLAG_IO_U8) ? 1 : sizeof(float);
+  const size_t esz = image_elem_bytes(flags);
   const uint8_t* x_host = static_cast<const uint8_t*>(x_host_v);
   uint8_t* y_host = static_cast<uint8_t*>(y_host_v);
   MZ_REQUIRE(m && x_host && y_host, "upscale_host: null pointer");
   MZ_REQUIRE(B > 0 && H > 0 && W > 0, "upscale_host: empty input (B %d, H %d, W %d)", B, H, W);
+  const int frc = check_image_flags(flags);  // (before the copies are enqueued)
+  if (frc != MZ_OK) return frc;
   if (m->F > 0) {
     MZ_REQUIRE(c_host != nullptr, "Control vector c is required for control models.");
     MZ_REQUIRE(c_rows == 1 || c_rows == B, "Batch size of c (%d) must match x (%d).", c_rows, B);

@@ -166,8 +166,18 @@ __device__ __forceinline__ void st_global_v2(void* p, uint32_t a, uint32_t b) {
   asm volatile("st.global.v2.b32 [%0], {%1, %2};" ::"l"(p), "r"(a), "r"(b) : "memory");
 }
 
+// element i of the image as float: fp32 as it is; 8 / 16 bits as the exact quotient x8 / 255, x16 / 65535 (IEEE
+// division, what ToDtype(float32, scale=True) computes): the network amplifies a 1-ulp difference of its input through
+// 20..40 layers of 16-bit rounding to ~1e-3 at the output
+__device__ __forceinline__ float stem_px(const float* __restrict__ x, const uint8_t* __restrict__ x8,
+                                         const uint16_t* __restrict__ x16, size_t i) {
+  if (x8 != nullptr) return __fdiv_rn(static_cast<float>(__ldg(x8 + i)), 255.f);
+  if (x16 != nullptr) return __fdiv_rn(static_cast<float>(__ldg(x16 + i)), 65535.f);
+  return __ldg(x + i);
+}
+
 __global__ void __launch_bounds__(256) stem_kernel(const float* __restrict__ x, const uint8_t* __restrict__ x8,
-                                                   const float* __restrict__ w,
+                                                   const uint16_t* __restrict__ x16, const float* __restrict__ w,
                                                    const float* __restrict__ bias, float* __restrict__ zf,
                                                    uint16_t* __restrict__ zb, int bf16, int B, int H, int W, int Cp,
                                                    int Cz, int ppb, unsigned int* sat, int x_nhwc) {
@@ -192,7 +202,7 @@ __global__ void __launch_bounds__(256) stem_kernel(const float* __restrict__ x, 
     const size_t e0 = p0 * 3;
     for (int e = tid; e < 3 * n; e += nt) {
       const int j = e / 3, c = e - 3 * j;
-      xs[c * ppb + j] = x8 != nullptr ? __fdiv_rn(static_cast<float>(__ldg(x8 + e0 + e)), 255.f) : __ldg(x + e0 + e);
+      xs[c * ppb + j] = stem_px(x, x8, x16, e0 + e);
     }
   } else {
     const size_t b0 = p0 / plane, rem0 = p0 - b0 * plane;  // (one division per block; the range may cross images)
@@ -205,12 +215,7 @@ __global__ void __launch_bounds__(256) stem_kernel(const float* __restrict__ x, 
       }
       const size_t xo = b * 3 * plane + rem;
 #pragma unroll
-      for (int c = 0; c < 3; ++c) {
-        // 8-bit input: exact x8 / 255 (IEEE division, what ToDtype(float32, scale=True) computes): the network
-        // amplifies a 1-ulp difference of its input through 20..40 layers of 16-bit rounding to ~1e-3 at the output
-        xs[c * ppb + j] = x8 != nullptr ? __fdiv_rn(static_cast<float>(__ldg(x8 + xo + c * plane)), 255.f)
-                                        : __ldg(x + xo + c * plane);
-      }
+      for (int c = 0; c < 3; ++c) xs[c * ppb + j] = stem_px(x, x8, x16, xo + c * plane);
     }
   }
   __syncthreads();
@@ -231,7 +236,8 @@ __global__ void __launch_bounds__(256) stem_kernel(const float* __restrict__ x, 
 }
 
 int launch_stem(const float* x, const uint8_t* x8, const float* w, const float* bias, float* zf, uint16_t* zb, int bf16,
-                int B, int H, int W, int Cp, int zb_pitch, cudaStream_t s, unsigned int* sat, bool x_nhwc) {
+                int B, int H, int W, int Cp, int zb_pitch, cudaStream_t s, unsigned int* sat, bool x_nhwc,
+                const uint16_t* x16) {
   MZ_REQUIRE(Cp > 0 && Cp % 8 == 0, "stem: padded channel count must be a multiple of 8, %d given", Cp);
   MZ_REQUIRE(B > 0 && H > 0 && W > 0, "stem: empty input");
   MZ_REQUIRE(zf != nullptr, "stem: null fp32 stream");
@@ -249,8 +255,8 @@ int launch_stem(const float* x, const uint8_t* x8, const float* w, const float* 
   const long long blocks = (npix + ppb - 1) / ppb;
   MZ_REQUIRE(blocks < (1LL << 31), "stem: too many pixels");
   const size_t smem = static_cast<size_t>(3) * ppb * sizeof(float);
-  stem_kernel<<<static_cast<unsigned>(blocks), dim3(groups, py), smem, s>>>(x, x8, w, bias, zf, zb, bf16, B, H, W, Cp, Cz,
-                                                                         static_cast<int>(ppb), sat, x_nhwc ? 1 : 0);
+  stem_kernel<<<static_cast<unsigned>(blocks), dim3(groups, py), smem, s>>>(x, x8, x16, w, bias, zf, zb, bf16, B, H, W, Cp,
+                                                                         Cz, static_cast<int>(ppb), sat, x_nhwc ? 1 : 0);
   MZ_CUDA(cudaGetLastError());
   return MZ_OK;
 }

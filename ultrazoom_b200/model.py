@@ -31,11 +31,14 @@ def _is_nhwc(t: Tensor) -> bool:
     return t.is_contiguous(memory_format=torch.channels_last) and not t.is_contiguous()
 
 
-def _input_image(x: Tensor, io8: bool):
-    """``(x, flag)``: the image as the kernels read it -- uint8 as it is, anything else as float32 -- kept interleaved
-    when it is (``MZ_FLAG_X_NHWC``, no transpose), otherwise made contiguous NCHW."""
+_INT_IMAGE_DTYPES = (torch.uint8, torch.uint16)   # images the kernels read and write as integers (MZ_FLAG_IO_U8 / _U16)
+
+
+def _input_image(x: Tensor, integer: bool):
+    """``(x, flag)``: the image as the kernels read it -- uint8 / uint16 as it is, anything else as float32 -- kept
+    interleaved when it is (``MZ_FLAG_X_NHWC``, no transpose), otherwise made contiguous NCHW."""
     nhwc = _is_nhwc(x)
-    x = x.detach() if io8 else x.detach().to(torch.float32)
+    x = x.detach() if integer else x.detach().to(torch.float32)
     x = x.contiguous(memory_format=torch.channels_last if nhwc else torch.contiguous_format)
     return x, (_native.FLAG_X_NHWC if nhwc else 0)
 
@@ -265,7 +268,7 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         self.residual_stream = residual_stream
         self._engines: dict = {}
         self._flags_extra = 0
-        self.u8_truncate = False
+        self.u8_truncate = False          # uint8 results: floor(255 y) instead of floor(255 y + 0.5); not for uint16
         self._auto_dtype = "float16"      # operand_dtype="auto": what the next call runs with
         self._param_cache = None
         self._host_keep: dict = {}          # (device, lane) -> (engine, x, c, out) of the frame in flight on that lane
@@ -421,6 +424,12 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         t = _native.tune(**kw)
         _native.check(eng.lib.mz_model_set_tune(eng.handle, which, C.byref(t)))
 
+    def _image_flags(self, dtype: torch.dtype) -> int:
+        """The element-type flags of an image: uint8 (rounded as ``u8_truncate`` says), uint16, or 0 for float32."""
+        if dtype == torch.uint8:
+            return _native.FLAG_IO_U8 | (_native.FLAG_U8_TRUNC if self.u8_truncate else 0)
+        return _native.FLAG_IO_U16 if dtype == torch.uint16 else 0
+
     def _check_inputs(self, x: Tensor, c: Optional[Tensor]) -> Optional[Tensor]:
         assert x.dim() == 4 and x.shape[1] == 3, f"Expected input of shape (B, 3, H, W), got {tuple(x.shape)}."
         assert x.shape[0] > 0 and x.shape[2] > 0 and x.shape[3] > 0, "Input must not be empty."
@@ -442,11 +451,12 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
             raise RuntimeError("ultrazoom_b200.MewZoom runs on sm_100a CUDA kernels only; move the input to a "
                                "B200 (`x.cuda()`). There is no CPU fallback.")
         dev = x.device
-        io8 = x.dtype == torch.uint8       # 8-bit images in and out (upscale only): see upscale()
-        if io8:
-            assert flags & _native.FLAG_CLAMP01, "uint8 images are supported by upscale(), not forward()"
-            flags |= _native.FLAG_IO_U8 | (_native.FLAG_U8_TRUNC if self.u8_truncate else 0)
-        x, xflag = _input_image(x, io8)
+        odt = x.dtype if x.dtype in _INT_IMAGE_DTYPES else torch.float32   # 8 / 16-bit images in and out: see upscale()
+        if odt != torch.float32:
+            assert flags & _native.FLAG_CLAMP01, (
+                f"{str(odt).replace('torch.', '')} images are supported by upscale(), not forward()")
+            flags |= self._image_flags(odt)
+        x, xflag = _input_image(x, odt != torch.float32)
         flags |= xflag | _output_flag(memory_format)
         if c is not None:
             c = c.detach().to(device=dev, dtype=torch.float32).contiguous()
@@ -460,8 +470,7 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
                 torch.cuda.synchronize(dev)    # (the flag of an earlier asynchronous call is not this call's to absorb)
             if not capturing:
                 self._range_guard(eng)
-            y = torch.empty((B, 3, H * r, W * r), dtype=torch.uint8 if io8 else torch.float32, device=dev,
-                            memory_format=memory_format)
+            y = torch.empty((B, 3, H * r, W * r), dtype=odt, device=dev, memory_format=memory_format)
             stream = torch.cuda.current_stream(dev)
             eng.begin(stream)
             w = ws if ws is not None else eng.workspace(B, H, W, stream)
@@ -491,6 +500,9 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         (``ToDtype(float32, scale=True)``, test_compare.py:55-57) and the result comes back as uint8,
         ``floor(255 * y + 0.5)`` as ``save_image`` writes it (test_compare.py:89) -- or ``floor(255 * y)`` as
         ``ToPILImage`` does (README.md:81) when ``model.u8_truncate`` is set: a quarter of the image traffic.
+        A ``torch.uint16`` image (16-bit PNG / TIFF, 10/12-bit video decoded to rgb48le) is read as ``x / 65535``, the
+        exact quotient, and comes back as uint16, ``floor(65535 * y + 0.5)``: the fp32 result on ``x.float() / 65535``,
+        quantised, at half the image traffic.  ``u8_truncate`` does not apply to it.
 
         Interleaved images need no transpose on either side: an ``x`` in ``channels_last`` strides (and not also plainly
         contiguous), e.g. ``torch.from_numpy(hwc_frames).permute(0, 3, 1, 2)``, is read as it is, and
@@ -505,7 +517,8 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         0.2.x model (validate.py:97).  The bicubic image comes from the stand-alone bicubic kernel (mz_bicubic_f32)."""
         from . import ops
 
-        return self.upscale(x, c), ops.bicubic(x.float() if x.dtype != torch.uint8 else x.float() / 255.0,
+        scale = {torch.uint8: 255.0, torch.uint16: 65535.0}.get(x.dtype)
+        return self.upscale(x, c), ops.bicubic(x.float() if scale is None else x.float() / scale,
                                                self.upscale_ratio).clamp_(0, 1)
 
     @torch.inference_mode()
@@ -525,11 +538,9 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
             torch.cuda.synchronize(dev)        # (as in upscale: only this call's flag may be absorbed by its re-run)
         self._range_guard(eng)
         x_in, c_in = x, c
-        io8 = x.dtype == torch.uint8
-        flags = _native.FLAG_CLAMP01 | self._flags_extra
-        if io8:
-            flags |= _native.FLAG_IO_U8 | (_native.FLAG_U8_TRUNC if self.u8_truncate else 0)
-        x, xflag = _input_image(x, io8)
+        odt = x.dtype if x.dtype in _INT_IMAGE_DTYPES else torch.float32
+        flags = _native.FLAG_CLAMP01 | self._flags_extra | self._image_flags(odt)
+        x, xflag = _input_image(x, odt != torch.float32)
         if c is not None:
             c = c.detach().to(device=dev, dtype=torch.float32).contiguous()
         B, _, H, W = x.shape
@@ -537,7 +548,7 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         y0, y1, x0, x1 = window
         fy, fx = at
         assert frame.is_cuda and frame.dim() == 4 and frame.shape[0] == B and frame.shape[1] == 3, "frame must be (B,3,H',W')"
-        assert frame.dtype == (torch.uint8 if io8 else torch.float32)
+        assert frame.dtype == odt, f"frame must be {odt} for a {odt} input, got {frame.dtype}"
         yflag, row_pitch, img_pitch = _frame_layout(frame)
         flags |= xflag | yflag
         assert 0 <= fy and fy + (y1 - y0) * r <= frame.shape[2] and 0 <= fx and fx + (x1 - x0) * r <= frame.shape[3], (
@@ -568,15 +579,14 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         num_encoder_layers``.  Between stages ``sharding.upscale_tiled_refresh`` overwrites the tile's halo with the
         neighbours' values (``stage_views``)."""
         c = self._check_inputs(x, c)
-        assert x.is_cuda and x.dtype in (torch.float32, torch.uint8), "upscale_stage takes a CUDA image (float32 or uint8)"
+        assert x.is_cuda and x.dtype in (torch.float32, torch.uint8, torch.uint16), (
+            "upscale_stage takes a CUDA image (float32, uint8 or uint16)")
         dev = x.device
         eng = self._engine(dev)
         self._range_guard(eng)            # (stages run asynchronously: a saturated stage is reported by the next call)
-        io8 = x.dtype == torch.uint8
-        flags = _native.FLAG_CLAMP01 | self._flags_extra
-        if io8:
-            flags |= _native.FLAG_IO_U8 | (_native.FLAG_U8_TRUNC if self.u8_truncate else 0)
-        x, xflag = _input_image(x, io8)
+        integer = x.dtype in _INT_IMAGE_DTYPES
+        flags = _native.FLAG_CLAMP01 | self._flags_extra | self._image_flags(x.dtype)
+        x, xflag = _input_image(x, integer)
         if c is not None:
             c = c.detach().to(device=dev, dtype=torch.float32).contiguous()
         B, _, H, W = x.shape
@@ -642,9 +652,10 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         and ``out`` should be pinned and must not be touched until the wait.  A frame clipped to the fp16 range raises
         in the synchronous call itself ("auto": it is repeated with bfloat16 operands), on a lane at ``host_wait``.
 
-        Layouts as in ``upscale``: a channels-last ``x`` is copied as it is (no transpose on the CPU), and the result is
-        interleaved with ``memory_format=torch.channels_last``.  A caller's ``out`` sets the output layout itself: it
-        must be contiguous NCHW or contiguous channels-last."""
+        Element types and layouts as in ``upscale`` (uint8 and uint16 frames come back as such): a channels-last ``x`` is
+        copied as it is (no transpose on the CPU), and the result is interleaved with
+        ``memory_format=torch.channels_last``.  A caller's ``out`` sets the output layout itself: it must be contiguous
+        NCHW or contiguous channels-last, of the input's element type."""
         c = self._check_inputs(x, c)
         assert not x.is_cuda, "upscale_host takes host tensors"
         assert lane in (None, 0, 1), "lane must be None, 0 or 1"
@@ -652,13 +663,12 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         if lane is None and self.operand_dtype == "auto" and eng.operand_dtype == "float16":
             torch.cuda.synchronize(torch.device("cuda", device))   # (as in upscale; lanes included)
         self._range_guard(eng)
-        io8 = x.dtype == torch.uint8
-        x, xflag = _input_image(x, io8)
+        odt = x.dtype if x.dtype in _INT_IMAGE_DTYPES else torch.float32
+        x, xflag = _input_image(x, odt != torch.float32)
         if c is not None:
             c = c.to(device="cpu", dtype=torch.float32).contiguous()
         B, _, H, W = x.shape
         r = self.upscale_ratio
-        odt = torch.uint8 if io8 else torch.float32
         if out is None:
             out = torch.empty((B, 3, H * r, W * r), dtype=odt, memory_format=memory_format)
             yflag = _output_flag(memory_format)
@@ -666,9 +676,7 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
             yflag = _native.FLAG_Y_NHWC if _is_nhwc(out) else 0
             assert out.is_contiguous() or yflag, "out must be contiguous NCHW or contiguous channels-last"
         assert tuple(out.shape) == (B, 3, H * r, W * r) and out.dtype == odt
-        flags = _native.FLAG_CLAMP01 | self._flags_extra | xflag | yflag
-        if io8:
-            flags |= _native.FLAG_IO_U8 | (_native.FLAG_U8_TRUNC if self.u8_truncate else 0)
+        flags = _native.FLAG_CLAMP01 | self._flags_extra | xflag | yflag | self._image_flags(odt)
         cp, cr = (c.data_ptr(), c.shape[0]) if c is not None else (None, 0)
         if lane is None:
             _native.check(eng.lib.mz_upscale_host(eng.handle, x.data_ptr(), cp, cr, out.data_ptr(), B, H, W, flags))
@@ -714,7 +722,7 @@ class GraphedUpscale:
             raise RuntimeError("MewZoom.capture needs a CUDA input (there is no CPU fallback).")
         self.model = model
         # (the input buffer keeps the layout of x: the graph reads it as _run reads x; a replay copies either layout in)
-        self.x = _input_image(x, x.dtype == torch.uint8)[0].clone()
+        self.x = _input_image(x, x.dtype in _INT_IMAGE_DTYPES)[0].clone()
         self.c = None if c is None else c.detach().to(device=x.device, dtype=torch.float32).contiguous().clone()
         # The graph bakes in raw pointers: it owns everything they point at -- its input / output tensors, a PRIVATE
         # workspace (the engine's cached one is dropped and re-allocated when a later call needs a larger one) and the
@@ -747,7 +755,8 @@ class GraphedUpscale:
     def __call__(self, x: Tensor, c: Optional[Tensor] = None) -> Tensor:
         """Copy ``x`` / ``c`` in and replay; raises first when an earlier replay was clipped to the fp16 range."""
         self.model._range_guard(self.engine)
-        assert tuple(x.shape) == tuple(self.x.shape) and (x.dtype == torch.uint8) == (self.x.dtype == torch.uint8), (
+        integer = x.dtype in _INT_IMAGE_DTYPES
+        assert tuple(x.shape) == tuple(self.x.shape) and (x.dtype == self.x.dtype if integer else self.x.dtype == torch.float32), (
             f"Graph was captured for input {tuple(self.x.shape)} {self.x.dtype}, got {tuple(x.shape)} {x.dtype}.")
         self.x.copy_(x, non_blocking=True)
         if self.c is not None:

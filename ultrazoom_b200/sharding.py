@@ -202,7 +202,7 @@ class SharedFrame:
                 dist.broadcast_object_list(box, src=owner, group=group)   # control plane: 64 bytes, once
             if not self.owner:
                 _native.check(self.lib.mz_ipc_frame_open(box[0], C.byref(self.ptr)))
-        typestr = {torch.float32: "<f4", torch.uint8: "|u1"}[dtype]
+        typestr = {torch.float32: "<f4", torch.uint8: "|u1", torch.uint16: "<u2"}[dtype]
 
         class _Mem:
             __cuda_array_interface__ = {"shape": tuple(int(d) for d in shape), "typestr": typestr,
