@@ -92,22 +92,23 @@ def bicubic_phase_table(r: int) -> list[tuple[int, list[float]]]:
 
 def bicubic_upsample_ref(x: Tensor, r: int) -> Tensor:
     """Pure index-arithmetic bicubic zoom (float64 accumulate), clamped tap
-    indices, no antialias, no output clamp.  x: (B,3,H,W)."""
+    indices, no antialias, no output clamp.  x: (B,3,H,W), on any device (the result stays there)."""
     B, C, H, W = x.shape
+    dev = x.device
     tab = bicubic_phase_table(r)
     xd = x.double()
     # horizontal pass
-    ox = torch.arange(W * r)
-    base_x = ox // r + torch.tensor([tab[p][0] for p in range(r)])[ox % r]
-    wx = torch.tensor([tab[p][1] for p in range(r)], dtype=torch.float64)[ox % r]  # (Wr,4)
-    tmp = torch.zeros(B, C, H, W * r, dtype=torch.float64)
+    ox = torch.arange(W * r, device=dev)
+    base_x = ox // r + torch.tensor([tab[p][0] for p in range(r)], device=dev)[ox % r]
+    wx = torch.tensor([tab[p][1] for p in range(r)], dtype=torch.float64, device=dev)[ox % r]  # (Wr,4)
+    tmp = torch.zeros(B, C, H, W * r, dtype=torch.float64, device=dev)
     for k in range(4):
         idx = (base_x - 1 + k).clamp(0, W - 1)
         tmp += xd[..., idx] * wx[:, k]
-    oy = torch.arange(H * r)
-    base_y = oy // r + torch.tensor([tab[p][0] for p in range(r)])[oy % r]
-    wy = torch.tensor([tab[p][1] for p in range(r)], dtype=torch.float64)[oy % r]
-    out = torch.zeros(B, C, H * r, W * r, dtype=torch.float64)
+    oy = torch.arange(H * r, device=dev)
+    base_y = oy // r + torch.tensor([tab[p][0] for p in range(r)], device=dev)[oy % r]
+    wy = torch.tensor([tab[p][1] for p in range(r)], dtype=torch.float64, device=dev)[oy % r]
+    out = torch.zeros(B, C, H * r, W * r, dtype=torch.float64, device=dev)
     for k in range(4):
         idx = (base_y - 1 + k).clamp(0, H - 1)
         out += tmp[:, :, idx, :] * wy[:, k][None, None, :, None]
