@@ -68,6 +68,24 @@ typedef enum mz_status {
  * (MZ_ERR_INVALID).  Applies to mz_upscale, mz_upscale_window, mz_upscale_stage, mz_upscale_host and
  * mz_upscale_host_async. */
 #define MZ_FLAG_IO_U16 128u
+/* 4:2:0 video frames, as decoders (NVDEC, ffmpeg -hwaccel cuda) produce and encoders (NVENC) take them: x and y are
+ * NV12 with MZ_FLAG_IO_U8, P010 with MZ_FLAG_IO_U16.  A frame is a luma plane of H x W elements, then an interleaved
+ * Cb,Cr plane of H/2 x W/2 pairs; frames are 3HW/2 elements apart, with no row pitch beyond W (HR frames: rH, rW).  P010
+ * words hold the 10-bit code in their top bits (word = code << 6): the low 6 bits are ignored on input, zero on output.
+ * The call is exactly
+ *   mz_yuv420_to_rgb16(x) -> the MZ_FLAG_IO_U16 planar upscale -> mz_rgb16_to_yuv420(y)
+ * with both 16-bit RGB images in the workspace (mz_workspace_bytes_flags).  Chroma siting is the H.264 / HEVC default
+ * (sample (i, j) at luma row 2i + 1/2, column 2j); see mz_yuv420_to_rgb16 for the filters and rounding.
+ * Needs MZ_FLAG_CLAMP01, exactly one of MZ_FLAG_IO_U8 / _U16 and even H and W; MZ_FLAG_X_NHWC, MZ_FLAG_Y_NHWC,
+ * MZ_FLAG_U8_TRUNC and MZ_FLAG_SKIP_FROM_BUFFER are refused (MZ_ERR_INVALID).  Applies to mz_upscale, mz_upscale_host
+ * and mz_upscale_host_async; mz_upscale_window and mz_upscale_stage refuse it.
+ * Colour: BT.709 (Kr 0.2126, Kb 0.0722) unless MZ_FLAG_YUV_BT601 (0.299, 0.114) or MZ_FLAG_YUV_BT2020 (0.2627, 0.0593,
+ * non-constant luminance) is set -- both is MZ_ERR_INVALID; limited range (8-bit Y 16..235, C 16..240; 10-bit 64..940,
+ * 64..960) unless MZ_FLAG_YUV_FULL_RANGE.  The colour bits without MZ_FLAG_YUV420 are refused. */
+#define MZ_FLAG_YUV420 256u
+#define MZ_FLAG_YUV_BT601 512u
+#define MZ_FLAG_YUV_BT2020 1024u
+#define MZ_FLAG_YUV_FULL_RANGE 2048u
 
 /* Constructor kwargs of the 0.2.x-style MewZoom (README.md:254-258, model.py:52-69). */
 typedef struct mz_config {
@@ -142,12 +160,17 @@ int mz_model_saturated(mz_model* m, int32_t reset, int32_t* saturated);
 
 /* Bytes of device scratch mz_upscale needs for a (B,3,H,W) input. */
 int mz_workspace_bytes(const mz_model* m, int32_t B, int32_t H, int32_t W, size_t* bytes);
+/* The same for a call with `flags`: equal to mz_workspace_bytes unless MZ_FLAG_YUV420 is set, which adds the two 16-bit
+ * RGB images (B,3,H,W) and (B,3,rH,rW), each rounded up to 1024 bytes, after everything mz_workspace_layout places. */
+int mz_workspace_bytes_flags(const mz_model* m, int32_t B, int32_t H, int32_t W, uint32_t flags, size_t* bytes);
 
 /* ---- the hot path: replaces MewZoom.forward / MewZoom.upscale (model.py:149-179) ----
- * x_dev : (B,3,H,W) fp32 NCHW in [0,1]   (uint8 / uint16 with MZ_FLAG_IO_U8 / _U16; (B,H,W,3) with MZ_FLAG_X_NHWC)
+ * x_dev : (B,3,H,W) fp32 NCHW in [0,1]   (uint8 / uint16 with MZ_FLAG_IO_U8 / _U16; (B,H,W,3) with MZ_FLAG_X_NHWC;
+ *         B 4:2:0 frames of H x W luma with MZ_FLAG_YUV420)
  * c_dev : NULL for non-control models, else (B, control_features) fp32 (c_rows == B)
  *         or (1, control_features) (c_rows == 1, broadcast) -- validate.py:73-94
- * y_dev : (B,3,rH,rW) fp32 NCHW          (uint8 / uint16 with MZ_FLAG_IO_U8 / _U16; (B,rH,rW,3) with MZ_FLAG_Y_NHWC)
+ * y_dev : (B,3,rH,rW) fp32 NCHW          (uint8 / uint16 with MZ_FLAG_IO_U8 / _U16; (B,rH,rW,3) with MZ_FLAG_Y_NHWC;
+ *         B 4:2:0 frames of rH x rW luma with MZ_FLAG_YUV420)
  * flags : MZ_FLAG_CLAMP01 => upscale(), 0 => forward()
  */
 int mz_upscale(mz_model* m, const void* x_dev, const float* c_dev, int32_t c_rows, void* y_dev,
@@ -295,6 +318,20 @@ int mz_head_shuffle_add(const void* zb_dev, const void* wpacked_dev, const float
                         int32_t B, int32_t H, int32_t W, int32_t cin_p, int32_t in_pitch, int32_t r,
                         int32_t skip_mode, int32_t clamp01, int32_t operand_dtype, int32_t use_tc,
                         const mz_conv_tune* tune, void* stream);
+
+/* The two halves of an MZ_FLAG_YUV420 call (flags: MZ_FLAG_YUV420, MZ_FLAG_IO_U8 for NV12 or MZ_FLAG_IO_U16 for P010,
+ * and the colour bits).  yuv_dev holds B frames of 3HW/2 elements (aligned to 2 bytes for NV12, 4 for P010); rgb_dev is
+ * (B,3,H,W) uint16 planar (4-byte aligned); H and W are the luma size and must be even.
+ * mz_yuv420_to_rgb16: chroma is upsampled separably with clamped edges, vertical first -- luma row 2i takes
+ *   3/4 C[i] + 1/4 C[i-1], row 2i+1 3/4 C[i] + 1/4 C[i+1]; column 2j takes C[j], column 2j+1 (C[j] + C[j+1]) / 2 -- then
+ *   R = Y' + 2(1-Kr) Cr', B = Y' + 2(1-Kb) Cb', G = (Y' - Kr R - Kb B) / Kg, clamped to [0, 1], rgb = floor(65535 v + 0.5).
+ * mz_rgb16_to_yuv420: v = rgb / 65535; Y' = Kr R + Kg G + Kb B per pixel; Cb' = (B - Y') / (2(1-Kb)) and
+ *   Cr' = (R - Y') / (2(1-Kr)) averaged over rows 2i and 2i+1, then filtered [1, 2, 1] / 4 over columns 2j-1, 2j, 2j+1
+ *   (column -1 clamped to 0); every code floor(offset + scale v + 0.5), clamped to [0, 2^bits - 1].
+ * Normalisation: 8-bit limited Y' = (Y - 16) / 219, C' = (C - 128) / 224; full Y / 255, (C - 128) / 255; 10-bit limited
+ * (Y - 64) / 876, (C - 512) / 896; full Y / 1023, (C - 512) / 1023. */
+int mz_yuv420_to_rgb16(const void* yuv_dev, uint16_t* rgb_dev, int32_t B, int32_t H, int32_t W, uint32_t flags, void* stream);
+int mz_rgb16_to_yuv420(const uint16_t* rgb_dev, void* yuv_dev, int32_t B, int32_t H, int32_t W, uint32_t flags, void* stream);
 
 /* Repack OIHW fp32 (host) -> device fp16|bf16 [tap = ky*3+kx][cout_p][cin_p] (K-major rows; the TMA
  * applies the shared-memory swizzle).  With dst_dev == NULL only *bytes is written. */

@@ -4,7 +4,7 @@
     from ultrazoom_b200.control import ControlVector
 """
 from .control import ControlVector  # noqa: F401
-from .model import MewZoom, ONNXModel  # noqa: F401
+from .model import MewZoom, ONNXModel, Yuv420  # noqa: F401
 
 MODEL_CONFIGS = {
     # reference README.md:35-42 (channels, encoder layers); hidden_ratio 2 = pretrain.py:74 default

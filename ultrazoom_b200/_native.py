@@ -29,6 +29,10 @@ FLAG_U8_TRUNC = 16
 FLAG_X_NHWC = 32
 FLAG_Y_NHWC = 64
 FLAG_IO_U16 = 128
+FLAG_YUV420 = 256
+FLAG_YUV_BT601 = 512
+FLAG_YUV_BT2020 = 1024
+FLAG_YUV_FULL_RANGE = 2048
 
 DTYPE_F16, DTYPE_BF16 = 0, 1
 MATH_TF32, MATH_FP32 = 0, 1
@@ -89,6 +93,7 @@ SIGNATURES = {
     "mz_model_enable_timing": (C.c_int, [_P, _I]),
     "mz_model_conv_stack_ms": (C.c_int, [_P, C.POINTER(C.c_float)]),
     "mz_workspace_bytes": (C.c_int, [_P, _I, _I, _I, C.POINTER(C.c_size_t)]),
+    "mz_workspace_bytes_flags": (C.c_int, [_P, _I, _I, _I, C.c_uint32, C.POINTER(C.c_size_t)]),
     "mz_model_fused_block": (C.c_int, [_P]),
     "mz_block_fused": (C.c_int, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
     "mz_upscale": (C.c_int, [_P, _P, _P, _I, _P, _I, _I, _I, _P, C.c_size_t, C.c_uint32, _P]),
@@ -110,6 +115,8 @@ SIGNATURES = {
     "mz_stem_pack": (C.c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
     "mz_conv3x3": (C.c_int, [_P, _P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, C.POINTER(MzConvTune), _P]),
     "mz_head_shuffle_add": (C.c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, C.POINTER(MzConvTune), _P]),
+    "mz_yuv420_to_rgb16": (C.c_int, [_P, _P, _I, _I, _I, C.c_uint32, _P]),
+    "mz_rgb16_to_yuv420": (C.c_int, [_P, _P, _I, _I, _I, C.c_uint32, _P]),
     "mz_pack_conv_weight": (C.c_int, [_P, _I, _I, _I, _I, _I, _P, C.POINTER(C.c_size_t)]),
     "mz_control_film": (C.c_int, [_P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "mz_adaptive_mix": (C.c_int, [_P, _P, _P, C.c_float, _P, _P, C.c_int64, _I, _I, _I, _I, _P]),

@@ -198,6 +198,18 @@ int launch_stem(const float* x, const uint8_t* x8, const float* w, const float* 
 int launch_film(const float* c, int c_rows, const float* w, const float* b, float* film, int L, int B, int F,
                 int hC, int hCp, int ns, cudaStream_t s);
 
+// 4:2:0 frames (yuv420.cu): colour matrix and code range of the MZ_FLAG_YUV* bits.  yuv_coef refuses (MZ_ERR_INVALID)
+// flags without MZ_FLAG_YUV420, without exactly one of MZ_FLAG_IO_U8 / _U16, or with both matrix bits.
+struct YuvCoef {
+  float kr, kb, kg;             // Kr, Kb, Kg = 1 - Kr - Kb
+  float yoff, yrange;           // Y = yoff + yrange Y'
+  float coff, crange, maxcode;  // C = coff + crange C'; codes 0..maxcode
+};
+int yuv_coef(uint32_t flags, YuvCoef* k);
+// yuv (B frames of 3HW/2 elements) <-> rgb16 (B,3,H,W); H and W even, the LR or HR luma size of the frame
+int launch_yuv420_to_rgb16(const void* yuv, uint16_t* rgb, int B, int H, int W, uint32_t flags, cudaStream_t s);
+int launch_rgb16_to_yuv420(const uint16_t* rgb, void* yuv, int B, int H, int W, uint32_t flags, cudaStream_t s);
+
 ConvTcTune to_tune(const mz_conv_tune* t);
 int current_device();
 bool dtype_ok(int d);

@@ -105,10 +105,14 @@ struct DeviceGuard {
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 struct WsPlan {
-  size_t zf, zb, hid, film, total;
+  size_t zf, zb, hid, film, rgb_lr, rgb_hr, total;
 };
 
-WsPlan plan_ws(const mz_model* m, int B, int H, int W) {
+constexpr uint32_t kYuvColourFlags = MZ_FLAG_YUV_BT601 | MZ_FLAG_YUV_BT2020 | MZ_FLAG_YUV_FULL_RANGE;
+
+// With MZ_FLAG_YUV420 the two 16-bit RGB images of the call follow everything else, so that mz_workspace_layout's offsets
+// are the same for every call.
+WsPlan plan_ws(const mz_model* m, int B, int H, int W, uint32_t flags = 0) {
   const size_t npix = static_cast<size_t>(B) * H * W;
   WsPlan p;
   size_t off = 0;
@@ -120,6 +124,13 @@ WsPlan plan_ws(const mz_model* m, int B, int H, int W) {
   off = align_up(off + npix * m->hCm * sizeof(uint16_t), 1024);
   p.film = off;
   if (m->F > 0) off = align_up(off + static_cast<size_t>(m->L) * B * 2 * m->hCp * sizeof(float), 1024);
+  p.rgb_lr = p.rgb_hr = off;
+  if (flags & MZ_FLAG_YUV420) {
+    const size_t lr = static_cast<size_t>(B) * 3 * H * W * sizeof(uint16_t);
+    off = align_up(off + lr, 1024);
+    p.rgb_hr = off;
+    off = align_up(off + lr * m->r * m->r, 1024);
+  }
   p.total = off;
   return p;
 }
@@ -557,6 +568,13 @@ int mz_workspace_bytes(const mz_model* m, int32_t B, int32_t H, int32_t W, size_
   return MZ_OK;
 }
 
+int mz_workspace_bytes_flags(const mz_model* m, int32_t B, int32_t H, int32_t W, uint32_t flags, size_t* bytes) {
+  MZ_REQUIRE(m && bytes, "workspace_bytes: null pointer");
+  MZ_REQUIRE(B > 0 && H > 0 && W > 0, "workspace_bytes: empty input (B %d, H %d, W %d)", B, H, W);
+  *bytes = plan_ws(m, B, H, W, flags).total;
+  return MZ_OK;
+}
+
 }  // extern "C"
 
 // output window of mz_upscale_window (nullptr: the whole image, densely)
@@ -565,19 +583,33 @@ struct OutWindow {
   long long row_pitch, plane_pitch;
 };
 
-// the image element type flags: 8 or 16 bits need MZ_FLAG_CLAMP01, recompute the skip and exclude each other
-static int check_image_flags(uint32_t flags) {
+// the image element type flags: 8 or 16 bits need MZ_FLAG_CLAMP01, recompute the skip and exclude each other; a 4:2:0
+// frame is one of them, planar on both sides, with even dimensions
+static int check_image_flags(uint32_t flags, int H, int W) {
   MZ_REQUIRE(!(flags & MZ_FLAG_IO_U8) || ((flags & MZ_FLAG_CLAMP01) && !(flags & MZ_FLAG_SKIP_FROM_BUFFER)),
              "upscale: 8-bit image I/O needs MZ_FLAG_CLAMP01 and recomputes the skip (no MZ_FLAG_SKIP_FROM_BUFFER)");
   MZ_REQUIRE(!(flags & MZ_FLAG_IO_U16) ||
                  ((flags & MZ_FLAG_CLAMP01) && !(flags & (MZ_FLAG_SKIP_FROM_BUFFER | MZ_FLAG_IO_U8 | MZ_FLAG_U8_TRUNC))),
              "upscale: 16-bit image I/O needs MZ_FLAG_CLAMP01, recomputes the skip (no MZ_FLAG_SKIP_FROM_BUFFER) and "
              "excludes MZ_FLAG_IO_U8 and MZ_FLAG_U8_TRUNC");
+  MZ_REQUIRE((flags & MZ_FLAG_YUV420) || !(flags & kYuvColourFlags),
+             "upscale: the colour bits MZ_FLAG_YUV_* apply to 4:2:0 frames only (MZ_FLAG_YUV420)");
+  if (flags & MZ_FLAG_YUV420) {
+    YuvCoef k;
+    const int rc = yuv_coef(flags, &k);  // (NV12 or P010, one colour matrix)
+    if (rc != MZ_OK) return rc;
+    MZ_REQUIRE(flags & MZ_FLAG_CLAMP01, "upscale: 4:2:0 frames need MZ_FLAG_CLAMP01");
+    MZ_REQUIRE(!(flags & (MZ_FLAG_X_NHWC | MZ_FLAG_Y_NHWC | MZ_FLAG_U8_TRUNC | MZ_FLAG_SKIP_FROM_BUFFER)),
+               "upscale: 4:2:0 frames exclude MZ_FLAG_X_NHWC, MZ_FLAG_Y_NHWC, MZ_FLAG_U8_TRUNC and MZ_FLAG_SKIP_FROM_BUFFER");
+    MZ_REQUIRE(H % 2 == 0 && W % 2 == 0, "upscale: a 4:2:0 frame has even dimensions, %d x %d given", H, W);
+  }
   return MZ_OK;
 }
-// bytes per image element: fp32, 8 or 16 bits
-static size_t image_elem_bytes(uint32_t flags) {
-  return (flags & MZ_FLAG_IO_U8) ? 1 : ((flags & MZ_FLAG_IO_U16) ? 2 : sizeof(float));
+// bytes of one image: 3HW elements of fp32, 8 or 16 bits, or a 4:2:0 frame of 3HW/2
+static size_t image_bytes(uint32_t flags, int H, int W) {
+  const size_t es = (flags & MZ_FLAG_IO_U8) ? 1 : ((flags & MZ_FLAG_IO_U16) ? 2 : sizeof(float));
+  const size_t px = static_cast<size_t>(H) * W;
+  return (flags & MZ_FLAG_YUV420) ? px * 3 / 2 * es : px * 3 * es;
 }
 
 // layer_begin / layer_end: the encoder blocks [layer_begin, layer_end) of this call (mz_upscale_stage).  The FiLM table and
@@ -590,8 +622,10 @@ static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, in
   MZ_REQUIRE(0 <= layer_begin && layer_begin <= layer_end && layer_end <= m->L, "upscale: bad layer range [%d, %d) of %d",
              layer_begin, layer_end, m->L);
   const bool front = layer_begin == 0, back = layer_end == m->L;
-  const int frc = check_image_flags(flags);
+  const int frc = check_image_flags(flags, H, W);
   if (frc != MZ_OK) return frc;
+  const bool yuv = (flags & MZ_FLAG_YUV420) != 0;
+  MZ_REQUIRE(!yuv || (!win && front && back), "upscale: 4:2:0 frames are neither windowed nor staged");
   const bool io8 = (flags & MZ_FLAG_IO_U8) != 0, io16 = (flags & MZ_FLAG_IO_U16) != 0;
   const bool x_nhwc = (flags & MZ_FLAG_X_NHWC) != 0, y_nhwc = (flags & MZ_FLAG_Y_NHWC) != 0;
   MZ_REQUIRE(!((x_nhwc || y_nhwc) && (flags & MZ_FLAG_SKIP_FROM_BUFFER)),
@@ -618,7 +652,7 @@ static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, in
       return MZ_ERR_STATE;
     }
   }
-  const WsPlan wp = plan_ws(m, B, H, W);
+  const WsPlan wp = plan_ws(m, B, H, W, flags);
   if (workspace_bytes < wp.total) {
     set_error("upscale: workspace too small (%zu < %zu bytes)", workspace_bytes, wp.total);
     return MZ_ERR_WORKSPACE;
@@ -634,6 +668,16 @@ static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, in
   float* film = reinterpret_cast<float*>(ws + wp.film);
   const bool simt = (flags & MZ_FLAG_SIMT_CONV) != 0;
   int rc;
+  if (yuv) {  // decode, the 16-bit planar upscale, encode (the intermediates follow its workspace)
+    uint16_t* lr = reinterpret_cast<uint16_t*>(ws + wp.rgb_lr);
+    uint16_t* hr = reinterpret_cast<uint16_t*>(ws + wp.rgb_hr);
+    rc = launch_yuv420_to_rgb16(x_dev_v, lr, B, H, W, flags, s);
+    if (rc != MZ_OK) return rc;
+    const uint32_t f16 = (flags & ~(MZ_FLAG_YUV420 | kYuvColourFlags | MZ_FLAG_IO_U8)) | MZ_FLAG_IO_U16;
+    rc = upscale_impl(m, lr, c_dev, c_rows, hr, B, H, W, workspace_dev, wp.rgb_lr, f16, stream, nullptr);
+    if (rc != MZ_OK) return rc;
+    return launch_rgb16_to_yuv420(hr, y_dev_v, B, H * m->r, W * m->r, flags, s);
+  }
 
   if (front && m->F > 0) {
     rc = launch_film(c_dev, c_rows, m->ctrl_w, m->ctrl_b, film, m->L, B, m->F, m->hC, m->hCp, m->ns, s);
@@ -801,6 +845,7 @@ int mz_upscale_window(mz_model* m, const void* x_dev, const float* c_dev, int32_
              "upscale_window: pitches (%lld, %lld) are smaller than the window", static_cast<long long>(y_row_pitch),
              static_cast<long long>(y_plane_pitch));
   MZ_REQUIRE(!(flags & MZ_FLAG_SKIP_FROM_BUFFER), "upscale_window: the bicubic skip is recomputed (no MZ_FLAG_SKIP_FROM_BUFFER)");
+  MZ_REQUIRE(!(flags & MZ_FLAG_YUV420), "upscale_window: 4:2:0 frames (MZ_FLAG_YUV420) cannot be windowed");
   // bytes of one vector store: the same in both layouts (an interleaved HR row segment of a pixel is three of them)
   const int es = (flags & MZ_FLAG_IO_U8) ? 1 : ((flags & MZ_FLAG_IO_U16) ? 2 : 4), vec = m->r == 3 ? es : es * m->r;
   MZ_REQUIRE(reinterpret_cast<uintptr_t>(y_dev) % vec == 0 && (y_row_pitch * es) % vec == 0 && (y_plane_pitch * es) % vec == 0,
@@ -815,6 +860,7 @@ int mz_upscale_stage(mz_model* m, const void* x_dev, const float* c_dev, int32_t
                      int32_t layer_begin, int32_t layer_end) {
   MZ_REQUIRE(m, "upscale_stage: null model");
   MZ_REQUIRE(!(flags & MZ_FLAG_SKIP_FROM_BUFFER), "upscale_stage: the bicubic skip is recomputed (no MZ_FLAG_SKIP_FROM_BUFFER)");
+  MZ_REQUIRE(!(flags & MZ_FLAG_YUV420), "upscale_stage: 4:2:0 frames (MZ_FLAG_YUV420) cannot be staged");
   if (win_y1 <= 0)  // dense output
     return upscale_impl(m, x_dev, c_dev, c_rows, y_dev, B, H, W, workspace_dev, workspace_bytes, flags, stream, nullptr,
                         layer_begin, layer_end);
@@ -842,11 +888,11 @@ int mz_workspace_layout(const mz_model* m, int32_t B, int32_t H, int32_t W, size
 static int host_enqueue(mz_model* m, int li, const void* x_host, const float* c_host, int32_t c_rows, void* y_host,
                         int32_t B, int32_t H, int32_t W, uint32_t flags) {
   mz_model::HostLane& L = m->lane[li];
-  const size_t xb = image_elem_bytes(flags) * 3 * B * H * W;
+  const size_t xb = image_bytes(flags, H, W) * B;
   const size_t yb = xb * m->r * m->r;
   const size_t cb = c_host ? sizeof(float) * c_rows * (m->F > 0 ? m->F : 1) : 0;
   size_t wsb = 0;
-  int rc = mz_workspace_bytes(m, B, H, W, &wsb);
+  int rc = mz_workspace_bytes_flags(m, B, H, W, flags, &wsb);
   if (rc != MZ_OK) return rc;
   auto ensure = [&](void** p, size_t* have, size_t need) -> int {
     if (*have >= need) return MZ_OK;
@@ -886,7 +932,7 @@ int mz_upscale_host_async(mz_model* m, int32_t lane, const void* x_host, const f
   MZ_REQUIRE(m && x_host && y_host, "upscale_host_async: null pointer");
   MZ_REQUIRE(lane == 0 || lane == 1, "upscale_host_async: lane must be 0 or 1, %d given", lane);
   MZ_REQUIRE(B > 0 && H > 0 && W > 0, "upscale_host_async: empty input (B %d, H %d, W %d)", B, H, W);
-  const int frc = check_image_flags(flags);  // (before the copies are enqueued)
+  const int frc = check_image_flags(flags, H, W);  // (before the copies are enqueued)
   if (frc != MZ_OK) return frc;
   DeviceGuard g(m->cfg.device);
   return host_enqueue(m, lane, x_host, c_host, c_rows, y_host, B, H, W, flags);
@@ -903,12 +949,11 @@ int mz_upscale_host_wait(mz_model* m, int32_t lane) {
 
 int mz_upscale_host(mz_model* m, const void* x_host_v, const float* c_host, int32_t c_rows, void* y_host_v, int32_t B,
                     int32_t H, int32_t W, uint32_t flags) {
-  const size_t esz = image_elem_bytes(flags);
   const uint8_t* x_host = static_cast<const uint8_t*>(x_host_v);
   uint8_t* y_host = static_cast<uint8_t*>(y_host_v);
   MZ_REQUIRE(m && x_host && y_host, "upscale_host: null pointer");
   MZ_REQUIRE(B > 0 && H > 0 && W > 0, "upscale_host: empty input (B %d, H %d, W %d)", B, H, W);
-  const int frc = check_image_flags(flags);  // (before the copies are enqueued)
+  const int frc = check_image_flags(flags, H, W);  // (before the copies are enqueued)
   if (frc != MZ_OK) return frc;
   if (m->F > 0) {
     MZ_REQUIRE(c_host != nullptr, "Control vector c is required for control models.");
@@ -918,7 +963,7 @@ int mz_upscale_host(mz_model* m, const void* x_host_v, const float* c_host, int3
   // A batch is cut into up to eight chunks that alternate between the two lanes: copies of chunk i+1 / i-1 run under
   // the kernels of chunk i.  (Images are independent: chunking does not change any result.)
   const int n_chunks = B >= 8 ? 8 : B;
-  const size_t x_img = static_cast<size_t>(3) * H * W * esz, y_img = x_img * m->r * m->r;  // bytes per image
+  const size_t x_img = image_bytes(flags, H, W), y_img = x_img * m->r * m->r;  // bytes per image
   const int F = m->F > 0 ? m->F : 1;
   int b0 = 0, rc = MZ_OK;
   for (int i = 0; i < n_chunks && rc == MZ_OK; ++i) {

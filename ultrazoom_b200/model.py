@@ -9,6 +9,7 @@ stream.  There is no CPU / eager fallback: a non-CUDA input or a missing native 
 from __future__ import annotations
 
 import ctypes as C
+from dataclasses import dataclass
 from typing import Optional
 
 import torch
@@ -41,6 +42,47 @@ def _input_image(x: Tensor, integer: bool):
     x = x.detach() if integer else x.detach().to(torch.float32)
     x = x.contiguous(memory_format=torch.channels_last if nhwc else torch.contiguous_format)
     return x, (_native.FLAG_X_NHWC if nhwc else 0)
+
+
+_YUV_MATRIX_FLAGS = {"bt709": 0, "bt601": _native.FLAG_YUV_BT601, "bt2020": _native.FLAG_YUV_BT2020}
+
+
+@dataclass(frozen=True)
+class Yuv420:
+    """4:2:0 video frames in and out of ``upscale`` (``yuv=Yuv420()``): NV12 as uint8, P010 as uint16 -- what NVDEC and
+    ``ffmpeg -hwaccel cuda`` decode to and NVENC encodes from.  A batch is a ``(B, 3H/2, W)`` tensor: per frame the H x W
+    luma plane, then H/2 rows of W/2 interleaved Cb,Cr pairs (no row pitch beyond W; H and W even).  P010 words hold
+    the 10-bit code in their top bits.
+
+    ``matrix``: "bt709" (default), "bt601" or "bt2020" (non-constant luminance); ``full_range``: full instead of limited
+    (studio) range.  Chroma siting is the H.264 / HEVC default.  The frame is converted to 16-bit RGB on the GPU, upscaled
+    exactly as a uint16 image is, and converted back (``ops.yuv420_to_rgb16`` / ``ops.rgb16_to_yuv420``; the filters
+    and rounding are stated at ``mz_yuv420_to_rgb16`` in include/mewzoom_b200.h)."""
+
+    matrix: str = "bt709"
+    full_range: bool = False
+
+    def __post_init__(self):
+        assert self.matrix in _YUV_MATRIX_FLAGS, f"matrix must be one of {sorted(_YUV_MATRIX_FLAGS)}, got {self.matrix!r}"
+
+    def flags(self, dtype: torch.dtype) -> int:
+        """The C ABI's flag bits for frames of ``dtype`` (uint8: NV12, uint16: P010)."""
+        assert dtype in _INT_IMAGE_DTYPES, f"4:2:0 frames are uint8 (NV12) or uint16 (P010), got {dtype}"
+        return (_native.FLAG_YUV420 | _YUV_MATRIX_FLAGS[self.matrix] | (_native.FLAG_YUV_FULL_RANGE if self.full_range else 0)
+                | (_native.FLAG_IO_U8 if dtype == torch.uint8 else _native.FLAG_IO_U16))
+
+
+def _yuv_dims(x: Tensor):
+    """``(B, H, W)`` of a batch of 4:2:0 frames ``(B, 3H/2, W)``."""
+    assert x.dim() == 3 and x.dtype in _INT_IMAGE_DTYPES, (
+        f"Expected 4:2:0 frames (B, 3H/2, W) of uint8 (NV12) or uint16 (P010), got {tuple(x.shape)} {x.dtype}.")
+    assert x.shape[0] > 0 and x.shape[1] > 0 and x.shape[2] > 0, "Input must not be empty."
+    assert x.shape[1] % 3 == 0, f"A 4:2:0 frame has 3H/2 rows for an even H, got {x.shape[1]}."
+    return x.shape[0], x.shape[1] // 3 * 2, x.shape[2]
+
+
+def _no_yuv(yuv, what: str) -> None:
+    assert yuv is None, f"4:2:0 frames are supported by upscale(), upscale_host() and capture(), not {what}()"
 
 
 def _output_flag(memory_format) -> int:
@@ -187,9 +229,9 @@ class _Engine:
         _native.check(self.lib.mz_model_saturated(self.handle, 1 if reset else 0, C.byref(flag)))
         return bool(flag.value)
 
-    def workspace(self, B: int, H: int, W: int, stream: "torch.cuda.Stream") -> Tensor:
+    def workspace(self, B: int, H: int, W: int, stream: "torch.cuda.Stream", flags: int = 0) -> Tensor:
         need = C.c_size_t()
-        _native.check(self.lib.mz_workspace_bytes(self.handle, B, H, W, C.byref(need)))
+        _native.check(self.lib.mz_workspace_bytes_flags(self.handle, B, H, W, flags, C.byref(need)))
         if self.ws is None or self.ws.numel() < need.value:
             self.ws = None     # (kernels still using the old buffer were recorded on it with record_stream)
             self.ws = torch.empty(need.value + 1024, dtype=torch.uint8, device=self.device)
@@ -430,9 +472,12 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
             return _native.FLAG_IO_U8 | (_native.FLAG_U8_TRUNC if self.u8_truncate else 0)
         return _native.FLAG_IO_U16 if dtype == torch.uint16 else 0
 
-    def _check_inputs(self, x: Tensor, c: Optional[Tensor]) -> Optional[Tensor]:
-        assert x.dim() == 4 and x.shape[1] == 3, f"Expected input of shape (B, 3, H, W), got {tuple(x.shape)}."
-        assert x.shape[0] > 0 and x.shape[2] > 0 and x.shape[3] > 0, "Input must not be empty."
+    def _check_inputs(self, x: Tensor, c: Optional[Tensor], yuv: Optional[Yuv420] = None) -> Optional[Tensor]:
+        if yuv is not None:
+            _yuv_dims(x)
+        else:
+            assert x.dim() == 4 and x.shape[1] == 3, f"Expected input of shape (B, 3, H, W), got {tuple(x.shape)}."
+            assert x.shape[0] > 0 and x.shape[2] > 0 and x.shape[3] > 0, "Input must not be empty."
         if self.control_features == 0:
             assert c is None, "This model has no control modules; c must be None."
             return None
@@ -445,23 +490,31 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         return c
 
     def _run(self, x: Tensor, c: Optional[Tensor], flags: int, ws: Optional[Tensor] = None,
-             memory_format=torch.contiguous_format) -> Tensor:
-        c = self._check_inputs(x, c)
+             memory_format=torch.contiguous_format, yuv: Optional[Yuv420] = None) -> Tensor:
+        c = self._check_inputs(x, c, yuv)
         if not x.is_cuda:
             raise RuntimeError("ultrazoom_b200.MewZoom runs on sm_100a CUDA kernels only; move the input to a "
                                "B200 (`x.cuda()`). There is no CPU fallback.")
         dev = x.device
         odt = x.dtype if x.dtype in _INT_IMAGE_DTYPES else torch.float32   # 8 / 16-bit images in and out: see upscale()
-        if odt != torch.float32:
-            assert flags & _native.FLAG_CLAMP01, (
-                f"{str(odt).replace('torch.', '')} images are supported by upscale(), not forward()")
-            flags |= self._image_flags(odt)
-        x, xflag = _input_image(x, odt != torch.float32)
-        flags |= xflag | _output_flag(memory_format)
+        r = self.upscale_ratio
+        if yuv is not None:
+            assert memory_format == torch.contiguous_format, "4:2:0 frames have one layout (no memory_format)"
+            B, H, W = _yuv_dims(x)
+            flags |= yuv.flags(odt)
+            x = x.detach().contiguous()
+            out_shape = (B, H * r * 3 // 2, W * r)
+        else:
+            if odt != torch.float32:
+                assert flags & _native.FLAG_CLAMP01, (
+                    f"{str(odt).replace('torch.', '')} images are supported by upscale(), not forward()")
+                flags |= self._image_flags(odt)
+            x, xflag = _input_image(x, odt != torch.float32)
+            flags |= xflag | _output_flag(memory_format)
+            B, _, H, W = x.shape
+            out_shape = (B, 3, H * r, W * r)
         if c is not None:
             c = c.detach().to(device=dev, dtype=torch.float32).contiguous()
-        B, _, H, W = x.shape
-        r = self.upscale_ratio
         capturing = torch.cuda.is_current_stream_capturing()
         auto = self.operand_dtype == "auto" and not capturing
         while True:
@@ -470,10 +523,10 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
                 torch.cuda.synchronize(dev)    # (the flag of an earlier asynchronous call is not this call's to absorb)
             if not capturing:
                 self._range_guard(eng)
-            y = torch.empty((B, 3, H * r, W * r), dtype=odt, device=dev, memory_format=memory_format)
+            y = torch.empty(out_shape, dtype=odt, device=dev, memory_format=memory_format)
             stream = torch.cuda.current_stream(dev)
             eng.begin(stream)
-            w = ws if ws is not None else eng.workspace(B, H, W, stream)
+            w = ws if ws is not None else eng.workspace(B, H, W, stream, flags)
             ws_ptr = (w.data_ptr() + 1023) // 1024 * 1024
             ws_bytes = w.numel() - (ws_ptr - w.data_ptr())
             _native.check(eng.lib.mz_upscale(
@@ -488,12 +541,15 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
             return y
 
     # ---- reference model.py:149-179 ----
-    def forward(self, x: Tensor, c: Optional[Tensor] = None, *, memory_format=torch.contiguous_format) -> Tensor:
+    def forward(self, x: Tensor, c: Optional[Tensor] = None, *, memory_format=torch.contiguous_format,
+                yuv: Optional[Yuv420] = None) -> Tensor:
         """bicubic(x) + residual network, un-clamped (reference model.py:149-164).  See ``upscale`` for the layouts."""
+        _no_yuv(yuv, "forward")
         return self._run(x, c, 0, memory_format=memory_format)
 
     @torch.inference_mode()
-    def upscale(self, x: Tensor, c: Optional[Tensor] = None, *, memory_format=torch.contiguous_format) -> Tensor:
+    def upscale(self, x: Tensor, c: Optional[Tensor] = None, *, memory_format=torch.contiguous_format,
+                yuv: Optional[Yuv420] = None) -> Tensor:
         """``clamp(forward(x, c), 0, 1)`` (reference model.py:166-179); the clamp is fused in the head kernel.
 
         A ``torch.uint8`` image (what ``decode_image`` returns, reference test_compare.py:53) is read as ``x / 255``
@@ -508,8 +564,12 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         contiguous), e.g. ``torch.from_numpy(hwc_frames).permute(0, 3, 1, 2)``, is read as it is, and
         ``memory_format=torch.channels_last`` returns ``y`` in channels-last strides, so ``y.permute(0, 2, 3, 1)`` is a
         contiguous (B,rH,rW,3) array.  The default output is contiguous NCHW whatever the input's layout.  The results
-        are bit-identical in every layout."""
-        return self._run(x, c, _native.FLAG_CLAMP01, memory_format=memory_format)
+        are bit-identical in every layout.
+
+        ``yuv=Yuv420(...)``: ``x`` is a batch of 4:2:0 video frames ``(B, 3H/2, W)``, uint8 NV12 or uint16 P010, and so is
+        the result, ``(B, 3rH/2, rW)``.  It equals ``ops.rgb16_to_yuv420(upscale(ops.yuv420_to_rgb16(x)))`` bit for bit:
+        the frame is upscaled as a 16-bit RGB image, whatever its depth."""
+        return self._run(x, c, _native.FLAG_CLAMP01, memory_format=memory_format, yuv=yuv)
 
     @torch.inference_mode()
     def test_compare(self, x: Tensor, c: Optional[Tensor] = None):
@@ -522,12 +582,15 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
                                                self.upscale_ratio).clamp_(0, 1)
 
     @torch.inference_mode()
-    def upscale_into(self, x: Tensor, c: Optional[Tensor], frame: Tensor, window: tuple, at: tuple) -> None:
+    def upscale_into(self, x: Tensor, c: Optional[Tensor], frame: Tensor, window: tuple, at: tuple, *,
+                     yuv: Optional[Yuv420] = None) -> None:
         """Halo-tiled inference without a tile output: ``upscale`` the LR tile ``x`` and write only its core -- the LR
         pixels ``window = (y0, y1, x0, x1)`` of the tile -- straight into ``frame`` (B,3,rH',rW'), whose HR pixel
         ``at = (fy, fx)`` receives the core's first pixel (mz_upscale_window).  ``frame`` may live on another GPU
         (``sharding.share_frame``): the head kernel's stores are then the transfer over NVLink.  ``frame`` is planar or
-        interleaved (channels-last strides, any row and image pitch, e.g. a view into a wider HWC buffer)."""
+        interleaved (channels-last strides, any row and image pitch, e.g. a view into a wider HWC buffer).  4:2:0 frames
+        cannot be windowed."""
+        _no_yuv(yuv, "upscale_into")
         c = self._check_inputs(x, c)
         if not x.is_cuda:
             raise RuntimeError("ultrazoom_b200.MewZoom runs on sm_100a CUDA kernels only (no CPU fallback).")
@@ -572,12 +635,13 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
 
     @torch.inference_mode()
     def upscale_stage(self, x: Tensor, c: Optional[Tensor], frame: Tensor, window: tuple, at: tuple, layer_begin: int,
-                      layer_end: int, ws: Tensor) -> None:
+                      layer_end: int, ws: Tensor, *, yuv: Optional[Yuv420] = None) -> None:
         """``upscale_into`` cut into stages along the depth of the network (mz_upscale_stage): run the encoder blocks
         ``[layer_begin, layer_end)`` on the state kept in the caller's workspace ``ws`` (``stage_workspace``); the stem
         runs first when ``layer_begin == 0``, the head -- storing the window into ``frame`` -- last when ``layer_end ==
         num_encoder_layers``.  Between stages ``sharding.upscale_tiled_refresh`` overwrites the tile's halo with the
-        neighbours' values (``stage_views``)."""
+        neighbours' values (``stage_views``).  4:2:0 frames cannot be staged."""
+        _no_yuv(yuv, "upscale_stage")
         c = self._check_inputs(x, c)
         assert x.is_cuda and x.dtype in (torch.float32, torch.uint8, torch.uint16), (
             "upscale_stage takes a CUDA image (float32, uint8 or uint16)")
@@ -632,18 +696,21 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         return zf, z16
 
     def capture(self, x: Tensor, c: Optional[Tensor] = None, clamp: bool = True, *,
-                memory_format=torch.contiguous_format) -> "GraphedUpscale":
+                memory_format=torch.contiguous_format, yuv: Optional[Yuv420] = None) -> "GraphedUpscale":
         """Record one ``upscale`` (``clamp=False``: ``forward``) call at the shape of ``x`` into a CUDA graph.
 
         A frame of a few hundred pixels a side is launch-bound (2L + 3 kernels, most of them cluster launches of
         15-20 us of host time each); replaying the recorded graph removes the host from that loop.  The dependent-launch
         edges between the kernels are kept by the capture.  The graph reads its input in the layout of ``x`` and writes
-        its output in ``memory_format`` (see ``upscale``).  See ``GraphedUpscale``."""
-        return GraphedUpscale(self, x, c, _native.FLAG_CLAMP01 if clamp else 0, memory_format)
+        its output in ``memory_format`` (see ``upscale``), or 4:2:0 frames in and out with ``yuv``.  See
+        ``GraphedUpscale``."""
+        assert yuv is None or clamp, "4:2:0 frames are supported by upscale(), not forward()"
+        return GraphedUpscale(self, x, c, _native.FLAG_CLAMP01 if clamp else 0, memory_format, yuv)
 
     @torch.inference_mode()
     def upscale_host(self, x: Tensor, c: Optional[Tensor] = None, out: Optional[Tensor] = None,
-                     device: int = 0, lane: Optional[int] = None, *, memory_format=torch.contiguous_format) -> Tensor:
+                     device: int = 0, lane: Optional[int] = None, *, memory_format=torch.contiguous_format,
+                     yuv: Optional[Yuv420] = None) -> Tensor:
         """End-to-end call with HOST tensors: H2D copy, kernels, D2H copy (mz_upscale_host).
 
         ``lane=None``: synchronous; a batch is cut into chunks whose copies overlap the kernels of their neighbours.
@@ -655,8 +722,9 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         Element types and layouts as in ``upscale`` (uint8 and uint16 frames come back as such): a channels-last ``x`` is
         copied as it is (no transpose on the CPU), and the result is interleaved with
         ``memory_format=torch.channels_last``.  A caller's ``out`` sets the output layout itself: it must be contiguous
-        NCHW or contiguous channels-last, of the input's element type."""
-        c = self._check_inputs(x, c)
+        NCHW or contiguous channels-last, of the input's element type.  With ``yuv``, ``x`` and ``out`` are 4:2:0 frames
+        as in ``upscale`` (contiguous), at 1.5 (NV12) or 3 (P010) bytes per pixel over PCIe."""
+        c = self._check_inputs(x, c, yuv)
         assert not x.is_cuda, "upscale_host takes host tensors"
         assert lane in (None, 0, 1), "lane must be None, 0 or 1"
         eng = self._engine(torch.device("cuda", device))
@@ -664,24 +732,35 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
             torch.cuda.synchronize(torch.device("cuda", device))   # (as in upscale; lanes included)
         self._range_guard(eng)
         odt = x.dtype if x.dtype in _INT_IMAGE_DTYPES else torch.float32
-        x, xflag = _input_image(x, odt != torch.float32)
         if c is not None:
             c = c.to(device="cpu", dtype=torch.float32).contiguous()
-        B, _, H, W = x.shape
         r = self.upscale_ratio
-        if out is None:
-            out = torch.empty((B, 3, H * r, W * r), dtype=odt, memory_format=memory_format)
-            yflag = _output_flag(memory_format)
+        if yuv is not None:
+            assert memory_format == torch.contiguous_format, "4:2:0 frames have one layout (no memory_format)"
+            B, H, W = _yuv_dims(x)
+            x = x.contiguous()
+            out_shape = (B, H * r * 3 // 2, W * r)
+            if out is None:
+                out = torch.empty(out_shape, dtype=odt)
+            assert out.is_contiguous(), "out must be contiguous"
+            flags = _native.FLAG_CLAMP01 | self._flags_extra | yuv.flags(odt)
         else:
-            yflag = _native.FLAG_Y_NHWC if _is_nhwc(out) else 0
-            assert out.is_contiguous() or yflag, "out must be contiguous NCHW or contiguous channels-last"
-        assert tuple(out.shape) == (B, 3, H * r, W * r) and out.dtype == odt
-        flags = _native.FLAG_CLAMP01 | self._flags_extra | xflag | yflag | self._image_flags(odt)
+            x, xflag = _input_image(x, odt != torch.float32)
+            B, _, H, W = x.shape
+            out_shape = (B, 3, H * r, W * r)
+            if out is None:
+                out = torch.empty(out_shape, dtype=odt, memory_format=memory_format)
+                yflag = _output_flag(memory_format)
+            else:
+                yflag = _native.FLAG_Y_NHWC if _is_nhwc(out) else 0
+                assert out.is_contiguous() or yflag, "out must be contiguous NCHW or contiguous channels-last"
+            flags = _native.FLAG_CLAMP01 | self._flags_extra | xflag | yflag | self._image_flags(odt)
+        assert tuple(out.shape) == out_shape and out.dtype == odt
         cp, cr = (c.data_ptr(), c.shape[0]) if c is not None else (None, 0)
         if lane is None:
             _native.check(eng.lib.mz_upscale_host(eng.handle, x.data_ptr(), cp, cr, out.data_ptr(), B, H, W, flags))
             if not self._range_guard(eng, rerun=True):     # (the call has synchronised: "auto" repeats it with bf16)
-                return self.upscale_host(x, c, out, device)
+                return self.upscale_host(x, c, out, device, yuv=yuv)
         else:
             # keep the (possibly converted) inputs alive until the wait, and the engine whose lane runs the frame
             self._host_keep[(device, lane)] = (eng, x, c, out)
@@ -716,13 +795,13 @@ class GraphedUpscale:
     capture are picked up by the next ordinary call (which re-packs them), not by a replay on its own."""
 
     def __init__(self, model: MewZoom, x: Tensor, c: Optional[Tensor], flags: int,
-                 memory_format=torch.contiguous_format):
-        c = model._check_inputs(x, c)
+                 memory_format=torch.contiguous_format, yuv: Optional[Yuv420] = None):
+        c = model._check_inputs(x, c, yuv)
         if not x.is_cuda:
             raise RuntimeError("MewZoom.capture needs a CUDA input (there is no CPU fallback).")
         self.model = model
         # (the input buffer keeps the layout of x: the graph reads it as _run reads x; a replay copies either layout in)
-        self.x = _input_image(x, x.dtype in _INT_IMAGE_DTYPES)[0].clone()
+        self.x = (x.detach().contiguous() if yuv is not None else _input_image(x, x.dtype in _INT_IMAGE_DTYPES)[0]).clone()
         self.c = None if c is None else c.detach().to(device=x.device, dtype=torch.float32).contiguous().clone()
         # The graph bakes in raw pointers: it owns everything they point at -- its input / output tensors, a PRIVATE
         # workspace (the engine's cached one is dropped and re-allocated when a later call needs a larger one) and the
@@ -730,21 +809,22 @@ class GraphedUpscale:
         # switched to bfloat16.
         eng = model._engine(x.device)
         need = C.c_size_t()
-        B, _, H, W = self.x.shape
-        _native.check(eng.lib.mz_workspace_bytes(eng.handle, B, H, W, C.byref(need)))
+        B, H, W = _yuv_dims(self.x) if yuv is not None else (self.x.shape[0], self.x.shape[2], self.x.shape[3])
+        wflags = yuv.flags(self.x.dtype) if yuv is not None else 0
+        _native.check(eng.lib.mz_workspace_bytes_flags(eng.handle, B, H, W, wflags, C.byref(need)))
         self.ws = torch.empty(need.value + 1024, dtype=torch.uint8, device=x.device)
         with torch.inference_mode():
             side = torch.cuda.Stream(device=x.device)
             side.wait_stream(torch.cuda.current_stream(x.device))
             with torch.cuda.stream(side):        # warm-up: packs the weights, prepares the launches
-                model._run(self.x, self.c, flags, ws=self.ws, memory_format=memory_format)
+                model._run(self.x, self.c, flags, ws=self.ws, memory_format=memory_format, yuv=yuv)
             side.synchronize()
             self.engine = model._engine(x.device)
             model._range_guard(self.engine)      # a checkpoint that saturates is not recorded
             torch.cuda.current_stream(x.device).wait_stream(side)
             self.graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(self.graph):
-                self.y = model._run(self.x, self.c, flags, ws=self.ws, memory_format=memory_format)
+                self.y = model._run(self.x, self.c, flags, ws=self.ws, memory_format=memory_format, yuv=yuv)
 
     def replay(self) -> Tensor:
         """Replay as it is: the 3-5 us path, so it does not consult the fp16 range flag.  A clipped replay is reported

@@ -40,6 +40,37 @@ def bicubic(x: Tensor, r: int) -> Tensor:
     return y
 
 
+def yuv420_to_rgb16(x: Tensor, yuv: Optional["Yuv420"] = None) -> Tensor:
+    """4:2:0 frames (B, 3H/2, W) -- uint8 NV12 or uint16 P010 -- to 16-bit planar RGB (B, 3, H, W) (mz_yuv420_to_rgb16);
+    ``yuv`` (default ``Yuv420()``) names the colour matrix and range."""
+    from .model import Yuv420, _yuv_dims
+
+    _need_cuda(x)
+    B, H, W = _yuv_dims(x)
+    flags = (yuv or Yuv420()).flags(x.dtype)
+    x = x.contiguous()
+    y = torch.empty((B, 3, H, W), dtype=torch.uint16, device=x.device)
+    with torch.cuda.device(x.device):
+        _native.check(_native.load().mz_yuv420_to_rgb16(x.data_ptr(), y.data_ptr(), B, H, W, flags, _stream(x)))
+    return y
+
+
+def rgb16_to_yuv420(rgb: Tensor, dtype: torch.dtype = torch.uint8, yuv: Optional["Yuv420"] = None) -> Tensor:
+    """16-bit planar RGB (B, 3, H, W) to 4:2:0 frames (B, 3H/2, W) of ``dtype``: uint8 NV12 or uint16 P010
+    (mz_rgb16_to_yuv420)."""
+    from .model import Yuv420
+
+    _need_cuda(rgb)
+    assert rgb.dim() == 4 and rgb.shape[1] == 3 and rgb.dtype == torch.uint16, "Expected a uint16 image (B, 3, H, W)."
+    B, _, H, W = rgb.shape
+    flags = (yuv or Yuv420()).flags(dtype)
+    rgb = rgb.contiguous()
+    y = torch.empty((B, H * 3 // 2, W), dtype=dtype, device=rgb.device)
+    with torch.cuda.device(rgb.device):
+        _native.check(_native.load().mz_rgb16_to_yuv420(rgb.data_ptr(), y.data_ptr(), B, H, W, flags, _stream(rgb)))
+    return y
+
+
 def pack_conv_weight(w: Tensor, device: torch.device, cout_p: Optional[int] = None,
                      cin_p: Optional[int] = None, dtype: torch.dtype = torch.float16) -> Tensor:
     """OIHW fp32 -> device fp16|bf16 [9][cout_p][cin_p]."""
