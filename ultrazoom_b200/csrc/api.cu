@@ -78,8 +78,8 @@ int mz_stem_pack(const float* x_dev, const float* w_dev, const float* bias_dev, 
                  int32_t H, int32_t W, int32_t Cp, int32_t zb_pitch, int32_t operand_dtype, void* stream) {
   MZ_REQUIRE(x_dev && w_dev && bias_dev && zf_dev && zb_dev, "stem: null pointer");
   MZ_REQUIRE(dtype_ok(operand_dtype), "operand_dtype must be MZ_DTYPE_F16 or MZ_DTYPE_BF16, %d given", operand_dtype);
-  return launch_stem(x_dev, nullptr, w_dev, bias_dev, zf_dev, static_cast<uint16_t*>(zb_dev), operand_dtype, B, H, W, Cp, zb_pitch,
-                     static_cast<cudaStream_t>(stream));
+  return launch_stem(x_dev, kImgF32, 0, w_dev, bias_dev, zf_dev, static_cast<uint16_t*>(zb_dev), operand_dtype, B, H, W, Cp,
+                     zb_pitch, static_cast<cudaStream_t>(stream));
 }
 
 int mz_conv3x3(const void* in_dev, const void* wpacked_dev, int32_t mode, const float* film_dev, void* out_bf16_dev,
@@ -135,11 +135,12 @@ int mz_head_shuffle_add(const void* zb_dev, const void* wpacked_dev, const float
   a.epi.H = H;
   a.epi.W = W;
   a.epi.n_pad = mz_padded_channels(3 * r * r);
-  a.epi.x = x_dev;
-  a.epi.y = y_dev;
+  a.epi.img.x = x_dev;
+  a.epi.img.y = y_dev;
+  a.epi.img.type = kImgF32;
+  a.epi.img.skip_mode = skip_mode;
+  a.epi.img.clamp01 = clamp01;
   a.epi.r = r;
-  a.epi.skip_mode = skip_mode;
-  a.epi.clamp01 = clamp01;
   make_bicubic_table(r, &a.epi.bt);
   if (use_tc) return launch_conv_tc(a, to_tune(tune), current_device(), static_cast<cudaStream_t>(stream));
   return launch_conv_simt(a, static_cast<cudaStream_t>(stream));

@@ -107,8 +107,8 @@ __host__ __device__ inline SmemPlan plan_smem(const TcParams& p) {
 // instead of 3R: the 128 x 16 activation tile -- 4 KB of shared-memory operand fetch per UMMA, what bounds the small-N
 // shapes -- is fetched once per input row instead of once per (output row, tap).  Every UMMA accumulates; the epilogue
 // zeroes each accumulator column group right after reading it.
-// LAY (head only): bit 0 interleaved input image, bit 1 interleaved output image (EpiParams::x_nhwc / y_nhwc), bit 2
-// 16-bit images (EpiParams::x16 / y16).
+// LAY (head only): bit 0 interleaved input image, bit 1 interleaved output image (ImageIo::x_nhwc / y_nhwc), bit 2
+// 16-bit images (ImageIo::type kImgU16).
 template <int MODE, int KT, int ROWS, int VAR, int LAY = 0>
 __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_constant__ TcParams p) {
   constexpr bool PAIR = VAR == 1, FUSE = VAR == 2;
@@ -1155,22 +1155,15 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
 // host side
 // ----------------------------------------------------------------------------------------------
 // ---- kernel lookup -------------------------------------------------------------------------------------------------
-// One lookup function per epilogue mode, so that the build can compile the instantiations of each mode in its own
-// translation unit: build.py compiles this file four times, with -DMZ_TC_PART=<mode> for the kernels of modes 0..2 and
-// -DMZ_TC_PART=4 for the host side, the heads for interleaved images (LAY 1..3) with -DMZ_TC_PART=5..7 and those for
-// 16-bit images (LAY 4..7) with -DMZ_TC_PART=8..11.  Without the define (a plain `nvcc -c conv_tc.cu`) everything lands
-// in one object.
+// One lookup function per epilogue mode and head layout, so that the build can compile the instantiations of each in
+// its own translation unit: build.py compiles this file with -DMZ_TC_PART=<mode> for the kernels of modes 0 and 1,
+// -DMZ_TC_PART=4 for the host side, -DMZ_TC_PART=2 for the planar head (LAY 0) and -DMZ_TC_PART=5..11 for the heads of
+// LAY 1..7.  Without the define (a plain `nvcc -c conv_tc.cu`) everything lands in one object.
 //   var 0: one CTA per patch, 1: CTA pair (cta_group::2), 2: fused rows.  Returns nullptr for a shape that has no kernel.
 const void* tc_kernel_mode0(int ks, int rows, int var);
 const void* tc_kernel_mode1(int ks, int rows, int var);
-const void* tc_kernel_mode2(int ks, int rows, int var);
-const void* tc_kernel_mode2_lay1(int ks, int rows, int var);
-const void* tc_kernel_mode2_lay2(int ks, int rows, int var);
-const void* tc_kernel_mode2_lay3(int ks, int rows, int var);
-const void* tc_kernel_mode2_lay4(int ks, int rows, int var);
-const void* tc_kernel_mode2_lay5(int ks, int rows, int var);
-const void* tc_kernel_mode2_lay6(int ks, int rows, int var);
-const void* tc_kernel_mode2_lay7(int ks, int rows, int var);
+template <int LAY>  // the head for image layouts LAY
+const void* tc_kernel_head_lay(int ks, int rows, int var);
 
 template <int M, int K, int LAY = 0>
 static const void* tc_kernel_rows(int rows, int var) {
@@ -1207,29 +1200,14 @@ const void* tc_kernel_mode0(int ks, int rows, int var) { return tc_kernel_lookup
 #if !defined(MZ_TC_PART) || MZ_TC_PART == 1
 const void* tc_kernel_mode1(int ks, int rows, int var) { return tc_kernel_lookup<1>(ks, rows, var); }
 #endif
-#if !defined(MZ_TC_PART) || MZ_TC_PART == 2
-const void* tc_kernel_mode2(int ks, int rows, int var) { return tc_kernel_lookup<2>(ks, rows, var); }
+#if !defined(MZ_TC_PART) || MZ_TC_PART == 2 || MZ_TC_PART >= 5
+template <int LAY>
+const void* tc_kernel_head_lay(int ks, int rows, int var) { return tc_kernel_lookup<2, LAY>(ks, rows, var); }
 #endif
-#if !defined(MZ_TC_PART) || MZ_TC_PART == 5
-const void* tc_kernel_mode2_lay1(int ks, int rows, int var) { return tc_kernel_lookup<2, 1>(ks, rows, var); }
-#endif
-#if !defined(MZ_TC_PART) || MZ_TC_PART == 6
-const void* tc_kernel_mode2_lay2(int ks, int rows, int var) { return tc_kernel_lookup<2, 2>(ks, rows, var); }
-#endif
-#if !defined(MZ_TC_PART) || MZ_TC_PART == 7
-const void* tc_kernel_mode2_lay3(int ks, int rows, int var) { return tc_kernel_lookup<2, 3>(ks, rows, var); }
-#endif
-#if !defined(MZ_TC_PART) || MZ_TC_PART == 8
-const void* tc_kernel_mode2_lay4(int ks, int rows, int var) { return tc_kernel_lookup<2, 4>(ks, rows, var); }
-#endif
-#if !defined(MZ_TC_PART) || MZ_TC_PART == 9
-const void* tc_kernel_mode2_lay5(int ks, int rows, int var) { return tc_kernel_lookup<2, 5>(ks, rows, var); }
-#endif
-#if !defined(MZ_TC_PART) || MZ_TC_PART == 10
-const void* tc_kernel_mode2_lay6(int ks, int rows, int var) { return tc_kernel_lookup<2, 6>(ks, rows, var); }
-#endif
-#if !defined(MZ_TC_PART) || MZ_TC_PART == 11
-const void* tc_kernel_mode2_lay7(int ks, int rows, int var) { return tc_kernel_lookup<2, 7>(ks, rows, var); }
+#if defined(MZ_TC_PART) && MZ_TC_PART == 2
+template const void* tc_kernel_head_lay<0>(int ks, int rows, int var);
+#elif defined(MZ_TC_PART) && MZ_TC_PART >= 5
+template const void* tc_kernel_head_lay<MZ_TC_PART - 4>(int ks, int rows, int var);
 #endif
 
 #if !defined(MZ_TC_PART) || MZ_TC_PART == 4  // ---- host side ----------------------------------------------------------
@@ -1304,19 +1282,13 @@ struct ConvLaunchImpl {
 
 // the head kernel for image layouts `lay` (bit 0 interleaved input, bit 1 interleaved output, bit 2 16-bit images)
 static const void* tc_kernel_head(int lay, int ks, int rows, int var) {
-  switch (lay) {
-    case 0: return tc_kernel_mode2(ks, rows, var);
-    case 1: return tc_kernel_mode2_lay1(ks, rows, var);
-    case 2: return tc_kernel_mode2_lay2(ks, rows, var);
-    case 3: return tc_kernel_mode2_lay3(ks, rows, var);
-    case 4: return tc_kernel_mode2_lay4(ks, rows, var);
-    case 5: return tc_kernel_mode2_lay5(ks, rows, var);
-    case 6: return tc_kernel_mode2_lay6(ks, rows, var);
-    default: return tc_kernel_mode2_lay7(ks, rows, var);
-  }
+  static const void* (*const heads[8])(int, int, int) = {tc_kernel_head_lay<0>, tc_kernel_head_lay<1>, tc_kernel_head_lay<2>,
+                                                         tc_kernel_head_lay<3>, tc_kernel_head_lay<4>, tc_kernel_head_lay<5>,
+                                                         tc_kernel_head_lay<6>, tc_kernel_head_lay<7>};
+  return heads[lay](ks, rows, var);
 }
 static int head_layout(const EpiParams& e) {
-  return (e.x_nhwc ? 1 : 0) | (e.y_nhwc ? 2 : 0) | (e.y16 != nullptr ? 4 : 0);
+  return (e.img.x_nhwc ? 1 : 0) | (e.img.y_nhwc ? 2 : 0) | (e.img.type == kImgU16 ? 4 : 0);
 }
 static_assert(sizeof(ConvLaunchImpl) <= sizeof(ConvLaunch::storage), "ConvLaunch::storage too small");
 
@@ -1386,24 +1358,7 @@ int patch_conv_epi(ConvLaunch& launch, const EpiParams& e) {
     L.fn = fn;
     L.lay = lay;
   }
-  EpiParams& d = L.p.epi;
-  d.x = e.x;
-  d.y = e.y;
-  d.x8 = e.x8;
-  d.y8 = e.y8;
-  d.x16 = e.x16;
-  d.y16 = e.y16;
-  d.u8_trunc = e.u8_trunc;
-  d.skip_mode = e.skip_mode;
-  d.clamp01 = e.clamp01;
-  d.wy0 = e.wy0;
-  d.wy1 = e.wy1;
-  d.wx0 = e.wx0;
-  d.wx1 = e.wx1;
-  d.y_row = e.y_row;
-  d.y_plane = e.y_plane;
-  d.x_nhwc = e.x_nhwc;
-  d.y_nhwc = e.y_nhwc;
+  L.p.epi.img = e.img;
   return MZ_OK;
 }
 

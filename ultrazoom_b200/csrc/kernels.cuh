@@ -26,10 +26,37 @@ struct BicubicTable {
 void make_bicubic_table(int r, BicubicTable* t);
 
 // ----------------------------------------------------------------------------------------------
+// The call's two images, as the stem reads x and the head reads x and writes y.
+// ----------------------------------------------------------------------------------------------
+// Element type of both images.  8 bits (MZ_FLAG_IO_U8): x holds round(255 * x), read back as x / 255 (ToDtype(float32,
+// scale=True), reference test_compare.py:53-57); y = floor(255 * clamp(v, 0, 1) + 0.5) (torchvision save_image,
+// test_compare.py:89) or floor(255 * clamp(v, 0, 1)) with u8_trunc (ToPILImage, README.md:81).  16 bits
+// (MZ_FLAG_IO_U16): x is read as the IEEE quotient x / 65535; y = floor(65535 * clamp(v, 0, 1) + 0.5).
+enum ImageType : int { kImgF32 = 0, kImgU8 = 1, kImgU16 = 2 };
+struct ImageIo {
+  const void* x;  // LR image (B,3,H,W)
+  void* y;        // HR image (B,3,rH,rW)
+  int type;       // ImageType
+  // Interleaved images (MZ_FLAG_X_NHWC / MZ_FLAG_Y_NHWC): x is (B,H,W,3), y is (B,rH,rW,3) -- colour c of a pixel at
+  // pixel * 3 + c, images 3HW (3 rH rW) elements apart as in the planar layout.
+  int x_nhwc, y_nhwc;
+  int u8_trunc;
+  int skip_mode;  // 0 none, 1 y already holds the bicubic image (fp32 only), 2 recompute bicubic from x
+  int clamp01;
+  // Windowed output (mz_upscale_window; all zero = the whole image, densely): only LR pixels wy0 <= y < wy1,
+  // wx0 <= x < wx1 are stored, pixel (wy0, wx0) of plane 0 of image 0 at y itself, HR rows y_row elements and colour
+  // planes y_plane elements apart -- a tile's core written straight into an assembled (possibly remote) frame.  For an
+  // interleaved output y points at colour 0 of HR pixel (wy0 r, wx0 r), y_row is the element pitch of HR rows and
+  // y_plane that of images.
+  int wy0, wy1, wx0, wx1;
+  long long y_row, y_plane;
+};
+
+// ----------------------------------------------------------------------------------------------
 // Epilogue parameters.
 //   mode 0: hidden = SiLU(scale[b,n] * acc + shift[b,n])   -> bf16 NHWC      (conv1 + control + SiLU)
 //   mode 1: zf += acc ; zb = bf16(zf)                                         (conv2 + ResidualConnection)
-//   mode 2: y = [clamp](skip + PixelShuffle_r(acc))         -> fp32 NCHW      (SubpixelConv2d + skip)
+//   mode 2: y = [clamp](skip + PixelShuffle_r(acc))         -> the HR image   (SubpixelConv2d + skip)
 // ----------------------------------------------------------------------------------------------
 struct EpiParams {
   int mode;
@@ -46,32 +73,9 @@ struct EpiParams {
   float* zf;                // mode 1: fp32 residual stream, updated in place
   int zf_pitch;             // channel pitch of zf in elements (0 = n_pad); > n_pad when this launch owns a channel slice
   int zf_extent;            // channels of zf that exist in memory (0 = n_pad), as out_extent
-  // mode 2
-  const float* x;  // LR image (B,3,H,W) fp32 -- only for skip_mode 2
-  float* y;        // HR image (B,3,rH,rW) fp32
-  // 8-bit image I/O (MZ_FLAG_IO_U8): when set they replace x / y.  x8 holds round(255 * x), read back as x8 / 255
-  // (ToDtype(float32, scale=True), reference test_compare.py:53-57); y8 = floor(255 * clamp(v, 0, 1) + 0.5)
-  // (torchvision save_image, test_compare.py:89) or floor(255 * clamp(v, 0, 1)) with u8_trunc (ToPILImage, README.md:81)
-  const uint8_t* x8;
-  uint8_t* y8;
-  int u8_trunc;
+  // mode 2: the images (a prepared launch takes them from each call: patch_conv_epi), the ratio and its bicubic table
+  ImageIo img;
   int r;
-  int skip_mode;  // 0 none, 1 y already holds the bicubic image, 2 recompute bicubic from x
-  int clamp01;
-  // Windowed output (mz_upscale_window; all zero = the whole image, densely): only LR pixels wy0 <= y < wy1,
-  // wx0 <= x < wx1 are stored, pixel (wy0, wx0) of plane 0 of image 0 at y / y8 itself, HR rows y_row elements and
-  // colour planes y_plane elements apart -- a tile's core written straight into an assembled (possibly remote) frame.
-  int wy0, wy1, wx0, wx1;
-  long long y_row, y_plane;
-  // Interleaved images (MZ_FLAG_X_NHWC / MZ_FLAG_Y_NHWC): x is (B,H,W,3), y is (B,rH,rW,3) -- colour c of a pixel at
-  // pixel * 3 + c, images 3HW (3 rH rW) elements apart as in the planar layout.  For a windowed y_nhwc output y / y8
-  // points at colour 0 of HR pixel (wy0 r, wx0 r), y_row is the element pitch of HR rows and y_plane that of images.
-  int x_nhwc, y_nhwc;
-  // 16-bit image I/O (MZ_FLAG_IO_U16), either layout: when set they replace x / y.  x16 is read as the IEEE quotient
-  // x16 / 65535 (ToDtype(float32, scale=True)); y16 = floor(65535 * clamp(v, 0, 1) + 0.5).  A head kernel of its own
-  // (conv_tc_kernel's LAY bit 2) reads and writes them.
-  const uint16_t* x16;
-  uint16_t* y16;
   // fp16 range guard: a kernel that is about to round a value beyond +-65504 into a 16-bit fp16 operand (where
   // cvt.rn.satfinite would clip it silently) writes 1 here.  Points at a host-mapped word owned by the mz_model
   // (mz_model_saturated); nullptr = not tracked (per-kernel entry points).
@@ -83,22 +87,23 @@ struct EpiParams {
 #define MZ_F16_MAX 65504.0f
 
 // address of colour c of HR pixel (y r + i, x r + j) of image b in the output of mode 2, or -1 outside the window;
-// YN: interleaved output (EpiParams::y_nhwc)
+// YN: interleaved output (ImageIo::y_nhwc)
 template <bool YN>
 __host__ __device__ inline long long head_out_index_l(const EpiParams& p, int b, int c, int y, int x, int i, int j) {
+  const ImageIo& io = p.img;
   const long long WR = static_cast<long long>(p.W) * p.r, HR = static_cast<long long>(p.H) * p.r;
-  if (p.wy1 > 0 && (y < p.wy0 || y >= p.wy1 || x < p.wx0 || x >= p.wx1)) return -1;
+  if (io.wy1 > 0 && (y < io.wy0 || y >= io.wy1 || x < io.wx0 || x >= io.wx1)) return -1;
   if (YN) {
-    const long long row = p.y_row ? p.y_row : 3 * WR, img = p.y_plane ? p.y_plane : 3 * HR * WR;
-    return static_cast<long long>(b) * img + (static_cast<long long>(y - p.wy0) * p.r + i) * row +
-           (static_cast<long long>(x - p.wx0) * p.r + j) * 3 + c;
+    const long long row = io.y_row ? io.y_row : 3 * WR, img = io.y_plane ? io.y_plane : 3 * HR * WR;
+    return static_cast<long long>(b) * img + (static_cast<long long>(y - io.wy0) * p.r + i) * row +
+           (static_cast<long long>(x - io.wx0) * p.r + j) * 3 + c;
   }
-  const long long row = p.y_row ? p.y_row : WR, plane = p.y_plane ? p.y_plane : HR * WR;
-  return (static_cast<long long>(b) * 3 + c) * plane + (static_cast<long long>(y - p.wy0) * p.r + i) * row +
-         static_cast<long long>(x - p.wx0) * p.r + j;
+  const long long row = io.y_row ? io.y_row : WR, plane = io.y_plane ? io.y_plane : HR * WR;
+  return (static_cast<long long>(b) * 3 + c) * plane + (static_cast<long long>(y - io.wy0) * p.r + i) * row +
+         static_cast<long long>(x - io.wx0) * p.r + j;
 }
 __host__ __device__ inline long long head_out_index(const EpiParams& p, int b, int c, int y, int x, int i, int j) {
-  return p.y_nhwc ? head_out_index_l<true>(p, b, c, y, x, i, j) : head_out_index_l<false>(p, b, c, y, x, i, j);
+  return p.img.y_nhwc ? head_out_index_l<true>(p, b, c, y, x, i, j) : head_out_index_l<false>(p, b, c, y, x, i, j);
 }
 
 // One 3x3 convolution launch (both kernels).
@@ -145,8 +150,8 @@ struct alignas(64) ConvLaunch {
 };
 int prepare_conv_tc(const ConvArgs& a, const ConvTcTune& tune, int device, ConvLaunch* out);
 int run_conv_tc(ConvLaunch& launch, cudaStream_t s);
-// head (mode 2) only: replace the image pointers, output window, image layouts and image-epilogue flags of a prepared
-// launch (a new layout swaps the kernel instantiation)
+// head (mode 2) only: replace the images (EpiParams::img) of a prepared launch (a new layout swaps the kernel
+// instantiation)
 int patch_conv_epi(ConvLaunch& launch, const EpiParams& e);
 // ---- one encoder block as one kernel (block_fused.cu): zf += conv2(SiLU(FiLM(conv1(zb_in)))), zb_out = round16(zf) ----
 struct FusedBlockArgs {
@@ -188,12 +193,9 @@ bool seg_gemm_tc_applies(const float* a0, const float* a1, const float* wt, cons
 int launch_seg_gemm_tc(const SgArgs& a, cudaStream_t s);
 
 int launch_bicubic(const float* x, float* y, int planes, int H, int W, int r, cudaStream_t s);
-// fp32 stream zf + 16-bit shadow zb (pitch zb_pitch).
-// x8 != nullptr: the image is 8-bit (B,3,H,W) and read as x8 / 255; x16 != nullptr: 16-bit, read as x16 / 65535.
-// x_nhwc: the image is interleaved (B,H,W,3).
-int launch_stem(const float* x, const uint8_t* x8, const float* w, const float* bias, float* zf, uint16_t* zb, int bf16,
-                int B, int H, int W, int Cp, int zb_pitch, cudaStream_t s, unsigned int* sat = nullptr,
-                bool x_nhwc = false, const uint16_t* x16 = nullptr);
+// image x (element type `type`, interleaved when x_nhwc: as ImageIo) -> fp32 stream zf + 16-bit shadow zb (pitch zb_pitch)
+int launch_stem(const void* x, int type, int x_nhwc, const float* w, const float* bias, float* zf, uint16_t* zb, int bf16,
+                int B, int H, int W, int Cp, int zb_pitch, cudaStream_t s, unsigned int* sat = nullptr);
 // film: [L][hCp / ns][B][2][ns] -- one [B][2][ns] table (scale row, shift row) per conv1 launch; ns == hCp normally
 int launch_film(const float* c, int c_rows, const float* w, const float* b, float* film, int L, int B, int F,
                 int hC, int hCp, int ns, cudaStream_t s);
@@ -323,6 +325,62 @@ __device__ __forceinline__ uint16_t to_u16(float v) {
 __device__ __forceinline__ uint32_t pack_u16x2(uint16_t lo, uint16_t hi) {
   return static_cast<uint32_t>(lo) | (static_cast<uint32_t>(hi) << 16);
 }
+// R contiguous values v of the HR image, quantised to T and stored at element d of y: fp32 clamped when clamp01 is set,
+// 8 and 16 bits always (to_u8 / to_u16).  R = 2 or 4 leave in one vector store (fp32: float2 / float4; 8 bits:
+// u16 / u32; 16 bits: u32 / 8 bytes), any other R element by element.
+template <typename T, int R>
+__device__ __forceinline__ void store_px(const ImageIo& io, size_t d, const float* v) {
+  T* dst = static_cast<T*>(io.y) + d;
+  if constexpr (std::is_same_v<T, float>) {
+    float q[R];
+#pragma unroll
+    for (int j = 0; j < R; ++j) q[j] = io.clamp01 ? fminf(fmaxf(v[j], 0.f), 1.f) : v[j];
+    if constexpr (R == 4) {
+      *reinterpret_cast<float4*>(dst) = make_float4(q[0], q[1], q[2], q[3]);
+    } else if constexpr (R == 2) {
+      *reinterpret_cast<float2*>(dst) = make_float2(q[0], q[1]);
+    } else {
+#pragma unroll
+      for (int j = 0; j < R; ++j) dst[j] = q[j];
+    }
+  } else if constexpr (std::is_same_v<T, uint8_t>) {
+    uint32_t w = 0;
+#pragma unroll
+    for (int j = 0; j < R; ++j) w |= static_cast<uint32_t>(to_u8(v[j], io.u8_trunc)) << (8 * j);
+    if constexpr (R == 4) {
+      *reinterpret_cast<uint32_t*>(dst) = w;
+    } else if constexpr (R == 2) {
+      *reinterpret_cast<uint16_t*>(dst) = static_cast<uint16_t>(w);
+    } else {
+#pragma unroll
+      for (int j = 0; j < R; ++j) dst[j] = static_cast<uint8_t>(w >> (8 * j));
+    }
+  } else {
+    static_assert(std::is_same_v<T, uint16_t>, "HR images are fp32, 8 or 16 bits");
+    uint16_t q[R];
+#pragma unroll
+    for (int j = 0; j < R; ++j) q[j] = to_u16(v[j]);
+    if constexpr (R == 4) {
+      *reinterpret_cast<uint2*>(dst) = make_uint2(pack_u16x2(q[0], q[1]), pack_u16x2(q[2], q[3]));
+    } else if constexpr (R == 2) {
+      *reinterpret_cast<uint32_t*>(dst) = pack_u16x2(q[0], q[1]);
+    } else {
+#pragma unroll
+      for (int j = 0; j < R; ++j) dst[j] = q[j];
+    }
+  }
+}
+// store_px with the output type chosen by the caller's kernel: 16 bits when o16 (a compile-time constant in the tcgen05
+// heads, whose LAY bit 2 selects 16-bit images), otherwise 8 bits or fp32 as io.type says (a runtime branch)
+template <int R>
+__device__ __forceinline__ void store_out(const ImageIo& io, size_t d, const float* v, bool o16) {
+  if (o16)
+    store_px<uint16_t, R>(io, d, v);
+  else if (io.type == kImgU8)
+    store_px<uint8_t, R>(io, d, v);
+  else
+    store_px<float, R>(io, d, v);
+}
 
 // Bicubic value of HR pixel (oy, ox) of one colour (H x W, fp32 | u8 | u16, pixels `ps` elements apart: 1 planar, 3
 // interleaved): 16 clamped taps, rows first.
@@ -362,87 +420,25 @@ __device__ __forceinline__ void epi_head(const EpiParams& p, int b, int y, int x
       const long long di = head_out_index(p, b, c, y, x, i, j);
       if (di < 0) continue;
       float v = acc[n];
-      if (p.skip_mode == 1) {
-        v += p.y[di];
-      } else if (p.skip_mode == 2) {
+      if (p.img.skip_mode == 1) {
+        v += static_cast<const float*>(p.img.y)[di];
+      } else if (p.img.skip_mode == 2) {
         const size_t HW = static_cast<size_t>(p.H) * p.W;
-        const size_t pl = p.x_nhwc ? static_cast<size_t>(b) * 3 * HW + c : (static_cast<size_t>(b) * 3 + c) * HW;
-        const int ps = p.x_nhwc ? 3 : 1;
-        v += p.x16 != nullptr ? bicubic_at(p.x16 + pl, p.H, p.W, ps, p.bt, oy, ox)
-             : p.x8 != nullptr ? bicubic_at(p.x8 + pl, p.H, p.W, ps, p.bt, oy, ox)
-                               : bicubic_at(p.x + pl, p.H, p.W, ps, p.bt, oy, ox);
+        const size_t pl = p.img.x_nhwc ? static_cast<size_t>(b) * 3 * HW + c : (static_cast<size_t>(b) * 3 + c) * HW;
+        const int ps = p.img.x_nhwc ? 3 : 1;
+        v += p.img.type == kImgU16 ? bicubic_at(static_cast<const uint16_t*>(p.img.x) + pl, p.H, p.W, ps, p.bt, oy, ox)
+             : p.img.type == kImgU8 ? bicubic_at(static_cast<const uint8_t*>(p.img.x) + pl, p.H, p.W, ps, p.bt, oy, ox)
+                                    : bicubic_at(static_cast<const float*>(p.img.x) + pl, p.H, p.W, ps, p.bt, oy, ox);
       }
-      if (p.clamp01) v = fminf(fmaxf(v, 0.f), 1.f);
-      if (p.y16 != nullptr)
-        p.y16[di] = to_u16(v);
-      else if (p.y8 != nullptr)
-        p.y8[di] = to_u8(v, p.u8_trunc);
-      else
-        p.y[di] = v;
+      store_out<1>(p.img, di, &v, p.img.type == kImgU16);
     }
   }
 }
-// One interleaved HR row segment of an LR pixel: v = R pixels x 3 colours, stored at element d of y / y8 / y16 as three
-// vectors (fp32: float2 at R = 2, float4 at R = 4; 8-bit: u16 / u32; 16-bit: u32 / 8 bytes) or, at R = 3, element by
-// element.  O16: the output is 16-bit (y16).
-template <int R, bool O16 = false>
-__device__ __forceinline__ void store_hr_row_nhwc(const EpiParams& p, size_t d, float (&v)[3 * R]) {
-  if constexpr (O16) {
-    uint16_t q[3 * R];
+// One interleaved HR row segment of an LR pixel: v = R pixels x 3 colours at element d, as three stores of R values
+template <int R, bool O16>
+__device__ __forceinline__ void store_hr_row_nhwc(const ImageIo& io, size_t d, const float (&v)[3 * R]) {
 #pragma unroll
-    for (int e = 0; e < 3 * R; ++e) q[e] = to_u16(v[e]);
-    uint16_t* rowp = p.y16 + d;
-    if constexpr (R == 4) {
-#pragma unroll
-      for (int k = 0; k < 3; ++k)
-        reinterpret_cast<uint2*>(rowp)[k] = make_uint2(pack_u16x2(q[4 * k], q[4 * k + 1]), pack_u16x2(q[4 * k + 2], q[4 * k + 3]));
-    } else if constexpr (R == 2) {
-#pragma unroll
-      for (int k = 0; k < 3; ++k) reinterpret_cast<uint32_t*>(rowp)[k] = pack_u16x2(q[2 * k], q[2 * k + 1]);
-    } else {
-#pragma unroll
-      for (int e = 0; e < 3 * R; ++e) rowp[e] = q[e];
-    }
-    return;
-  }
-  if (p.y8 != nullptr) {
-    uint8_t q[3 * R];
-#pragma unroll
-    for (int e = 0; e < 3 * R; ++e) q[e] = to_u8(v[e], p.u8_trunc);
-    uint8_t* rowp = p.y8 + d;
-    if constexpr (R == 4) {
-#pragma unroll
-      for (int k = 0; k < 3; ++k)
-        reinterpret_cast<uint32_t*>(rowp)[k] = static_cast<uint32_t>(q[4 * k]) | (static_cast<uint32_t>(q[4 * k + 1]) << 8) |
-                                               (static_cast<uint32_t>(q[4 * k + 2]) << 16) |
-                                               (static_cast<uint32_t>(q[4 * k + 3]) << 24);
-    } else if constexpr (R == 2) {
-#pragma unroll
-      for (int k = 0; k < 3; ++k)
-        reinterpret_cast<uint16_t*>(rowp)[k] =
-            static_cast<uint16_t>(static_cast<uint32_t>(q[2 * k]) | (static_cast<uint32_t>(q[2 * k + 1]) << 8));
-    } else {
-#pragma unroll
-      for (int e = 0; e < 3 * R; ++e) rowp[e] = q[e];
-    }
-    return;
-  }
-  if (p.clamp01) {
-#pragma unroll
-    for (int e = 0; e < 3 * R; ++e) v[e] = fminf(fmaxf(v[e], 0.f), 1.f);
-  }
-  float* rowp = p.y + d;
-  if constexpr (R == 4) {
-#pragma unroll
-    for (int k = 0; k < 3; ++k)
-      reinterpret_cast<float4*>(rowp)[k] = make_float4(v[4 * k], v[4 * k + 1], v[4 * k + 2], v[4 * k + 3]);
-  } else if constexpr (R == 2) {
-#pragma unroll
-    for (int k = 0; k < 3; ++k) reinterpret_cast<float2*>(rowp)[k] = make_float2(v[2 * k], v[2 * k + 1]);
-  } else {
-#pragma unroll
-    for (int e = 0; e < 3 * R; ++e) rowp[e] = v[e];
-  }
+  for (int k = 0; k < 3; ++k) store_out<R>(io, d + k * R, v + k * R, O16);
 }
 
 // Same as epi_head with the ratio known at compile time: the 5x5 LR neighbourhood of the pixel is loaded once per
@@ -455,10 +451,10 @@ __device__ __forceinline__ void store_hr_row_nhwc(const EpiParams& p, size_t d, 
 // the first FMA; skip-from-buffer reads all its row segments before the first store (a store to y orders every
 // later load from y behind it).  Columns are only clamped in the first and last warp of an image row: the others
 // (interior) read each neighbourhood row through one pointer with immediate offsets.
-// XN / YN: interleaved input / output (EpiParams::x_nhwc / y_nhwc) -- compile-time, so that the planar instantiation is
+// XN / YN: interleaved input / output (ImageIo::x_nhwc / y_nhwc) -- compile-time, so that the planar instantiation is
 // the code it was.  Interleaved, the taps of one colour are 3 elements apart (same FMA order per colour: bit-identical
 // results) and each HR row of the pixel leaves as 3R contiguous values.
-// T = uint16_t: 16-bit images on both sides (MZ_FLAG_IO_U16, y16) -- the 16-bit heads are instantiations of their own.
+// T = uint16_t: 16-bit images on both sides (MZ_FLAG_IO_U16) -- the 16-bit heads are instantiations of their own.
 template <int R, typename T, bool XN, bool YN>
 __device__ __forceinline__ void epi_head_rt(const EpiParams& p, const T* __restrict__ lr, int b, int y, int x,
                                             const float (&acc)[48], bool interior) {
@@ -466,8 +462,8 @@ __device__ __forceinline__ void epi_head_rt(const EpiParams& p, const T* __restr
   const int H = p.H, W = p.W;
   const long long first = head_out_index_l<YN>(p, b, 0, y, x, 0, 0);
   if (first < 0) return;  // outside the output window
-  const size_t row_pitch = p.y_row ? static_cast<size_t>(p.y_row) : static_cast<size_t>(W) * R * (YN ? 3 : 1);
-  const size_t plane_pitch = p.y_plane ? static_cast<size_t>(p.y_plane) : static_cast<size_t>(H) * R * W * R;
+  const size_t row_pitch = p.img.y_row ? static_cast<size_t>(p.img.y_row) : static_cast<size_t>(W) * R * (YN ? 3 : 1);
+  const size_t plane_pitch = p.img.y_plane ? static_cast<size_t>(p.img.y_plane) : static_cast<size_t>(H) * R * W * R;
   constexpr int NC = (R == 2) ? 3 : 1;  // colours whose taps are in flight together
   constexpr int PS = XN ? 3 : 1;        // elements between horizontally adjacent LR pixels of one colour
   float out[3][R][R];
@@ -478,7 +474,7 @@ __device__ __forceinline__ void epi_head_rt(const EpiParams& p, const T* __restr
 #pragma unroll
       for (int j = 0; j < R; ++j) out[c][i][j] = acc[c * R * R + i * R + j];
 
-  if (p.skip_mode == 2) {
+  if (p.img.skip_mode == 2) {
     const size_t HW = static_cast<size_t>(H) * W;
     const T* img = lr + static_cast<size_t>(b) * 3 * HW;
     int xo[5], ro[5];  // (a colour plane is below 2^31 pixels: prepare_conv_tc checks; an interleaved image is below
@@ -543,53 +539,14 @@ __device__ __forceinline__ void epi_head_rt(const EpiParams& p, const T* __restr
       for (int j = 0; j < R; ++j)
 #pragma unroll
         for (int c = 0; c < 3; ++c) v[3 * j + c] = out[c][i][j];
-      store_hr_row_nhwc<R, O16>(p, static_cast<size_t>(first) + static_cast<size_t>(i) * row_pitch, v);
+      store_hr_row_nhwc<R, O16>(p.img, static_cast<size_t>(first) + static_cast<size_t>(i) * row_pitch, v);
     }
     return;
   }
-  if constexpr (O16) {  // 16-bit output: 2R bytes per HR row segment -- one u32 at R = 2, one 8-byte store at R = 4
-#pragma unroll
-    for (int c = 0; c < 3; ++c)
-#pragma unroll
-      for (int i = 0; i < R; ++i) {
-        uint16_t* rowp = p.y16 + static_cast<size_t>(first) + c * plane_pitch + static_cast<size_t>(i) * row_pitch;
-        uint16_t q[R];
-#pragma unroll
-        for (int j = 0; j < R; ++j) q[j] = to_u16(out[c][i][j]);
-        if constexpr (R == 4) {
-          *reinterpret_cast<uint2*>(rowp) = make_uint2(pack_u16x2(q[0], q[1]), pack_u16x2(q[2], q[3]));
-        } else if constexpr (R == 2) {
-          *reinterpret_cast<uint32_t*>(rowp) = pack_u16x2(q[0], q[1]);
-        } else {
-#pragma unroll
-          for (int j = 0; j < R; ++j) rowp[j] = q[j];
-        }
-      }
-    return;
-  }
-  if (p.y8 != nullptr) {  // 8-bit output: R bytes per HR row segment (a warp writes 32 * R contiguous bytes)
-#pragma unroll
-    for (int c = 0; c < 3; ++c)
-#pragma unroll
-      for (int i = 0; i < R; ++i) {
-        uint8_t* rowp = p.y8 + static_cast<size_t>(first) + c * plane_pitch + static_cast<size_t>(i) * row_pitch;
-        uint32_t w = 0;
-#pragma unroll
-        for (int j = 0; j < R; ++j) w |= static_cast<uint32_t>(to_u8(out[c][i][j], p.u8_trunc)) << (8 * j);
-        if (R == 4) {
-          *reinterpret_cast<uint32_t*>(rowp) = w;
-        } else if (R == 2) {
-          *reinterpret_cast<uint16_t*>(rowp) = static_cast<uint16_t>(w);
-        } else {
-#pragma unroll
-          for (int j = 0; j < R; ++j) rowp[j] = static_cast<uint8_t>(w >> (8 * j));
-        }
-      }
-    return;
-  }
-
-  float* dst = p.y + static_cast<size_t>(first);
-  if (p.skip_mode == 1) {  // y already holds the bicubic image: all of this pixel's segments first, then the stores
+  // y already holds the bicubic image (fp32: 8 and 16 bits recompute the skip): all of this pixel's segments first,
+  // then the stores
+  if (!O16 && p.img.skip_mode == 1) {
+    const float* dst = static_cast<const float*>(p.img.y) + static_cast<size_t>(first);
     float sk[3][R][R];
 #pragma unroll
     for (int c = 0; c < 3; ++c)
@@ -617,22 +574,8 @@ __device__ __forceinline__ void epi_head_rt(const EpiParams& p, const T* __restr
 #pragma unroll
   for (int c = 0; c < 3; ++c)
 #pragma unroll
-    for (int i = 0; i < R; ++i) {
-      float* rowp = dst + c * plane_pitch + static_cast<size_t>(i) * row_pitch;
-      if (p.clamp01) {
-#pragma unroll
-        for (int j = 0; j < R; ++j) out[c][i][j] = fminf(fmaxf(out[c][i][j], 0.f), 1.f);
-      }
-      if (R == 4) {
-        *reinterpret_cast<float4*>(rowp) =
-            make_float4(out[c][i][0], out[c][i][1], out[c][i][R > 2 ? 2 : 0], out[c][i][R - 1]);
-      } else if (R == 2) {
-        *reinterpret_cast<float2*>(rowp) = make_float2(out[c][i][0], out[c][i][1]);
-      } else {
-#pragma unroll
-        for (int j = 0; j < R; ++j) rowp[j] = out[c][i][j];
-      }
-    }
+    for (int i = 0; i < R; ++i)
+      store_out<R>(p.img, static_cast<size_t>(first) + c * plane_pitch + static_cast<size_t>(i) * row_pitch, out[c][i], O16);
 }
 // interior: warp-uniform promise that x - 2 >= 0 and x + 2 < W for every lane of the calling warp
 // (the layouts and the 16-bit image type, I16, are template parameters of the calling kernel: one runtime branch over
@@ -640,11 +583,11 @@ __device__ __forceinline__ void epi_head_rt(const EpiParams& p, const T* __restr
 template <int R, bool XN, bool YN, bool I16>
 __device__ __forceinline__ void epi_head_r(const EpiParams& p, int b, int y, int x, const float (&acc)[48], bool interior) {
   if constexpr (I16)
-    epi_head_rt<R, uint16_t, XN, YN>(p, p.x16, b, y, x, acc, interior);
-  else if (p.x8 != nullptr)
-    epi_head_rt<R, uint8_t, XN, YN>(p, p.x8, b, y, x, acc, interior);
+    epi_head_rt<R, uint16_t, XN, YN>(p, static_cast<const uint16_t*>(p.img.x), b, y, x, acc, interior);
+  else if (p.img.type == kImgU8)
+    epi_head_rt<R, uint8_t, XN, YN>(p, static_cast<const uint8_t*>(p.img.x), b, y, x, acc, interior);
   else
-    epi_head_rt<R, float, XN, YN>(p, p.x, b, y, x, acc, interior);
+    epi_head_rt<R, float, XN, YN>(p, static_cast<const float*>(p.img.x), b, y, x, acc, interior);
 }
 // r = 2, TWO vertically adjacent LR pixels (y, x) and (y + 1, x) per thread: their 5x5 neighbourhoods share four of
 // five rows, so the pair costs 6 x 5 loads and 6 x 2 horizontal interpolations per colour instead of 2 x (5 x 5) and
@@ -661,9 +604,9 @@ __device__ __forceinline__ void epi_head2_pair(const EpiParams& p, const T* __re
   first[0] = head_out_index_l<YN>(p, b, 0, y, x, 0, 0);
   first[1] = second ? head_out_index_l<YN>(p, b, 0, y + 1, x, 0, 0) : -1;
   if (first[0] < 0 && first[1] < 0) return;  // both outside the output window
-  const size_t row_pitch = p.y_row ? static_cast<size_t>(p.y_row) : static_cast<size_t>(W) * 2 * (YN ? 3 : 1);
+  const size_t row_pitch = p.img.y_row ? static_cast<size_t>(p.img.y_row) : static_cast<size_t>(W) * 2 * (YN ? 3 : 1);
   constexpr int PS = XN ? 3 : 1;  // elements between horizontally adjacent LR pixels of one colour
-  const size_t plane_pitch = p.y_plane ? static_cast<size_t>(p.y_plane) : static_cast<size_t>(H) * 2 * W * 2;
+  const size_t plane_pitch = p.img.y_plane ? static_cast<size_t>(p.img.y_plane) : static_cast<size_t>(H) * 2 * W * 2;
   float out[2][3][2][2];
 #pragma unroll
   for (int c = 0; c < 3; ++c)
@@ -674,7 +617,7 @@ __device__ __forceinline__ void epi_head2_pair(const EpiParams& p, const T* __re
         out[0][c][i][j] = __uint_as_float(v0[c * 4 + i * 2 + j]);
         out[1][c][i][j] = __uint_as_float(v1[c * 4 + i * 2 + j]);
       }
-  if (p.skip_mode == 2) {
+  if (p.img.skip_mode == 2) {
     const size_t HW = static_cast<size_t>(H) * W;
     const T* img = lr + static_cast<size_t>(b) * 3 * HW;
     int xo[5], ro[6];
@@ -736,12 +679,13 @@ __device__ __forceinline__ void epi_head2_pair(const EpiParams& p, const T* __re
         for (int j = 0; j < 2; ++j)
 #pragma unroll
           for (int c = 0; c < 3; ++c) v[3 * j + c] = out[rr][c][i][j];
-        store_hr_row_nhwc<2, O16>(p, static_cast<size_t>(first[rr]) + static_cast<size_t>(i) * row_pitch, v);
+        store_hr_row_nhwc<2, O16>(p.img, static_cast<size_t>(first[rr]) + static_cast<size_t>(i) * row_pitch, v);
       }
     }
     return;
   }
-  if (!O16 && p.skip_mode == 1 && p.y8 == nullptr) {  // y already holds the bicubic image: every segment is read before the first store
+  if (!O16 && p.img.skip_mode == 1) {  // y already holds the bicubic image (fp32): every segment is read before the first store
+    const float* sy = static_cast<const float*>(p.img.y);
     float2 sk[2][3][2];
 #pragma unroll
     for (int rr = 0; rr < 2; ++rr)
@@ -750,7 +694,7 @@ __device__ __forceinline__ void epi_head2_pair(const EpiParams& p, const T* __re
 #pragma unroll
         for (int i = 0; i < 2; ++i)
           sk[rr][c][i] = first[rr] < 0 ? make_float2(0.f, 0.f)
-                                       : *reinterpret_cast<const float2*>(p.y + static_cast<size_t>(first[rr]) + c * plane_pitch +
+                                       : *reinterpret_cast<const float2*>(sy + static_cast<size_t>(first[rr]) + c * plane_pitch +
                                                                           static_cast<size_t>(i) * row_pitch);
 #pragma unroll
     for (int rr = 0; rr < 2; ++rr)
@@ -768,31 +712,20 @@ __device__ __forceinline__ void epi_head2_pair(const EpiParams& p, const T* __re
 #pragma unroll
     for (int c = 0; c < 3; ++c)
 #pragma unroll
-      for (int i = 0; i < 2; ++i) {
-        const size_t d = static_cast<size_t>(first[rr]) + c * plane_pitch + static_cast<size_t>(i) * row_pitch;
-        if constexpr (O16) {
-          *reinterpret_cast<uint32_t*>(p.y16 + d) = pack_u16x2(to_u16(out[rr][c][i][0]), to_u16(out[rr][c][i][1]));
-        } else if (p.y8 != nullptr) {
-          const uint32_t w = static_cast<uint32_t>(to_u8(out[rr][c][i][0], p.u8_trunc)) |
-                             (static_cast<uint32_t>(to_u8(out[rr][c][i][1], p.u8_trunc)) << 8);
-          *reinterpret_cast<uint16_t*>(p.y8 + d) = static_cast<uint16_t>(w);
-        } else {
-          float a0 = out[rr][c][i][0], a1 = out[rr][c][i][1];
-          if (p.clamp01) a0 = fminf(fmaxf(a0, 0.f), 1.f), a1 = fminf(fmaxf(a1, 0.f), 1.f);
-          *reinterpret_cast<float2*>(p.y + d) = make_float2(a0, a1);
-        }
-      }
+      for (int i = 0; i < 2; ++i)
+        store_out<2>(p.img, static_cast<size_t>(first[rr]) + c * plane_pitch + static_cast<size_t>(i) * row_pitch,
+                     out[rr][c][i], O16);
   }
 }
 template <bool XN, bool YN, bool I16>
 __device__ __forceinline__ void epi_head2(const EpiParams& p, int b, int y, int x, const uint32_t (&v0)[16],
                                           const uint32_t (&v1)[16], bool interior, bool second) {
   if constexpr (I16)
-    epi_head2_pair<uint16_t, XN, YN>(p, p.x16, b, y, x, v0, v1, interior, second);
-  else if (p.x8 != nullptr)
-    epi_head2_pair<uint8_t, XN, YN>(p, p.x8, b, y, x, v0, v1, interior, second);
+    epi_head2_pair<uint16_t, XN, YN>(p, static_cast<const uint16_t*>(p.img.x), b, y, x, v0, v1, interior, second);
+  else if (p.img.type == kImgU8)
+    epi_head2_pair<uint8_t, XN, YN>(p, static_cast<const uint8_t*>(p.img.x), b, y, x, v0, v1, interior, second);
   else
-    epi_head2_pair<float, XN, YN>(p, p.x, b, y, x, v0, v1, interior, second);
+    epi_head2_pair<float, XN, YN>(p, static_cast<const float*>(p.img.x), b, y, x, v0, v1, interior, second);
 }
 #endif  // __CUDACC__
 

@@ -162,19 +162,10 @@ static int run_conv(mz_model* m, int slot, const ConvArgs& a, const ConvTcTune& 
   key.a = a;
   key.t = t;
   if (a.epi.mode == 2) {
-    // The head reads the LR image and writes the HR image through plain pointers (no tensor map): they, the output
-    // window and the flags of the image epilogue are not part of what was prepared -- a fresh output tensor per call
-    // must not cost a geometry search and two tensor-map encodes.  They are patched into the prepared launch below.
-    key.a.epi.x = nullptr;
-    key.a.epi.y = nullptr;
-    key.a.epi.x8 = nullptr;
-    key.a.epi.y8 = nullptr;
-    key.a.epi.x16 = nullptr;
-    key.a.epi.y16 = nullptr;
-    key.a.epi.u8_trunc = key.a.epi.skip_mode = key.a.epi.clamp01 = 0;
-    key.a.epi.wy0 = key.a.epi.wy1 = key.a.epi.wx0 = key.a.epi.wx1 = 0;
-    key.a.epi.y_row = key.a.epi.y_plane = 0;
-    key.a.epi.x_nhwc = key.a.epi.y_nhwc = 0;
+    // The head reads the LR image and writes the HR image through plain pointers (no tensor map): the images are not
+    // part of what was prepared -- a fresh output tensor per call must not cost a geometry search and two tensor-map
+    // encodes.  They are patched into the prepared launch below.
+    key.a.epi.img = ImageIo{};
   }
   // kWays prepared launches per convolution: the host lanes, the engine workspace and captured graphs alternate operands
   for (int way = 0; way < kWays; ++way) {
@@ -626,18 +617,27 @@ static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, in
   if (frc != MZ_OK) return frc;
   const bool yuv = (flags & MZ_FLAG_YUV420) != 0;
   MZ_REQUIRE(!yuv || (!win && front && back), "upscale: 4:2:0 frames are neither windowed nor staged");
-  const bool io8 = (flags & MZ_FLAG_IO_U8) != 0, io16 = (flags & MZ_FLAG_IO_U16) != 0;
-  const bool x_nhwc = (flags & MZ_FLAG_X_NHWC) != 0, y_nhwc = (flags & MZ_FLAG_Y_NHWC) != 0;
-  MZ_REQUIRE(!((x_nhwc || y_nhwc) && (flags & MZ_FLAG_SKIP_FROM_BUFFER)),
+  ImageIo img{};
+  img.x = x_dev_v;
+  img.y = y_dev_v;
+  img.type = (flags & MZ_FLAG_IO_U8) ? kImgU8 : ((flags & MZ_FLAG_IO_U16) ? kImgU16 : kImgF32);
+  img.x_nhwc = (flags & MZ_FLAG_X_NHWC) ? 1 : 0;
+  img.y_nhwc = (flags & MZ_FLAG_Y_NHWC) ? 1 : 0;
+  img.u8_trunc = (flags & MZ_FLAG_U8_TRUNC) ? 1 : 0;
+  img.skip_mode = (flags & MZ_FLAG_SKIP_FROM_BUFFER) ? 1 : 2;
+  img.clamp01 = (flags & MZ_FLAG_CLAMP01) ? 1 : 0;
+  if (win) {
+    img.wy0 = win->y0;
+    img.wy1 = win->y1;
+    img.wx0 = win->x0;
+    img.wx1 = win->x1;
+    img.y_row = win->row_pitch;
+    img.y_plane = win->plane_pitch;
+  }
+  MZ_REQUIRE(!((img.x_nhwc || img.y_nhwc) && img.skip_mode == 1),
              "upscale: interleaved images (MZ_FLAG_X_NHWC / MZ_FLAG_Y_NHWC) recompute the skip (no MZ_FLAG_SKIP_FROM_BUFFER)");
-  MZ_REQUIRE(!(x_nhwc || y_nhwc) || static_cast<long long>(H) * W * 3 < (1LL << 31),
+  MZ_REQUIRE(!(img.x_nhwc || img.y_nhwc) || static_cast<long long>(H) * W * 3 < (1LL << 31),
              "upscale: an interleaved %d x %d image exceeds 2^31 elements", H, W);
-  const float* x_dev = io8 || io16 ? nullptr : static_cast<const float*>(x_dev_v);
-  float* y_dev = io8 || io16 ? nullptr : static_cast<float*>(y_dev_v);
-  const uint8_t* x8 = io8 ? static_cast<const uint8_t*>(x_dev_v) : nullptr;
-  uint8_t* y8 = io8 ? static_cast<uint8_t*>(y_dev_v) : nullptr;
-  const uint16_t* x16 = io16 ? static_cast<const uint16_t*>(x_dev_v) : nullptr;
-  uint16_t* y16 = io16 ? static_cast<uint16_t*>(y_dev_v) : nullptr;
   MZ_REQUIRE(B > 0 && H > 0 && W > 0, "upscale: empty input (B %d, H %d, W %d)", B, H, W);
   if (m->F > 0) {
     MZ_REQUIRE(c_dev != nullptr, "Control vector c is required for control models.");
@@ -685,8 +685,8 @@ static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, in
   }
   rc = MZ_OK;
   if (front)
-    rc = launch_stem(x_dev, x8, m->stem_w, m->stem_b, zf, zb, m->bf16, B, H, W, m->Cpm, m->Czm, s,
-                     m->sat_dev, x_nhwc, x16);
+    rc = launch_stem(img.x, img.type, img.x_nhwc, m->stem_w, m->stem_b, zf, zb, m->bf16, B, H, W, m->Cpm, m->Czm, s,
+                     m->sat_dev);
   if (rc != MZ_OK) return rc;
 
   const int slot = m->timing_calls % kTimingSlots;
@@ -782,11 +782,9 @@ static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, in
   }
   if (!back) return MZ_OK;
 
-  int skip_mode = 2;
-  if (flags & MZ_FLAG_SKIP_FROM_BUFFER) {
-    rc = launch_bicubic(x_dev, y_dev, B * 3, H, W, m->r, s);
+  if (img.skip_mode == 1) {  // (fp32 only: check_image_flags)
+    rc = launch_bicubic(static_cast<const float*>(img.x), static_cast<float*>(img.y), B * 3, H, W, m->r, s);
     if (rc != MZ_OK) return rc;
-    skip_mode = 1;
   }
   ConvArgs a;
   memset(&a, 0, sizeof(a));
@@ -801,26 +799,8 @@ static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, in
   a.epi.H = H;
   a.epi.W = W;
   a.epi.n_pad = m->headNp;
-  a.epi.x = x_dev;
-  a.epi.y = y_dev;
-  a.epi.x8 = x8;
-  a.epi.y8 = y8;
-  a.epi.x16 = x16;
-  a.epi.y16 = y16;
-  a.epi.u8_trunc = (flags & MZ_FLAG_U8_TRUNC) ? 1 : 0;
+  a.epi.img = img;
   a.epi.r = m->r;
-  a.epi.skip_mode = skip_mode;
-  a.epi.clamp01 = (flags & MZ_FLAG_CLAMP01) ? 1 : 0;
-  a.epi.x_nhwc = x_nhwc ? 1 : 0;
-  a.epi.y_nhwc = y_nhwc ? 1 : 0;
-  if (win) {
-    a.epi.wy0 = win->y0;
-    a.epi.wy1 = win->y1;
-    a.epi.wx0 = win->x0;
-    a.epi.wx1 = win->x1;
-    a.epi.y_row = win->row_pitch;
-    a.epi.y_plane = win->plane_pitch;
-  }
   make_bicubic_table(m->r, &a.epi.bt);
   return simt ? launch_conv_simt(a, s) : run_conv(m, m->L * (S + S2), a, m->tune[2], s);
 }

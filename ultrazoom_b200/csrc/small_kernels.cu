@@ -152,7 +152,7 @@ int launch_bicubic(const float* x, float* y, int planes, int H, int W, int r, cu
 }
 
 // ----------------------------------------------------------------------------------------------
-// stem: x (B,3,H,W) fp32 NCHW -> zf (B,H,W,Cp) fp32 and zb (B,H,W,Cz) 16-bit; z = W x + bias,
+// stem: x (B,3,H,W) -> zf (B,H,W,Cp) fp32 and zb (B,H,W,Cz) 16-bit; z = W x + bias,
 // channels >= C are written as zero (w/bias are zero-padded to Cp by the caller).
 // A store-only stream (12 B read, 6 Cp B written per pixel).  One thread -> 4 channels of one pixel, threads of a
 // block laid out channel-fastest over consecutive pixels: a warp's fp32 store is 512 contiguous bytes, its 16-bit
@@ -166,21 +166,21 @@ __device__ __forceinline__ void st_global_v2(void* p, uint32_t a, uint32_t b) {
   asm volatile("st.global.v2.b32 [%0], {%1, %2};" ::"l"(p), "r"(a), "r"(b) : "memory");
 }
 
-// element i of the image as float: fp32 as it is; 8 / 16 bits as the exact quotient x8 / 255, x16 / 65535 (IEEE
-// division, what ToDtype(float32, scale=True) computes): the network amplifies a 1-ulp difference of its input through
-// 20..40 layers of 16-bit rounding to ~1e-3 at the output
-__device__ __forceinline__ float stem_px(const float* __restrict__ x, const uint8_t* __restrict__ x8,
-                                         const uint16_t* __restrict__ x16, size_t i) {
-  if (x8 != nullptr) return __fdiv_rn(static_cast<float>(__ldg(x8 + i)), 255.f);
-  if (x16 != nullptr) return __fdiv_rn(static_cast<float>(__ldg(x16 + i)), 65535.f);
-  return __ldg(x + i);
+// element i of the image (ImageType `type`) as float: fp32 as it is; 8 / 16 bits as the exact quotient x / 255,
+// x / 65535 (IEEE division, what ToDtype(float32, scale=True) computes): the network amplifies a 1-ulp difference of its
+// input through 20..40 layers of 16-bit rounding to ~1e-3 at the output
+__device__ __forceinline__ float stem_px(const void* __restrict__ x, int type, size_t i) {
+  switch (type) {
+    case kImgU8: return __fdiv_rn(static_cast<float>(static_cast<const uint8_t*>(x)[i]), 255.f);
+    case kImgU16: return __fdiv_rn(static_cast<float>(static_cast<const uint16_t*>(x)[i]), 65535.f);
+    default: return static_cast<const float*>(x)[i];
+  }
 }
 
-__global__ void __launch_bounds__(256) stem_kernel(const float* __restrict__ x, const uint8_t* __restrict__ x8,
-                                                   const uint16_t* __restrict__ x16, const float* __restrict__ w,
-                                                   const float* __restrict__ bias, float* __restrict__ zf,
-                                                   uint16_t* __restrict__ zb, int bf16, int B, int H, int W, int Cp,
-                                                   int Cz, int ppb, unsigned int* sat, int x_nhwc) {
+__global__ void __launch_bounds__(256) stem_kernel(const void* __restrict__ x, int type, int x_nhwc,
+                                                   const float* __restrict__ w, const float* __restrict__ bias,
+                                                   float* __restrict__ zf, uint16_t* __restrict__ zb, int bf16, int B,
+                                                   int H, int W, int Cp, int Cz, int ppb, unsigned int* sat) {
   extern __shared__ float xs[];  // [3][ppb]: the block's pixels, colour planes apart
   // blockDim = (channel groups of 4, pixels per pass): a thread keeps ITS four channels' weights and bias in registers
   const int g = threadIdx.x;
@@ -202,7 +202,7 @@ __global__ void __launch_bounds__(256) stem_kernel(const float* __restrict__ x, 
     const size_t e0 = p0 * 3;
     for (int e = tid; e < 3 * n; e += nt) {
       const int j = e / 3, c = e - 3 * j;
-      xs[c * ppb + j] = stem_px(x, x8, x16, e0 + e);
+      xs[c * ppb + j] = stem_px(x, type, e0 + e);
     }
   } else {
     const size_t b0 = p0 / plane, rem0 = p0 - b0 * plane;  // (one division per block; the range may cross images)
@@ -215,7 +215,7 @@ __global__ void __launch_bounds__(256) stem_kernel(const float* __restrict__ x, 
       }
       const size_t xo = b * 3 * plane + rem;
 #pragma unroll
-      for (int c = 0; c < 3; ++c) xs[c * ppb + j] = stem_px(x, x8, x16, xo + c * plane);
+      for (int c = 0; c < 3; ++c) xs[c * ppb + j] = stem_px(x, type, xo + c * plane);
     }
   }
   __syncthreads();
@@ -235,9 +235,8 @@ __global__ void __launch_bounds__(256) stem_kernel(const float* __restrict__ x, 
   if (!bf16 && sat != nullptr && !(amax <= MZ_F16_MAX)) *sat = 1u;  // fp16 range guard (see EpiParams::sat)
 }
 
-int launch_stem(const float* x, const uint8_t* x8, const float* w, const float* bias, float* zf, uint16_t* zb, int bf16,
-                int B, int H, int W, int Cp, int zb_pitch, cudaStream_t s, unsigned int* sat, bool x_nhwc,
-                const uint16_t* x16) {
+int launch_stem(const void* x, int type, int x_nhwc, const float* w, const float* bias, float* zf, uint16_t* zb, int bf16,
+                int B, int H, int W, int Cp, int zb_pitch, cudaStream_t s, unsigned int* sat) {
   MZ_REQUIRE(Cp > 0 && Cp % 8 == 0, "stem: padded channel count must be a multiple of 8, %d given", Cp);
   MZ_REQUIRE(B > 0 && H > 0 && W > 0, "stem: empty input");
   MZ_REQUIRE(zf != nullptr, "stem: null fp32 stream");
@@ -255,8 +254,8 @@ int launch_stem(const float* x, const uint8_t* x8, const float* w, const float* 
   const long long blocks = (npix + ppb - 1) / ppb;
   MZ_REQUIRE(blocks < (1LL << 31), "stem: too many pixels");
   const size_t smem = static_cast<size_t>(3) * ppb * sizeof(float);
-  stem_kernel<<<static_cast<unsigned>(blocks), dim3(groups, py), smem, s>>>(x, x8, x16, w, bias, zf, zb, bf16, B, H, W, Cp,
-                                                                         Cz, static_cast<int>(ppb), sat, x_nhwc ? 1 : 0);
+  stem_kernel<<<static_cast<unsigned>(blocks), dim3(groups, py), smem, s>>>(x, type, x_nhwc, w, bias, zf, zb, bf16, B, H, W,
+                                                                         Cp, Cz, static_cast<int>(ppb), sat);
   MZ_CUDA(cudaGetLastError());
   return MZ_OK;
 }
