@@ -86,6 +86,21 @@ typedef enum mz_status {
 #define MZ_FLAG_YUV_BT601 512u
 #define MZ_FLAG_YUV_BT2020 1024u
 #define MZ_FLAG_YUV_FULL_RANGE 2048u
+/* Images with an alpha channel (PNG / WebP / TIFF stills with transparency): x is (B,4,H,W), y is (B,4,rH,rW) -- colour
+ * 0..2, then a straight (not premultiplied) alpha.  Planar, an image is four planes (4HW elements); interleaved
+ * (MZ_FLAG_X_NHWC / MZ_FLAG_Y_NHWC), channel c of a pixel is at pixel * 4 + c.  Element types, layouts and quantisation
+ * as for RGB.
+ *   colour: y[:, :3] equals, bit for bit, the 3-channel call on x[:, :3] with the same flags otherwise -- the network never
+ *           reads the alpha and is unchanged;
+ *   alpha:  y[:, 3] = Q(clamp?(bicubic_r(x[:, 3]))) -- the global skip's resampling (Keys cubic, A = -0.75, half-pixel
+ *           centres, clamped taps; integer inputs read as the colour skip reads them), computed by the head in the same
+ *           FMA order as a colour's skip but started from 0 instead of from the accumulator, clamped with
+ *           MZ_FLAG_CLAMP01 and quantised as the colour is.  So with all head weights zero an alpha equal to a colour
+ *           plane gives a bit-identical output channel.
+ * MZ_FLAG_YUV420 and MZ_FLAG_SKIP_FROM_BUFFER are refused (MZ_ERR_INVALID).  Applies to mz_upscale, mz_upscale_window,
+ * mz_upscale_stage, mz_upscale_host and mz_upscale_host_async (MZ_FLAG_SIMT_CONV included); mz_workspace_bytes is
+ * unchanged (the alpha needs no workspace) and mz_head_shuffle_add stays RGB. */
+#define MZ_FLAG_RGBA 4096u
 
 /* Constructor kwargs of the 0.2.x-style MewZoom (README.md:254-258, model.py:52-69). */
 typedef struct mz_config {
@@ -166,11 +181,11 @@ int mz_workspace_bytes_flags(const mz_model* m, int32_t B, int32_t H, int32_t W,
 
 /* ---- the hot path: replaces MewZoom.forward / MewZoom.upscale (model.py:149-179) ----
  * x_dev : (B,3,H,W) fp32 NCHW in [0,1]   (uint8 / uint16 with MZ_FLAG_IO_U8 / _U16; (B,H,W,3) with MZ_FLAG_X_NHWC;
- *         B 4:2:0 frames of H x W luma with MZ_FLAG_YUV420)
+ *         B 4:2:0 frames of H x W luma with MZ_FLAG_YUV420; 4 channels with MZ_FLAG_RGBA)
  * c_dev : NULL for non-control models, else (B, control_features) fp32 (c_rows == B)
  *         or (1, control_features) (c_rows == 1, broadcast) -- validate.py:73-94
  * y_dev : (B,3,rH,rW) fp32 NCHW          (uint8 / uint16 with MZ_FLAG_IO_U8 / _U16; (B,rH,rW,3) with MZ_FLAG_Y_NHWC;
- *         B 4:2:0 frames of rH x rW luma with MZ_FLAG_YUV420)
+ *         B 4:2:0 frames of rH x rW luma with MZ_FLAG_YUV420; 4 channels with MZ_FLAG_RGBA)
  * flags : MZ_FLAG_CLAMP01 => upscale(), 0 => forward()
  */
 int mz_upscale(mz_model* m, const void* x_dev, const float* c_dev, int32_t c_rows, void* y_dev,
@@ -180,14 +195,17 @@ int mz_upscale(mz_model* m, const void* x_dev, const float* c_dev, int32_t c_row
 /* The same call with a WINDOWED output, for halo-tiled inference (SURVEY.md 8(e), partitioning 2): of the (H, W) input
  * tile only the LR pixels win_y0 <= y < win_y1, win_x0 <= x < win_x1 (the tile's core) are written, and they go
  * straight into an assembled frame: y_dev is where HR pixel (win_y0 * r, win_x0 * r) of plane 0 of image 0 lands,
- * HR rows are y_row_pitch elements apart and the three colour planes (and then the images) y_plane_pitch elements.
+ * HR rows are y_row_pitch elements apart and the three colour planes (four with MZ_FLAG_RGBA; then the images)
+ * y_plane_pitch elements.
  * y_dev may be another GPU's memory with peer access enabled (mz_enable_peer_access): the head kernel's stores then ARE
  * the transfer over NVLink -- no tile output buffer, no copy, no collective.  The bicubic skip is always recomputed.
  * With MZ_FLAG_Y_NHWC (interleaved output): y_dev is where colour 0 of HR pixel (win_y0 * r, win_x0 * r) of image 0
- * lands, y_row_pitch is the number of elements between HR rows (at least 3 * r * (win_x1 - win_x0)) and y_plane_pitch the
- * number between images.
+ * lands, y_row_pitch is the number of elements between HR rows (at least 3 * r * (win_x1 - win_x0), 4 * r * ... with
+ * MZ_FLAG_RGBA) and y_plane_pitch the number between images.
  * y_dev and both pitches must be aligned to the head's vector stores: fp32 8 / 16 / 4 bytes at r = 2 / 4 / 3, 8-bit
- * 2 / 4 / 1 bytes, 16-bit 4 / 8 / 2 bytes -- in either layout. */
+ * 2 / 4 / 1 bytes, 16-bit 4 / 8 / 2 bytes -- in either layout, except interleaved RGBA output (MZ_FLAG_RGBA with
+ * MZ_FLAG_Y_NHWC), whose row segment of a pixel (4r values) leaves in the widest vectors dividing it: fp32 16 bytes at
+ * every r, 8-bit 8 / 16 / 4 bytes at r = 2 / 4 / 3, 16-bit 16 / 16 / 8 bytes. */
 int mz_upscale_window(mz_model* m, const void* x_dev, const float* c_dev, int32_t c_rows, void* y_dev,
                       int64_t y_row_pitch, int64_t y_plane_pitch, int32_t B, int32_t H, int32_t W, int32_t win_y0,
                       int32_t win_y1, int32_t win_x0, int32_t win_x1, void* workspace_dev, size_t workspace_bytes,

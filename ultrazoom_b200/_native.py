@@ -33,6 +33,7 @@ FLAG_YUV420 = 256
 FLAG_YUV_BT601 = 512
 FLAG_YUV_BT2020 = 1024
 FLAG_YUV_FULL_RANGE = 2048
+FLAG_RGBA = 4096
 
 DTYPE_F16, DTYPE_BF16 = 0, 1
 MATH_TF32, MATH_FP32 = 0, 1

@@ -21,9 +21,10 @@ LIB = os.path.join(LIBDIR, "libmewzoom_b200.so")
 STAMP = os.path.join(LIBDIR, "libmewzoom_b200.sha256")
 # (source, extra defines, object name).  conv_tc.cu is compiled once per epilogue mode 0..2 (its template instantiations
 # dominate the build time), once (part 4) for its host side, once per interleaved image layout of the head (parts
-# 5..7) and once per layout of the 16-bit image head (parts 8..11); see the MZ_TC_PART comment in the file.
+# 5..7), once per layout of the 16-bit image head (parts 8..11) and once per layout of the RGBA head (parts 12..19); see
+# the MZ_TC_PART comment in the file.
 SOURCES = [(f"{n}.cu", [], f"{n}.o") for n in ("host_util", "small_kernels", "yuv420", "api", "model", "probe", "block_fused", "unet_ops", "unet_tc")] + [
-    ("conv_tc.cu", [f"-DMZ_TC_PART={part}"], f"conv_tc_p{part}.o") for part in (0, 1, 2, 4, 5, 6, 7, 8, 9, 10, 11)
+    ("conv_tc.cu", [f"-DMZ_TC_PART={part}"], f"conv_tc_p{part}.o") for part in (0, 1, 2, 4, *range(5, 20))
 ]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

@@ -78,7 +78,7 @@ int mz_stem_pack(const float* x_dev, const float* w_dev, const float* bias_dev, 
                  int32_t H, int32_t W, int32_t Cp, int32_t zb_pitch, int32_t operand_dtype, void* stream) {
   MZ_REQUIRE(x_dev && w_dev && bias_dev && zf_dev && zb_dev, "stem: null pointer");
   MZ_REQUIRE(dtype_ok(operand_dtype), "operand_dtype must be MZ_DTYPE_F16 or MZ_DTYPE_BF16, %d given", operand_dtype);
-  return launch_stem(x_dev, kImgF32, 0, w_dev, bias_dev, zf_dev, static_cast<uint16_t*>(zb_dev), operand_dtype, B, H, W, Cp,
+  return launch_stem(x_dev, kImgF32, 0, 3, w_dev, bias_dev, zf_dev, static_cast<uint16_t*>(zb_dev), operand_dtype, B, H, W, Cp,
                      zb_pitch, static_cast<cudaStream_t>(stream));
 }
 
@@ -138,6 +138,7 @@ int mz_head_shuffle_add(const void* zb_dev, const void* wpacked_dev, const float
   a.epi.img.x = x_dev;
   a.epi.img.y = y_dev;
   a.epi.img.type = kImgF32;
+  a.epi.nc = 3;
   a.epi.img.skip_mode = skip_mode;
   a.epi.img.clamp01 = clamp01;
   a.epi.r = r;

@@ -108,7 +108,7 @@ __host__ __device__ inline SmemPlan plan_smem(const TcParams& p) {
 // shapes -- is fetched once per input row instead of once per (output row, tap).  Every UMMA accumulates; the epilogue
 // zeroes each accumulator column group right after reading it.
 // LAY (head only): bit 0 interleaved input image, bit 1 interleaved output image (ImageIo::x_nhwc / y_nhwc), bit 2
-// 16-bit images (ImageIo::type kImgU16).
+// 16-bit images (ImageIo::type kImgU16), bit 3 RGBA images (EpiParams::nc == 4).
 template <int MODE, int KT, int ROWS, int VAR, int LAY = 0>
 __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_constant__ TcParams p) {
   constexpr bool PAIR = VAR == 1, FUSE = VAR == 2;
@@ -937,7 +937,8 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
             if (ok) {
               const bool interior = xw >= 2 && xw + 33 < p.epi.W;  // (warp-uniform) no clamped column in this warp
               const bool second = y + 1 < p.epi.H;
-              epi_head2<(LAY & 1) != 0, (LAY & 2) != 0, (LAY & 4) != 0>(p.epi, b, y, x, v0, v1, interior, second);
+              epi_head2<(LAY & 1) != 0, (LAY & 2) != 0, (LAY & 4) != 0, (LAY & 8) ? 4 : 3>(p.epi, b, y, x, v0, v1, interior,
+                                                                                           second);
             }
           }
         }
@@ -980,12 +981,13 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
           if (ok) {
             const bool interior = xw >= 2 && xw + 33 < p.epi.W;  // (warp-uniform) no clamped column in this warp
             constexpr bool XN = (LAY & 1) != 0, YN = (LAY & 2) != 0, I16 = (LAY & 4) != 0;
+            constexpr int CH = (LAY & 8) ? 4 : 3;
             if (p.epi.r == 4)
-              epi_head_r<4, XN, YN, I16>(p.epi, b, y, x, acc, interior);
+              epi_head_r<4, XN, YN, I16, CH>(p.epi, b, y, x, acc, interior);
             else if (p.epi.r == 2)
-              epi_head_r<2, XN, YN, I16>(p.epi, b, y, x, acc, interior);
+              epi_head_r<2, XN, YN, I16, CH>(p.epi, b, y, x, acc, interior);
             else
-              epi_head_r<3, XN, YN, I16>(p.epi, b, y, x, acc, interior);
+              epi_head_r<3, XN, YN, I16, CH>(p.epi, b, y, x, acc, interior);
           }
         } else if (MODE == 1) {
           if (k > 0 && !all_rows) load_residual(k, k + 1);
@@ -1157,8 +1159,8 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
 // ---- kernel lookup -------------------------------------------------------------------------------------------------
 // One lookup function per epilogue mode and head layout, so that the build can compile the instantiations of each in
 // its own translation unit: build.py compiles this file with -DMZ_TC_PART=<mode> for the kernels of modes 0 and 1,
-// -DMZ_TC_PART=4 for the host side, -DMZ_TC_PART=2 for the planar head (LAY 0) and -DMZ_TC_PART=5..11 for the heads of
-// LAY 1..7.  Without the define (a plain `nvcc -c conv_tc.cu`) everything lands in one object.
+// -DMZ_TC_PART=4 for the host side, -DMZ_TC_PART=2 for the planar head (LAY 0) and -DMZ_TC_PART=5..11 / 12..19 for the
+// heads of LAY 1..7 / 8..15 (RGBA).  Without the define (a plain `nvcc -c conv_tc.cu`) everything lands in one object.
 //   var 0: one CTA per patch, 1: CTA pair (cta_group::2), 2: fused rows.  Returns nullptr for a shape that has no kernel.
 const void* tc_kernel_mode0(int ks, int rows, int var);
 const void* tc_kernel_mode1(int ks, int rows, int var);
@@ -1280,15 +1282,18 @@ struct ConvLaunchImpl {
   int ks, var, lay;  // what `fn` was looked up for (the head's image layouts are patched per call)
 };
 
-// the head kernel for image layouts `lay` (bit 0 interleaved input, bit 1 interleaved output, bit 2 16-bit images)
+// the head kernel for image layouts `lay` (bit 0 interleaved input, bit 1 interleaved output, bit 2 16-bit images,
+// bit 3 RGBA)
 static const void* tc_kernel_head(int lay, int ks, int rows, int var) {
-  static const void* (*const heads[8])(int, int, int) = {tc_kernel_head_lay<0>, tc_kernel_head_lay<1>, tc_kernel_head_lay<2>,
-                                                         tc_kernel_head_lay<3>, tc_kernel_head_lay<4>, tc_kernel_head_lay<5>,
-                                                         tc_kernel_head_lay<6>, tc_kernel_head_lay<7>};
+  static const void* (*const heads[16])(int, int, int) = {
+      tc_kernel_head_lay<0>,  tc_kernel_head_lay<1>,  tc_kernel_head_lay<2>,  tc_kernel_head_lay<3>,
+      tc_kernel_head_lay<4>,  tc_kernel_head_lay<5>,  tc_kernel_head_lay<6>,  tc_kernel_head_lay<7>,
+      tc_kernel_head_lay<8>,  tc_kernel_head_lay<9>,  tc_kernel_head_lay<10>, tc_kernel_head_lay<11>,
+      tc_kernel_head_lay<12>, tc_kernel_head_lay<13>, tc_kernel_head_lay<14>, tc_kernel_head_lay<15>};
   return heads[lay](ks, rows, var);
 }
 static int head_layout(const EpiParams& e) {
-  return (e.img.x_nhwc ? 1 : 0) | (e.img.y_nhwc ? 2 : 0) | (e.img.type == kImgU16 ? 4 : 0);
+  return (e.img.x_nhwc ? 1 : 0) | (e.img.y_nhwc ? 2 : 0) | (e.img.type == kImgU16 ? 4 : 0) | (e.nc == 4 ? 8 : 0);
 }
 static_assert(sizeof(ConvLaunchImpl) <= sizeof(ConvLaunch::storage), "ConvLaunch::storage too small");
 
@@ -1359,6 +1364,7 @@ int patch_conv_epi(ConvLaunch& launch, const EpiParams& e) {
     L.lay = lay;
   }
   L.p.epi.img = e.img;
+  L.p.epi.nc = e.nc;
   return MZ_OK;
 }
 

@@ -34,18 +34,19 @@ void make_bicubic_table(int r, BicubicTable* t);
 // (MZ_FLAG_IO_U16): x is read as the IEEE quotient x / 65535; y = floor(65535 * clamp(v, 0, 1) + 0.5).
 enum ImageType : int { kImgF32 = 0, kImgU8 = 1, kImgU16 = 2 };
 struct ImageIo {
-  const void* x;  // LR image (B,3,H,W)
-  void* y;        // HR image (B,3,rH,rW)
+  const void* x;  // LR image (B,nc,H,W), nc = EpiParams::nc
+  void* y;        // HR image (B,nc,rH,rW)
   int type;       // ImageType
-  // Interleaved images (MZ_FLAG_X_NHWC / MZ_FLAG_Y_NHWC): x is (B,H,W,3), y is (B,rH,rW,3) -- colour c of a pixel at
-  // pixel * 3 + c, images 3HW (3 rH rW) elements apart as in the planar layout.
+  // Interleaved images (MZ_FLAG_X_NHWC / MZ_FLAG_Y_NHWC): x is (B,H,W,nc), y is (B,rH,rW,nc) -- channel c of a pixel at
+  // pixel * nc + c, images nc HW (nc rH rW) elements apart as in the planar layout.
   int x_nhwc, y_nhwc;
   int u8_trunc;
   int skip_mode;  // 0 none, 1 y already holds the bicubic image (fp32 only), 2 recompute bicubic from x
   int clamp01;
   // Windowed output (mz_upscale_window; all zero = the whole image, densely): only LR pixels wy0 <= y < wy1,
   // wx0 <= x < wx1 are stored, pixel (wy0, wx0) of plane 0 of image 0 at y itself, HR rows y_row elements and colour
-  // planes y_plane elements apart -- a tile's core written straight into an assembled (possibly remote) frame.  For an
+  // planes y_plane elements apart (images nc planes) -- a tile's core written straight into an assembled (possibly
+  // remote) frame.  For an
   // interleaved output y points at colour 0 of HR pixel (wy0 r, wx0 r), y_row is the element pitch of HR rows and
   // y_plane that of images.
   int wy0, wy1, wx0, wx1;
@@ -73,9 +74,15 @@ struct EpiParams {
   float* zf;                // mode 1: fp32 residual stream, updated in place
   int zf_pitch;             // channel pitch of zf in elements (0 = n_pad); > n_pad when this launch owns a channel slice
   int zf_extent;            // channels of zf that exist in memory (0 = n_pad), as out_extent
-  // mode 2: the images (a prepared launch takes them from each call: patch_conv_epi), the ratio and its bicubic table
+  // mode 2: the images (a prepared launch takes them from each call: patch_conv_epi), the ratio, their channel count and
+  // the bicubic table
   ImageIo img;
   int r;
+  // Channels per pixel of both images: 3 (RGB) or 4 (RGBA, MZ_FLAG_RGBA: colour 0..2, then a straight alpha that the
+  // network never reads; the head writes its bicubic resampling -- a colour skip's arithmetic started from 0 instead of
+  // the accumulator).  Part of the images (patch_conv_epi replaces it with img), kept here, in what was padding after r,
+  // so that every field the RGB kernels read stays where it was.
+  int nc;
   // fp16 range guard: a kernel that is about to round a value beyond +-65504 into a 16-bit fp16 operand (where
   // cvt.rn.satfinite would clip it silently) writes 1 here.  Points at a host-mapped word owned by the mz_model
   // (mz_model_saturated); nullptr = not tracked (per-kernel entry points).
@@ -86,23 +93,25 @@ struct EpiParams {
 // largest finite fp16: a pre-rounding magnitude above it saturates the operand
 #define MZ_F16_MAX 65504.0f
 
-// address of colour c of HR pixel (y r + i, x r + j) of image b in the output of mode 2, or -1 outside the window;
-// YN: interleaved output (ImageIo::y_nhwc)
-template <bool YN>
+// address of channel c of HR pixel (y r + i, x r + j) of image b in the output of mode 2, or -1 outside the window;
+// YN: interleaved output (ImageIo::y_nhwc); CH: channels per pixel (EpiParams::nc)
+template <bool YN, int CH = 3>
 __host__ __device__ inline long long head_out_index_l(const EpiParams& p, int b, int c, int y, int x, int i, int j) {
   const ImageIo& io = p.img;
   const long long WR = static_cast<long long>(p.W) * p.r, HR = static_cast<long long>(p.H) * p.r;
   if (io.wy1 > 0 && (y < io.wy0 || y >= io.wy1 || x < io.wx0 || x >= io.wx1)) return -1;
   if (YN) {
-    const long long row = io.y_row ? io.y_row : 3 * WR, img = io.y_plane ? io.y_plane : 3 * HR * WR;
+    const long long row = io.y_row ? io.y_row : CH * WR, img = io.y_plane ? io.y_plane : CH * HR * WR;
     return static_cast<long long>(b) * img + (static_cast<long long>(y - io.wy0) * p.r + i) * row +
-           (static_cast<long long>(x - io.wx0) * p.r + j) * 3 + c;
+           (static_cast<long long>(x - io.wx0) * p.r + j) * CH + c;
   }
   const long long row = io.y_row ? io.y_row : WR, plane = io.y_plane ? io.y_plane : HR * WR;
-  return (static_cast<long long>(b) * 3 + c) * plane + (static_cast<long long>(y - io.wy0) * p.r + i) * row +
+  return (static_cast<long long>(b) * CH + c) * plane + (static_cast<long long>(y - io.wy0) * p.r + i) * row +
          static_cast<long long>(x - io.wx0) * p.r + j;
 }
 __host__ __device__ inline long long head_out_index(const EpiParams& p, int b, int c, int y, int x, int i, int j) {
+  if (p.nc == 4)
+    return p.img.y_nhwc ? head_out_index_l<true, 4>(p, b, c, y, x, i, j) : head_out_index_l<false, 4>(p, b, c, y, x, i, j);
   return p.img.y_nhwc ? head_out_index_l<true>(p, b, c, y, x, i, j) : head_out_index_l<false>(p, b, c, y, x, i, j);
 }
 
@@ -150,8 +159,8 @@ struct alignas(64) ConvLaunch {
 };
 int prepare_conv_tc(const ConvArgs& a, const ConvTcTune& tune, int device, ConvLaunch* out);
 int run_conv_tc(ConvLaunch& launch, cudaStream_t s);
-// head (mode 2) only: replace the images (EpiParams::img) of a prepared launch (a new layout swaps the kernel
-// instantiation)
+// head (mode 2) only: replace the images (EpiParams::img and nc) of a prepared launch (a new layout or channel count
+// swaps the kernel instantiation)
 int patch_conv_epi(ConvLaunch& launch, const EpiParams& e);
 // ---- one encoder block as one kernel (block_fused.cu): zf += conv2(SiLU(FiLM(conv1(zb_in)))), zb_out = round16(zf) ----
 struct FusedBlockArgs {
@@ -193,9 +202,10 @@ bool seg_gemm_tc_applies(const float* a0, const float* a1, const float* wt, cons
 int launch_seg_gemm_tc(const SgArgs& a, cudaStream_t s);
 
 int launch_bicubic(const float* x, float* y, int planes, int H, int W, int r, cudaStream_t s);
-// image x (element type `type`, interleaved when x_nhwc: as ImageIo) -> fp32 stream zf + 16-bit shadow zb (pitch zb_pitch)
-int launch_stem(const void* x, int type, int x_nhwc, const float* w, const float* bias, float* zf, uint16_t* zb, int bf16,
-                int B, int H, int W, int Cp, int zb_pitch, cudaStream_t s, unsigned int* sat = nullptr);
+// image x (element type `type`, interleaved when x_nhwc, nc = 3 or 4 channels: as ImageIo; colour 0..2 only is read)
+// -> fp32 stream zf + 16-bit shadow zb (pitch zb_pitch)
+int launch_stem(const void* x, int type, int x_nhwc, int nc, const float* w, const float* bias, float* zf, uint16_t* zb,
+                int bf16, int B, int H, int W, int Cp, int zb_pitch, cudaStream_t s, unsigned int* sat = nullptr);
 // film: [L][hCp / ns][B][2][ns] -- one [B][2][ns] table (scale row, shift row) per conv1 launch; ns == hCp normally
 int launch_film(const float* c, int c_rows, const float* w, const float* b, float* film, int L, int B, int F,
                 int hC, int hCp, int ns, cudaStream_t s);
@@ -327,11 +337,42 @@ __device__ __forceinline__ uint32_t pack_u16x2(uint16_t lo, uint16_t hi) {
 }
 // R contiguous values v of the HR image, quantised to T and stored at element d of y: fp32 clamped when clamp01 is set,
 // 8 and 16 bits always (to_u8 / to_u16).  R = 2 or 4 leave in one vector store (fp32: float2 / float4; 8 bits:
-// u16 / u32; 16 bits: u32 / 8 bytes), any other R element by element.
+// u16 / u32; 16 bits: u32 / 8 bytes), any other R up to 4 element by element.  R = 8, 12, 16 (an interleaved RGBA row
+// segment of a pixel at r = 2, 3, 4) are packed into 32-bit words and leave in the widest vectors that divide their
+// R * sizeof(T) bytes, up to 16: fp32 in 16-byte stores; 16 bits in 16-byte stores at R = 8 and 16, 8-byte ones at
+// R = 12; 8 bits in one 8-byte store at R = 8, three 4-byte ones at R = 12 and one 16-byte store at R = 16.
 template <typename T, int R>
 __device__ __forceinline__ void store_px(const ImageIo& io, size_t d, const float* v) {
   T* dst = static_cast<T*>(io.y) + d;
-  if constexpr (std::is_same_v<T, float>) {
+  if constexpr (R > 4) {
+    static_assert(R % 4 == 0, "a wide run is whole RGBA pixels");
+    constexpr int NW = R * static_cast<int>(sizeof(T)) / 4;  // 32-bit words of the run
+    constexpr int VB = (NW % 4 == 0) ? 16 : ((NW % 2 == 0) ? 8 : 4);
+    uint32_t w[NW];
+#pragma unroll
+    for (int k = 0; k < NW; ++k) {
+      if constexpr (std::is_same_v<T, float>) {
+        w[k] = __float_as_uint(io.clamp01 ? fminf(fmaxf(v[k], 0.f), 1.f) : v[k]);
+      } else if constexpr (std::is_same_v<T, uint8_t>) {
+        w[k] = 0;
+#pragma unroll
+        for (int q = 0; q < 4; ++q) w[k] |= static_cast<uint32_t>(to_u8(v[4 * k + q], io.u8_trunc)) << (8 * q);
+      } else {
+        static_assert(std::is_same_v<T, uint16_t>, "HR images are fp32, 8 or 16 bits");
+        w[k] = pack_u16x2(to_u16(v[2 * k]), to_u16(v[2 * k + 1]));
+      }
+    }
+    char* b = reinterpret_cast<char*>(dst);
+#pragma unroll
+    for (int k = 0; k < NW; k += VB / 4) {
+      if constexpr (VB == 16)
+        *reinterpret_cast<uint4*>(b + 4 * k) = make_uint4(w[k], w[k + 1], w[k + 2], w[k + 3]);
+      else if constexpr (VB == 8)
+        *reinterpret_cast<uint2*>(b + 4 * k) = make_uint2(w[k], w[k + 1]);
+      else
+        *reinterpret_cast<uint32_t*>(b + 4 * k) = w[k];
+    }
+  } else if constexpr (std::is_same_v<T, float>) {
     float q[R];
 #pragma unroll
     for (int j = 0; j < R; ++j) q[j] = io.clamp01 ? fminf(fmaxf(v[j], 0.f), 1.f) : v[j];
@@ -382,8 +423,8 @@ __device__ __forceinline__ void store_out(const ImageIo& io, size_t d, const flo
     store_px<float, R>(io, d, v);
 }
 
-// Bicubic value of HR pixel (oy, ox) of one colour (H x W, fp32 | u8 | u16, pixels `ps` elements apart: 1 planar, 3
-// interleaved): 16 clamped taps, rows first.
+// Bicubic value of HR pixel (oy, ox) of one channel (H x W, fp32 | u8 | u16, pixels `ps` elements apart: 1 planar, 3
+// or 4 interleaved): 16 clamped taps, rows first.
 template <typename T>
 __device__ __forceinline__ float bicubic_at(const T* __restrict__ plane, int H, int W, int ps, const BicubicTable& bt,
                                             int oy, int ox) {
@@ -406,9 +447,20 @@ __device__ __forceinline__ float bicubic_at(const T* __restrict__ plane, int H, 
   return acc;
 }
 
+// skip of channel c at HR pixel (oy, ox) of image b, read from x in its element type and layout (epi_head)
+__device__ __forceinline__ float head_skip_at(const EpiParams& p, int b, int c, int oy, int ox) {
+  const int nc = p.nc == 4 ? 4 : 3;
+  const size_t HW = static_cast<size_t>(p.H) * p.W;
+  const size_t pl = p.img.x_nhwc ? static_cast<size_t>(b) * nc * HW + c : (static_cast<size_t>(b) * nc + c) * HW;
+  const int ps = p.img.x_nhwc ? nc : 1;
+  return p.img.type == kImgU16 ? bicubic_at(static_cast<const uint16_t*>(p.img.x) + pl, p.H, p.W, ps, p.bt, oy, ox)
+         : p.img.type == kImgU8 ? bicubic_at(static_cast<const uint8_t*>(p.img.x) + pl, p.H, p.W, ps, p.bt, oy, ox)
+                                : bicubic_at(static_cast<const float*>(p.img.x) + pl, p.H, p.W, ps, p.bt, oy, ox);
+}
 // mode 2: all head channels of LR pixel (b, y, x): acc[n], n = c*r*r + i*r + j  ->  y[b, c, y*r+i, x*r+j]
 // (PixelShuffle index rule, reference model.py:911,928) plus the global skip (model.py:162) and the clamp
-// of upscale() (model.py:177).
+// of upscale() (model.py:177).  An RGBA image's alpha (EpiParams::nc == 4) is the skip alone, channel 3's bicubic
+// resampling with no accumulator (a loop over its r*r phases at run time).
 template <int NMAX>
 __device__ __forceinline__ void epi_head(const EpiParams& p, int b, int y, int x, const float (&acc)[NMAX]) {
   const int r = p.r, rr = r * r;
@@ -416,29 +468,136 @@ __device__ __forceinline__ void epi_head(const EpiParams& p, int b, int y, int x
   for (int n = 0; n < NMAX; ++n) {
     if (n < 3 * rr) {
       const int c = n / rr, i = (n % rr) / r, j = n % r;
-      const int oy = y * r + i, ox = x * r + j;
       const long long di = head_out_index(p, b, c, y, x, i, j);
       if (di < 0) continue;
       float v = acc[n];
-      if (p.img.skip_mode == 1) {
+      if (p.img.skip_mode == 1)
         v += static_cast<const float*>(p.img.y)[di];
-      } else if (p.img.skip_mode == 2) {
-        const size_t HW = static_cast<size_t>(p.H) * p.W;
-        const size_t pl = p.img.x_nhwc ? static_cast<size_t>(b) * 3 * HW + c : (static_cast<size_t>(b) * 3 + c) * HW;
-        const int ps = p.img.x_nhwc ? 3 : 1;
-        v += p.img.type == kImgU16 ? bicubic_at(static_cast<const uint16_t*>(p.img.x) + pl, p.H, p.W, ps, p.bt, oy, ox)
-             : p.img.type == kImgU8 ? bicubic_at(static_cast<const uint8_t*>(p.img.x) + pl, p.H, p.W, ps, p.bt, oy, ox)
-                                    : bicubic_at(static_cast<const float*>(p.img.x) + pl, p.H, p.W, ps, p.bt, oy, ox);
-      }
+      else if (p.img.skip_mode == 2)
+        v += head_skip_at(p, b, c, y * r + i, x * r + j);
+      store_out<1>(p.img, di, &v, p.img.type == kImgU16);
+    }
+  }
+  if (p.nc == 4 && p.img.skip_mode == 2) {  // (RGBA recomputes the skip: check_image_flags)
+    for (int n = 0; n < rr; ++n) {
+      const int i = n / r, j = n % r;
+      const long long di = head_out_index(p, b, 3, y, x, i, j);
+      if (di < 0) continue;
+      const float v = head_skip_at(p, b, 3, y * r + i, x * r + j);
       store_out<1>(p.img, di, &v, p.img.type == kImgU16);
     }
   }
 }
-// One interleaved HR row segment of an LR pixel: v = R pixels x 3 colours at element d, as three stores of R values
-template <int R, bool O16>
-__device__ __forceinline__ void store_hr_row_nhwc(const ImageIo& io, size_t d, const float (&v)[3 * R]) {
+// One interleaved HR row segment of an LR pixel: v = R pixels x CH channels at element d -- RGB as three stores of R
+// values, RGBA (whole pixels, 4R values) as one run in the widest aligned vectors (store_px)
+template <int R, bool O16, int CH = 3>
+__device__ __forceinline__ void store_hr_row_nhwc(const ImageIo& io, size_t d, const float (&v)[CH * R]) {
+  if constexpr (CH == 4) {
+    store_out<4 * R>(io, d, v, O16);
+  } else {
 #pragma unroll
-  for (int k = 0; k < 3; ++k) store_out<R>(io, d + k * R, v + k * R, O16);
+    for (int k = 0; k < 3; ++k) store_out<R>(io, d + k * R, v + k * R, O16);
+  }
+}
+
+// channel 3 (alpha) of image b of an RGBA LR image: interleaved, its first element; planar, its plane
+template <int CH, bool XN, typename T>
+__device__ __forceinline__ const T* alpha_plane(const T* lr, int b, int H, int W) {
+  const size_t HW = static_cast<size_t>(H) * W;
+  return lr + static_cast<size_t>(b) * CH * HW + (XN ? 3 : 3 * HW);
+}
+// The alpha of an RGBA image (EpiParams::nc == 4) at ratio R: the bicubic skip of one channel of LR pixel (y, x), with
+// the loads and FMAs of a colour's skip in epi_head_rt in the same order, each sum started from 0 instead of from the
+// accumulator -- o[i][j] for HR pixel (y R + i, x R + j).  pl: the channel's plane in image b (pixels PS elements
+// apart); interior as in epi_head_rt.
+template <int R, typename T, int PS>
+__device__ __forceinline__ void alpha_skip(const EpiParams& p, const T* __restrict__ pl, int y, int x, bool interior,
+                                           float (&o)[R][R]) {
+  const int H = p.H, W = p.W;
+  int ro[5];
+#pragma unroll
+  for (int k = 0; k < 5; ++k) ro[k] = min(max(y - 2 + k, 0), H - 1) * W * PS;
+  float nb[5][5];
+  if (interior) {
+#pragma unroll
+    for (int k = 0; k < 5; ++k) {
+      const T* rp = pl + (ro[k] + (x - 2) * PS);
+#pragma unroll
+      for (int m = 0; m < 5; ++m) nb[k][m] = lr_px(rp + m * PS);
+    }
+  } else {
+#pragma unroll
+    for (int k = 0; k < 5; ++k)
+#pragma unroll
+      for (int m = 0; m < 5; ++m) nb[k][m] = lr_px(pl + (ro[k] + min(max(x - 2 + m, 0), W - 1) * PS));
+  }
+  float hz[5][R];
+#pragma unroll
+  for (int k = 0; k < 5; ++k)
+#pragma unroll
+    for (int j = 0; j < R; ++j) {
+      const int s = (2 * j + 1 < R) ? 0 : 1;
+      float a = 0.f;
+#pragma unroll
+      for (int m = 0; m < 4; ++m) a = fmaf(nb[k][s + m], p.bt.w[j][m], a);
+      hz[k][j] = a;
+    }
+#pragma unroll
+  for (int i = 0; i < R; ++i) {
+    const int s = (2 * i + 1 < R) ? 0 : 1;
+#pragma unroll
+    for (int j = 0; j < R; ++j) {
+      float a = 0.f;
+#pragma unroll
+      for (int k = 0; k < 4; ++k) a = fmaf(hz[s + k][j], p.bt.w[i][k], a);
+      o[i][j] = a;
+    }
+  }
+}
+// The same for the two LR pixels (y, x) and (y + 1, x) of epi_head2_pair at r = 2: o[rr][i][j] for HR pixel
+// (2 (y + rr) + i, 2 x + j), in epi_head2_pair's order
+template <typename T, int PS>
+__device__ __forceinline__ void alpha_skip_pair(const EpiParams& p, const T* __restrict__ pl, int y, int x, bool interior,
+                                                float (&o)[2][2][2]) {
+  const int H = p.H, W = p.W;
+  int ro[6];
+#pragma unroll
+  for (int k = 0; k < 6; ++k) ro[k] = min(max(y - 2 + k, 0), H - 1) * W * PS;
+  float nb[6][5];
+  if (interior) {
+#pragma unroll
+    for (int k = 0; k < 6; ++k) {
+      const T* rp = pl + (ro[k] + (x - 2) * PS);
+#pragma unroll
+      for (int m = 0; m < 5; ++m) nb[k][m] = lr_px(rp + m * PS);
+    }
+  } else {
+#pragma unroll
+    for (int k = 0; k < 6; ++k)
+#pragma unroll
+      for (int m = 0; m < 5; ++m) nb[k][m] = lr_px(pl + (ro[k] + min(max(x - 2 + m, 0), W - 1) * PS));
+  }
+  float hz[6][2];
+#pragma unroll
+  for (int k = 0; k < 6; ++k)
+#pragma unroll
+    for (int j = 0; j < 2; ++j) {
+      float a = 0.f;
+#pragma unroll
+      for (int m = 0; m < 4; ++m) a = fmaf(nb[k][j + m], p.bt.w[j][m], a);
+      hz[k][j] = a;
+    }
+#pragma unroll
+  for (int rr = 0; rr < 2; ++rr)
+#pragma unroll
+    for (int i = 0; i < 2; ++i)
+#pragma unroll
+      for (int j = 0; j < 2; ++j) {
+        float a = 0.f;
+#pragma unroll
+        for (int k = 0; k < 4; ++k) a = fmaf(hz[rr + i + k][j], p.bt.w[i][k], a);
+        o[rr][i][j] = a;
+      }
 }
 
 // Same as epi_head with the ratio known at compile time: the 5x5 LR neighbourhood of the pixel is loaded once per
@@ -455,17 +614,21 @@ __device__ __forceinline__ void store_hr_row_nhwc(const ImageIo& io, size_t d, c
 // the code it was.  Interleaved, the taps of one colour are 3 elements apart (same FMA order per colour: bit-identical
 // results) and each HR row of the pixel leaves as 3R contiguous values.
 // T = uint16_t: 16-bit images on both sides (MZ_FLAG_IO_U16) -- the 16-bit heads are instantiations of their own.
-template <int R, typename T, bool XN, bool YN>
+// CH = 4: RGBA images (EpiParams::nc) -- pixels 4 elements apart when interleaved, images 4 planes apart when planar, and
+// the alpha (alpha_skip) written beside the colour: interleaved output computes it before the stores and leaves every
+// HR row segment of the pixel as one run of 4R values (alpha live with the colour: 4R^2 more registers at the peak);
+// planar output computes it after the colour stores, once out[3][R][R] is dead, and stores it as a fourth plane.
+template <int R, typename T, bool XN, bool YN, int CH = 3>
 __device__ __forceinline__ void epi_head_rt(const EpiParams& p, const T* __restrict__ lr, int b, int y, int x,
                                             const float (&acc)[48], bool interior) {
   constexpr bool O16 = std::is_same_v<T, uint16_t>;
   const int H = p.H, W = p.W;
-  const long long first = head_out_index_l<YN>(p, b, 0, y, x, 0, 0);
+  const long long first = head_out_index_l<YN, CH>(p, b, 0, y, x, 0, 0);
   if (first < 0) return;  // outside the output window
-  const size_t row_pitch = p.img.y_row ? static_cast<size_t>(p.img.y_row) : static_cast<size_t>(W) * R * (YN ? 3 : 1);
+  const size_t row_pitch = p.img.y_row ? static_cast<size_t>(p.img.y_row) : static_cast<size_t>(W) * R * (YN ? CH : 1);
   const size_t plane_pitch = p.img.y_plane ? static_cast<size_t>(p.img.y_plane) : static_cast<size_t>(H) * R * W * R;
   constexpr int NC = (R == 2) ? 3 : 1;  // colours whose taps are in flight together
-  constexpr int PS = XN ? 3 : 1;        // elements between horizontally adjacent LR pixels of one colour
+  constexpr int PS = XN ? CH : 1;       // elements between horizontally adjacent LR pixels of one channel
   float out[3][R][R];
 #pragma unroll
   for (int c = 0; c < 3; ++c)
@@ -476,7 +639,7 @@ __device__ __forceinline__ void epi_head_rt(const EpiParams& p, const T* __restr
 
   if (p.img.skip_mode == 2) {
     const size_t HW = static_cast<size_t>(H) * W;
-    const T* img = lr + static_cast<size_t>(b) * 3 * HW;
+    const T* img = lr + static_cast<size_t>(b) * CH * HW;
     int xo[5], ro[5];  // (a colour plane is below 2^31 pixels: prepare_conv_tc checks; an interleaved image is below
                        // 2^31 elements: upscale_impl checks)
 #pragma unroll
@@ -532,14 +695,18 @@ __device__ __forceinline__ void epi_head_rt(const EpiParams& p, const T* __restr
   }
 
   if constexpr (YN) {  // (no skip-from-buffer: the API refuses it with interleaved images)
+    float al[R][R];
+    if constexpr (CH == 4) alpha_skip<R, T, PS>(p, alpha_plane<CH, XN>(lr, b, H, W), y, x, interior, al);
 #pragma unroll
     for (int i = 0; i < R; ++i) {
-      float v[3 * R];
+      float v[CH * R];
 #pragma unroll
-      for (int j = 0; j < R; ++j)
+      for (int j = 0; j < R; ++j) {
 #pragma unroll
-        for (int c = 0; c < 3; ++c) v[3 * j + c] = out[c][i][j];
-      store_hr_row_nhwc<R, O16>(p.img, static_cast<size_t>(first) + static_cast<size_t>(i) * row_pitch, v);
+        for (int c = 0; c < 3; ++c) v[CH * j + c] = out[c][i][j];
+        if constexpr (CH == 4) v[CH * j + 3] = al[i][j];
+      }
+      store_hr_row_nhwc<R, O16, CH>(p.img, static_cast<size_t>(first) + static_cast<size_t>(i) * row_pitch, v);
     }
     return;
   }
@@ -576,36 +743,44 @@ __device__ __forceinline__ void epi_head_rt(const EpiParams& p, const T* __restr
 #pragma unroll
     for (int i = 0; i < R; ++i)
       store_out<R>(p.img, static_cast<size_t>(first) + c * plane_pitch + static_cast<size_t>(i) * row_pitch, out[c][i], O16);
+  if constexpr (CH == 4) {  // (RGBA always recomputes the skip: check_image_flags)
+    float al[R][R];
+    alpha_skip<R, T, PS>(p, alpha_plane<CH, XN>(lr, b, H, W), y, x, interior, al);
+#pragma unroll
+    for (int i = 0; i < R; ++i)
+      store_out<R>(p.img, static_cast<size_t>(first) + 3 * plane_pitch + static_cast<size_t>(i) * row_pitch, al[i], O16);
+  }
 }
 // interior: warp-uniform promise that x - 2 >= 0 and x + 2 < W for every lane of the calling warp
 // (the layouts and the 16-bit image type, I16, are template parameters of the calling kernel: one runtime branch over
 // four layouts in the same kernel raises the planar head's registers and makes it spill)
-template <int R, bool XN, bool YN, bool I16>
+template <int R, bool XN, bool YN, bool I16, int CH = 3>
 __device__ __forceinline__ void epi_head_r(const EpiParams& p, int b, int y, int x, const float (&acc)[48], bool interior) {
   if constexpr (I16)
-    epi_head_rt<R, uint16_t, XN, YN>(p, static_cast<const uint16_t*>(p.img.x), b, y, x, acc, interior);
+    epi_head_rt<R, uint16_t, XN, YN, CH>(p, static_cast<const uint16_t*>(p.img.x), b, y, x, acc, interior);
   else if (p.img.type == kImgU8)
-    epi_head_rt<R, uint8_t, XN, YN>(p, static_cast<const uint8_t*>(p.img.x), b, y, x, acc, interior);
+    epi_head_rt<R, uint8_t, XN, YN, CH>(p, static_cast<const uint8_t*>(p.img.x), b, y, x, acc, interior);
   else
-    epi_head_rt<R, float, XN, YN>(p, static_cast<const float*>(p.img.x), b, y, x, acc, interior);
+    epi_head_rt<R, float, XN, YN, CH>(p, static_cast<const float*>(p.img.x), b, y, x, acc, interior);
 }
 // r = 2, TWO vertically adjacent LR pixels (y, x) and (y + 1, x) per thread: their 5x5 neighbourhoods share four of
 // five rows, so the pair costs 6 x 5 loads and 6 x 2 horizontal interpolations per colour instead of 2 x (5 x 5) and
 // 2 x (5 x 2), and -- what matters for the latency-bound epilogue warps -- ONE exposed load latency instead of two.
 // Same FMA order per output as epi_head_rt<2>: the results are bit-identical.  v0 / v1: the twelve head channels of the
-// two pixels as they come out of TMEM; second: row y + 1 exists (y + 1 < H).  XN / YN as in epi_head_rt.
-template <typename T, bool XN, bool YN>
+// two pixels as they come out of TMEM; second: row y + 1 exists (y + 1 < H).  XN / YN / CH as in epi_head_rt (the alpha
+// of both pixels: alpha_skip_pair).
+template <typename T, bool XN, bool YN, int CH = 3>
 __device__ __forceinline__ void epi_head2_pair(const EpiParams& p, const T* __restrict__ lr, int b, int y, int x,
                                                const uint32_t (&v0)[16], const uint32_t (&v1)[16], bool interior,
                                                bool second) {
   constexpr bool O16 = std::is_same_v<T, uint16_t>;  // 16-bit images on both sides, as in epi_head_rt
   const int H = p.H, W = p.W;
   long long first[2];
-  first[0] = head_out_index_l<YN>(p, b, 0, y, x, 0, 0);
-  first[1] = second ? head_out_index_l<YN>(p, b, 0, y + 1, x, 0, 0) : -1;
+  first[0] = head_out_index_l<YN, CH>(p, b, 0, y, x, 0, 0);
+  first[1] = second ? head_out_index_l<YN, CH>(p, b, 0, y + 1, x, 0, 0) : -1;
   if (first[0] < 0 && first[1] < 0) return;  // both outside the output window
-  const size_t row_pitch = p.img.y_row ? static_cast<size_t>(p.img.y_row) : static_cast<size_t>(W) * 2 * (YN ? 3 : 1);
-  constexpr int PS = XN ? 3 : 1;  // elements between horizontally adjacent LR pixels of one colour
+  const size_t row_pitch = p.img.y_row ? static_cast<size_t>(p.img.y_row) : static_cast<size_t>(W) * 2 * (YN ? CH : 1);
+  constexpr int PS = XN ? CH : 1;  // elements between horizontally adjacent LR pixels of one channel
   const size_t plane_pitch = p.img.y_plane ? static_cast<size_t>(p.img.y_plane) : static_cast<size_t>(H) * 2 * W * 2;
   float out[2][3][2][2];
 #pragma unroll
@@ -619,7 +794,7 @@ __device__ __forceinline__ void epi_head2_pair(const EpiParams& p, const T* __re
       }
   if (p.img.skip_mode == 2) {
     const size_t HW = static_cast<size_t>(H) * W;
-    const T* img = lr + static_cast<size_t>(b) * 3 * HW;
+    const T* img = lr + static_cast<size_t>(b) * CH * HW;
     int xo[5], ro[6];
 #pragma unroll
     for (int m = 0; m < 5; ++m) xo[m] = min(max(x - 2 + m, 0), W - 1) * PS;
@@ -669,17 +844,21 @@ __device__ __forceinline__ void epi_head2_pair(const EpiParams& p, const T* __re
     }
   }
   if constexpr (YN) {  // (no skip-from-buffer: the API refuses it with interleaved images)
+    float al[2][2][2];
+    if constexpr (CH == 4) alpha_skip_pair<T, PS>(p, alpha_plane<CH, XN>(lr, b, H, W), y, x, interior, al);
 #pragma unroll
     for (int rr = 0; rr < 2; ++rr) {
       if (first[rr] < 0) continue;
 #pragma unroll
       for (int i = 0; i < 2; ++i) {
-        float v[6];
+        float v[2 * CH];
 #pragma unroll
-        for (int j = 0; j < 2; ++j)
+        for (int j = 0; j < 2; ++j) {
 #pragma unroll
-          for (int c = 0; c < 3; ++c) v[3 * j + c] = out[rr][c][i][j];
-        store_hr_row_nhwc<2, O16>(p.img, static_cast<size_t>(first[rr]) + static_cast<size_t>(i) * row_pitch, v);
+          for (int c = 0; c < 3; ++c) v[CH * j + c] = out[rr][c][i][j];
+          if constexpr (CH == 4) v[CH * j + 3] = al[rr][i][j];
+        }
+        store_hr_row_nhwc<2, O16, CH>(p.img, static_cast<size_t>(first[rr]) + static_cast<size_t>(i) * row_pitch, v);
       }
     }
     return;
@@ -716,16 +895,28 @@ __device__ __forceinline__ void epi_head2_pair(const EpiParams& p, const T* __re
         store_out<2>(p.img, static_cast<size_t>(first[rr]) + c * plane_pitch + static_cast<size_t>(i) * row_pitch,
                      out[rr][c][i], O16);
   }
+  if constexpr (CH == 4) {  // after the colour stores (out is dead); RGBA always recomputes the skip
+    float al[2][2][2];
+    alpha_skip_pair<T, PS>(p, alpha_plane<CH, XN>(lr, b, H, W), y, x, interior, al);
+#pragma unroll
+    for (int rr = 0; rr < 2; ++rr) {
+      if (first[rr] < 0) continue;
+#pragma unroll
+      for (int i = 0; i < 2; ++i)
+        store_out<2>(p.img, static_cast<size_t>(first[rr]) + 3 * plane_pitch + static_cast<size_t>(i) * row_pitch, al[rr][i],
+                     O16);
+    }
+  }
 }
-template <bool XN, bool YN, bool I16>
+template <bool XN, bool YN, bool I16, int CH = 3>
 __device__ __forceinline__ void epi_head2(const EpiParams& p, int b, int y, int x, const uint32_t (&v0)[16],
                                           const uint32_t (&v1)[16], bool interior, bool second) {
   if constexpr (I16)
-    epi_head2_pair<uint16_t, XN, YN>(p, static_cast<const uint16_t*>(p.img.x), b, y, x, v0, v1, interior, second);
+    epi_head2_pair<uint16_t, XN, YN, CH>(p, static_cast<const uint16_t*>(p.img.x), b, y, x, v0, v1, interior, second);
   else if (p.img.type == kImgU8)
-    epi_head2_pair<uint8_t, XN, YN>(p, static_cast<const uint8_t*>(p.img.x), b, y, x, v0, v1, interior, second);
+    epi_head2_pair<uint8_t, XN, YN, CH>(p, static_cast<const uint8_t*>(p.img.x), b, y, x, v0, v1, interior, second);
   else
-    epi_head2_pair<float, XN, YN>(p, static_cast<const float*>(p.img.x), b, y, x, v0, v1, interior, second);
+    epi_head2_pair<float, XN, YN, CH>(p, static_cast<const float*>(p.img.x), b, y, x, v0, v1, interior, second);
 }
 #endif  // __CUDACC__
 

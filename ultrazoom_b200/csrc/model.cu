@@ -164,8 +164,9 @@ static int run_conv(mz_model* m, int slot, const ConvArgs& a, const ConvTcTune& 
   if (a.epi.mode == 2) {
     // The head reads the LR image and writes the HR image through plain pointers (no tensor map): the images are not
     // part of what was prepared -- a fresh output tensor per call must not cost a geometry search and two tensor-map
-    // encodes.  They are patched into the prepared launch below.
+    // encodes.  They and their channel count are patched into the prepared launch below (RGB <-> RGBA swaps the head).
     key.a.epi.img = ImageIo{};
+    key.a.epi.nc = 0;
   }
   // kWays prepared launches per convolution: the host lanes, the engine workspace and captured graphs alternate operands
   for (int way = 0; way < kWays; ++way) {
@@ -594,13 +595,17 @@ static int check_image_flags(uint32_t flags, int H, int W) {
                "upscale: 4:2:0 frames exclude MZ_FLAG_X_NHWC, MZ_FLAG_Y_NHWC, MZ_FLAG_U8_TRUNC and MZ_FLAG_SKIP_FROM_BUFFER");
     MZ_REQUIRE(H % 2 == 0 && W % 2 == 0, "upscale: a 4:2:0 frame has even dimensions, %d x %d given", H, W);
   }
+  MZ_REQUIRE(!(flags & MZ_FLAG_RGBA) || !(flags & (MZ_FLAG_YUV420 | MZ_FLAG_SKIP_FROM_BUFFER)),
+             "upscale: RGBA images (MZ_FLAG_RGBA) exclude MZ_FLAG_YUV420 and MZ_FLAG_SKIP_FROM_BUFFER");
   return MZ_OK;
 }
-// bytes of one image: 3HW elements of fp32, 8 or 16 bits, or a 4:2:0 frame of 3HW/2
+// channels per pixel of an image: 4 with MZ_FLAG_RGBA, otherwise 3
+static int image_channels(uint32_t flags) { return (flags & MZ_FLAG_RGBA) ? 4 : 3; }
+// bytes of one image: 3HW (RGBA: 4HW) elements of fp32, 8 or 16 bits, or a 4:2:0 frame of 3HW/2
 static size_t image_bytes(uint32_t flags, int H, int W) {
   const size_t es = (flags & MZ_FLAG_IO_U8) ? 1 : ((flags & MZ_FLAG_IO_U16) ? 2 : sizeof(float));
   const size_t px = static_cast<size_t>(H) * W;
-  return (flags & MZ_FLAG_YUV420) ? px * 3 / 2 * es : px * 3 * es;
+  return (flags & MZ_FLAG_YUV420) ? px * 3 / 2 * es : px * image_channels(flags) * es;
 }
 
 // layer_begin / layer_end: the encoder blocks [layer_begin, layer_end) of this call (mz_upscale_stage).  The FiLM table and
@@ -618,6 +623,7 @@ static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, in
   const bool yuv = (flags & MZ_FLAG_YUV420) != 0;
   MZ_REQUIRE(!yuv || (!win && front && back), "upscale: 4:2:0 frames are neither windowed nor staged");
   ImageIo img{};
+  const int nc = image_channels(flags);
   img.x = x_dev_v;
   img.y = y_dev_v;
   img.type = (flags & MZ_FLAG_IO_U8) ? kImgU8 : ((flags & MZ_FLAG_IO_U16) ? kImgU16 : kImgF32);
@@ -636,8 +642,8 @@ static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, in
   }
   MZ_REQUIRE(!((img.x_nhwc || img.y_nhwc) && img.skip_mode == 1),
              "upscale: interleaved images (MZ_FLAG_X_NHWC / MZ_FLAG_Y_NHWC) recompute the skip (no MZ_FLAG_SKIP_FROM_BUFFER)");
-  MZ_REQUIRE(!(img.x_nhwc || img.y_nhwc) || static_cast<long long>(H) * W * 3 < (1LL << 31),
-             "upscale: an interleaved %d x %d image exceeds 2^31 elements", H, W);
+  MZ_REQUIRE(!(img.x_nhwc || img.y_nhwc) || static_cast<long long>(H) * W * nc < (1LL << 31),
+             "upscale: an interleaved %d x %d x %d image exceeds 2^31 elements", H, W, nc);
   MZ_REQUIRE(B > 0 && H > 0 && W > 0, "upscale: empty input (B %d, H %d, W %d)", B, H, W);
   if (m->F > 0) {
     MZ_REQUIRE(c_dev != nullptr, "Control vector c is required for control models.");
@@ -685,7 +691,7 @@ static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, in
   }
   rc = MZ_OK;
   if (front)
-    rc = launch_stem(img.x, img.type, img.x_nhwc, m->stem_w, m->stem_b, zf, zb, m->bf16, B, H, W, m->Cpm, m->Czm, s,
+    rc = launch_stem(img.x, img.type, img.x_nhwc, nc, m->stem_w, m->stem_b, zf, zb, m->bf16, B, H, W, m->Cpm, m->Czm, s,
                      m->sat_dev);
   if (rc != MZ_OK) return rc;
 
@@ -801,6 +807,7 @@ static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, in
   a.epi.n_pad = m->headNp;
   a.epi.img = img;
   a.epi.r = m->r;
+  a.epi.nc = nc;
   make_bicubic_table(m->r, &a.epi.bt);
   return simt ? launch_conv_simt(a, s) : run_conv(m, m->L * (S + S2), a, m->tune[2], s);
 }
@@ -820,14 +827,18 @@ int mz_upscale_window(mz_model* m, const void* x_dev, const float* c_dev, int32_
   MZ_REQUIRE(0 <= win_y0 && win_y0 < win_y1 && win_y1 <= H && 0 <= win_x0 && win_x0 < win_x1 && win_x1 <= W,
              "upscale_window: window [%d, %d) x [%d, %d) is not inside the %d x %d input", win_y0, win_y1, win_x0, win_x1,
              H, W);
-  const int64_t r = m->r, ch = (flags & MZ_FLAG_Y_NHWC) ? 3 : 1;  // (elements per HR pixel in a row)
+  const int64_t r = m->r, ch = (flags & MZ_FLAG_Y_NHWC) ? image_channels(flags) : 1;  // (elements per HR pixel in a row)
   MZ_REQUIRE(y_row_pitch >= (win_x1 - win_x0) * r * ch && y_plane_pitch >= y_row_pitch * (win_y1 - win_y0) * r,
              "upscale_window: pitches (%lld, %lld) are smaller than the window", static_cast<long long>(y_row_pitch),
              static_cast<long long>(y_plane_pitch));
   MZ_REQUIRE(!(flags & MZ_FLAG_SKIP_FROM_BUFFER), "upscale_window: the bicubic skip is recomputed (no MZ_FLAG_SKIP_FROM_BUFFER)");
   MZ_REQUIRE(!(flags & MZ_FLAG_YUV420), "upscale_window: 4:2:0 frames (MZ_FLAG_YUV420) cannot be windowed");
-  // bytes of one vector store: the same in both layouts (an interleaved HR row segment of a pixel is three of them)
-  const int es = (flags & MZ_FLAG_IO_U8) ? 1 : ((flags & MZ_FLAG_IO_U16) ? 2 : 4), vec = m->r == 3 ? es : es * m->r;
+  // bytes of one vector store: RGB the same in both layouts (an interleaved HR row segment of a pixel is three of them);
+  // interleaved RGBA stores a pixel's row segment of 4r values in the widest vectors that divide its 4r es bytes, up to 16
+  const int es = (flags & MZ_FLAG_IO_U8) ? 1 : ((flags & MZ_FLAG_IO_U16) ? 2 : 4), seg = 4 * m->r * es;
+  const int vec = ((flags & MZ_FLAG_RGBA) && (flags & MZ_FLAG_Y_NHWC)) ? (seg % 16 == 0 ? 16 : (seg % 8 == 0 ? 8 : 4))
+                  : m->r == 3                                        ? es
+                                                                     : es * m->r;
   MZ_REQUIRE(reinterpret_cast<uintptr_t>(y_dev) % vec == 0 && (y_row_pitch * es) % vec == 0 && (y_plane_pitch * es) % vec == 0,
              "upscale_window: y and its pitches must be aligned to %d bytes", vec);
   const OutWindow w{win_y0, win_y1, win_x0, win_x1, y_row_pitch, y_plane_pitch};

@@ -152,15 +152,17 @@ int launch_bicubic(const float* x, float* y, int planes, int H, int W, int r, cu
 }
 
 // ----------------------------------------------------------------------------------------------
-// stem: x (B,3,H,W) -> zf (B,H,W,Cp) fp32 and zb (B,H,W,Cz) 16-bit; z = W x + bias,
+// stem: x (B,3,H,W) or (B,4,H,W) -> zf (B,H,W,Cp) fp32 and zb (B,H,W,Cz) 16-bit; z = W x + bias,
 // channels >= C are written as zero (w/bias are zero-padded to Cp by the caller).
 // A store-only stream (12 B read, 6 Cp B written per pixel).  One thread -> 4 channels of one pixel, threads of a
 // block laid out channel-fastest over consecutive pixels: a warp's fp32 store is 512 contiguous bytes, its 16-bit
 // store 256 (the first version's 8 channels per thread wrote every other 16 bytes of a 1 KB span per instruction:
 // 1.67 x the L2 sectors, ncu l1tex 75 % busy at 62 % of the DRAM peak).  The block first stages the three colour
 // planes of its pixel range in shared memory with coalesced loads, so the store loop never waits for a global load.
-// x_nhwc: x is interleaved (B,H,W,3); images are 3HW elements apart in both layouts, so the block's pixel range is one
-// contiguous run of 3n elements even across images, read with coalesced loads into the same planar staging.
+// x_nhwc: x is interleaved (B,H,W,nc); images are nc HW elements apart in both layouts, so the block's pixel range is
+// one contiguous run of nc n elements even across images, read with coalesced loads into the same planar staging.
+// nc = 4 (RGBA): the alpha is skipped (interleaved: not loaded; planar: its plane is not read) -- the stem reads
+// channels 0..2 only and its arithmetic per pixel is the RGB stem's.
 // ----------------------------------------------------------------------------------------------
 __device__ __forceinline__ void st_global_v2(void* p, uint32_t a, uint32_t b) {
   asm volatile("st.global.v2.b32 [%0], {%1, %2};" ::"l"(p), "r"(a), "r"(b) : "memory");
@@ -177,7 +179,7 @@ __device__ __forceinline__ float stem_px(const void* __restrict__ x, int type, s
   }
 }
 
-__global__ void __launch_bounds__(256) stem_kernel(const void* __restrict__ x, int type, int x_nhwc,
+__global__ void __launch_bounds__(256) stem_kernel(const void* __restrict__ x, int type, int x_nhwc, int nc,
                                                    const float* __restrict__ w, const float* __restrict__ bias,
                                                    float* __restrict__ zf, uint16_t* __restrict__ zb, int bf16, int B,
                                                    int H, int W, int Cp, int Cz, int ppb, unsigned int* sat) {
@@ -199,10 +201,10 @@ __global__ void __launch_bounds__(256) stem_kernel(const void* __restrict__ x, i
   const int n = static_cast<int>((p0 + ppb < npix ? p0 + ppb : npix) - p0);
   if (x_nhwc) {
     const int tid = threadIdx.y * blockDim.x + threadIdx.x, nt = blockDim.x * blockDim.y;
-    const size_t e0 = p0 * 3;
-    for (int e = tid; e < 3 * n; e += nt) {
-      const int j = e / 3, c = e - 3 * j;
-      xs[c * ppb + j] = stem_px(x, type, e0 + e);
+    const size_t e0 = p0 * nc;
+    for (int e = tid; e < nc * n; e += nt) {
+      const int j = nc == 4 ? e >> 2 : e / 3, c = e - nc * j;
+      if (c < 3) xs[c * ppb + j] = stem_px(x, type, e0 + e);
     }
   } else {
     const size_t b0 = p0 / plane, rem0 = p0 - b0 * plane;  // (one division per block; the range may cross images)
@@ -213,7 +215,7 @@ __global__ void __launch_bounds__(256) stem_kernel(const void* __restrict__ x, i
         rem -= plane;
         ++b;
       }
-      const size_t xo = b * 3 * plane + rem;
+      const size_t xo = b * nc * plane + rem;
 #pragma unroll
       for (int c = 0; c < 3; ++c) xs[c * ppb + j] = stem_px(x, type, xo + c * plane);
     }
@@ -235,9 +237,10 @@ __global__ void __launch_bounds__(256) stem_kernel(const void* __restrict__ x, i
   if (!bf16 && sat != nullptr && !(amax <= MZ_F16_MAX)) *sat = 1u;  // fp16 range guard (see EpiParams::sat)
 }
 
-int launch_stem(const void* x, int type, int x_nhwc, const float* w, const float* bias, float* zf, uint16_t* zb, int bf16,
-                int B, int H, int W, int Cp, int zb_pitch, cudaStream_t s, unsigned int* sat) {
+int launch_stem(const void* x, int type, int x_nhwc, int nc, const float* w, const float* bias, float* zf, uint16_t* zb,
+                int bf16, int B, int H, int W, int Cp, int zb_pitch, cudaStream_t s, unsigned int* sat) {
   MZ_REQUIRE(Cp > 0 && Cp % 8 == 0, "stem: padded channel count must be a multiple of 8, %d given", Cp);
+  MZ_REQUIRE(nc == 3 || nc == 4, "stem: an image has 3 or 4 channels, %d given", nc);
   MZ_REQUIRE(B > 0 && H > 0 && W > 0, "stem: empty input");
   MZ_REQUIRE(zf != nullptr, "stem: null fp32 stream");
   const int Cz = zb_pitch ? zb_pitch : Cp;
@@ -254,8 +257,8 @@ int launch_stem(const void* x, int type, int x_nhwc, const float* w, const float
   const long long blocks = (npix + ppb - 1) / ppb;
   MZ_REQUIRE(blocks < (1LL << 31), "stem: too many pixels");
   const size_t smem = static_cast<size_t>(3) * ppb * sizeof(float);
-  stem_kernel<<<static_cast<unsigned>(blocks), dim3(groups, py), smem, s>>>(x, type, x_nhwc, w, bias, zf, zb, bf16, B, H, W,
-                                                                         Cp, Cz, static_cast<int>(ppb), sat);
+  stem_kernel<<<static_cast<unsigned>(blocks), dim3(groups, py), smem, s>>>(x, type, x_nhwc, nc, w, bias, zf, zb, bf16, B, H,
+                                                                         W, Cp, Cz, static_cast<int>(ppb), sat);
   MZ_CUDA(cudaGetLastError());
   return MZ_OK;
 }

@@ -27,7 +27,7 @@ from . import _native
 
 
 def _is_nhwc(t: Tensor) -> bool:
-    """``t`` holds interleaved pixels: (B,3,H,W) in ``channels_last`` strides -- what a numpy / PIL / video frame becomes
+    """``t`` holds interleaved pixels: (B,C,H,W) in ``channels_last`` strides -- what a numpy / PIL / video frame becomes
     through ``torch.from_numpy(frames).permute(0, 3, 1, 2)`` -- and not also plainly contiguous."""
     return t.is_contiguous(memory_format=torch.channels_last) and not t.is_contiguous()
 
@@ -85,20 +85,27 @@ def _no_yuv(yuv, what: str) -> None:
     assert yuv is None, f"4:2:0 frames are supported by upscale(), upscale_host() and capture(), not {what}()"
 
 
+def _channel_flag(x: Tensor) -> int:
+    """``MZ_FLAG_RGBA`` for a 4-channel image (colour, then a straight alpha that is resampled, not run through the
+    network), 0 for RGB."""
+    return _native.FLAG_RGBA if x.shape[1] == 4 else 0
+
+
 def _output_flag(memory_format) -> int:
     assert memory_format in (torch.contiguous_format, torch.channels_last), (
         "memory_format must be torch.contiguous_format or torch.channels_last")
     return _native.FLAG_Y_NHWC if memory_format == torch.channels_last else 0
 
 
-def _frame_layout(frame: Tensor):
-    """``(flag, row pitch, image-or-plane pitch)`` of an assembled output frame (B,3,H',W'): interleaved (channels-last
-    strides: ``stride(1) == 1``, ``stride(3) == 3``; rows and images at any pitch) or planar (``stride(3) == 1``, evenly
-    spaced planes)."""
-    if frame.stride(1) == 1 and frame.stride(3) == 3:
+def _frame_layout(frame: Tensor, channels: int = 3):
+    """``(flag, row pitch, image-or-plane pitch)`` of an assembled output frame (B,C,H',W') of ``channels`` channels:
+    interleaved (channels-last strides: ``stride(1) == 1``, ``stride(3) == C``; rows and images at any pitch) or planar
+    (``stride(3) == 1``, evenly spaced planes, images C planes apart)."""
+    if frame.stride(1) == 1 and frame.stride(3) == channels:
         return _native.FLAG_Y_NHWC, frame.stride(2), frame.stride(0)
-    assert frame.stride(3) == 1, "frame must be planar (stride(3) == 1) or interleaved (stride(1) == 1, stride(3) == 3)"
-    assert frame.stride(0) == 3 * frame.stride(1), "frame planes must be evenly spaced"
+    assert frame.stride(3) == 1, (
+        f"frame must be planar (stride(3) == 1) or interleaved (stride(1) == 1, stride(3) == {channels})")
+    assert frame.stride(0) == channels * frame.stride(1), "frame planes must be evenly spaced"
     return 0, frame.stride(2), frame.stride(1)
 
 
@@ -476,7 +483,8 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         if yuv is not None:
             _yuv_dims(x)
         else:
-            assert x.dim() == 4 and x.shape[1] == 3, f"Expected input of shape (B, 3, H, W), got {tuple(x.shape)}."
+            assert x.dim() == 4 and x.shape[1] in (3, 4), (
+                f"Expected input of shape (B, 3, H, W) (RGB) or (B, 4, H, W) (RGBA), got {tuple(x.shape)}.")
             assert x.shape[0] > 0 and x.shape[2] > 0 and x.shape[3] > 0, "Input must not be empty."
         if self.control_features == 0:
             assert c is None, "This model has no control modules; c must be None."
@@ -510,9 +518,9 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
                     f"{str(odt).replace('torch.', '')} images are supported by upscale(), not forward()")
                 flags |= self._image_flags(odt)
             x, xflag = _input_image(x, odt != torch.float32)
-            flags |= xflag | _output_flag(memory_format)
-            B, _, H, W = x.shape
-            out_shape = (B, 3, H * r, W * r)
+            flags |= xflag | _output_flag(memory_format) | _channel_flag(x)
+            B, C_, H, W = x.shape
+            out_shape = (B, C_, H * r, W * r)
         if c is not None:
             c = c.detach().to(device=dev, dtype=torch.float32).contiguous()
         capturing = torch.cuda.is_current_stream_capturing()
@@ -568,7 +576,13 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
 
         ``yuv=Yuv420(...)``: ``x`` is a batch of 4:2:0 video frames ``(B, 3H/2, W)``, uint8 NV12 or uint16 P010, and so is
         the result, ``(B, 3rH/2, rW)``.  It equals ``ops.rgb16_to_yuv420(upscale(ops.yuv420_to_rgb16(x)))`` bit for bit:
-        the frame is upscaled as a 16-bit RGB image, whatever its depth."""
+        the frame is upscaled as a 16-bit RGB image, whatever its depth.
+
+        A 4-channel ``x`` (B, 4, H, W) is RGBA -- ``decode_image(..., mode=ImageReadMode.RGB_ALPHA)``, or an (H, W, 4)
+        PIL / numpy array permuted to channels-last -- and the result is (B, 4, rH, rW) in the same element type and
+        layouts: ``y[:, :3]`` equals ``upscale(x[:, :3])`` bit for bit (the network never reads the alpha), and
+        ``y[:, 3]`` is the bicubic resampling of the straight alpha, the global skip alone, clamped and quantised as the
+        colour is (``forward``: unclamped).  4:2:0 frames have no alpha."""
         return self._run(x, c, _native.FLAG_CLAMP01, memory_format=memory_format, yuv=yuv)
 
     @torch.inference_mode()
@@ -588,8 +602,8 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         pixels ``window = (y0, y1, x0, x1)`` of the tile -- straight into ``frame`` (B,3,rH',rW'), whose HR pixel
         ``at = (fy, fx)`` receives the core's first pixel (mz_upscale_window).  ``frame`` may live on another GPU
         (``sharding.share_frame``): the head kernel's stores are then the transfer over NVLink.  ``frame`` is planar or
-        interleaved (channels-last strides, any row and image pitch, e.g. a view into a wider HWC buffer).  4:2:0 frames
-        cannot be windowed."""
+        interleaved (channels-last strides, any row and image pitch, e.g. a view into a wider HWC buffer).  An RGBA tile
+        (B,4,h,w) goes into a (B,4,rH',rW') frame.  4:2:0 frames cannot be windowed."""
         _no_yuv(yuv, "upscale_into")
         c = self._check_inputs(x, c)
         if not x.is_cuda:
@@ -610,10 +624,11 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         r = self.upscale_ratio
         y0, y1, x0, x1 = window
         fy, fx = at
-        assert frame.is_cuda and frame.dim() == 4 and frame.shape[0] == B and frame.shape[1] == 3, "frame must be (B,3,H',W')"
+        assert frame.is_cuda and frame.dim() == 4 and frame.shape[0] == B and frame.shape[1] == x.shape[1], (
+            f"frame must be (B,{x.shape[1]},H',W') for a {x.shape[1]}-channel input")
         assert frame.dtype == odt, f"frame must be {odt} for a {odt} input, got {frame.dtype}"
-        yflag, row_pitch, img_pitch = _frame_layout(frame)
-        flags |= xflag | yflag
+        yflag, row_pitch, img_pitch = _frame_layout(frame, x.shape[1])
+        flags |= xflag | yflag | _channel_flag(x)
         assert 0 <= fy and fy + (y1 - y0) * r <= frame.shape[2] and 0 <= fx and fx + (x1 - x0) * r <= frame.shape[3], (
             "the window does not fit into the frame at that position")
         if frame.device != dev:
@@ -657,9 +672,10 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         r = self.upscale_ratio
         y0, y1, x0, x1 = window
         fy, fx = at
-        assert frame.is_cuda and frame.dim() == 4 and frame.shape[0] == B and frame.shape[1] == 3
-        yflag, row_pitch, img_pitch = _frame_layout(frame)
-        flags |= xflag | yflag
+        assert frame.is_cuda and frame.dim() == 4 and frame.shape[0] == B and frame.shape[1] == x.shape[1], (
+            f"frame must be (B,{x.shape[1]},H',W') for a {x.shape[1]}-channel input")
+        yflag, row_pitch, img_pitch = _frame_layout(frame, x.shape[1])
+        flags |= xflag | yflag | _channel_flag(x)
         if frame.device != dev:
             _native.check(eng.lib.mz_enable_peer_access(dev.index or 0, frame.device.index or 0))
         stream = torch.cuda.current_stream(dev)
@@ -671,7 +687,8 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
             flags, stream.cuda_stream, layer_begin, layer_end))
 
     def stage_workspace(self, shape, device: torch.device) -> Tensor:
-        """A private workspace for ``upscale_stage`` calls on a (B,3,H,W) tile (the state between stages lives in it)."""
+        """A private workspace for ``upscale_stage`` calls on a (B,3,H,W) or (B,4,H,W) tile (the state between stages
+        lives in it; an alpha channel needs none)."""
         eng = self._engine(torch.device(device))
         need = C.c_size_t()
         _native.check(eng.lib.mz_workspace_bytes(eng.handle, shape[0], shape[2], shape[3], C.byref(need)))
@@ -722,8 +739,9 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         Element types and layouts as in ``upscale`` (uint8 and uint16 frames come back as such): a channels-last ``x`` is
         copied as it is (no transpose on the CPU), and the result is interleaved with
         ``memory_format=torch.channels_last``.  A caller's ``out`` sets the output layout itself: it must be contiguous
-        NCHW or contiguous channels-last, of the input's element type.  With ``yuv``, ``x`` and ``out`` are 4:2:0 frames
-        as in ``upscale`` (contiguous), at 1.5 (NV12) or 3 (P010) bytes per pixel over PCIe."""
+        NCHW or contiguous channels-last, of the input's element type and channel count (RGBA: 4).  With ``yuv``, ``x``
+        and ``out`` are 4:2:0 frames as in ``upscale`` (contiguous), at 1.5 (NV12) or 3 (P010) bytes per pixel over
+        PCIe."""
         c = self._check_inputs(x, c, yuv)
         assert not x.is_cuda, "upscale_host takes host tensors"
         assert lane in (None, 0, 1), "lane must be None, 0 or 1"
@@ -746,15 +764,15 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
             flags = _native.FLAG_CLAMP01 | self._flags_extra | yuv.flags(odt)
         else:
             x, xflag = _input_image(x, odt != torch.float32)
-            B, _, H, W = x.shape
-            out_shape = (B, 3, H * r, W * r)
+            B, C_, H, W = x.shape
+            out_shape = (B, C_, H * r, W * r)
             if out is None:
                 out = torch.empty(out_shape, dtype=odt, memory_format=memory_format)
                 yflag = _output_flag(memory_format)
             else:
                 yflag = _native.FLAG_Y_NHWC if _is_nhwc(out) else 0
                 assert out.is_contiguous() or yflag, "out must be contiguous NCHW or contiguous channels-last"
-            flags = _native.FLAG_CLAMP01 | self._flags_extra | xflag | yflag | self._image_flags(odt)
+            flags = _native.FLAG_CLAMP01 | self._flags_extra | xflag | yflag | self._image_flags(odt) | _channel_flag(x)
         assert tuple(out.shape) == out_shape and out.dtype == odt
         cp, cr = (c.data_ptr(), c.shape[0]) if c is not None else (None, 0)
         if lane is None:

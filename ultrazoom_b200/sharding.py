@@ -162,10 +162,10 @@ def upscale_tiled(fn: Callable[[Tensor, Optional[Tensor]], Tensor], x: Tensor, c
     """Tiled inference, exact w.r.t. the full-image result.  ``tiles`` selects which tile indices THIS
     caller computes (e.g. ``frames_for_rank(rows*cols, rank, world)``); the others are left untouched in
     ``out`` so ranks can fill disjoint parts of a shared / gathered buffer."""
-    B, _, H, W = x.shape
+    B, _, H, W = x.shape      # (3 or 4 channels: the output has x's)
     plan = plan_tiles(H, W, rows, cols, halo_radius(num_encoder_layers), align_w)
     if out is None:
-        out = torch.zeros((B, 3, H * r, W * r), dtype=torch.float32, device=x.device)
+        out = torch.zeros((B, x.shape[1], H * r, W * r), dtype=torch.float32, device=x.device)
     for t in plan:
         if tiles is not None and t.index not in tiles:
             continue
