@@ -342,12 +342,17 @@ def test_invalid_interleaved_calls(dev):
         return eng.lib.mz_upscale_window(eng.handle, x.data_ptr(), c.data_ptr(), B, dst, row, img, B, H, W, 0, H, 0, x1,
                                          ws_ptr, ws_bytes, flags, s)
 
+    def stage(dst, row, img):                                          # the same window, stored by a stage's head
+        return eng.lib.mz_upscale_stage(eng.handle, x.data_ptr(), c.data_ptr(), B, dst, row, img, B, H, W, 0, H, 0, W,
+                                        ws_ptr, ws_bytes, flags, s, 0, m.num_encoder_layers)
+
     assert window(f.data_ptr(), rp, ip) == N.MZ_OK
-    assert window(f.data_ptr() + 8, rp, ip) == N.MZ_ERR_INVALID      # 8 B: not 16-byte aligned
-    assert window(f.data_ptr(), rp - 2, ip) == N.MZ_ERR_INVALID      # row pitch 8 B off alignment
-    assert window(f.data_ptr(), rp, ip - 2) == N.MZ_ERR_INVALID      # image pitch 8 B off alignment
-    assert window(f.data_ptr(), 3 * r * W - 4, ip) == N.MZ_ERR_INVALID  # row pitch smaller than the window's 3 r w
-    assert window(f.data_ptr(), r * W, ip) == N.MZ_ERR_INVALID       # a planar row pitch is too small interleaved
+    for call in (window, stage):
+        assert call(f.data_ptr() + 8, rp, ip) == N.MZ_ERR_INVALID      # 8 B: not 16-byte aligned
+        assert call(f.data_ptr(), rp - 2, ip) == N.MZ_ERR_INVALID      # row pitch 8 B off alignment
+        assert call(f.data_ptr(), rp, ip - 2) == N.MZ_ERR_INVALID      # image pitch 8 B off alignment
+        assert call(f.data_ptr(), 3 * r * W - 4, ip) == N.MZ_ERR_INVALID  # row pitch smaller than the window's 3 r w
+        assert call(f.data_ptr(), r * W, ip) == N.MZ_ERR_INVALID       # a planar row pitch is too small interleaved
     torch.cuda.synchronize()
     # Python: frames in neither layout
     bad = [torch.empty(B, 3, H * r, 2 * W * r, device=dev)[..., ::2],                    # stride(3) == 2

@@ -451,10 +451,15 @@ def test_invalid_rgba_calls(dev):
         return eng.lib.mz_upscale_window(eng.handle, x.data_ptr(), c.data_ptr(), B, dst, row, img, B, H, W, 0, H, 0, W,
                                          ws_ptr, ws_bytes, flags, s)
 
-    assert window(f.data_ptr() + 8, rp, ip) == N.MZ_ERR_INVALID       # 8 B: not 16-byte aligned
-    assert window(f.data_ptr(), rp - 2, ip) == N.MZ_ERR_INVALID       # row pitch 8 B off
-    assert window(f.data_ptr(), rp, ip - 2) == N.MZ_ERR_INVALID       # image pitch 8 B off
-    assert window(f.data_ptr(), 3 * r * W, ip) == N.MZ_ERR_INVALID    # an RGB row pitch is too small for RGBA
+    def stage(dst, row, img):                                          # the same window, stored by a stage's head
+        return eng.lib.mz_upscale_stage(eng.handle, x.data_ptr(), c.data_ptr(), B, dst, row, img, B, H, W, 0, H, 0, W,
+                                        ws_ptr, ws_bytes, flags, s, 0, m.num_encoder_layers)
+
+    for call in (window, stage):
+        assert call(f.data_ptr() + 8, rp, ip) == N.MZ_ERR_INVALID       # 8 B: not 16-byte aligned
+        assert call(f.data_ptr(), rp - 2, ip) == N.MZ_ERR_INVALID       # row pitch 8 B off
+        assert call(f.data_ptr(), rp, ip - 2) == N.MZ_ERR_INVALID       # image pitch 8 B off
+        assert call(f.data_ptr(), 3 * r * W, ip) == N.MZ_ERR_INVALID    # an RGB row pitch is too small for RGBA
     torch.cuda.synchronize()
     assert bool((f == -1.0).all()), "a refused window wrote its frame"
     assert window(f.data_ptr(), rp, ip) == N.MZ_OK

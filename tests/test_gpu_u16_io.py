@@ -400,11 +400,16 @@ def test_invalid_u16_calls(dev):
             return eng.lib.mz_upscale_window(eng.handle, x16.data_ptr(), c.data_ptr(), B, dst, row, img, B, H, W, 0, H, 0,
                                              W, ws_ptr, ws_bytes, flags, s)
 
+        def stage(dst, row, img):                                      # the same window, stored by a stage's head
+            return eng.lib.mz_upscale_stage(eng.handle, x16.data_ptr(), c.data_ptr(), B, dst, row, img, B, H, W, 0, H, 0,
+                                            W, ws_ptr, ws_bytes, flags, s, 0, m.num_encoder_layers)
+
         assert window(f.data_ptr(), rp, ip) == N.MZ_OK
-        assert window(f.data_ptr() + 2, rp, ip) == N.MZ_ERR_INVALID   # 2 B: not 8-byte aligned
-        assert window(f.data_ptr() + 4, rp, ip) == N.MZ_ERR_INVALID   # 4 B: not 8-byte aligned
-        assert window(f.data_ptr(), rp + 2, ip) == N.MZ_ERR_INVALID   # row pitch 4 B off alignment
-        assert window(f.data_ptr(), rp, ip + 1) == N.MZ_ERR_INVALID   # image pitch 2 B off alignment
+        for call in (window, stage):
+            assert call(f.data_ptr() + 2, rp, ip) == N.MZ_ERR_INVALID   # 2 B: not 8-byte aligned
+            assert call(f.data_ptr() + 4, rp, ip) == N.MZ_ERR_INVALID   # 4 B: not 8-byte aligned
+            assert call(f.data_ptr(), rp + 2, ip) == N.MZ_ERR_INVALID   # row pitch 4 B off alignment
+            assert call(f.data_ptr(), rp, ip + 1) == N.MZ_ERR_INVALID   # image pitch 2 B off alignment
     torch.cuda.synchronize()
     # Python
     with pytest.raises(AssertionError):
@@ -415,7 +420,15 @@ def test_invalid_u16_calls(dev):
         m.upscale_host(x16.cpu(), c.cpu(), out=torch.empty(B, 3, H * r, W * r, dtype=torch.uint8))   # uint8 out
     with pytest.raises(AssertionError):
         m.upscale_host(xf.cpu(), c.cpu(), out=torch.empty(B, 3, H * r, W * r, dtype=torch.uint16))   # uint16 out, fp32 in
-    with pytest.raises(AssertionError):
-        m.upscale_into(x16, c, torch.empty(B, 3, H * r, W * r, device=dev), (0, H, 0, W), (0, 0))
-    with pytest.raises(AssertionError):
-        m.upscale_into(xf, c, torch.empty(B, 3, H * r, W * r, dtype=torch.uint16, device=dev), (0, H, 0, W), (0, 0))
+    ws = m.stage_workspace(x16.shape, dev)
+    for call in (lambda xx, frame, at: m.upscale_into(xx, c, frame, (0, H, 0, W), at),
+                 lambda xx, frame, at: m.upscale_stage(xx, c, frame, (0, H, 0, W), at, 0, m.num_encoder_layers, ws)):
+        with pytest.raises(AssertionError):
+            call(x16, torch.empty(B, 3, H * r, W * r, device=dev), (0, 0))
+        with pytest.raises(AssertionError):
+            call(xf, torch.empty(B, 3, H * r, W * r, dtype=torch.uint16, device=dev), (0, 0))
+        frame = torch.full((B, 3, H * r, W * r), 0x2345, dtype=torch.int16, device=dev)
+        with pytest.raises(AssertionError):                            # the window at (r, 0) overruns the frame
+            call(x16, frame.view(torch.uint16), (r, 0))
+        torch.cuda.synchronize()
+        assert bool((frame == 0x2345).all()), "a refused call wrote its frame"

@@ -569,81 +569,101 @@ int mz_workspace_bytes_flags(const mz_model* m, int32_t B, int32_t H, int32_t W,
 
 }  // extern "C"
 
-// output window of mz_upscale_window (nullptr: the whole image, densely)
+// output window of mz_upscale_window and mz_upscale_stage (nullptr: the whole image, densely)
 struct OutWindow {
   int y0, y1, x0, x1;
   long long row_pitch, plane_pitch;
 };
 
-// the image element type flags: 8 or 16 bits need MZ_FLAG_CLAMP01, recompute the skip and exclude each other; a 4:2:0
-// frame is one of them, planar on both sides, with even dimensions
-static int check_image_flags(uint32_t flags, int H, int W) {
-  MZ_REQUIRE(!(flags & MZ_FLAG_IO_U8) || ((flags & MZ_FLAG_CLAMP01) && !(flags & MZ_FLAG_SKIP_FROM_BUFFER)),
-             "upscale: 8-bit image I/O needs MZ_FLAG_CLAMP01 and recomputes the skip (no MZ_FLAG_SKIP_FROM_BUFFER)");
-  MZ_REQUIRE(!(flags & MZ_FLAG_IO_U16) ||
-                 ((flags & MZ_FLAG_CLAMP01) && !(flags & (MZ_FLAG_SKIP_FROM_BUFFER | MZ_FLAG_IO_U8 | MZ_FLAG_U8_TRUNC))),
-             "upscale: 16-bit image I/O needs MZ_FLAG_CLAMP01, recomputes the skip (no MZ_FLAG_SKIP_FROM_BUFFER) and "
-             "excludes MZ_FLAG_IO_U8 and MZ_FLAG_U8_TRUNC");
+// element type of both images: fp32, 8 bits (MZ_FLAG_IO_U8) or 16 bits (MZ_FLAG_IO_U16), and its size in bytes
+static int image_type(uint32_t flags) {
+  return (flags & MZ_FLAG_IO_U8) ? kImgU8 : ((flags & MZ_FLAG_IO_U16) ? kImgU16 : kImgF32);
+}
+static int type_bytes(int type) { return type == kImgU8 ? 1 : (type == kImgU16 ? 2 : 4); }
+// channels per pixel of an image: 4 with MZ_FLAG_RGBA, otherwise 3
+static int image_channels(uint32_t flags) { return (flags & MZ_FLAG_RGBA) ? 4 : 3; }
+// bytes of one image: 3HW (RGBA: 4HW) elements of fp32, 8 or 16 bits, or a 4:2:0 frame of 3HW/2
+static size_t image_bytes(uint32_t flags, int H, int W) {
+  const size_t es = type_bytes(image_type(flags));
+  const size_t px = static_cast<size_t>(H) * W;
+  return (flags & MZ_FLAG_YUV420) ? px * 3 / 2 * es : px * image_channels(flags) * es;
+}
+
+// The images of a call -- its flags, the H x W input x, the output y and its window (nullptr: the whole image, densely)
+// -- as the stem and head read them (*img, *nc channels per pixel), or MZ_ERR_INVALID.  staged: a call of
+// mz_upscale_stage.  Every entry point refuses here, before anything is enqueued.
+static int image_io(const mz_model* m, const void* x, void* y, uint32_t flags, int H, int W, const OutWindow* win,
+                    bool staged, ImageIo* img, int* nc) {
+  // y holds the bicubic image of a planar fp32 RGB x, whole: every other image recomputes the skip
+  MZ_REQUIRE(!(flags & MZ_FLAG_SKIP_FROM_BUFFER) ||
+                 !(win || staged || (flags & (MZ_FLAG_IO_U8 | MZ_FLAG_IO_U16 | MZ_FLAG_YUV420 | MZ_FLAG_RGBA |
+                                              MZ_FLAG_X_NHWC | MZ_FLAG_Y_NHWC))),
+             "upscale: MZ_FLAG_SKIP_FROM_BUFFER takes a planar fp32 RGB image, neither windowed nor staged");
+  MZ_REQUIRE(!(flags & (MZ_FLAG_IO_U8 | MZ_FLAG_IO_U16)) || (flags & MZ_FLAG_CLAMP01),
+             "upscale: 8- and 16-bit image I/O needs MZ_FLAG_CLAMP01");
+  MZ_REQUIRE(!(flags & MZ_FLAG_IO_U16) || !(flags & (MZ_FLAG_IO_U8 | MZ_FLAG_U8_TRUNC)),
+             "upscale: 16-bit image I/O excludes MZ_FLAG_IO_U8 and MZ_FLAG_U8_TRUNC");
   MZ_REQUIRE((flags & MZ_FLAG_YUV420) || !(flags & kYuvColourFlags),
              "upscale: the colour bits MZ_FLAG_YUV_* apply to 4:2:0 frames only (MZ_FLAG_YUV420)");
   if (flags & MZ_FLAG_YUV420) {
     YuvCoef k;
     const int rc = yuv_coef(flags, &k);  // (NV12 or P010, one colour matrix)
     if (rc != MZ_OK) return rc;
-    MZ_REQUIRE(flags & MZ_FLAG_CLAMP01, "upscale: 4:2:0 frames need MZ_FLAG_CLAMP01");
-    MZ_REQUIRE(!(flags & (MZ_FLAG_X_NHWC | MZ_FLAG_Y_NHWC | MZ_FLAG_U8_TRUNC | MZ_FLAG_SKIP_FROM_BUFFER)),
-               "upscale: 4:2:0 frames exclude MZ_FLAG_X_NHWC, MZ_FLAG_Y_NHWC, MZ_FLAG_U8_TRUNC and MZ_FLAG_SKIP_FROM_BUFFER");
+    MZ_REQUIRE(!(flags & (MZ_FLAG_X_NHWC | MZ_FLAG_Y_NHWC | MZ_FLAG_U8_TRUNC | MZ_FLAG_RGBA)),
+               "upscale: 4:2:0 frames exclude MZ_FLAG_X_NHWC, MZ_FLAG_Y_NHWC, MZ_FLAG_U8_TRUNC and MZ_FLAG_RGBA");
+    MZ_REQUIRE(!win && !staged, "upscale: 4:2:0 frames are neither windowed nor staged");
     MZ_REQUIRE(H % 2 == 0 && W % 2 == 0, "upscale: a 4:2:0 frame has even dimensions, %d x %d given", H, W);
   }
-  MZ_REQUIRE(!(flags & MZ_FLAG_RGBA) || !(flags & (MZ_FLAG_YUV420 | MZ_FLAG_SKIP_FROM_BUFFER)),
-             "upscale: RGBA images (MZ_FLAG_RGBA) exclude MZ_FLAG_YUV420 and MZ_FLAG_SKIP_FROM_BUFFER");
+  *img = ImageIo{};
+  *nc = image_channels(flags);
+  img->x = x;
+  img->y = y;
+  img->type = image_type(flags);
+  img->x_nhwc = (flags & MZ_FLAG_X_NHWC) ? 1 : 0;
+  img->y_nhwc = (flags & MZ_FLAG_Y_NHWC) ? 1 : 0;
+  img->u8_trunc = (flags & MZ_FLAG_U8_TRUNC) ? 1 : 0;
+  img->skip_mode = (flags & MZ_FLAG_SKIP_FROM_BUFFER) ? 1 : 2;
+  img->clamp01 = (flags & MZ_FLAG_CLAMP01) ? 1 : 0;
+  MZ_REQUIRE(!(img->x_nhwc || img->y_nhwc) || static_cast<long long>(H) * W * *nc < (1LL << 31),
+             "upscale: an interleaved %d x %d x %d image exceeds 2^31 elements", H, W, *nc);
+  if (!win) return MZ_OK;
+  MZ_REQUIRE(0 <= win->y0 && win->y0 < win->y1 && win->y1 <= H && 0 <= win->x0 && win->x0 < win->x1 && win->x1 <= W,
+             "upscale: window [%d, %d) x [%d, %d) is not inside the %d x %d input", win->y0, win->y1, win->x0, win->x1, H,
+             W);
+  const long long r = m->r, ch = img->y_nhwc ? *nc : 1;  // (elements per HR pixel in a row)
+  MZ_REQUIRE(win->row_pitch >= (win->x1 - win->x0) * r * ch && win->plane_pitch >= win->row_pitch * (win->y1 - win->y0) * r,
+             "upscale: pitches (%lld, %lld) are smaller than the window", win->row_pitch, win->plane_pitch);
+  // bytes of one vector store: RGB the same in both layouts (an interleaved HR row segment of a pixel is three of them);
+  // interleaved RGBA stores a pixel's row segment of 4r values in the widest vectors that divide its 4r es bytes, up to 16
+  const int es = type_bytes(img->type), seg = 4 * m->r * es;
+  const int vec = (*nc == 4 && img->y_nhwc) ? (seg % 16 == 0 ? 16 : (seg % 8 == 0 ? 8 : 4)) : m->r == 3 ? es : es * m->r;
+  MZ_REQUIRE(reinterpret_cast<uintptr_t>(y) % vec == 0 && (win->row_pitch * es) % vec == 0 &&
+                 (win->plane_pitch * es) % vec == 0,
+             "upscale: y and its pitches must be aligned to %d bytes", vec);
+  img->wy0 = win->y0;
+  img->wy1 = win->y1;
+  img->wx0 = win->x0;
+  img->wx1 = win->x1;
+  img->y_row = win->row_pitch;
+  img->y_plane = win->plane_pitch;
   return MZ_OK;
-}
-// channels per pixel of an image: 4 with MZ_FLAG_RGBA, otherwise 3
-static int image_channels(uint32_t flags) { return (flags & MZ_FLAG_RGBA) ? 4 : 3; }
-// bytes of one image: 3HW (RGBA: 4HW) elements of fp32, 8 or 16 bits, or a 4:2:0 frame of 3HW/2
-static size_t image_bytes(uint32_t flags, int H, int W) {
-  const size_t es = (flags & MZ_FLAG_IO_U8) ? 1 : ((flags & MZ_FLAG_IO_U16) ? 2 : sizeof(float));
-  const size_t px = static_cast<size_t>(H) * W;
-  return (flags & MZ_FLAG_YUV420) ? px * 3 / 2 * es : px * image_channels(flags) * es;
 }
 
 // layer_begin / layer_end: the encoder blocks [layer_begin, layer_end) of this call (mz_upscale_stage).  The FiLM table and
 // the stem run when layer_begin == 0, the head when layer_end == L; in between the state lives in the workspace.
 static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, int32_t c_rows, void* y_dev_v, int32_t B,
                         int32_t H, int32_t W, void* workspace_dev, size_t workspace_bytes, uint32_t flags, void* stream,
-                        const OutWindow* win, int layer_begin = 0, int layer_end = -1) {
+                        const OutWindow* win, bool staged = false, int layer_begin = 0, int layer_end = -1) {
   MZ_REQUIRE(m && x_dev_v && y_dev_v && workspace_dev, "upscale: null pointer");
   if (layer_end < 0) layer_end = m->L;
   MZ_REQUIRE(0 <= layer_begin && layer_begin <= layer_end && layer_end <= m->L, "upscale: bad layer range [%d, %d) of %d",
              layer_begin, layer_end, m->L);
   const bool front = layer_begin == 0, back = layer_end == m->L;
-  const int frc = check_image_flags(flags, H, W);
-  if (frc != MZ_OK) return frc;
+  ImageIo img;
+  int nc;
+  const int irc = image_io(m, x_dev_v, y_dev_v, flags, H, W, win, staged, &img, &nc);
+  if (irc != MZ_OK) return irc;
   const bool yuv = (flags & MZ_FLAG_YUV420) != 0;
-  MZ_REQUIRE(!yuv || (!win && front && back), "upscale: 4:2:0 frames are neither windowed nor staged");
-  ImageIo img{};
-  const int nc = image_channels(flags);
-  img.x = x_dev_v;
-  img.y = y_dev_v;
-  img.type = (flags & MZ_FLAG_IO_U8) ? kImgU8 : ((flags & MZ_FLAG_IO_U16) ? kImgU16 : kImgF32);
-  img.x_nhwc = (flags & MZ_FLAG_X_NHWC) ? 1 : 0;
-  img.y_nhwc = (flags & MZ_FLAG_Y_NHWC) ? 1 : 0;
-  img.u8_trunc = (flags & MZ_FLAG_U8_TRUNC) ? 1 : 0;
-  img.skip_mode = (flags & MZ_FLAG_SKIP_FROM_BUFFER) ? 1 : 2;
-  img.clamp01 = (flags & MZ_FLAG_CLAMP01) ? 1 : 0;
-  if (win) {
-    img.wy0 = win->y0;
-    img.wy1 = win->y1;
-    img.wx0 = win->x0;
-    img.wx1 = win->x1;
-    img.y_row = win->row_pitch;
-    img.y_plane = win->plane_pitch;
-  }
-  MZ_REQUIRE(!((img.x_nhwc || img.y_nhwc) && img.skip_mode == 1),
-             "upscale: interleaved images (MZ_FLAG_X_NHWC / MZ_FLAG_Y_NHWC) recompute the skip (no MZ_FLAG_SKIP_FROM_BUFFER)");
-  MZ_REQUIRE(!(img.x_nhwc || img.y_nhwc) || static_cast<long long>(H) * W * nc < (1LL << 31),
-             "upscale: an interleaved %d x %d x %d image exceeds 2^31 elements", H, W, nc);
   MZ_REQUIRE(B > 0 && H > 0 && W > 0, "upscale: empty input (B %d, H %d, W %d)", B, H, W);
   if (m->F > 0) {
     MZ_REQUIRE(c_dev != nullptr, "Control vector c is required for control models.");
@@ -788,7 +808,7 @@ static int upscale_impl(mz_model* m, const void* x_dev_v, const float* c_dev, in
   }
   if (!back) return MZ_OK;
 
-  if (img.skip_mode == 1) {  // (fp32 only: check_image_flags)
+  if (img.skip_mode == 1) {  // (planar fp32 RGB only: image_io)
     rc = launch_bicubic(static_cast<const float*>(img.x), static_cast<float*>(img.y), B * 3, H, W, m->r, s);
     if (rc != MZ_OK) return rc;
   }
@@ -823,24 +843,6 @@ int mz_upscale_window(mz_model* m, const void* x_dev, const float* c_dev, int32_
                       int64_t y_plane_pitch, int32_t B, int32_t H, int32_t W, int32_t win_y0, int32_t win_y1,
                       int32_t win_x0, int32_t win_x1, void* workspace_dev, size_t workspace_bytes, uint32_t flags,
                       void* stream) {
-  MZ_REQUIRE(m, "upscale_window: null model");
-  MZ_REQUIRE(0 <= win_y0 && win_y0 < win_y1 && win_y1 <= H && 0 <= win_x0 && win_x0 < win_x1 && win_x1 <= W,
-             "upscale_window: window [%d, %d) x [%d, %d) is not inside the %d x %d input", win_y0, win_y1, win_x0, win_x1,
-             H, W);
-  const int64_t r = m->r, ch = (flags & MZ_FLAG_Y_NHWC) ? image_channels(flags) : 1;  // (elements per HR pixel in a row)
-  MZ_REQUIRE(y_row_pitch >= (win_x1 - win_x0) * r * ch && y_plane_pitch >= y_row_pitch * (win_y1 - win_y0) * r,
-             "upscale_window: pitches (%lld, %lld) are smaller than the window", static_cast<long long>(y_row_pitch),
-             static_cast<long long>(y_plane_pitch));
-  MZ_REQUIRE(!(flags & MZ_FLAG_SKIP_FROM_BUFFER), "upscale_window: the bicubic skip is recomputed (no MZ_FLAG_SKIP_FROM_BUFFER)");
-  MZ_REQUIRE(!(flags & MZ_FLAG_YUV420), "upscale_window: 4:2:0 frames (MZ_FLAG_YUV420) cannot be windowed");
-  // bytes of one vector store: RGB the same in both layouts (an interleaved HR row segment of a pixel is three of them);
-  // interleaved RGBA stores a pixel's row segment of 4r values in the widest vectors that divide its 4r es bytes, up to 16
-  const int es = (flags & MZ_FLAG_IO_U8) ? 1 : ((flags & MZ_FLAG_IO_U16) ? 2 : 4), seg = 4 * m->r * es;
-  const int vec = ((flags & MZ_FLAG_RGBA) && (flags & MZ_FLAG_Y_NHWC)) ? (seg % 16 == 0 ? 16 : (seg % 8 == 0 ? 8 : 4))
-                  : m->r == 3                                        ? es
-                                                                     : es * m->r;
-  MZ_REQUIRE(reinterpret_cast<uintptr_t>(y_dev) % vec == 0 && (y_row_pitch * es) % vec == 0 && (y_plane_pitch * es) % vec == 0,
-             "upscale_window: y and its pitches must be aligned to %d bytes", vec);
   const OutWindow w{win_y0, win_y1, win_x0, win_x1, y_row_pitch, y_plane_pitch};
   return upscale_impl(m, x_dev, c_dev, c_rows, y_dev, B, H, W, workspace_dev, workspace_bytes, flags, stream, &w);
 }
@@ -849,17 +851,9 @@ int mz_upscale_stage(mz_model* m, const void* x_dev, const float* c_dev, int32_t
                      int64_t y_plane_pitch, int32_t B, int32_t H, int32_t W, int32_t win_y0, int32_t win_y1, int32_t win_x0,
                      int32_t win_x1, void* workspace_dev, size_t workspace_bytes, uint32_t flags, void* stream,
                      int32_t layer_begin, int32_t layer_end) {
-  MZ_REQUIRE(m, "upscale_stage: null model");
-  MZ_REQUIRE(!(flags & MZ_FLAG_SKIP_FROM_BUFFER), "upscale_stage: the bicubic skip is recomputed (no MZ_FLAG_SKIP_FROM_BUFFER)");
-  MZ_REQUIRE(!(flags & MZ_FLAG_YUV420), "upscale_stage: 4:2:0 frames (MZ_FLAG_YUV420) cannot be staged");
-  if (win_y1 <= 0)  // dense output
-    return upscale_impl(m, x_dev, c_dev, c_rows, y_dev, B, H, W, workspace_dev, workspace_bytes, flags, stream, nullptr,
-                        layer_begin, layer_end);
-  MZ_REQUIRE(0 <= win_y0 && win_y0 < win_y1 && win_y1 <= H && 0 <= win_x0 && win_x0 < win_x1 && win_x1 <= W,
-             "upscale_stage: window [%d, %d) x [%d, %d) is not inside the %d x %d input", win_y0, win_y1, win_x0, win_x1, H, W);
   const OutWindow w{win_y0, win_y1, win_x0, win_x1, y_row_pitch, y_plane_pitch};
-  return upscale_impl(m, x_dev, c_dev, c_rows, y_dev, B, H, W, workspace_dev, workspace_bytes, flags, stream, &w, layer_begin,
-                      layer_end);
+  return upscale_impl(m, x_dev, c_dev, c_rows, y_dev, B, H, W, workspace_dev, workspace_bytes, flags, stream,
+                      win_y1 > 0 ? &w : nullptr, true, layer_begin, layer_end);  // (win_y1 <= 0: dense output)
 }
 
 int mz_workspace_layout(const mz_model* m, int32_t B, int32_t H, int32_t W, size_t* zf_offset, size_t* zb_offset,
@@ -923,8 +917,10 @@ int mz_upscale_host_async(mz_model* m, int32_t lane, const void* x_host, const f
   MZ_REQUIRE(m && x_host && y_host, "upscale_host_async: null pointer");
   MZ_REQUIRE(lane == 0 || lane == 1, "upscale_host_async: lane must be 0 or 1, %d given", lane);
   MZ_REQUIRE(B > 0 && H > 0 && W > 0, "upscale_host_async: empty input (B %d, H %d, W %d)", B, H, W);
-  const int frc = check_image_flags(flags, H, W);  // (before the copies are enqueued)
-  if (frc != MZ_OK) return frc;
+  ImageIo img;
+  int nc;
+  const int irc = image_io(m, x_host, y_host, flags, H, W, nullptr, false, &img, &nc);  // (before the copies are enqueued)
+  if (irc != MZ_OK) return irc;
   DeviceGuard g(m->cfg.device);
   return host_enqueue(m, lane, x_host, c_host, c_rows, y_host, B, H, W, flags);
 }
@@ -944,8 +940,10 @@ int mz_upscale_host(mz_model* m, const void* x_host_v, const float* c_host, int3
   uint8_t* y_host = static_cast<uint8_t*>(y_host_v);
   MZ_REQUIRE(m && x_host && y_host, "upscale_host: null pointer");
   MZ_REQUIRE(B > 0 && H > 0 && W > 0, "upscale_host: empty input (B %d, H %d, W %d)", B, H, W);
-  const int frc = check_image_flags(flags, H, W);  // (before the copies are enqueued)
-  if (frc != MZ_OK) return frc;
+  ImageIo img;
+  int nc;
+  const int irc = image_io(m, x_host, y_host, flags, H, W, nullptr, false, &img, &nc);  // (before the copies are enqueued)
+  if (irc != MZ_OK) return irc;
   if (m->F > 0) {
     MZ_REQUIRE(c_host != nullptr, "Control vector c is required for control models.");
     MZ_REQUIRE(c_rows == 1 || c_rows == B, "Batch size of c (%d) must match x (%d).", c_rows, B);

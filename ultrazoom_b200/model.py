@@ -10,7 +10,7 @@ from __future__ import annotations
 
 import ctypes as C
 from dataclasses import dataclass
-from typing import Optional
+from typing import NamedTuple, Optional
 
 import torch
 from torch import Tensor, nn
@@ -35,13 +35,22 @@ def _is_nhwc(t: Tensor) -> bool:
 _INT_IMAGE_DTYPES = (torch.uint8, torch.uint16)   # images the kernels read and write as integers (MZ_FLAG_IO_U8 / _U16)
 
 
-def _input_image(x: Tensor, integer: bool):
-    """``(x, flag)``: the image as the kernels read it -- uint8 / uint16 as it is, anything else as float32 -- kept
-    interleaved when it is (``MZ_FLAG_X_NHWC``, no transpose), otherwise made contiguous NCHW."""
-    nhwc = _is_nhwc(x)
-    x = x.detach() if integer else x.detach().to(torch.float32)
-    x = x.contiguous(memory_format=torch.channels_last if nhwc else torch.contiguous_format)
-    return x, (_native.FLAG_X_NHWC if nhwc else 0)
+def _io_dtype(dtype: torch.dtype) -> torch.dtype:
+    """The element type the kernels read and write an image of ``dtype`` in: uint8 / uint16 as it is, else float32."""
+    return dtype if dtype in _INT_IMAGE_DTYPES else torch.float32
+
+
+def _cuda_device(x: Tensor) -> torch.device:
+    if not x.is_cuda:
+        raise RuntimeError("ultrazoom_b200.MewZoom runs on sm_100a CUDA kernels only; move the input to a B200 "
+                           "(`x.cuda()`). There is no CPU fallback.")
+    return x.device
+
+
+def _aligned(ws: Tensor):
+    """``(pointer, bytes)`` of a workspace tensor from its first 1024-byte boundary, where the kernels want it."""
+    ptr = (ws.data_ptr() + 1023) // 1024 * 1024
+    return ptr, ws.numel() - (ptr - ws.data_ptr())
 
 
 _YUV_MATRIX_FLAGS = {"bt709": 0, "bt601": _native.FLAG_YUV_BT601, "bt2020": _native.FLAG_YUV_BT2020}
@@ -85,16 +94,18 @@ def _no_yuv(yuv, what: str) -> None:
     assert yuv is None, f"4:2:0 frames are supported by upscale(), upscale_host() and capture(), not {what}()"
 
 
-def _channel_flag(x: Tensor) -> int:
-    """``MZ_FLAG_RGBA`` for a 4-channel image (colour, then a straight alpha that is resampled, not run through the
-    network), 0 for RGB."""
-    return _native.FLAG_RGBA if x.shape[1] == 4 else 0
+class _Images(NamedTuple):
+    """The images of one call (``MewZoom._images``): ``x`` as the kernels read it, the C ABI's image flags (element type,
+    ``MZ_FLAG_X_NHWC`` / ``MZ_FLAG_Y_NHWC``, ``MZ_FLAG_RGBA``, the 4:2:0 bits), the input's size and the output's element
+    type and shape."""
 
-
-def _output_flag(memory_format) -> int:
-    assert memory_format in (torch.contiguous_format, torch.channels_last), (
-        "memory_format must be torch.contiguous_format or torch.channels_last")
-    return _native.FLAG_Y_NHWC if memory_format == torch.channels_last else 0
+    x: Tensor
+    flags: int
+    B: int
+    H: int
+    W: int
+    dtype: torch.dtype
+    shape: tuple
 
 
 def _frame_layout(frame: Tensor, channels: int = 3):
@@ -473,16 +484,31 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         t = _native.tune(**kw)
         _native.check(eng.lib.mz_model_set_tune(eng.handle, which, C.byref(t)))
 
-    def _image_flags(self, dtype: torch.dtype) -> int:
-        """The element-type flags of an image: uint8 (rounded as ``u8_truncate`` says), uint16, or 0 for float32."""
-        if dtype == torch.uint8:
-            return _native.FLAG_IO_U8 | (_native.FLAG_U8_TRUNC if self.u8_truncate else 0)
-        return _native.FLAG_IO_U16 if dtype == torch.uint16 else 0
+    def _launch(self, dev: torch.device, enqueue, repeat: bool, synchronous: bool = False):
+        """Run one call under the fp16 range policy and return what ``enqueue(engine)`` returns; it enqueues the call on
+        the current engine of ``dev``.  A flag left up by an earlier call raises first (``_range_guard``).  A call that
+        may ``repeat`` is checked after itself while "auto" still runs fp16 -- the device is synchronised before it and
+        after it, so the flag is its own -- and is repeated with bfloat16 operands when it clipped.  A ``synchronous``
+        call (it has waited for its kernels) is checked after itself with "float16" too.  Every other call returns at
+        once and the next call reports it.  A capturing stream is neither checked nor synchronised."""
+        capturing = torch.cuda.is_current_stream_capturing()
+        while True:
+            eng = self._engine(dev)
+            auto = repeat and not capturing and self.operand_dtype == "auto" and eng.operand_dtype == "float16"
+            if auto:
+                torch.cuda.synchronize(dev)    # (the flag of an earlier asynchronous call is not this call's to absorb)
+            if not capturing:
+                self._range_guard(eng)
+            result = enqueue(eng)
+            if auto and not synchronous:
+                torch.cuda.current_stream(dev).synchronize()
+            if (auto or synchronous) and not self._range_guard(eng, rerun=True):
+                continue
+            return result
 
     def _check_inputs(self, x: Tensor, c: Optional[Tensor], yuv: Optional[Yuv420] = None) -> Optional[Tensor]:
-        if yuv is not None:
-            _yuv_dims(x)
-        else:
+        """Checks the shapes of ``x`` (4:2:0 frames: ``_images``) and ``c``; returns ``c`` as the kernels read it."""
+        if yuv is None:
             assert x.dim() == 4 and x.shape[1] in (3, 4), (
                 f"Expected input of shape (B, 3, H, W) (RGB) or (B, 4, H, W) (RGBA), got {tuple(x.shape)}.")
             assert x.shape[0] > 0 and x.shape[2] > 0 and x.shape[3] > 0, "Input must not be empty."
@@ -495,58 +521,82 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         assert c.dim() == 2 and c.shape[1] == self.control_features, (
             f"Expected {self.control_features} control features, got {c.shape[-1]}.")
         assert c.shape[0] in (1, x.shape[0]), "Batch size of c must match x."
-        return c
+        return c.detach().to(device=x.device, dtype=torch.float32).contiguous()
+
+    def _images(self, x: Tensor, yuv: Optional[Yuv420] = None, out=torch.contiguous_format) -> _Images:
+        """The images of a call on ``x`` (RGB or RGBA; with ``yuv`` 4:2:0 frames).  ``out`` is the output's memory format,
+        or a caller's output tensor -- contiguous NCHW or contiguous channels-last, of the output's dtype and shape --
+        whose layout the call writes.  (A frame's layout is ``_frame_target``'s.)"""
+        dtype = _io_dtype(x.dtype)            # 8 / 16-bit images in and out: see upscale()
+        r = self.upscale_ratio
+        if yuv is not None:
+            B, H, W = _yuv_dims(x)
+            x, flags, shape = x.detach().contiguous(), yuv.flags(dtype), (B, H * r * 3 // 2, W * r)
+        else:
+            # an interleaved x is read as it is (MZ_FLAG_X_NHWC, no transpose), anything else as contiguous NCHW
+            x_nhwc = _is_nhwc(x)
+            x = x.detach().to(dtype).contiguous(memory_format=torch.channels_last if x_nhwc else torch.contiguous_format)
+            B, C_, H, W = x.shape
+            shape = (B, C_, H * r, W * r)
+            flags = (_native.FLAG_X_NHWC if x_nhwc else 0) | (_native.FLAG_RGBA if C_ == 4 else 0)
+            if dtype == torch.uint8:
+                flags |= _native.FLAG_IO_U8 | (_native.FLAG_U8_TRUNC if self.u8_truncate else 0)
+            elif dtype == torch.uint16:
+                flags |= _native.FLAG_IO_U16
+        if isinstance(out, Tensor):
+            y_nhwc = yuv is None and _is_nhwc(out)
+            assert out.is_contiguous() or y_nhwc, "out must be contiguous NCHW or contiguous channels-last"
+            assert tuple(out.shape) == shape and out.dtype == dtype, (
+                f"out must be {shape} {dtype}, got {tuple(out.shape)} {out.dtype}")
+        else:
+            assert out in (torch.contiguous_format, torch.channels_last), (
+                "memory_format must be torch.contiguous_format or torch.channels_last")
+            assert yuv is None or out == torch.contiguous_format, "4:2:0 frames have one layout (no memory_format)"
+            y_nhwc = out == torch.channels_last
+        return _Images(x, flags | (_native.FLAG_Y_NHWC if y_nhwc else 0), B, H, W, dtype, shape)
+
+    def _frame_target(self, img: _Images, frame: Tensor, window: tuple, at: tuple, dev: torch.device,
+                      stores: bool = True):
+        """``(layout flag, destination pointer, row pitch, image pitch)`` of the LR ``window = (y0, y1, x0, x1)`` of a
+        call's output -- all of it, dense, when ``y1 <= 0`` (stages) -- placed at the HR pixel ``at = (fy, fx)`` of
+        ``frame``.  When the call ``stores`` (runs the head), the frame must hold the window whole, in the output's
+        element type.  A frame on another GPU gets peer access from ``dev``."""
+        B, C_, rH, rW = img.shape
+        assert frame.is_cuda and frame.dim() == 4 and frame.shape[0] == B and frame.shape[1] == C_, (
+            f"frame must be (B,{C_},H',W') for a {C_}-channel input")
+        yflag, row_pitch, img_pitch = _frame_layout(frame, C_)
+        y0, y1, x0, x1 = window
+        fy, fx = at
+        if stores:
+            assert frame.dtype == img.dtype, f"frame must be {img.dtype} for a {img.dtype} input, got {frame.dtype}"
+            h, w = ((y1 - y0) * self.upscale_ratio, (x1 - x0) * self.upscale_ratio) if y1 > 0 else (rH, rW)
+            assert 0 <= fy and fy + h <= frame.shape[2] and 0 <= fx and fx + w <= frame.shape[3], (
+                "the window does not fit into the frame at that position")
+        if frame.device != dev:
+            _native.check(_native.load().mz_enable_peer_access(dev.index or 0, frame.device.index or 0))
+        return yflag, (frame[0, 0, fy, fx].data_ptr() if frame.numel() else 0), row_pitch, img_pitch
 
     def _run(self, x: Tensor, c: Optional[Tensor], flags: int, ws: Optional[Tensor] = None,
              memory_format=torch.contiguous_format, yuv: Optional[Yuv420] = None) -> Tensor:
         c = self._check_inputs(x, c, yuv)
-        if not x.is_cuda:
-            raise RuntimeError("ultrazoom_b200.MewZoom runs on sm_100a CUDA kernels only; move the input to a "
-                               "B200 (`x.cuda()`). There is no CPU fallback.")
-        dev = x.device
-        odt = x.dtype if x.dtype in _INT_IMAGE_DTYPES else torch.float32   # 8 / 16-bit images in and out: see upscale()
-        r = self.upscale_ratio
-        if yuv is not None:
-            assert memory_format == torch.contiguous_format, "4:2:0 frames have one layout (no memory_format)"
-            B, H, W = _yuv_dims(x)
-            flags |= yuv.flags(odt)
-            x = x.detach().contiguous()
-            out_shape = (B, H * r * 3 // 2, W * r)
-        else:
-            if odt != torch.float32:
-                assert flags & _native.FLAG_CLAMP01, (
-                    f"{str(odt).replace('torch.', '')} images are supported by upscale(), not forward()")
-                flags |= self._image_flags(odt)
-            x, xflag = _input_image(x, odt != torch.float32)
-            flags |= xflag | _output_flag(memory_format) | _channel_flag(x)
-            B, C_, H, W = x.shape
-            out_shape = (B, C_, H * r, W * r)
-        if c is not None:
-            c = c.detach().to(device=dev, dtype=torch.float32).contiguous()
-        capturing = torch.cuda.is_current_stream_capturing()
-        auto = self.operand_dtype == "auto" and not capturing
-        while True:
-            eng = self._engine(dev)
-            if auto and eng.operand_dtype == "float16":
-                torch.cuda.synchronize(dev)    # (the flag of an earlier asynchronous call is not this call's to absorb)
-            if not capturing:
-                self._range_guard(eng)
-            y = torch.empty(out_shape, dtype=odt, device=dev, memory_format=memory_format)
+        dev = _cuda_device(x)
+        img = self._images(x, yuv, memory_format)
+        assert img.dtype == torch.float32 or flags & _native.FLAG_CLAMP01, (
+            f"{str(img.dtype).replace('torch.', '')} images are supported by upscale(), not forward()")
+        flags |= img.flags
+        cp, cr = (c.data_ptr(), c.shape[0]) if c is not None else (None, 0)
+
+        def enqueue(eng: _Engine) -> Tensor:
+            y = torch.empty(img.shape, dtype=img.dtype, device=dev, memory_format=memory_format)
             stream = torch.cuda.current_stream(dev)
             eng.begin(stream)
-            w = ws if ws is not None else eng.workspace(B, H, W, stream, flags)
-            ws_ptr = (w.data_ptr() + 1023) // 1024 * 1024
-            ws_bytes = w.numel() - (ws_ptr - w.data_ptr())
-            _native.check(eng.lib.mz_upscale(
-                eng.handle, x.data_ptr(), c.data_ptr() if c is not None else None,
-                c.shape[0] if c is not None else 0, y.data_ptr(), B, H, W, ws_ptr, ws_bytes,
-                flags | self._flags_extra, stream.cuda_stream))
+            ws_ptr, ws_bytes = _aligned(ws if ws is not None else eng.workspace(img.B, img.H, img.W, stream, flags))
+            _native.check(eng.lib.mz_upscale(eng.handle, img.x.data_ptr(), cp, cr, y.data_ptr(), img.B, img.H, img.W,
+                                             ws_ptr, ws_bytes, flags | self._flags_extra, stream.cuda_stream))
             eng.end(stream)
-            if auto and eng.operand_dtype == "float16":
-                stream.synchronize()       # "auto": a saturated fp16 call is repeated with bfloat16 operands
-                if not self._range_guard(eng, rerun=True):
-                    continue
             return y
+
+        return self._launch(dev, enqueue, repeat=True)
 
     # ---- reference model.py:149-179 ----
     def forward(self, x: Tensor, c: Optional[Tensor] = None, *, memory_format=torch.contiguous_format,
@@ -606,47 +656,22 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         (B,4,h,w) goes into a (B,4,rH',rW') frame.  4:2:0 frames cannot be windowed."""
         _no_yuv(yuv, "upscale_into")
         c = self._check_inputs(x, c)
-        if not x.is_cuda:
-            raise RuntimeError("ultrazoom_b200.MewZoom runs on sm_100a CUDA kernels only (no CPU fallback).")
-        dev = x.device
-        eng = self._engine(dev)
-        auto = self.operand_dtype == "auto" and eng.operand_dtype == "float16"
-        if auto:
-            torch.cuda.synchronize(dev)        # (as in upscale: only this call's flag may be absorbed by its re-run)
-        self._range_guard(eng)
-        x_in, c_in = x, c
-        odt = x.dtype if x.dtype in _INT_IMAGE_DTYPES else torch.float32
-        flags = _native.FLAG_CLAMP01 | self._flags_extra | self._image_flags(odt)
-        x, xflag = _input_image(x, odt != torch.float32)
-        if c is not None:
-            c = c.detach().to(device=dev, dtype=torch.float32).contiguous()
-        B, _, H, W = x.shape
-        r = self.upscale_ratio
-        y0, y1, x0, x1 = window
-        fy, fx = at
-        assert frame.is_cuda and frame.dim() == 4 and frame.shape[0] == B and frame.shape[1] == x.shape[1], (
-            f"frame must be (B,{x.shape[1]},H',W') for a {x.shape[1]}-channel input")
-        assert frame.dtype == odt, f"frame must be {odt} for a {odt} input, got {frame.dtype}"
-        yflag, row_pitch, img_pitch = _frame_layout(frame, x.shape[1])
-        flags |= xflag | yflag | _channel_flag(x)
-        assert 0 <= fy and fy + (y1 - y0) * r <= frame.shape[2] and 0 <= fx and fx + (x1 - x0) * r <= frame.shape[3], (
-            "the window does not fit into the frame at that position")
-        if frame.device != dev:
-            _native.check(eng.lib.mz_enable_peer_access(dev.index or 0, frame.device.index or 0))
-        stream = torch.cuda.current_stream(dev)
-        eng.begin(stream)
-        ws = eng.workspace(B, H, W, stream)
-        ws_ptr = (ws.data_ptr() + 1023) // 1024 * 1024
-        dst = frame[0, 0, fy, fx].data_ptr() if frame.numel() else 0
-        _native.check(eng.lib.mz_upscale_window(
-            eng.handle, x.data_ptr(), c.data_ptr() if c is not None else None, c.shape[0] if c is not None else 0,
-            dst, row_pitch, img_pitch, B, H, W, y0, y1, x0, x1, ws_ptr,
-            ws.numel() - (ws_ptr - ws.data_ptr()), flags, stream.cuda_stream))
-        eng.end(stream)
-        if auto:
-            stream.synchronize()          # as in upscale: a saturated window is written again with bfloat16 operands
-            if not self._range_guard(eng, rerun=True):
-                self.upscale_into(x_in, c_in, frame, window, at)
+        dev = _cuda_device(x)
+        img = self._images(x)
+        yflag, dst, row_pitch, img_pitch = self._frame_target(img, frame, window, at, dev)
+        flags = _native.FLAG_CLAMP01 | self._flags_extra | img.flags | yflag
+        cp, cr = (c.data_ptr(), c.shape[0]) if c is not None else (None, 0)
+
+        def enqueue(eng: _Engine) -> None:
+            stream = torch.cuda.current_stream(dev)
+            eng.begin(stream)
+            ws_ptr, ws_bytes = _aligned(eng.workspace(img.B, img.H, img.W, stream))
+            _native.check(eng.lib.mz_upscale_window(eng.handle, img.x.data_ptr(), cp, cr, dst, row_pitch, img_pitch,
+                                                    img.B, img.H, img.W, *window, ws_ptr, ws_bytes, flags,
+                                                    stream.cuda_stream))
+            eng.end(stream)
+
+        self._launch(dev, enqueue, repeat=True)
 
     @torch.inference_mode()
     def upscale_stage(self, x: Tensor, c: Optional[Tensor], frame: Tensor, window: tuple, at: tuple, layer_begin: int,
@@ -658,33 +683,22 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         neighbours' values (``stage_views``).  4:2:0 frames cannot be staged."""
         _no_yuv(yuv, "upscale_stage")
         c = self._check_inputs(x, c)
-        assert x.is_cuda and x.dtype in (torch.float32, torch.uint8, torch.uint16), (
-            "upscale_stage takes a CUDA image (float32, uint8 or uint16)")
-        dev = x.device
-        eng = self._engine(dev)
-        self._range_guard(eng)            # (stages run asynchronously: a saturated stage is reported by the next call)
-        integer = x.dtype in _INT_IMAGE_DTYPES
-        flags = _native.FLAG_CLAMP01 | self._flags_extra | self._image_flags(x.dtype)
-        x, xflag = _input_image(x, integer)
-        if c is not None:
-            c = c.detach().to(device=dev, dtype=torch.float32).contiguous()
-        B, _, H, W = x.shape
-        r = self.upscale_ratio
-        y0, y1, x0, x1 = window
-        fy, fx = at
-        assert frame.is_cuda and frame.dim() == 4 and frame.shape[0] == B and frame.shape[1] == x.shape[1], (
-            f"frame must be (B,{x.shape[1]},H',W') for a {x.shape[1]}-channel input")
-        yflag, row_pitch, img_pitch = _frame_layout(frame, x.shape[1])
-        flags |= xflag | yflag | _channel_flag(x)
-        if frame.device != dev:
-            _native.check(eng.lib.mz_enable_peer_access(dev.index or 0, frame.device.index or 0))
-        stream = torch.cuda.current_stream(dev)
-        ws_ptr = (ws.data_ptr() + 1023) // 1024 * 1024
-        dst = frame[0, 0, fy, fx].data_ptr()
-        _native.check(eng.lib.mz_upscale_stage(
-            eng.handle, x.data_ptr(), c.data_ptr() if c is not None else None, c.shape[0] if c is not None else 0,
-            dst, row_pitch, img_pitch, B, H, W, y0, y1, x0, x1, ws_ptr, ws.numel() - (ws_ptr - ws.data_ptr()),
-            flags, stream.cuda_stream, layer_begin, layer_end))
+        dev = _cuda_device(x)
+        img = self._images(x)
+        # (a stage that ends before the head leaves the frame alone; a negative layer_end runs to the end)
+        head = not 0 <= layer_end < self.num_encoder_layers
+        yflag, dst, row_pitch, img_pitch = self._frame_target(img, frame, window, at, dev, stores=head)
+        flags = _native.FLAG_CLAMP01 | self._flags_extra | img.flags | yflag
+        cp, cr = (c.data_ptr(), c.shape[0]) if c is not None else (None, 0)
+        ws_ptr, ws_bytes = _aligned(ws)
+
+        def enqueue(eng: _Engine) -> None:
+            _native.check(eng.lib.mz_upscale_stage(eng.handle, img.x.data_ptr(), cp, cr, dst, row_pitch, img_pitch, img.B,
+                                                   img.H, img.W, *window, ws_ptr, ws_bytes, flags,
+                                                   torch.cuda.current_stream(dev).cuda_stream, layer_begin, layer_end))
+
+        # (stages run asynchronously and cannot be repeated: a saturated stage is reported by the next call)
+        self._launch(dev, enqueue, repeat=False)
 
     def stage_workspace(self, shape, device: torch.device) -> Tensor:
         """A private workspace for ``upscale_stage`` calls on a (B,3,H,W) or (B,4,H,W) tile (the state between stages
@@ -703,7 +717,7 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         cp, zp = C.c_int32(), C.c_int32()
         _native.check(eng.lib.mz_workspace_layout(eng.handle, B, H, W, C.byref(zf_o), C.byref(zb_o), C.byref(hid_o),
                                                   C.byref(cp), C.byref(zp)))
-        base = (ws.data_ptr() + 1023) // 1024 * 1024 - ws.data_ptr()
+        base = _aligned(ws)[0] - ws.data_ptr()
         npix = B * H * W
         dt16 = torch.bfloat16 if eng.operand_dtype == "bfloat16" else torch.float16
         zf = ws[base + zf_o.value: base + zf_o.value + npix * cp.value * 4].view(torch.float32).view(B, H, W, cp.value)
@@ -745,45 +759,22 @@ class MewZoom(nn.Module, PyTorchModelHubMixin):
         c = self._check_inputs(x, c, yuv)
         assert not x.is_cuda, "upscale_host takes host tensors"
         assert lane in (None, 0, 1), "lane must be None, 0 or 1"
-        eng = self._engine(torch.device("cuda", device))
-        if lane is None and self.operand_dtype == "auto" and eng.operand_dtype == "float16":
-            torch.cuda.synchronize(torch.device("cuda", device))   # (as in upscale; lanes included)
-        self._range_guard(eng)
-        odt = x.dtype if x.dtype in _INT_IMAGE_DTYPES else torch.float32
-        if c is not None:
-            c = c.to(device="cpu", dtype=torch.float32).contiguous()
-        r = self.upscale_ratio
-        if yuv is not None:
-            assert memory_format == torch.contiguous_format, "4:2:0 frames have one layout (no memory_format)"
-            B, H, W = _yuv_dims(x)
-            x = x.contiguous()
-            out_shape = (B, H * r * 3 // 2, W * r)
-            if out is None:
-                out = torch.empty(out_shape, dtype=odt)
-            assert out.is_contiguous(), "out must be contiguous"
-            flags = _native.FLAG_CLAMP01 | self._flags_extra | yuv.flags(odt)
-        else:
-            x, xflag = _input_image(x, odt != torch.float32)
-            B, C_, H, W = x.shape
-            out_shape = (B, C_, H * r, W * r)
-            if out is None:
-                out = torch.empty(out_shape, dtype=odt, memory_format=memory_format)
-                yflag = _output_flag(memory_format)
-            else:
-                yflag = _native.FLAG_Y_NHWC if _is_nhwc(out) else 0
-                assert out.is_contiguous() or yflag, "out must be contiguous NCHW or contiguous channels-last"
-            flags = _native.FLAG_CLAMP01 | self._flags_extra | xflag | yflag | self._image_flags(odt) | _channel_flag(x)
-        assert tuple(out.shape) == out_shape and out.dtype == odt
+        img = self._images(x, yuv, memory_format if out is None else out)
+        if out is None:
+            out = torch.empty(img.shape, dtype=img.dtype, memory_format=memory_format)
         cp, cr = (c.data_ptr(), c.shape[0]) if c is not None else (None, 0)
-        if lane is None:
-            _native.check(eng.lib.mz_upscale_host(eng.handle, x.data_ptr(), cp, cr, out.data_ptr(), B, H, W, flags))
-            if not self._range_guard(eng, rerun=True):     # (the call has synchronised: "auto" repeats it with bf16)
-                return self.upscale_host(x, c, out, device, yuv=yuv)
-        else:
-            # keep the (possibly converted) inputs alive until the wait, and the engine whose lane runs the frame
-            self._host_keep[(device, lane)] = (eng, x, c, out)
-            _native.check(eng.lib.mz_upscale_host_async(eng.handle, lane, x.data_ptr(), cp, cr, out.data_ptr(), B, H, W,
-                                                        flags))
+        args = (img.x.data_ptr(), cp, cr, out.data_ptr(), img.B, img.H, img.W,
+                _native.FLAG_CLAMP01 | self._flags_extra | img.flags)
+
+        def enqueue(eng: _Engine) -> None:
+            if lane is None:
+                _native.check(eng.lib.mz_upscale_host(eng.handle, *args))
+            else:
+                # keep the (possibly converted) inputs alive until the wait, and the engine whose lane runs the frame
+                self._host_keep[(device, lane)] = (eng, img.x, c, out)
+                _native.check(eng.lib.mz_upscale_host_async(eng.handle, lane, *args))
+
+        self._launch(torch.device("cuda", device), enqueue, repeat=lane is None, synchronous=lane is None)
         return out
 
     def host_wait(self, lane: int = -1, device: int = 0) -> None:
@@ -815,31 +806,29 @@ class GraphedUpscale:
     def __init__(self, model: MewZoom, x: Tensor, c: Optional[Tensor], flags: int,
                  memory_format=torch.contiguous_format, yuv: Optional[Yuv420] = None):
         c = model._check_inputs(x, c, yuv)
-        if not x.is_cuda:
-            raise RuntimeError("MewZoom.capture needs a CUDA input (there is no CPU fallback).")
+        dev = _cuda_device(x)
         self.model = model
+        img = model._images(x, yuv, memory_format)
         # (the input buffer keeps the layout of x: the graph reads it as _run reads x; a replay copies either layout in)
-        self.x = (x.detach().contiguous() if yuv is not None else _input_image(x, x.dtype in _INT_IMAGE_DTYPES)[0]).clone()
-        self.c = None if c is None else c.detach().to(device=x.device, dtype=torch.float32).contiguous().clone()
+        self.x = img.x.clone()
+        self.c = None if c is None else c.clone()
         # The graph bakes in raw pointers: it owns everything they point at -- its input / output tensors, a PRIVATE
         # workspace (the engine's cached one is dropped and re-allocated when a later call needs a larger one) and the
         # engine itself (packed weights, FiLM parameters): the one the warm-up left current, which "auto" may have
         # switched to bfloat16.
-        eng = model._engine(x.device)
+        eng = model._engine(dev)
         need = C.c_size_t()
-        B, H, W = _yuv_dims(self.x) if yuv is not None else (self.x.shape[0], self.x.shape[2], self.x.shape[3])
-        wflags = yuv.flags(self.x.dtype) if yuv is not None else 0
-        _native.check(eng.lib.mz_workspace_bytes_flags(eng.handle, B, H, W, wflags, C.byref(need)))
-        self.ws = torch.empty(need.value + 1024, dtype=torch.uint8, device=x.device)
+        _native.check(eng.lib.mz_workspace_bytes_flags(eng.handle, img.B, img.H, img.W, img.flags, C.byref(need)))
+        self.ws = torch.empty(need.value + 1024, dtype=torch.uint8, device=dev)
         with torch.inference_mode():
-            side = torch.cuda.Stream(device=x.device)
-            side.wait_stream(torch.cuda.current_stream(x.device))
+            side = torch.cuda.Stream(device=dev)
+            side.wait_stream(torch.cuda.current_stream(dev))
             with torch.cuda.stream(side):        # warm-up: packs the weights, prepares the launches
                 model._run(self.x, self.c, flags, ws=self.ws, memory_format=memory_format, yuv=yuv)
             side.synchronize()
-            self.engine = model._engine(x.device)
+            self.engine = model._engine(dev)
             model._range_guard(self.engine)      # a checkpoint that saturates is not recorded
-            torch.cuda.current_stream(x.device).wait_stream(side)
+            torch.cuda.current_stream(dev).wait_stream(side)
             self.graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(self.graph):
                 self.y = model._run(self.x, self.c, flags, ws=self.ws, memory_format=memory_format, yuv=yuv)
@@ -853,8 +842,7 @@ class GraphedUpscale:
     def __call__(self, x: Tensor, c: Optional[Tensor] = None) -> Tensor:
         """Copy ``x`` / ``c`` in and replay; raises first when an earlier replay was clipped to the fp16 range."""
         self.model._range_guard(self.engine)
-        integer = x.dtype in _INT_IMAGE_DTYPES
-        assert tuple(x.shape) == tuple(self.x.shape) and (x.dtype == self.x.dtype if integer else self.x.dtype == torch.float32), (
+        assert tuple(x.shape) == tuple(self.x.shape) and _io_dtype(x.dtype) == self.x.dtype, (
             f"Graph was captured for input {tuple(self.x.shape)} {self.x.dtype}, got {tuple(x.shape)} {x.dtype}.")
         self.x.copy_(x, non_blocking=True)
         if self.c is not None:
