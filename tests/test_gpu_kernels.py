@@ -291,6 +291,41 @@ def test_head_with_stacked_taps(dev, r, tol, cin, shape):
     assert (got - (u + s)).abs().max().item() <= tol
 
 
+def test_2x_pair_form_equals_row_form(dev):
+    """The 2X head finishes two vertically adjacent LR rows per epilogue warp (pair form: four-row patches, eight epilogue
+    warps) unless told to go row by row (tune dbg 128).  Every value is the same FMA chain in both, so they agree bit for
+    bit, in every element type and layout pair, RGB and RGBA, with the skip recomputed: on a width that is not a multiple
+    of 128 (clamped edge warps) and an odd height (a pair whose second row is below the image).  Eight epilogue warps are
+    required (the launch fails rather than take four) and the head kernel's name shows its four-row patches, so the pair
+    form is what ran."""
+    from torch.profiler import ProfilerActivity, profile
+
+    from tests.test_gpu_memory_contract import bits
+    from tests.test_gpu_rgba_io import CL, _build, _cl, _is_cl, _rand4, _types
+
+    m = _build("2x-fused-f16", dev)
+    x, c = _rand4((2, 4, 9, 131), 31, dev)
+    try:
+        m.set_conv_tune(2, dev, epi_warps=8)
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            m.upscale(x, c)
+            torch.cuda.synchronize()
+        heads = {e.key for e in prof.key_averages() if "conv_tc_kernel<2," in e.key}
+        assert heads and all(", 4, 2, 8>" in k for k in heads), heads   # <2, K, ROWS = 4, VAR 2, LAY 8 (RGBA)>
+        for ch in (3, 4):
+            for tag, xx, trunc in _types(x[:, :ch].contiguous()):
+                m.u8_truncate = trunc
+                for x_in in (xx, _cl(xx)):
+                    for fmt in (torch.contiguous_format, CL):
+                        m.set_conv_tune(2, dev, epi_warps=8)
+                        pair = m.upscale(x_in, c, memory_format=fmt)
+                        m.set_conv_tune(2, dev, epi_warps=8, dbg=128)
+                        row = m.upscale(x_in, c, memory_format=fmt)
+                        assert torch.equal(bits(pair), bits(row)), (ch, tag, _is_cl(x_in), fmt)
+    finally:
+        m.set_conv_tune(2, dev)
+        m.u8_truncate = False
+
 def test_shifted_umma_descriptor_probe(dev):
     """The hardware property the shared-halo conv relies on (DESIGN.md): a K-major swizzled A descriptor may
     start at ANY row of a TMA-written tile when base_offset stays 0."""

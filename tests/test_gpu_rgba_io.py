@@ -494,3 +494,4 @@ def test_rgba_against_reference(dev):
             y = fn(x_in.to(dev), c.to(dev), memory_format=fmt).cpu()
             assert (y[:, :3] - want[:, :3]).abs().max().item() <= 2e-2, (clamp, fmt)
             assert (y[:, 3] - want[:, 3]).abs().max().item() <= 1e-6, (clamp, fmt)
+

@@ -913,7 +913,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
       bool rows_done = false;
       if constexpr (MODE == 2 && ROWS == 4) {
         // 2X head, eight epilogue warps: each warp finishes two ADJACENT rows of the patch in one pass (their bicubic
-        // neighbourhoods share four of five LR rows, and one load latency is exposed instead of two: epi_head2_pair)
+        // neighbourhoods share four of five LR rows, and one load latency is exposed instead of two: epi_head_tc<2, 2>)
         if (nh == 2 && p.epi.r == 2 && !(p.dbg & 128)) {  // (warp-uniform; dbg 128: row-by-row form)
           rows_done = true;
           const int r0 = 2 * half, y = y0 + r0;
@@ -935,10 +935,13 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
               tmem_zero16(t1);
             }
             if (ok) {
+              float acc[2][12];
+#pragma unroll
+              for (int i = 0; i < 12; ++i) acc[0][i] = __uint_as_float(v0[i]), acc[1][i] = __uint_as_float(v1[i]);
               const bool interior = xw >= 2 && xw + 33 < p.epi.W;  // (warp-uniform) no clamped column in this warp
               const bool second = y + 1 < p.epi.H;
-              epi_head2<(LAY & 1) != 0, (LAY & 2) != 0, (LAY & 4) != 0, (LAY & 8) ? 4 : 3>(p.epi, b, y, x, v0, v1, interior,
-                                                                                           second);
+              epi_head_tc<2, 2, (LAY & 1) != 0, (LAY & 2) != 0, (LAY & 4) != 0, (LAY & 8) ? 4 : 3>(p.epi, b, y, x, acc,
+                                                                                                interior, second);
             }
           }
         }
@@ -963,7 +966,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
           }
         }
         if (MODE == 2) {
-          float acc[48];
+          float acc[1][48];
           uint32_t v[16];
 #pragma unroll
           for (int j = 0; j < 3; ++j) {
@@ -972,10 +975,10 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
               tmem_ld_wait();
               if (FUSE) tmem_zero16(taddr + j * 16);
 #pragma unroll
-              for (int i = 0; i < 16; ++i) acc[j * 16 + i] = __uint_as_float(v[i]);
+              for (int i = 0; i < 16; ++i) acc[0][j * 16 + i] = __uint_as_float(v[i]);
             } else {
 #pragma unroll
-              for (int i = 0; i < 16; ++i) acc[j * 16 + i] = 0.f;
+              for (int i = 0; i < 16; ++i) acc[0][j * 16 + i] = 0.f;
             }
           }
           if (ok) {
@@ -983,11 +986,11 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
             constexpr bool XN = (LAY & 1) != 0, YN = (LAY & 2) != 0, I16 = (LAY & 4) != 0;
             constexpr int CH = (LAY & 8) ? 4 : 3;
             if (p.epi.r == 4)
-              epi_head_r<4, XN, YN, I16, CH>(p.epi, b, y, x, acc, interior);
+              epi_head_tc<4, 1, XN, YN, I16, CH>(p.epi, b, y, x, acc, interior);
             else if (p.epi.r == 2)
-              epi_head_r<2, XN, YN, I16, CH>(p.epi, b, y, x, acc, interior);
+              epi_head_tc<2, 1, XN, YN, I16, CH>(p.epi, b, y, x, acc, interior);
             else
-              epi_head_r<3, XN, YN, I16, CH>(p.epi, b, y, x, acc, interior);
+              epi_head_tc<3, 1, XN, YN, I16, CH>(p.epi, b, y, x, acc, interior);
           }
         } else if (MODE == 1) {
           if (k > 0 && !all_rows) load_residual(k, k + 1);

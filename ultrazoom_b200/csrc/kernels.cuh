@@ -500,423 +500,258 @@ __device__ __forceinline__ void store_hr_row_nhwc(const ImageIo& io, size_t d, c
   }
 }
 
-// channel 3 (alpha) of image b of an RGBA LR image: interleaved, its first element; planar, its plane
-template <int CH, bool XN, typename T>
-__device__ __forceinline__ const T* alpha_plane(const T* lr, int b, int H, int W) {
-  const size_t HW = static_cast<size_t>(H) * W;
-  return lr + static_cast<size_t>(b) * CH * HW + (XN ? 3 : 3 * HW);
-}
-// The alpha of an RGBA image (EpiParams::nc == 4) at ratio R: the bicubic skip of one channel of LR pixel (y, x), with
-// the loads and FMAs of a colour's skip in epi_head_rt in the same order, each sum started from 0 instead of from the
-// accumulator -- o[i][j] for HR pixel (y R + i, x R + j).  pl: the channel's plane in image b (pixels PS elements
-// apart); interior as in epi_head_rt.
-template <int R, typename T, int PS>
-__device__ __forceinline__ void alpha_skip(const EpiParams& p, const T* __restrict__ pl, int y, int x, bool interior,
-                                           float (&o)[R][R]) {
-  const int H = p.H, W = p.W;
-  int ro[5];
+// ---- the tcgen05 head's epilogue (mode 2) ----
+// The epilogue warps are few (two per scheduler) and this code is latency-bound, so: the skip source's type is a
+// template parameter (one load per tap instead of a predicated fp32 / 8-bit pair), the clamped row / column offsets are
+// computed once per pixel for every colour, at r = 2 all 75 colour taps (pair: 90; r > 2: the 25 of a colour) are
+// requested before the first FMA, and columns are only clamped in the first and last warp of an image row: the others
+// (interior) read each neighbourhood row through one pointer with immediate offsets.
+
+// Clamped offsets of the NR x 5 LR neighbourhood of pixel (y, x) -- rows y - 2 .. y + NR - 3, columns x - 2 .. x + 2 --
+// in elements from the start of a channel plane whose pixels are PS elements apart (a colour plane is below 2^31 pixels:
+// prepare_conv_tc checks; an interleaved image is below 2^31 elements: upscale_impl checks)
+template <int NR, int PS>
+struct NbOffsets {
+  int ro[NR], xo[5];
+  __device__ __forceinline__ NbOffsets(int y, int x, int H, int W) {
 #pragma unroll
-  for (int k = 0; k < 5; ++k) ro[k] = min(max(y - 2 + k, 0), H - 1) * W * PS;
-  float nb[5][5];
+    for (int m = 0; m < 5; ++m) xo[m] = min(max(x - 2 + m, 0), W - 1) * PS;
+#pragma unroll
+    for (int k = 0; k < NR; ++k) ro[k] = min(max(y - 2 + k, 0), H - 1) * W * PS;
+  }
+};
+// That neighbourhood of channel plane pl as float.  interior: warp-uniform promise that x - 2 >= 0 and x + 2 < W for
+// every lane of the calling warp (no column of its neighbourhoods is clamped -> one pointer per row)
+template <int NR, int PS, typename T>
+__device__ __forceinline__ void load_nb(const T* __restrict__ pl, int x, const NbOffsets<NR, PS>& o, bool interior,
+                                        float (&nb)[NR][5]) {
   if (interior) {
 #pragma unroll
-    for (int k = 0; k < 5; ++k) {
-      const T* rp = pl + (ro[k] + (x - 2) * PS);
+    for (int k = 0; k < NR; ++k) {
+      const T* rp = pl + (o.ro[k] + (x - 2) * PS);
 #pragma unroll
       for (int m = 0; m < 5; ++m) nb[k][m] = lr_px(rp + m * PS);
     }
   } else {
 #pragma unroll
-    for (int k = 0; k < 5; ++k)
+    for (int k = 0; k < NR; ++k)
 #pragma unroll
-      for (int m = 0; m < 5; ++m) nb[k][m] = lr_px(pl + (ro[k] + min(max(x - 2 + m, 0), W - 1) * PS));
-  }
-  float hz[5][R];
-#pragma unroll
-  for (int k = 0; k < 5; ++k)
-#pragma unroll
-    for (int j = 0; j < R; ++j) {
-      const int s = (2 * j + 1 < R) ? 0 : 1;
-      float a = 0.f;
-#pragma unroll
-      for (int m = 0; m < 4; ++m) a = fmaf(nb[k][s + m], p.bt.w[j][m], a);
-      hz[k][j] = a;
-    }
-#pragma unroll
-  for (int i = 0; i < R; ++i) {
-    const int s = (2 * i + 1 < R) ? 0 : 1;
-#pragma unroll
-    for (int j = 0; j < R; ++j) {
-      float a = 0.f;
-#pragma unroll
-      for (int k = 0; k < 4; ++k) a = fmaf(hz[s + k][j], p.bt.w[i][k], a);
-      o[i][j] = a;
-    }
+      for (int m = 0; m < 5; ++m) nb[k][m] = lr_px(pl + (o.ro[k] + o.xo[m]));
   }
 }
-// The same for the two LR pixels (y, x) and (y + 1, x) of epi_head2_pair at r = 2: o[rr][i][j] for HR pixel
-// (2 (y + rr) + i, 2 x + j), in epi_head2_pair's order
-template <typename T, int PS>
-__device__ __forceinline__ void alpha_skip_pair(const EpiParams& p, const T* __restrict__ pl, int y, int x, bool interior,
-                                                float (&o)[2][2][2]) {
-  const int H = p.H, W = p.W;
-  int ro[6];
+// Bicubic skip of one channel at ratio R for the P vertically adjacent LR pixels (y + rr, x) whose neighbourhoods are
+// the rows of nb (rr + 0 .. rr + 4): the 4 + P rows interpolated horizontally for the R phases, then vertically --
+// s[rr][i][j] for HR pixel ((y + rr) R + i, x R + j).  Phase i's first tap is at offset -2 + (2i + 1 < R ? 0 : 1) from
+// the pixel, in both directions.  Each sum starts from 0 and takes its four taps in order, so a value is the same FMA
+// chain whatever P: two pixels at r = 2 cost 6 x 5 loads and 6 x 2 horizontal interpolations per channel instead of
+// 2 x (5 x 5) and 2 x (5 x 2), with one exposed load latency instead of two, and give bit-identical results.
+template <int R, int P>
+__device__ __forceinline__ void skip_interp(const BicubicTable& bt, const float (&nb)[4 + P][5], float (&s)[P][R][R]) {
+  float hz[4 + P][R];
 #pragma unroll
-  for (int k = 0; k < 6; ++k) ro[k] = min(max(y - 2 + k, 0), H - 1) * W * PS;
-  float nb[6][5];
-  if (interior) {
+  for (int k = 0; k < 4 + P; ++k)
 #pragma unroll
-    for (int k = 0; k < 6; ++k) {
-      const T* rp = pl + (ro[k] + (x - 2) * PS);
-#pragma unroll
-      for (int m = 0; m < 5; ++m) nb[k][m] = lr_px(rp + m * PS);
-    }
-  } else {
-#pragma unroll
-    for (int k = 0; k < 6; ++k)
-#pragma unroll
-      for (int m = 0; m < 5; ++m) nb[k][m] = lr_px(pl + (ro[k] + min(max(x - 2 + m, 0), W - 1) * PS));
-  }
-  float hz[6][2];
-#pragma unroll
-  for (int k = 0; k < 6; ++k)
-#pragma unroll
-    for (int j = 0; j < 2; ++j) {
+    for (int j = 0; j < R; ++j) {
+      const int sh = (2 * j + 1 < R) ? 0 : 1;
       float a = 0.f;
 #pragma unroll
-      for (int m = 0; m < 4; ++m) a = fmaf(nb[k][j + m], p.bt.w[j][m], a);
+      for (int m = 0; m < 4; ++m) a = fmaf(nb[k][sh + m], bt.w[j][m], a);
       hz[k][j] = a;
     }
 #pragma unroll
-  for (int rr = 0; rr < 2; ++rr)
+  for (int rr = 0; rr < P; ++rr)
 #pragma unroll
-    for (int i = 0; i < 2; ++i)
+    for (int i = 0; i < R; ++i) {
+      const int sh = (2 * i + 1 < R) ? 0 : 1;
 #pragma unroll
-      for (int j = 0; j < 2; ++j) {
+      for (int j = 0; j < R; ++j) {
         float a = 0.f;
 #pragma unroll
-        for (int k = 0; k < 4; ++k) a = fmaf(hz[rr + i + k][j], p.bt.w[i][k], a);
-        o[rr][i][j] = a;
+        for (int k = 0; k < 4; ++k) a = fmaf(hz[rr + sh + k][j], bt.w[i][k], a);
+        s[rr][i][j] = a;
       }
+    }
+}
+// R contiguous fp32 values of an HR image at src: the load counterpart of store_px<float, R> (one float4 / float2 at
+// R = 4 / 2, element by element otherwise)
+template <int R>
+__device__ __forceinline__ void load_px(const float* src, float (&v)[R]) {
+  if constexpr (R == 4) {
+    const float4 q = *reinterpret_cast<const float4*>(src);
+    v[0] = q.x, v[1] = q.y, v[2] = q.z, v[3] = q.w;
+  } else if constexpr (R == 2) {
+    const float2 q = *reinterpret_cast<const float2*>(src);
+    v[0] = q.x, v[1] = q.y;
+  } else {
+#pragma unroll
+    for (int j = 0; j < R; ++j) v[j] = src[j];
+  }
 }
 
-// Same as epi_head with the ratio known at compile time: the 5x5 LR neighbourhood of the pixel is loaded once per
-// colour, interpolated horizontally for the R phases (5 rows x R values) and then vertically (R x R values) --
-// 25 loads + 20R + 4R^2 FMAs per colour instead of 16 loads + 20 FMAs per HR pixel -- and every HR row segment of
-// the pixel (R contiguous floats) leaves in one vector store, so a warp writes 32*R contiguous floats.
-// The epilogue warps are few (two per scheduler) and this code is latency-bound, so: the skip source's type is a
-// template parameter (one load per tap instead of a predicated fp32 / 8-bit pair), the clamped row / column offsets
-// are computed once for the three colours, and at R = 2 all 75 taps (R > 2: the 25 of a colour) are requested before
-// the first FMA; skip-from-buffer reads all its row segments before the first store (a store to y orders every
-// later load from y behind it).  Columns are only clamped in the first and last warp of an image row: the others
-// (interior) read each neighbourhood row through one pointer with immediate offsets.
+// The alpha of an RGBA image (EpiParams::nc == 4): the skip of its channel plane pl alone -- a colour's loads and FMAs
+// in the same order, each sum started from 0 instead of from the accumulator.  A function of its own, with its plane
+// pointer formed at the call rather than by epi_head_t's plane(): written inline or given plane(3), the compiler folds
+// the RGBA heads' address arithmetic worse (2-5 % more instructions; 10 % more head time with planar input and
+// interleaved output).
+template <int R, int P, int PS, typename T>
+__device__ __forceinline__ void alpha_skip(const EpiParams& p, const T* __restrict__ pl, int y, int x, bool interior,
+                                           float (&al)[P][R][R]) {
+  const NbOffsets<4 + P, PS> o(y, x, p.H, p.W);
+  float nb[4 + P][5];
+  load_nb(pl, x, o, interior, nb);
+  skip_interp<R, P>(p.bt, nb, al);
+}
+// epi_head with the ratio R known at compile time, for P = 1 LR pixel (y, x) (any ratio) or P = 2 vertically adjacent
+// pixels (y, x) and (y + 1, x) (r = 2; second: row y + 1 exists).  acc[rr][n]: the head channels of pixel (y + rr, x) as
+// they come out of TMEM, n = c R^2 + i R + j for HR pixel ((y + rr) R + i, x R + j) of colour c.  The 5 x 5 (pair:
+// 6 x 5) LR neighbourhood is loaded once per colour and interpolated by skip_interp -- 25 loads + 20R + 4R^2 FMAs per
+// colour of a pixel instead of 16 loads + 20 FMAs per HR pixel -- and every HR row segment of a pixel (R contiguous
+// values) leaves in one vector store, so a warp writes 32R contiguous values.  Skip-from-buffer reads all of a pixel's
+// row segments before the first store (a store to y orders every later load from y behind it).
 // XN / YN: interleaved input / output (ImageIo::x_nhwc / y_nhwc) -- compile-time, so that the planar instantiation is
-// the code it was.  Interleaved, the taps of one colour are 3 elements apart (same FMA order per colour: bit-identical
-// results) and each HR row of the pixel leaves as 3R contiguous values.
+// the code it was.  Interleaved, the taps of one colour are CH elements apart (same FMA order per colour: bit-identical
+// results) and each HR row of the pixel leaves as CH R contiguous values.
 // T = uint16_t: 16-bit images on both sides (MZ_FLAG_IO_U16) -- the 16-bit heads are instantiations of their own.
 // CH = 4: RGBA images (EpiParams::nc) -- pixels 4 elements apart when interleaved, images 4 planes apart when planar, and
-// the alpha (alpha_skip) written beside the colour: interleaved output computes it before the stores and leaves every
-// HR row segment of the pixel as one run of 4R values (alpha live with the colour: 4R^2 more registers at the peak);
-// planar output computes it after the colour stores, once out[3][R][R] is dead, and stores it as a fourth plane.
-template <int R, typename T, bool XN, bool YN, int CH = 3>
-__device__ __forceinline__ void epi_head_rt(const EpiParams& p, const T* __restrict__ lr, int b, int y, int x,
-                                            const float (&acc)[48], bool interior) {
+// the alpha (channel 3's skip alone: skip_interp started from 0 instead of from the accumulator; RGBA always recomputes
+// the skip, image_io refuses skip-from-buffer) written beside the colour: interleaved output computes it before the
+// stores and leaves every HR row segment of the pixel as one run of 4R values (alpha live with the colour: 4R^2 more
+// registers at the peak); planar output computes it after the colour stores, once out is dead, and stores it as a
+// fourth plane.
+template <int R, int P, typename T, bool XN, bool YN, int CH, int NA>
+__device__ __forceinline__ void epi_head_t(const EpiParams& p, const T* __restrict__ lr, int b, int y, int x,
+                                           const float (&acc)[P][NA], bool interior, bool second) {
+  static_assert(P == 1 || R == 2, "pixel pairs at r = 2 only");
+  static_assert(NA >= 3 * R * R, "every colour's R x R accumulators");
   constexpr bool O16 = std::is_same_v<T, uint16_t>;
   const int H = p.H, W = p.W;
-  const long long first = head_out_index_l<YN, CH>(p, b, 0, y, x, 0, 0);
-  if (first < 0) return;  // outside the output window
+  long long first[P];
+  first[0] = head_out_index_l<YN, CH>(p, b, 0, y, x, 0, 0);
+  if constexpr (P == 2) first[1] = second ? head_out_index_l<YN, CH>(p, b, 0, y + 1, x, 0, 0) : -1;
+  if (first[0] < 0 && first[P - 1] < 0) return;  // outside the output window
   const size_t row_pitch = p.img.y_row ? static_cast<size_t>(p.img.y_row) : static_cast<size_t>(W) * R * (YN ? CH : 1);
   const size_t plane_pitch = p.img.y_plane ? static_cast<size_t>(p.img.y_plane) : static_cast<size_t>(H) * R * W * R;
   constexpr int NC = (R == 2) ? 3 : 1;  // colours whose taps are in flight together
   constexpr int PS = XN ? CH : 1;       // elements between horizontally adjacent LR pixels of one channel
-  float out[3][R][R];
-#pragma unroll
-  for (int c = 0; c < 3; ++c)
-#pragma unroll
-    for (int i = 0; i < R; ++i)
-#pragma unroll
-      for (int j = 0; j < R; ++j) out[c][i][j] = acc[c * R * R + i * R + j];
-
-  if (p.img.skip_mode == 2) {
+  auto plane = [&](int c) {             // channel c of LR image b
     const size_t HW = static_cast<size_t>(H) * W;
-    const T* img = lr + static_cast<size_t>(b) * CH * HW;
-    int xo[5], ro[5];  // (a colour plane is below 2^31 pixels: prepare_conv_tc checks; an interleaved image is below
-                       // 2^31 elements: upscale_impl checks)
+    return lr + static_cast<size_t>(b) * CH * HW + (XN ? c : c * HW);
+  };
+  auto alpha = [&](float (&al)[P][R][R]) {  // (the plane formed here, not by plane(3): see alpha_skip)
+    const size_t HW = static_cast<size_t>(H) * W;
+    alpha_skip<R, P, PS>(p, lr + static_cast<size_t>(b) * CH * HW + (XN ? 3 : 3 * HW), y, x, interior, al);
+  };
+  float out[P][3][R][R];
 #pragma unroll
-    for (int m = 0; m < 5; ++m) xo[m] = min(max(x - 2 + m, 0), W - 1) * PS;
-#pragma unroll
-    for (int k = 0; k < 5; ++k) ro[k] = min(max(y - 2 + k, 0), H - 1) * W * PS;
-#pragma unroll
-    for (int c0 = 0; c0 < 3; c0 += NC) {
-      float nb[NC][5][5];
-#pragma unroll
-      for (int cc = 0; cc < NC; ++cc) {
-        const T* pl = img + (XN ? (c0 + cc) : (c0 + cc) * HW);
-        if (interior) {  // warp-uniform: no column of the warp's neighbourhoods is clamped -> one pointer per row
-#pragma unroll
-          for (int k = 0; k < 5; ++k) {
-            const T* rp = pl + (ro[k] + (x - 2) * PS);
-#pragma unroll
-            for (int m = 0; m < 5; ++m) nb[cc][k][m] = lr_px(rp + m * PS);
-          }
-        } else {
-#pragma unroll
-          for (int k = 0; k < 5; ++k)
-#pragma unroll
-            for (int m = 0; m < 5; ++m) nb[cc][k][m] = lr_px(pl + (ro[k] + xo[m]));
-        }
-      }
-#pragma unroll
-      for (int cc = 0; cc < NC; ++cc) {
-        float hz[5][R];
-#pragma unroll
-        for (int k = 0; k < 5; ++k)
-#pragma unroll
-          for (int j = 0; j < R; ++j) {
-            const int s = (2 * j + 1 < R) ? 0 : 1;  // first tap relative to x-2 (phase offset -1 or 0)
-            float a = 0.f;
-#pragma unroll
-            for (int m = 0; m < 4; ++m) a = fmaf(nb[cc][k][s + m], p.bt.w[j][m], a);
-            hz[k][j] = a;
-          }
-#pragma unroll
-        for (int i = 0; i < R; ++i) {
-          const int s = (2 * i + 1 < R) ? 0 : 1;
-#pragma unroll
-          for (int j = 0; j < R; ++j) {
-            float a = 0.f;
-#pragma unroll
-            for (int k = 0; k < 4; ++k) a = fmaf(hz[s + k][j], p.bt.w[i][k], a);
-            out[c0 + cc][i][j] += a;
-          }
-        }
-      }
-    }
-  }
-
-  if constexpr (YN) {  // (no skip-from-buffer: the API refuses it with interleaved images)
-    float al[R][R];
-    if constexpr (CH == 4) alpha_skip<R, T, PS>(p, alpha_plane<CH, XN>(lr, b, H, W), y, x, interior, al);
-#pragma unroll
-    for (int i = 0; i < R; ++i) {
-      float v[CH * R];
-#pragma unroll
-      for (int j = 0; j < R; ++j) {
-#pragma unroll
-        for (int c = 0; c < 3; ++c) v[CH * j + c] = out[c][i][j];
-        if constexpr (CH == 4) v[CH * j + 3] = al[i][j];
-      }
-      store_hr_row_nhwc<R, O16, CH>(p.img, static_cast<size_t>(first) + static_cast<size_t>(i) * row_pitch, v);
-    }
-    return;
-  }
-  // y already holds the bicubic image (fp32: 8 and 16 bits recompute the skip): all of this pixel's segments first,
-  // then the stores
-  if (!O16 && p.img.skip_mode == 1) {
-    const float* dst = static_cast<const float*>(p.img.y) + static_cast<size_t>(first);
-    float sk[3][R][R];
-#pragma unroll
-    for (int c = 0; c < 3; ++c)
-#pragma unroll
-      for (int i = 0; i < R; ++i) {
-        const float* rowp = dst + c * plane_pitch + static_cast<size_t>(i) * row_pitch;
-        if (R == 4) {
-          const float4 v = *reinterpret_cast<const float4*>(rowp);
-          sk[c][i][0] = v.x, sk[c][i][1] = v.y, sk[c][i][R > 2 ? 2 : 0] = v.z, sk[c][i][R - 1] = v.w;
-        } else if (R == 2) {
-          const float2 v = *reinterpret_cast<const float2*>(rowp);
-          sk[c][i][0] = v.x, sk[c][i][1] = v.y;
-        } else {
-#pragma unroll
-          for (int j = 0; j < R; ++j) sk[c][i][j] = rowp[j];
-        }
-      }
+  for (int rr = 0; rr < P; ++rr)
 #pragma unroll
     for (int c = 0; c < 3; ++c)
 #pragma unroll
       for (int i = 0; i < R; ++i)
 #pragma unroll
-        for (int j = 0; j < R; ++j) out[c][i][j] += sk[c][i][j];
-  }
-#pragma unroll
-  for (int c = 0; c < 3; ++c)
-#pragma unroll
-    for (int i = 0; i < R; ++i)
-      store_out<R>(p.img, static_cast<size_t>(first) + c * plane_pitch + static_cast<size_t>(i) * row_pitch, out[c][i], O16);
-  if constexpr (CH == 4) {  // (RGBA always recomputes the skip: check_image_flags)
-    float al[R][R];
-    alpha_skip<R, T, PS>(p, alpha_plane<CH, XN>(lr, b, H, W), y, x, interior, al);
-#pragma unroll
-    for (int i = 0; i < R; ++i)
-      store_out<R>(p.img, static_cast<size_t>(first) + 3 * plane_pitch + static_cast<size_t>(i) * row_pitch, al[i], O16);
-  }
-}
-// interior: warp-uniform promise that x - 2 >= 0 and x + 2 < W for every lane of the calling warp
-// (the layouts and the 16-bit image type, I16, are template parameters of the calling kernel: one runtime branch over
-// four layouts in the same kernel raises the planar head's registers and makes it spill)
-template <int R, bool XN, bool YN, bool I16, int CH = 3>
-__device__ __forceinline__ void epi_head_r(const EpiParams& p, int b, int y, int x, const float (&acc)[48], bool interior) {
-  if constexpr (I16)
-    epi_head_rt<R, uint16_t, XN, YN, CH>(p, static_cast<const uint16_t*>(p.img.x), b, y, x, acc, interior);
-  else if (p.img.type == kImgU8)
-    epi_head_rt<R, uint8_t, XN, YN, CH>(p, static_cast<const uint8_t*>(p.img.x), b, y, x, acc, interior);
-  else
-    epi_head_rt<R, float, XN, YN, CH>(p, static_cast<const float*>(p.img.x), b, y, x, acc, interior);
-}
-// r = 2, TWO vertically adjacent LR pixels (y, x) and (y + 1, x) per thread: their 5x5 neighbourhoods share four of
-// five rows, so the pair costs 6 x 5 loads and 6 x 2 horizontal interpolations per colour instead of 2 x (5 x 5) and
-// 2 x (5 x 2), and -- what matters for the latency-bound epilogue warps -- ONE exposed load latency instead of two.
-// Same FMA order per output as epi_head_rt<2>: the results are bit-identical.  v0 / v1: the twelve head channels of the
-// two pixels as they come out of TMEM; second: row y + 1 exists (y + 1 < H).  XN / YN / CH as in epi_head_rt (the alpha
-// of both pixels: alpha_skip_pair).
-template <typename T, bool XN, bool YN, int CH = 3>
-__device__ __forceinline__ void epi_head2_pair(const EpiParams& p, const T* __restrict__ lr, int b, int y, int x,
-                                               const uint32_t (&v0)[16], const uint32_t (&v1)[16], bool interior,
-                                               bool second) {
-  constexpr bool O16 = std::is_same_v<T, uint16_t>;  // 16-bit images on both sides, as in epi_head_rt
-  const int H = p.H, W = p.W;
-  long long first[2];
-  first[0] = head_out_index_l<YN, CH>(p, b, 0, y, x, 0, 0);
-  first[1] = second ? head_out_index_l<YN, CH>(p, b, 0, y + 1, x, 0, 0) : -1;
-  if (first[0] < 0 && first[1] < 0) return;  // both outside the output window
-  const size_t row_pitch = p.img.y_row ? static_cast<size_t>(p.img.y_row) : static_cast<size_t>(W) * 2 * (YN ? CH : 1);
-  constexpr int PS = XN ? CH : 1;  // elements between horizontally adjacent LR pixels of one channel
-  const size_t plane_pitch = p.img.y_plane ? static_cast<size_t>(p.img.y_plane) : static_cast<size_t>(H) * 2 * W * 2;
-  float out[2][3][2][2];
-#pragma unroll
-  for (int c = 0; c < 3; ++c)
-#pragma unroll
-    for (int i = 0; i < 2; ++i)
-#pragma unroll
-      for (int j = 0; j < 2; ++j) {
-        out[0][c][i][j] = __uint_as_float(v0[c * 4 + i * 2 + j]);
-        out[1][c][i][j] = __uint_as_float(v1[c * 4 + i * 2 + j]);
-      }
+        for (int j = 0; j < R; ++j) out[rr][c][i][j] = acc[rr][c * R * R + i * R + j];
+
   if (p.img.skip_mode == 2) {
-    const size_t HW = static_cast<size_t>(H) * W;
-    const T* img = lr + static_cast<size_t>(b) * CH * HW;
-    int xo[5], ro[6];
+    const NbOffsets<4 + P, PS> o(y, x, H, W);
 #pragma unroll
-    for (int m = 0; m < 5; ++m) xo[m] = min(max(x - 2 + m, 0), W - 1) * PS;
+    for (int c0 = 0; c0 < 3; c0 += NC) {
+      float nb[NC][4 + P][5];
 #pragma unroll
-    for (int k = 0; k < 6; ++k) ro[k] = min(max(y - 2 + k, 0), H - 1) * W * PS;
-    float nb[3][6][5];
+      for (int cc = 0; cc < NC; ++cc) load_nb(plane(c0 + cc), x, o, interior, nb[cc]);
 #pragma unroll
-    for (int c = 0; c < 3; ++c) {
-      const T* pl = img + (XN ? c : c * HW);
-      if (interior) {
+      for (int cc = 0; cc < NC; ++cc) {
+        float s[P][R][R];
+        skip_interp<R, P>(p.bt, nb[cc], s);
 #pragma unroll
-        for (int k = 0; k < 6; ++k) {
-          const T* rp = pl + (ro[k] + (x - 2) * PS);
+        for (int rr = 0; rr < P; ++rr)
 #pragma unroll
-          for (int m = 0; m < 5; ++m) nb[c][k][m] = lr_px(rp + m * PS);
-        }
-      } else {
+          for (int i = 0; i < R; ++i)
 #pragma unroll
-        for (int k = 0; k < 6; ++k)
-#pragma unroll
-          for (int m = 0; m < 5; ++m) nb[c][k][m] = lr_px(pl + (ro[k] + xo[m]));
+            for (int j = 0; j < R; ++j) out[rr][c0 + cc][i][j] += s[rr][i][j];
       }
     }
-#pragma unroll
-    for (int c = 0; c < 3; ++c) {
-      float hz[6][2];
-#pragma unroll
-      for (int k = 0; k < 6; ++k)
-#pragma unroll
-        for (int j = 0; j < 2; ++j) {  // phase j: first tap at x - 2 + j
-          float a = 0.f;
-#pragma unroll
-          for (int m = 0; m < 4; ++m) a = fmaf(nb[c][k][j + m], p.bt.w[j][m], a);
-          hz[k][j] = a;
-        }
-#pragma unroll
-      for (int rr = 0; rr < 2; ++rr)
-#pragma unroll
-        for (int i = 0; i < 2; ++i)
-#pragma unroll
-          for (int j = 0; j < 2; ++j) {  // pixel row y + rr, phase i: first tap at LR row y + rr - 2 + i
-            float a = 0.f;
-#pragma unroll
-            for (int k = 0; k < 4; ++k) a = fmaf(hz[rr + i + k][j], p.bt.w[i][k], a);
-            out[rr][c][i][j] += a;
-          }
-    }
   }
+
   if constexpr (YN) {  // (no skip-from-buffer: the API refuses it with interleaved images)
-    float al[2][2][2];
-    if constexpr (CH == 4) alpha_skip_pair<T, PS>(p, alpha_plane<CH, XN>(lr, b, H, W), y, x, interior, al);
+    float al[P][R][R];
+    if constexpr (CH == 4) alpha(al);
 #pragma unroll
-    for (int rr = 0; rr < 2; ++rr) {
+    for (int rr = 0; rr < P; ++rr) {
       if (first[rr] < 0) continue;
 #pragma unroll
-      for (int i = 0; i < 2; ++i) {
-        float v[2 * CH];
+      for (int i = 0; i < R; ++i) {
+        float v[CH * R];
 #pragma unroll
-        for (int j = 0; j < 2; ++j) {
+        for (int j = 0; j < R; ++j) {
 #pragma unroll
           for (int c = 0; c < 3; ++c) v[CH * j + c] = out[rr][c][i][j];
           if constexpr (CH == 4) v[CH * j + 3] = al[rr][i][j];
         }
-        store_hr_row_nhwc<2, O16, CH>(p.img, static_cast<size_t>(first[rr]) + static_cast<size_t>(i) * row_pitch, v);
+        store_hr_row_nhwc<R, O16, CH>(p.img, static_cast<size_t>(first[rr]) + static_cast<size_t>(i) * row_pitch, v);
       }
     }
     return;
   }
-  if (!O16 && p.img.skip_mode == 1) {  // y already holds the bicubic image (fp32): every segment is read before the first store
+  if (!O16 && p.img.skip_mode == 1) {  // y already holds the bicubic image (fp32: 8 and 16 bits recompute the skip)
     const float* sy = static_cast<const float*>(p.img.y);
-    float2 sk[2][3][2];
+    float sk[P][3][R][R];
 #pragma unroll
-    for (int rr = 0; rr < 2; ++rr)
-#pragma unroll
-      for (int c = 0; c < 3; ++c)
-#pragma unroll
-        for (int i = 0; i < 2; ++i)
-          sk[rr][c][i] = first[rr] < 0 ? make_float2(0.f, 0.f)
-                                       : *reinterpret_cast<const float2*>(sy + static_cast<size_t>(first[rr]) + c * plane_pitch +
-                                                                          static_cast<size_t>(i) * row_pitch);
-#pragma unroll
-    for (int rr = 0; rr < 2; ++rr)
+    for (int rr = 0; rr < P; ++rr)
 #pragma unroll
       for (int c = 0; c < 3; ++c)
 #pragma unroll
-        for (int i = 0; i < 2; ++i) {
-          out[rr][c][i][0] += sk[rr][c][i].x;
-          out[rr][c][i][1] += sk[rr][c][i].y;
+        for (int i = 0; i < R; ++i) {
+          if (first[rr] < 0) {
+#pragma unroll
+            for (int j = 0; j < R; ++j) sk[rr][c][i][j] = 0.f;
+          } else {
+            load_px<R>(sy + static_cast<size_t>(first[rr]) + c * plane_pitch + static_cast<size_t>(i) * row_pitch,
+                       sk[rr][c][i]);
+          }
         }
+#pragma unroll
+    for (int rr = 0; rr < P; ++rr)
+#pragma unroll
+      for (int c = 0; c < 3; ++c)
+#pragma unroll
+        for (int i = 0; i < R; ++i)
+#pragma unroll
+          for (int j = 0; j < R; ++j) out[rr][c][i][j] += sk[rr][c][i][j];
   }
 #pragma unroll
-  for (int rr = 0; rr < 2; ++rr) {
+  for (int rr = 0; rr < P; ++rr) {
     if (first[rr] < 0) continue;
 #pragma unroll
     for (int c = 0; c < 3; ++c)
 #pragma unroll
-      for (int i = 0; i < 2; ++i)
-        store_out<2>(p.img, static_cast<size_t>(first[rr]) + c * plane_pitch + static_cast<size_t>(i) * row_pitch,
+      for (int i = 0; i < R; ++i)
+        store_out<R>(p.img, static_cast<size_t>(first[rr]) + c * plane_pitch + static_cast<size_t>(i) * row_pitch,
                      out[rr][c][i], O16);
   }
-  if constexpr (CH == 4) {  // after the colour stores (out is dead); RGBA always recomputes the skip
-    float al[2][2][2];
-    alpha_skip_pair<T, PS>(p, alpha_plane<CH, XN>(lr, b, H, W), y, x, interior, al);
+  if constexpr (CH == 4) {
+    float al[P][R][R];
+    alpha(al);
 #pragma unroll
-    for (int rr = 0; rr < 2; ++rr) {
+    for (int rr = 0; rr < P; ++rr) {
       if (first[rr] < 0) continue;
 #pragma unroll
-      for (int i = 0; i < 2; ++i)
-        store_out<2>(p.img, static_cast<size_t>(first[rr]) + 3 * plane_pitch + static_cast<size_t>(i) * row_pitch, al[rr][i],
-                     O16);
+      for (int i = 0; i < R; ++i)
+        store_out<R>(p.img, static_cast<size_t>(first[rr]) + 3 * plane_pitch + static_cast<size_t>(i) * row_pitch,
+                     al[rr][i], O16);
     }
   }
 }
-template <bool XN, bool YN, bool I16, int CH = 3>
-__device__ __forceinline__ void epi_head2(const EpiParams& p, int b, int y, int x, const uint32_t (&v0)[16],
-                                          const uint32_t (&v1)[16], bool interior, bool second) {
+// The layouts and the 16-bit image type (I16) are template parameters of the calling kernel: one runtime branch over four
+// layouts in the same kernel raises the planar head's registers and makes it spill.  8 bits or fp32 is a runtime choice.
+template <int R, int P, bool XN, bool YN, bool I16, int CH, int NA>
+__device__ __forceinline__ void epi_head_tc(const EpiParams& p, int b, int y, int x, const float (&acc)[P][NA],
+                                            bool interior, bool second = false) {
   if constexpr (I16)
-    epi_head2_pair<uint16_t, XN, YN, CH>(p, static_cast<const uint16_t*>(p.img.x), b, y, x, v0, v1, interior, second);
+    epi_head_t<R, P, uint16_t, XN, YN, CH>(p, static_cast<const uint16_t*>(p.img.x), b, y, x, acc, interior, second);
   else if (p.img.type == kImgU8)
-    epi_head2_pair<uint8_t, XN, YN, CH>(p, static_cast<const uint8_t*>(p.img.x), b, y, x, v0, v1, interior, second);
+    epi_head_t<R, P, uint8_t, XN, YN, CH>(p, static_cast<const uint8_t*>(p.img.x), b, y, x, acc, interior, second);
   else
-    epi_head2_pair<float, XN, YN, CH>(p, static_cast<const float*>(p.img.x), b, y, x, v0, v1, interior, second);
+    epi_head_t<R, P, float, XN, YN, CH>(p, static_cast<const float*>(p.img.x), b, y, x, acc, interior, second);
 }
 #endif  // __CUDACC__
 
